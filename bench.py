@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: grid points/sec of the fused MLP + finite-difference physics loss at 256^3.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--hidden H] [--grid n] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--hidden H] [--grid n] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the whole synthetic grid: three MLP evaluations per
 point (t-dt, t, t+dt), the PDE residuals and the reduction to {L_sigma, L_u}.  Synthetic inputs as
@@ -192,6 +192,17 @@ def cpu_reference_rate(H: int, nxy: int, planes: int, threads: int):
     return g.N / dt, "port", 1, (float(r["loss_sigma"]), float(r["loss_u"]))
 
 
+def dump_outputs(out_dir: str, **arrays) -> None:
+    """--dump-outputs: what the timed path returned in its last step, one <out_dir>/<name>.npy per array, so that
+    two builds run with the same arguments (same seeded inputs) can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def host_threads() -> int:
     try:
         return len(os.sched_getaffinity(0))
@@ -240,6 +251,9 @@ def run_reference_arm(args, rank: int, world: int):
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        import numpy as np
+        dump_outputs(args.dump_outputs, loss=np.array(losses, np.float32))
     print(json.dumps(line), flush=True)
 
 
@@ -264,7 +278,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-clocks", action="store_true", help="skip the NVML clock sampler thread (diagnostics)")
     ap.add_argument("--no-extra", action="store_true", help="skip the H=32 / H=128 width sweep reported under 'extra' (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step to DIR/<name>.npy: "
+                         "sums (float64 [sum R_sigma^2, sum |R_u|^2] over the whole grid) and loss (float32 [L_sigma, L_u]); "
+                         "the reference arm writes loss")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.emulate_rank_of > 1:
+        ap.error("--dump-outputs does not apply to --emulate-rank-of (that mode times one slab only)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -370,7 +392,10 @@ def main():
     sampler = ClockSampler(local) if (rank == 0 and not args.no_clocks) else None
     total_ms, per, launches, clocks, wall = timed(args.steps, max(3, args.warmup), sampler)
     value = g.N * args.steps / (total_ms * 1e-3)
-    ls, lu = ctx.finalize(acc.cpu().numpy(), pw, g.N)
+    sums = acc.cpu().numpy()     # every launch overwrites acc: these are the last timed step's global sums
+    ls, lu = ctx.finalize(sums, pw, g.N)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sums=sums, loss=np.array([ls, lu], np.float32))
 
     # kernel-only duration on this rank (no all-reduce inside the events) for the roofline
     def kernel_only(K):

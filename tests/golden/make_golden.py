@@ -109,5 +109,32 @@ def main():
     print("wrote", len(out), "arrays;", os.path.getsize(os.path.join(HERE, "golden.npz")), "bytes")
 
 
+def full_size_128():
+    """tests/golden/full128.npz: BASELINE config 3 (128^3, H = 64 and 128, seed 777, scale 0.25, t 0.25, dt 2e-3,
+    periodic) for tests/test_gpu_parity.py::test_fused_full_size_128_properties -- both losses, the whole-grid max|R| of
+    each residual and the residuals at a fixed seeded sample of 4096 points.  Computed by the reference library when it
+    is built, else by the C port, which the golden vectors above pin bit for bit to the reference's CPU path.
+        python tests/golden/make_golden.py --full128"""
+    chk = oracle.reference() or oracle.port()
+    g = Grid(128, 128, 128, 1, 1, 1, 2e-3, True)
+    idx = np.sort(np.random.default_rng(128).choice(g.N, 4096, replace=False)).astype(np.int64)
+    out = {"idx": idx}
+    for H in (64, 128):
+        w = chk.mlp_random_init(H, 777, 0.25)
+        if chk.kind == "reference":
+            r = chk.fused_loss(g, w, 0.25, 2e-3, threads=len(os.sched_getaffinity(0)), want_residuals=True)
+        else:
+            r = chk.fused_loss(g, w, 0.25, 2e-3, want_residuals=True)
+        out[f"h{H}_loss"] = np.array([r["loss_sigma"], r["loss_u"]], np.float32)
+        out[f"h{H}_Rmax"] = np.array([np.max(np.abs(a)) for a in r["R"]], np.float64)
+        out[f"h{H}_R"] = np.stack([a[idx] for a in r["R"]])
+    path = os.path.join(HERE, "full128.npz")
+    np.savez_compressed(path, source=np.array(chk.kind), **out)
+    print("wrote", path, os.path.getsize(path), "bytes from the", chk.kind)
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["--full128"]:
+        full_size_128()
+    else:
+        main()

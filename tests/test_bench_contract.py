@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -20,20 +21,35 @@ def _run(args, timeout=600):
     return json.loads(lines[0])
 
 
-def test_reference_arm_json_contract():
+def test_reference_arm_json_contract(tmp_path):
     """--impl reference runs without a GPU: the reference's CPU path on the host cores, bounded sample."""
-    d = _run(["--impl", "reference", "--grid", "32", "--ref-planes", "4", "--steps", "2", "--warmup", "1"])
+    d = _run(["--impl", "reference", "--grid", "32", "--ref-planes", "4", "--steps", "2", "--warmup", "1",
+              "--dump-outputs", str(tmp_path)])
     assert d["impl"] == "reference" and BASE_KEYS <= set(d)
     assert d["value"] > 0 and d["unit"] == "points/s" and d["higher_is_better"] is True
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["cores"] >= 1
     assert d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"] and d["vs_baseline"] is None
+    # --dump-outputs: the last timed step ran on 32 x 32 x 4 planes; the same seeded inputs give the same losses again
+    assert sorted(os.listdir(tmp_path)) == ["loss.npy"]
+    loss = np.load(tmp_path / "loss.npy")
+    assert loss.dtype == np.float32 and loss.shape == (2,) and np.all(loss > 0)
+    again = tmp_path / "again"
+    _run(["--impl", "reference", "--grid", "32", "--ref-planes", "4", "--steps", "2", "--warmup", "1",
+          "--dump-outputs", str(again)])
+    assert np.array_equal(np.load(again / "loss.npy"), loss)
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=60, cwd=ROOT)
+    assert r.returncode != 0 and "--steps" in r.stderr and not r.stdout.strip()
 
 
 @pytest.mark.gpu
-def test_b200_arm_json_contract():
-    d = _run(["--grid", "64", "--steps", "4", "--warmup", "3", "--no-extra"])
+def test_b200_arm_json_contract(tmp_path):
+    d = _run(["--grid", "64", "--steps", "4", "--warmup", "3", "--no-extra", "--dump-outputs", str(tmp_path)])
     assert BASE_KEYS | {"clocks", "roofline"} <= set(d)
     assert d["n_gpus"] == 1 and d["steps"] == 4 and d["warmup"] >= 3 and d["gpu_launches"] == 4
     assert d["dtype"] == "f32" and d["data"] == "synthetic" and "workload" in d["config"] and "l2" in d["config"]
@@ -50,3 +66,9 @@ def test_b200_arm_json_contract():
         assert k in d["cpu_baseline"]
     # the two loss values of the timed path and of the end-to-end path agree
     assert d["e2e"]["loss"] == [d["loss"]["sigma"], d["loss"]["u"]]
+    # --dump-outputs: the last timed step's sums and losses, the losses being the ones the JSON line reports
+    assert sorted(os.listdir(tmp_path)) == ["loss.npy", "sums.npy"]
+    sums, loss = np.load(tmp_path / "sums.npy"), np.load(tmp_path / "loss.npy")
+    assert sums.dtype == np.float64 and sums.shape == (2,) and np.all(sums > 0)
+    assert loss.dtype == np.float32 and loss.tolist() == [d["loss"]["sigma"], d["loss"]["u"]]
+    assert loss.tolist() == [float(np.float32(s * (1.0 / 64 ** 3))) for s in sums]   # weights (1, 1): L = float(acc * (1/N))

@@ -764,14 +764,22 @@ def test_slab_partials_sum_to_whole(ctx, checker):
 
 
 def test_fused_full_size_128_properties(ctx, checker):
-    """BASELINE config 3 (128^3, H=64 and 128) against the reference on all host threads."""
+    """BASELINE config 3 (128^3, H=64 and 128) against the reference on all host threads where its library is built,
+    and always against tests/golden/full128.npz (make_golden.py --full128): both losses and a seeded 4096-point sample
+    of every residual, at the same tolerances and relative to the same whole-grid max|R|."""
+    import os
     import oracle
     R = oracle.reference()
+    stored = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "full128.npz"))
     og = OGrid(128, 128, 128, 1, 1, 1, 2e-3, True)
     for H in (64, 128):
         w = checker.mlp_random_init(H, 777, 0.25)
         got = ctx.fused_loss_host(_g(og), _cfg(H), *w, _pw(), 0.25, 2e-3, want_residuals=True)
         assert all(np.all(np.isfinite(r)) for r in got[2])
+        ws, wu = (float(v) for v in stored[f"h{H}_loss"])
+        assert abs(got[0] - ws) <= TOL_LOSS * ws and abs(got[1] - wu) <= TOL_LOSS * wu, (H, got[:2], ws, wu)
+        for a, b, m in zip(got[2], stored[f"h{H}_R"], stored[f"h{H}_Rmax"]):
+            assert np.max(np.abs(a[stored["idx"]].astype(np.float64) - b)) <= TOL_FIELD * m, H
         if R is not None:
             want = R.fused_loss(og, w, 0.25, 2e-3, threads=max(1, R.hardware_threads()), want_residuals=True)
             for a, b in zip(got[2], want["R"]):
