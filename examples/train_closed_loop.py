@@ -1,12 +1,13 @@
 """Closed-loop training of the coordinate MLP against the physics loss (the reference's planned milestone M6,
 REQUIREMENT.md:155-169), on 1..N GPUs:
 
-  python examples/train_closed_loop.py [--n 128] [--hidden 64] [--steps 200]
+  python examples/train_closed_loop.py [--loss fd|tangent] [--n 128] [--hidden 64] [--steps 200]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 examples/train_closed_loop.py
 
 Every rank differentiates its z-slab of the grid (physad_fused_loss_grad_slab_dev), one all-reduce of 9H+6 doubles
 gives every rank the same losses and gradient, and every rank applies the same Adam update to its copy of the
-580 (H=64) parameters -- no parameter broadcast is needed.  Prints one JSON line per 20 steps and a summary."""
+580 (H=64) parameters -- no parameter broadcast is needed.  --loss tangent trains on the analytic loss instead
+(derivatives propagated through the MLP, physad_tangent_loss_grad_dev): same slabs, same single all-reduce.  Prints one JSON line per 20 steps and a summary."""
 import argparse
 import json
 import os
@@ -26,6 +27,7 @@ def main():
     ap.add_argument("--hidden", type=int, default=64)
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--lr", type=float, default=3e-3)
+    ap.add_argument("--loss", choices=("fd", "tangent"), default="fd")
     a = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank, local = int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0"))
@@ -44,7 +46,10 @@ def main():
     for k in range(1, a.steps + 1):
         w = [th[:4 * H], th[4 * H:5 * H], th[5 * H:9 * H], th[9 * H:]]
         ctx.set_weights(cfg, *[x.astype(np.float32) for x in w])
-        ls, lu, grad = ctx.fused_loss_grad(g, pw, 0.25, 2e-3)      # slab per rank + all-reduce when world > 1
+        if a.loss == "tangent":
+            ls, lu, grad = ctx.tangent_loss_grad(g, pw, 0.25)      # slab per rank + all-reduce when world > 1
+        else:
+            ls, lu, grad = ctx.fused_loss_grad(g, pw, 0.25, 2e-3)
         last = float(ls) + float(lu)
         first = last if first is None else first
         m = 0.9 * m + 0.1 * grad
@@ -54,7 +59,7 @@ def main():
             print(json.dumps({"step": k, "loss_sigma": float(ls), "loss_u": float(lu)}), flush=True)
     dt = time.perf_counter() - t0
     if rank == 0:
-        print(json.dumps({"summary": f"{a.n}^3 H={H} on {world} GPU(s)", "steps": a.steps, "loss_first": first,
+        print(json.dumps({"summary": f"{a.n}^3 H={H} {a.loss} loss on {world} GPU(s)", "steps": a.steps, "loss_first": first,
                           "loss_last": last, "reduction_pct": 100 * (1 - last / first),
                           "wall_ms_per_step_incl_host_adam": 1e3 * dt / a.steps}))
     if world > 1:

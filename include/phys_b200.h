@@ -50,6 +50,11 @@ void mlp_phys_loss_deep_cuda(const GridSpec& g, const MLPGridConfig& cfg, const 
 void mlp_phys_loss_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const MLPWeights& w, const PhysWeights& pw,
                              float t, float dt, float* out_loss_sigma, float* out_loss_u, MLPWeights& grad);
 
+// The closed loop of the analytic loss: the two losses of mlp_phys_loss_tangent_cuda AND d(L_sigma + L_u)/d(weights), reverse
+// mode over its forward-mode tangents in one kernel.  `grad` is resized to the shapes of `w`.  Same requirements as above.
+void mlp_phys_loss_tangent_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const MLPWeights& w, const PhysWeights& pw,
+                                     float t, float* out_loss_sigma, float* out_loss_u, MLPWeights& grad);
+
 }  // namespace phys
 
 #endif  // PHYS_AUTODIFF_PHYS_B200_H

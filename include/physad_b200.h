@@ -326,6 +326,23 @@ int physad_fused_loss_grad_host(physad_ctx* ctx, const physad_grid* g, const phy
                                 const float* b1, const float* W2, const float* b2, const physad_phys_weights* w, float t,
                                 float dt, float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dW2, float* db2);
 
+/* ---- closed loop of the analytic loss (ADDITIVE, no reference counterpart) ---------------------------------------------
+ * physad_tangent_loss_dev's sums AND the gradient of L_sigma + L_u (weights w included, mean over the GLOBAL N) with
+ * respect to the weights set by physad_set_weights: reverse mode over the forward-mode tangents, one persistent kernel
+ * per call (points are independent: no stencil adjoint, no halo, no per-point workspace).  The forward arithmetic is
+ * physad_tangent_loss_dev's, so acc equals its sums.  acc: 2 device doubles (sum R_sigma^2, sum |R_u|^2 over the slab);
+ * grad: 9H+4 device doubles  dW1[H*4] | db1[H] | dW2[4*H] | db2[4]  (the reference's layouts), the slab's share already
+ * scaled by 2w/N of the whole grid -- so an all-reduce(sum) of the 9H+6 doubles over the ranks' slabs gives the
+ * whole-grid result.  slab NULL = whole grid; an empty slab gives zeros.  Requires In = Out = 4, H <= 128 and a
+ * one-hidden-layer network (physad_set_weights_deep with L > 1: PHYSAD_E_UNSUPPORTED).  Bitwise repeatable. */
+int physad_tangent_loss_grad_dev(physad_ctx* ctx, const physad_grid* g, const physad_slab* slab, const physad_phys_weights* w,
+                                 float t, double* acc, double* grad, void* stream);
+/* Host-buffer form on the whole grid: (optionally) new weights in, the two losses and the gradient out (any output
+ * pointer may be null). */
+int physad_tangent_loss_grad_host(physad_ctx* ctx, const physad_grid* g, const physad_mlp_config* cfg, const float* W1,
+                                  const float* b1, const float* W2, const float* b2, const physad_phys_weights* w, float t,
+                                  float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dW2, float* db2);
+
 /* Host-only: the work partition the fused kernel is launched with.  The sequence of tiles x planes
  * tile-planes (tile-major) is cut into at most `slots` contiguous ranges of equal cost, a range paying
  * ~0.9 plane-equivalents for every z-segment it starts (its recomputed halo planes).  Writes the

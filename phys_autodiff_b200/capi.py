@@ -94,6 +94,7 @@ EXPORTS = [
     "physad_fused_loss_grad_dev", "physad_fused_loss_grad_slab_dev", "physad_fused_loss_grad_host", "physad_plan_ranges", "physad_xchg_export", "physad_xchg_connect", "physad_xchg_disconnect", "physad_fused_loss_allreduce_dev",
     "physad_xchg_status", "physad_set_fused_trace", "physad_set_advection",
     "physad_mlp_generate_fields_lp_dev", "physad_phys_loss_lp_dev", "physad_tangent_loss_dev", "physad_tangent_loss_host",
+    "physad_tangent_loss_grad_dev", "physad_tangent_loss_grad_host",
 ]
 
 

@@ -7,6 +7,7 @@
 #include "dense_kernels.cuh"
 #include "grad_kernels.cuh"
 #include "stage_kernels.cuh"
+#include "tangent_grad_kernels.cuh"
 #include "tangent_kernels.cuh"
 
 #include <algorithm>
@@ -71,6 +72,7 @@ struct physad_ctx {
     double* d_grad = nullptr;   // [9 * 128 + 4]
     double* h_grad = nullptr;   // pinned, same size
     int grad_blocks_per_sm[3] = {0, 0, 0};   // HT = 32, 64, 128 on this device
+    int tgrad_blocks_per_sm[3] = {0, 0, 0};  // the same for the tangent-loss gradient (physad_tangent_loss_grad_*)
     uint64_t launches = 0;
     int fused_variant = 0;
     int exact_residuals = 0;  // 1: residual arithmetic in double exactly as the CPU reference; 0: fp32 with FMAs
@@ -1559,6 +1561,107 @@ int physad_fused_loss_grad_host(physad_ctx* c, const physad_grid* g, const physa
     if (!c->d_grad) CU(cudaMalloc(&c->d_grad, cap * sizeof(double)));
     if (!c->h_grad) CU(cudaMallocHost(&c->h_grad, cap * sizeof(double)));
     if (int rc = physad_fused_loss_grad_dev(c, g, w, t, dt, c->d_acc, c->d_grad, c->stream)) return rc;
+    const int H = c->cfg.H;
+    CU(cudaMemcpyAsync(c->h_acc, c->d_acc, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(c->h_grad, c->d_grad, size_t(9 * H + 4) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    physad_finalize_loss(c->h_acc, w, size_t(g->nx) * g->ny * g->nz, loss_sigma, loss_u);
+    const double* gd = c->h_grad;
+    if (dW1) for (int i = 0; i < 4 * H; ++i) dW1[i] = float(gd[i]);
+    if (db1) for (int i = 0; i < H; ++i) db1[i] = float(gd[4 * H + i]);
+    if (dW2) for (int i = 0; i < 4 * H; ++i) dW2[i] = float(gd[5 * H + i]);
+    if (db2) for (int i = 0; i < 4; ++i) db2[i] = float(gd[9 * H + i]);
+    return 0;
+}
+
+// ---- closed loop of the analytic loss: its gradient with respect to the MLP weights (tangent_grad_kernels.cuh) ----
+}  // extern "C"  (templates below)
+namespace {
+int ensure_grad_partials(physad_ctx* c, size_t doubles) {
+    if (doubles <= c->gpart_cap) return 0;
+    if (c->gpart) CU(cudaFree(c->gpart));
+    c->gpart = nullptr; c->gpart_cap = 0;
+    CU(cudaMalloc(&c->gpart, doubles * sizeof(double)));
+    c->gpart_cap = doubles;
+    return 0;
+}
+
+template <int H>
+int launch_tangent_grad_t(physad_ctx* c, const TangentGradArgs& a, float tcoord, size_t chunks, cudaStream_t st) {
+    int& bps = c->tgrad_blocks_per_sm[H == 32 ? 0 : (H == 64 ? 1 : 2)];
+    if (!bps) {
+        CU(cudaError_t(tangent_grad_blocks_per_sm(H, &bps)));
+        if (bps < 1) return fail(PHYSAD_E_UNSUPPORTED, "tangent_loss_grad: kernel does not fit an SM");
+    }
+    const size_t blocks = std::max<size_t>(1, std::min<size_t>(chunks, size_t(c->sm_count) * bps));
+    if (int rc = ensure_grad_partials(c, blocks * (TGRAD_NACC * H + 6))) return rc;
+    TangentGradArgs k = a;
+    k.partials = c->gpart;
+    TangentConst<H> w;
+    fill_tangent<H>(c, tcoord, w);
+    CU(cudaError_t(tangent_grad_launch(H, &w, k, unsigned(blocks), st)));
+    c->launches++;
+    return 0;
+}
+}  // namespace
+extern "C" {
+
+int physad_tangent_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad_slab* slab, const physad_phys_weights* w,
+                                 float t, double* acc, double* grad, void* stream) {
+    if (!c || !w || !acc || !grad) return fail(PHYSAD_E_INVALID, "tangent_loss_grad: null argument");
+    if (int rc = check_grid(g)) return rc;
+    if (int rc = need_4x4(c, "tangent_loss_grad")) return rc;
+    if (c->deep_layers > 1)
+        return fail(PHYSAD_E_UNSUPPORTED, "tangent_loss_grad: the gradient is of the one-hidden-layer network (set_weights_deep L > 1)");
+    physad_slab s;
+    if (int rc = check_slab(g, slab, &s)) return rc;
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    const int H = c->cfg.H;
+    if (s.z_end == s.z_begin) {
+        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
+        CU(cudaMemsetAsync(grad, 0, size_t(9 * H + 4) * sizeof(double), st));
+        return 0;
+    }
+    if (int rc = upload_weights_if_stale(c, st)) return rc;
+    if (int rc = ensure_coord_tables(c, g, st)) return rc;
+    TangentGradArgs a{};
+    a.nx = g->nx; a.ny = g->ny; a.nz = g->nz; a.z_begin = s.z_begin; a.z_end = s.z_end;
+    a.cxs = c->tab.dev; a.cys = a.cxs + g->nx; a.czs = a.cys + g->ny;
+    // dc/dx exactly as physad_tangent_loss_dev forms it (0 for an extent of 1)
+    const double f = c->cfg.norm == 1 ? 2.0 : 1.0;
+    a.sx = g->nx > 1 ? float(f / (double(g->nx - 1) * double(g->hx))) : 0.f;
+    a.sy = g->ny > 1 ? float(f / (double(g->ny - 1) * double(g->hy))) : 0.f;
+    a.sz = g->nz > 1 ? float(f / (double(g->nz - 1) * double(g->hz))) : 0.f;
+    vjp_scales(g, w, &a.scale_s, &a.scale_u);   // 2 w / float(N) of the whole grid: slab results add up to the grid's
+    a.ct = time_coord(t, c->cfg.norm);
+    a.W1 = c->dW1; a.W2 = c->dW2;
+    a.H = H;
+    a.ticket = c->ticket;
+    a.acc = acc; a.grad = grad;
+    const size_t chunks = (size_t(s.z_end - s.z_begin) * g->ny * g->nx + TGRAD_THREADS - 1) / TGRAD_THREADS;
+    switch (template_h(H)) {
+        case 32: return launch_tangent_grad_t<32>(c, a, a.ct, chunks, st);
+        case 64: return launch_tangent_grad_t<64>(c, a, a.ct, chunks, st);
+        case 128: return launch_tangent_grad_t<128>(c, a, a.ct, chunks, st);
+    }
+    return fail(PHYSAD_E_UNSUPPORTED, "H > 128 not built");
+}
+
+int physad_tangent_loss_grad_host(physad_ctx* c, const physad_grid* g, const physad_mlp_config* cfg, const float* W1,
+                                  const float* b1, const float* W2, const float* b2, const physad_phys_weights* w, float t,
+                                  float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dW2, float* db2) {
+    if (!c || !w) return fail(PHYSAD_E_INVALID, "tangent_loss_grad: null argument");
+    if (int rc = check_grid(g)) return rc;
+    if (cfg) {
+        if (int rc = physad_set_weights(c, cfg, W1, b1, W2, b2)) return rc;
+    }
+    if (int rc = need_4x4(c, "tangent_loss_grad")) return rc;
+    DeviceGuard dg(c->device);
+    constexpr size_t cap = 9 * 128 + 4;
+    if (!c->d_grad) CU(cudaMalloc(&c->d_grad, cap * sizeof(double)));
+    if (!c->h_grad) CU(cudaMallocHost(&c->h_grad, cap * sizeof(double)));
+    if (int rc = physad_tangent_loss_grad_dev(c, g, nullptr, w, t, c->d_acc, c->d_grad, c->stream)) return rc;
     const int H = c->cfg.H;
     CU(cudaMemcpyAsync(c->h_acc, c->d_acc, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(c->h_grad, c->d_grad, size_t(9 * H + 4) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));

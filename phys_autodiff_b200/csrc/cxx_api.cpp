@@ -312,6 +312,22 @@ void mlp_phys_loss_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const 
         die("mlp_phys_loss_grad_cuda", rc);
 }
 
+void mlp_phys_loss_tangent_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const MLPWeights& w, const PhysWeights& pw,
+                                     float t, float* out_loss_sigma, float* out_loss_u, MLPWeights& grad) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    const physad_grid cg = to_c(g);
+    const physad_phys_weights cw = to_c(pw);
+    const physad_mlp_config mc{int(cfg.dims.In), int(cfg.dims.H), int(cfg.dims.Out), norm_of(cfg.norm)};
+    grad.W1.resize(w.W1.size());
+    grad.b1.resize(w.b1.size());
+    grad.W2.resize(w.W2.size());
+    grad.b2.resize(w.b2.size());
+    if (int rc = physad_tangent_loss_grad_host(ctx(), &cg, &mc, w.W1.data(), w.b1.data(), w.W2.data(), w.b2.data(), &cw, t,
+                                               out_loss_sigma, out_loss_u, grad.W1.data(), grad.b1.data(), grad.W2.data(),
+                                               grad.b2.data()))
+        die("mlp_phys_loss_tangent_grad_cuda", rc);
+}
+
 }  // namespace phys
 
 // C-ABI access to the weight generator for non-C++ hosts (bench.py, tests): see include/physad_b200.h.

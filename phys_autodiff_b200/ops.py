@@ -431,6 +431,42 @@ class Context:
                                                 *[ptr(r) for r in R], self._stream()), "tangent_loss")
         return acc
 
+    # -- closed loop of the analytic loss: its sums + gradient with respect to the MLP weights (additive) -----
+    def tangent_loss_grad_acc(self, g: Grid, pw: PhysWeights, t: float, slab=None, out=None):
+        """Device form: a float64 device tensor [acc_sigma, acc_u, grad(9H+4)] of the slab (None = whole grid); grad =
+        dW1 | db1 | dW2 | db2, already scaled by 2w/N of the whole grid, so the slabs' tensors add up (all-reduce)."""
+        import torch
+        out = out if out is not None else self._empty(9 * self.cfg.H + 6, torch.float64)
+        cs, _ = self._slab(g, slab)
+        cg, cw = g.c(), pw.c()
+        check(self._lib.physad_tangent_loss_grad_dev(self._h, C.byref(cg), C.byref(cs), C.byref(cw), C.c_float(t), ptr(out),
+                                                     ptr(out[2:]), self._stream()), "tangent_loss_grad")
+        return out
+
+    def tangent_loss_grad(self, g: Grid, pw: PhysWeights, t: float, group=None):
+        """(L_sigma, L_u, grad float64 ndarray[9H+4]) of the analytic loss for the weights set by set_weights().  With
+        torch.distributed initialised each rank differentiates its z-slab and ONE all-reduce of 9H+6 doubles combines them."""
+        import torch.distributed as dist
+        world, rank = (dist.get_world_size(group), dist.get_rank(group)) if dist.is_initialized() else (1, 0)
+        buf = self.tangent_loss_grad_acc(g, pw, t, slab_for_rank(g.nz, rank, world))
+        if world > 1:
+            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+        h = buf.cpu().numpy()
+        ls, lu = self.finalize(h[:2], pw, g.N)
+        return ls, lu, h[2:].copy()
+
+    def tangent_loss_grad_host(self, g: Grid, cfg: MLPConfig, W1, b1, W2, b2, pw: PhysWeights, t: float):
+        """Host-buffer form: weights in, (L_sigma, L_u, dW1, db1, dW2, db2) of the analytic loss out (float32)."""
+        W1, b1, W2, b2 = _f32(W1), _f32(b1), _f32(W2), _f32(b2)
+        d = [np.empty(4 * cfg.H, np.float32), np.empty(cfg.H, np.float32), np.empty(4 * cfg.H, np.float32), np.empty(4, np.float32)]
+        ls, lu = C.c_float(), C.c_float()
+        cg, cc, cw = g.c(), cfg.c(), pw.c()
+        check(self._lib.physad_tangent_loss_grad_host(self._h, C.byref(cg), C.byref(cc), ptr(W1), ptr(b1), ptr(W2), ptr(b2),
+                                                      C.byref(cw), C.c_float(t), C.byref(ls), C.byref(lu),
+                                                      *[ptr(x) for x in d]), "tangent_loss_grad_host")
+        self.cfg = cfg
+        return (np.float32(ls.value), np.float32(lu.value), *d)
+
     # -- closed loop: loss + gradient with respect to the MLP weights (additive) ----------------------------
     def fused_loss_grad_acc(self, g: Grid, pw: PhysWeights, t: float, dt: float, acc=None, grad=None):
         """Device form: returns (acc[2], grad[9H+4]) float64 device tensors; grad = dW1 | db1 | dW2 | db2."""
@@ -669,3 +705,8 @@ def mlp_phys_loss_tangent_cuda(g: Grid, cfg: MLPConfig, w, pw: PhysWeights, t: f
 def mlp_phys_loss_grad_cuda(g: Grid, cfg: MLPConfig, w, pw: PhysWeights, t: float, dt: float):
     """Closed loop (additive): losses and d(L_sigma + L_u)/d(W1, b1, W2, b2)."""
     return default_context().fused_loss_grad_host(g, cfg, *w, pw, t, dt)
+
+
+def mlp_phys_loss_tangent_grad_cuda(g: Grid, cfg: MLPConfig, w, pw: PhysWeights, t: float):
+    """Closed loop of the analytic loss (additive): (L_sigma, L_u, dW1, db1, dW2, db2)."""
+    return default_context().tangent_loss_grad_host(g, cfg, *w, pw, t)

@@ -1,9 +1,12 @@
 """Times the closed-loop step (loss + gradient w.r.t. the MLP weights): CUDA events around the launches of one
 step (fields, residuals + sums, stencil adjoint, MLP backward [+ the all-reduce of 9H+6 doubles under torchrun]).
-  python tools/bench_grad.py [--n 256] [--hidden 64] [--steps 20]
+--loss tangent times the closed loop of the analytic loss instead (one kernel, physad_tangent_loss_grad_dev) and reports,
+from the same process, the analytic forward alone, the finite-difference step, the counted flops and the GPU it ran on.
+  python tools/bench_grad.py [--loss fd|tangent] [--n 256] [--hidden 64] [--steps 20]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/bench_grad.py   (z-slab per rank)"""
 import argparse
 import json
+import subprocess
 import sys, os
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -17,10 +20,13 @@ def main():
     ap.add_argument("--n", type=int, default=256)
     ap.add_argument("--hidden", type=int, default=64)
     ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--loss", choices=("fd", "tangent"), default="fd")
     a = ap.parse_args()
     g = Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True)
     if "RANK" in os.environ and int(os.environ.get("WORLD_SIZE", "1")) > 1:
         return distributed(a, g)
+    if a.loss == "tangent":
+        return tangent(a, g)
     ctx = ops.Context()
     ctx.set_weights(MLPConfig(4, a.hidden, 4, True), *ops.mlp_random_init(a.hidden, 777, 0.25))
     pw = PhysWeights(1, 1)
@@ -51,6 +57,62 @@ def main():
                       "grad_norm": float(grad.norm()), "acc": acc.tolist()}))
 
 
+def _times(fn, steps):
+    """Sorted per-call milliseconds: CUDA events around each call, one sync at the end."""
+    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
+    for e0, e1 in ev:
+        e0.record()
+        fn()
+        e1.record()
+    torch.cuda.synchronize()
+    return sorted(e0.elapsed_time(e1) for e0, e1 in ev)
+
+
+def _gpu():
+    """Name and power limit of the current GPU (the limit read with nvidia-smi, None where it cannot be read)."""
+    name = torch.cuda.get_device_name()
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader,nounits",
+                            f"--id={torch.cuda.current_device()}"], capture_output=True, text=True, timeout=30)
+        return name, float(q.stdout.strip().splitlines()[0])
+    except (OSError, ValueError, IndexError, subprocess.TimeoutExpired):
+        return name, None
+
+
+# counted work of the analytic gradient per point and hidden unit (tangent_grad_kernels.cu): stage phase 7 (z) + 8 (y, 4 FMA)
+# + 16 (the Jacobian's masked adds); backward 7 (z again) + 8 (W2^T yb) + 8 (yb a) + 6 (dz c) + 1 (dz) + 16 (the masked sums)
+TANGENT_GRAD_FLOPS_PER_UNIT = 77
+
+
+def tangent(a, g):
+    ctx = ops.Context()
+    ctx.set_weights(MLPConfig(4, a.hidden, 4, True), *ops.mlp_random_init(a.hidden, 777, 0.25))
+    pw = PhysWeights(1, 1)
+    out = ctx.tangent_loss_grad_acc(g, pw, 0.25)
+    acc, grad = ctx.fused_loss_grad_acc(g, pw, 0.25, 2e-3)
+    for _ in range(3):
+        ctx.tangent_loss_grad_acc(g, pw, 0.25, out=out)
+        ctx.tangent_loss_acc(g, 0.25, acc=acc)
+        ctx.fused_loss_grad_acc(g, pw, 0.25, 2e-3, acc, grad)
+    torch.cuda.synchronize()
+    # the three are timed in alternation, so that they share whatever else the GPU is doing
+    tg, tf, fd = [], [], []
+    for _ in range(a.steps):
+        tg += _times(lambda: ctx.tangent_loss_grad_acc(g, pw, 0.25, out=out), 1)
+        tf += _times(lambda: ctx.tangent_loss_acc(g, 0.25, acc=acc), 1)
+        fd += _times(lambda: ctx.fused_loss_grad_acc(g, pw, 0.25, 2e-3, acc, grad), 1)
+    tg.sort(); tf.sort(); fd.sort()
+    med = tg[len(tg) // 2]
+    flops_pt = TANGENT_GRAD_FLOPS_PER_UNIT * a.hidden
+    name, plim = _gpu()
+    h = out.cpu().numpy()
+    print(json.dumps({"workload": f"{a.n}^3 H={a.hidden} analytic loss+grad", "ms_median": med, "ms_min": tg[0],
+                      "gpts_per_s": g.N / med / 1e6, "tangent_forward_ms": tf[len(tf) // 2],
+                      "fd_loss_grad_ms": fd[len(fd) // 2], "flops_per_point": flops_pt,
+                      "counted_tflops": flops_pt * g.N / (med * 1e-3) / 1e12, "gpu": name, "power_limit_w": plim,
+                      "grad_norm": float(abs(h[2:]).max()), "acc": h[:2].tolist()}))
+
+
 def distributed(a, g):
     import torch.distributed as dist
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
@@ -60,10 +122,16 @@ def distributed(a, g):
     ctx.set_weights(MLPConfig(4, a.hidden, 4, True), *ops.mlp_random_init(a.hidden, 777, 0.25))
     pw = PhysWeights(1, 1)
     slab = ops.slab_for_rank(g.nz, rank, world)
-    buf = ctx.fused_loss_grad_slab_acc(g, pw, 0.25, 2e-3, slab)
+    if a.loss == "tangent":
+        buf = ctx.tangent_loss_grad_acc(g, pw, 0.25, slab)
+    else:
+        buf = ctx.fused_loss_grad_slab_acc(g, pw, 0.25, 2e-3, slab)
 
     def step():
-        ctx.fused_loss_grad_slab_acc(g, pw, 0.25, 2e-3, slab, buf)
+        if a.loss == "tangent":
+            ctx.tangent_loss_grad_acc(g, pw, 0.25, slab, buf)
+        else:
+            ctx.fused_loss_grad_slab_acc(g, pw, 0.25, 2e-3, slab, buf)
         dist.all_reduce(buf, op=dist.ReduceOp.SUM)
 
     for _ in range(5):
@@ -80,7 +148,8 @@ def distributed(a, g):
     t = torch.tensor([e0.elapsed_time(e1) / a.steps], device="cuda")
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
     if rank == 0:
-        print(json.dumps({"workload": f"{a.n}^3 H={a.hidden} loss+grad, z-slab per rank, 1 all-reduce of 9H+6 doubles",
+        kind = "analytic loss+grad" if a.loss == "tangent" else "loss+grad"
+        print(json.dumps({"workload": f"{a.n}^3 H={a.hidden} {kind}, z-slab per rank, 1 all-reduce of 9H+6 doubles",
                           "n_gpus": world, "ms_per_step_max_over_ranks": t.item(), "gpts_per_s": g.N / t.item() / 1e6,
                           "grad_norm": float(buf[2:].norm()), "acc": buf[:2].tolist()}))
     dist.destroy_process_group()
