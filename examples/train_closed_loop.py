@@ -1,13 +1,16 @@
 """Closed-loop training of the coordinate MLP against the physics loss (the reference's planned milestone M6,
 REQUIREMENT.md:155-169), on 1..N GPUs:
 
-  python examples/train_closed_loop.py [--loss fd|tangent] [--n 128] [--hidden 64] [--steps 200]
+  python examples/train_closed_loop.py [--loss fd|tangent] [--layers 1] [--n 128] [--hidden 64] [--steps 200]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 examples/train_closed_loop.py
 
 Every rank differentiates its z-slab of the grid (physad_fused_loss_grad_slab_dev), one all-reduce of 9H+6 doubles
 gives every rank the same losses and gradient, and every rank applies the same Adam update to its copy of the
 580 (H=64) parameters -- no parameter broadcast is needed.  --loss tangent trains on the analytic loss instead
-(derivatives propagated through the MLP, physad_tangent_loss_grad_dev): same slabs, same single all-reduce.  Prints one JSON line per 20 steps and a summary."""
+(derivatives propagated through the MLP, physad_tangent_loss_grad_dev): same slabs, same single all-reduce.  --layers L > 1
+trains a deep network (4 -> H -> ... -> H -> 4, L hidden layers; hidden weights drawn uniform in +-0.2) on the
+finite-difference loss through physad_deep_loss_grad_dev, again with one all-reduce of P+2 doubles.  Prints one JSON
+line per 20 steps and a summary."""
 import argparse
 import json
 import os
@@ -28,7 +31,10 @@ def main():
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--lr", type=float, default=3e-3)
     ap.add_argument("--loss", choices=("fd", "tangent"), default="fd")
+    ap.add_argument("--layers", type=int, default=1, help="hidden layers (> 1: a deep network, finite-difference loss only)")
     a = ap.parse_args()
+    if a.layers > 1 and a.loss != "fd":
+        ap.error("--layers > 1 trains on the finite-difference loss only")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank, local = int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
@@ -39,16 +45,27 @@ def main():
     g = Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True)
     cfg, pw = MLPConfig(4, H, 4, True), PhysWeights(1, 1)
     ctx = ops.Context(local)
-    th = np.concatenate([np.asarray(x, np.float64) for x in ops.mlp_random_init(H, 777, 0.25)])
+    W1, b1, W2, b2 = ops.mlp_random_init(H, 777, 0.25)
+    L = a.layers
+    rng = np.random.default_rng(L)
+    Wh = rng.uniform(-0.2, 0.2, (L - 1) * H * H).astype(np.float32)
+    bh = rng.uniform(-0.2, 0.2, (L - 1) * H).astype(np.float32)
+    parts = [W1, b1, W2, b2] if L == 1 else [W1, b1, Wh, bh, W2, b2]
+    th = np.concatenate([np.asarray(x, np.float64) for x in parts])
+    cuts = np.cumsum([x.size for x in parts])[:-1]
     m, v = np.zeros_like(th), np.zeros_like(th)
     first = last = None
     t0 = time.perf_counter()
     for k in range(1, a.steps + 1):
-        w = [th[:4 * H], th[4 * H:5 * H], th[5 * H:9 * H], th[9 * H:]]
-        ctx.set_weights(cfg, *[x.astype(np.float32) for x in w])
-        if a.loss == "tangent":
+        w = np.split(th.astype(np.float32), cuts)
+        if L > 1:
+            ctx.set_weights_deep(cfg, L, *w)
+            ls, lu, grad = ctx.deep_loss_grad(g, pw, 0.25, 2e-3)     # slab per rank + all-reduce when world > 1
+        elif a.loss == "tangent":
+            ctx.set_weights(cfg, *w)
             ls, lu, grad = ctx.tangent_loss_grad(g, pw, 0.25)      # slab per rank + all-reduce when world > 1
         else:
+            ctx.set_weights(cfg, *w)
             ls, lu, grad = ctx.fused_loss_grad(g, pw, 0.25, 2e-3)
         last = float(ls) + float(lu)
         first = last if first is None else first
@@ -59,7 +76,7 @@ def main():
             print(json.dumps({"step": k, "loss_sigma": float(ls), "loss_u": float(lu)}), flush=True)
     dt = time.perf_counter() - t0
     if rank == 0:
-        print(json.dumps({"summary": f"{a.n}^3 H={H} {a.loss} loss on {world} GPU(s)", "steps": a.steps, "loss_first": first,
+        print(json.dumps({"summary": f"{a.n}^3 H={H} L={L} {a.loss} loss on {world} GPU(s)", "steps": a.steps, "loss_first": first,
                           "loss_last": last, "reduction_pct": 100 * (1 - last / first),
                           "wall_ms_per_step_incl_host_adam": 1e3 * dt / a.steps}))
     if world > 1:

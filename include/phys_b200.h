@@ -55,6 +55,11 @@ void mlp_phys_loss_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const 
 void mlp_phys_loss_tangent_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const MLPWeights& w, const PhysWeights& pw,
                                      float t, float* out_loss_sigma, float* out_loss_u, MLPWeights& grad);
 
+// The closed loop of deeper networks: the two losses of mlp_phys_loss_deep_cuda (strict fp32) AND d(L_sigma + L_u) with
+// respect to every layer's weights.  `grad` is resized to the shapes of `w` (grad.hidden_layers = w.hidden_layers).
+void mlp_phys_loss_deep_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
+                                  float t, float dt, float* out_loss_sigma, float* out_loss_u, DeepMLPWeights& grad);
+
 }  // namespace phys
 
 #endif  // PHYS_AUTODIFF_PHYS_B200_H

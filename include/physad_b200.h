@@ -343,6 +343,33 @@ int physad_tangent_loss_grad_host(physad_ctx* ctx, const physad_grid* g, const p
                                   const float* b1, const float* W2, const float* b2, const physad_phys_weights* w, float t,
                                   float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dW2, float* db2);
 
+/* ---- closed loop of deeper networks (ADDITIVE, no reference counterpart) -------------------------------------------------
+ * The finite-difference loss of physad_deep_loss_host AND the gradient of L_sigma + L_u (weights w included, mean over the
+ * GLOBAL N) with respect to every layer of the network set by physad_set_weights_deep (strict fp32 arithmetic, mode 0).
+ * Forward stage-wise on the device (the deep fields of the three slices, residuals and the stencil adjoint in the
+ * context's workspace of 80 B/point), then one persistent kernel that recomputes the hidden layers tile by tile in the
+ * forward's exact order (so the ReLU masks are those of the fields that produced R), keeps each layer's activations in a
+ * per-block checkpoint area (L x 96 KB per SM) and back-propagates through every layer, and a reduction of the block
+ * partials in block order (bitwise repeatable).
+ * acc: 2 device doubles (sum R_sigma^2, sum |R_u|^2 over the slab); grad: P = physad_deep_grad_len(H, L) device doubles
+ *   dW1[H*4] | db1[H] | dWh[(L-1)*H*H, row-major [out][in]] | dbh[(L-1)*H] | dW2[4*H] | db2[4]
+ * (the argument order of physad_set_weights_deep), the slab's share already scaled by 2w/N of the whole grid -- so an
+ * all-reduce(sum) of the P+2 doubles over the ranks' slabs gives the whole-grid result.  slab NULL = whole grid; an empty
+ * slab gives zeros; a slab recomputes the field planes two around it locally (no halo exchange).  L = 1 is the
+ * one-hidden-layer closed loop (physad_fused_loss_grad_dev / _slab_dev), bit for bit.
+ * Errors: no deep weights (or a physad_set_weights after them): PHYSAD_E_NOWEIGHTS; physad_set_deep_mode(1) or upwind
+ * advection: PHYSAD_E_UNSUPPORTED; bad slab or null pointer: PHYSAD_E_INVALID; a recomputed window of 2^31 points or
+ * more: PHYSAD_E_UNSUPPORTED.
+ * physad_deep_grad_len: host-only, P(H, L) = 9H + 4 + (L-1)(H^2 + H), 0 for shapes that are not built. */
+size_t physad_deep_grad_len(int H, int hidden_layers);
+int physad_deep_loss_grad_dev(physad_ctx* ctx, const physad_grid* g, const physad_slab* slab, const physad_phys_weights* w,
+                              float t, float dt, double* acc, double* grad, void* stream);
+/* Host-buffer form on the whole grid with the context's deep weights: the two losses and the gradient out, split into the
+ * six arrays of physad_set_weights_deep's layouts (any output pointer may be null). */
+int physad_deep_loss_grad_host(physad_ctx* ctx, const physad_grid* g, const physad_phys_weights* w, float t, float dt,
+                               float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dWh, float* dbh, float* dW2,
+                               float* db2);
+
 /* Host-only: the work partition the fused kernel is launched with.  The sequence of tiles x planes
  * tile-planes (tile-major) is cut into at most `slots` contiguous ranges of equal cost, a range paying
  * ~0.9 plane-equivalents for every z-segment it starts (its recomputed halo planes).  Writes the

@@ -95,6 +95,7 @@ EXPORTS = [
     "physad_xchg_status", "physad_set_fused_trace", "physad_set_advection",
     "physad_mlp_generate_fields_lp_dev", "physad_phys_loss_lp_dev", "physad_tangent_loss_dev", "physad_tangent_loss_host",
     "physad_tangent_loss_grad_dev", "physad_tangent_loss_grad_host",
+    "physad_deep_grad_len", "physad_deep_loss_grad_dev", "physad_deep_loss_grad_host",
 ]
 
 
@@ -126,6 +127,7 @@ def lib() -> C.CDLL:
         _LIB.physad_launch_count.restype = C.c_uint64
         _LIB.physad_finalize_loss.restype = None
         _LIB.physad_deep_tc_layer_bytes.restype = C.c_size_t
+        _LIB.physad_deep_grad_len.restype = C.c_size_t
     return _LIB
 
 

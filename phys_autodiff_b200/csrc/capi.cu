@@ -2,6 +2,7 @@
 // the host-pointer staging wrappers.  All arithmetic lives in the kernels (*.cuh); this file only
 // decides shapes, fills the kernel-parameter weight block and moves bytes.
 #include "../../include/physad_b200.h"
+#include "deep_grad_kernels.cuh"
 #include "deep_kernels.cuh"
 #include "deep_tc_kernels.cuh"
 #include "dense_kernels.cuh"
@@ -73,6 +74,12 @@ struct physad_ctx {
     double* h_grad = nullptr;   // pinned, same size
     int grad_blocks_per_sm[3] = {0, 0, 0};   // HT = 32, 64, 128 on this device
     int tgrad_blocks_per_sm[3] = {0, 0, 0};  // the same for the tangent-loss gradient (physad_tangent_loss_grad_*)
+    // deep closed loop (physad_deep_loss_grad_*): per-block activation checkpoints, host-form result buffers
+    float* dckpt = nullptr;
+    size_t dckpt_cap = 0;
+    double* d_dgrad = nullptr;   // [P + 2]
+    double* h_dgrad = nullptr;   // pinned, same size
+    size_t dgrad_cap = 0;
     uint64_t launches = 0;
     int fused_variant = 0;
     int exact_residuals = 0;  // 1: residual arithmetic in double exactly as the CPU reference; 0: fp32 with FMAs
@@ -696,6 +703,8 @@ int physad_ctx_destroy(physad_ctx* c) {
     cudaFree(c->partials); cudaFree(c->ticket); cudaFree(c->d_acc); cudaFree(c->scratch);
     cudaFree(c->gws); cudaFree(c->gpart); cudaFree(c->d_grad);
     if (c->h_grad) cudaFreeHost(c->h_grad);
+    cudaFree(c->dckpt); cudaFree(c->d_dgrad);
+    if (c->h_dgrad) cudaFreeHost(c->h_dgrad);
     if (c->h_acc) cudaFreeHost(c->h_acc);
     if (c->h_res) cudaFreeHost(c->h_res);
     cudaFree(c->d_status);
@@ -1672,6 +1681,150 @@ int physad_tangent_loss_grad_host(physad_ctx* c, const physad_grid* g, const phy
     if (db1) for (int i = 0; i < H; ++i) db1[i] = float(gd[4 * H + i]);
     if (dW2) for (int i = 0; i < 4 * H; ++i) dW2[i] = float(gd[5 * H + i]);
     if (db2) for (int i = 0; i < 4; ++i) db2[i] = float(gd[9 * H + i]);
+    return 0;
+}
+
+// ---- closed loop of deeper networks (deep_grad_kernels.cuh) ----------------------------------------------------------
+size_t physad_deep_grad_len(int H, int hidden_layers) { return deep_grad_len(H, hidden_layers); }
+
+int physad_deep_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad_slab* slab, const physad_phys_weights* w,
+                              float t, float dt, double* acc, double* grad, void* stream) {
+    if (!c || !w || !acc || !grad) return fail(PHYSAD_E_INVALID, "deep_loss_grad: null argument");
+    if (int rc = check_grid(g)) return rc;
+    if (int rc = deep_ready(c, "deep_loss_grad")) return rc;
+    if (c->deep_mode != 0)
+        return fail(PHYSAD_E_UNSUPPORTED, "deep_loss_grad: the gradient is of the strict fp32 network (set_deep_mode(0))");
+    if (c->advection != 0) return fail(PHYSAD_E_UNSUPPORTED, "deep_loss_grad: the stencil adjoint is that of the central scheme");
+    physad_slab s;
+    if (int rc = check_slab(g, slab, &s)) return rc;
+    const bool whole = s.z_begin == 0 && s.z_end == g->nz;
+    // one hidden layer: the one-hidden-layer closed loop, whose gradient layout is the same
+    if (c->deep_layers == 1)
+        return whole ? physad_fused_loss_grad_dev(c, g, w, t, dt, acc, grad, stream)
+                     : physad_fused_loss_grad_slab_dev(c, g, &s, w, t, dt, acc, grad, stream);
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (s.z_begin == s.z_end) {
+        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
+        CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
+        return 0;
+    }
+    // window of VIRTUAL planes [zlo, zhi) whose fields the slab's gradient needs (as physad_fused_loss_grad_slab_dev)
+    const bool per = g->periodic != 0;
+    const int zlo = whole ? 0 : (per ? s.z_begin - 2 : std::max(0, s.z_begin - 2));
+    const int zhi = whole ? g->nz : (per ? s.z_end + 2 : std::min(g->nz, s.z_end + 2));
+    const int npl = zhi - zlo;
+    const size_t pln = size_t(g->nx) * g->ny, NL = pln * npl;
+    if (NL >= (size_t(1) << 31)) return fail(PHYSAD_E_UNSUPPORTED, "deep_loss_grad: window of 2^31 points or more");
+    if (int rc = ensure_grad_workspace(c, 20 * NL)) return rc;   // 12 NL fields, 4 NL residuals, 4 NL time-t adjoint
+    float* f = c->gws;
+    float *s_m = f, *s_0 = f + NL, *s_p = f + 2 * NL, *u_m = f + 3 * NL, *u_0 = f + 6 * NL, *u_p = f + 9 * NL, *R = f + 12 * NL;
+    if (whole) {
+        // the arithmetic of physad_deep_loss_host: same fields, same residual kernel, same sums
+        if (int rc = physad_mlp_generate_fields_deep_dev(c, g, nullptr, t, dt, s_m, s_0, s_p, u_m, u_0, u_p, stream)) return rc;
+        if (int rc = physad_phys_loss_dev(c, g, s_m, s_0, s_p, u_m, u_0, u_p, acc, R, R + NL, R + 2 * NL, R + 3 * NL, stream))
+            return rc;
+    } else {
+        // fields: the deep kernel writes u with the channel stride of its own launch, so each run of consecutive global
+        // planes goes to a contiguous scratch buffer and its 12 channel blocks are copied into the window arrays
+        int max_run = 0;
+        for (int zv = zlo; zv < zhi;) {
+            const int ga = ((zv % g->nz) + g->nz) % g->nz, run = std::min(zhi - zv, g->nz - ga);
+            max_run = std::max(max_run, run);
+            zv += run;
+        }
+        if (int rc = ensure_scratch(c, 12 * pln * size_t(max_run) * sizeof(float))) return rc;
+        float* sc = reinterpret_cast<float*>(c->scratch);
+        for (int zv = zlo; zv < zhi;) {
+            const int ga = ((zv % g->nz) + g->nz) % g->nz, run = std::min(zhi - zv, g->nz - ga);
+            const size_t nr = pln * size_t(run), off = size_t(zv - zlo) * pln;
+            const physad_slab rs{ga, ga + run};
+            if (int rc = physad_mlp_generate_fields_deep_dev(c, g, &rs, t, dt, sc, sc + nr, sc + 2 * nr, sc + 3 * nr, sc + 6 * nr,
+                                                             sc + 9 * nr, stream))
+                return rc;
+            float* dst[12] = {s_m + off, s_0 + off, s_p + off};
+            for (int k = 0; k < 3; ++k)
+                for (int ch = 0; ch < 3; ++ch) dst[3 + 3 * k + ch] = (k == 0 ? u_m : (k == 1 ? u_0 : u_p)) + ch * NL + off;
+            for (int b = 0; b < 12; ++b)
+                CU(cudaMemcpyAsync(dst[b], sc + size_t(b) * nr, nr * sizeof(float), cudaMemcpyDeviceToDevice, st));
+            zv += run;
+        }
+        // residuals of every window plane with the z neighbours clamped at its ends (exact on the planes the slab uses)
+        PhysArgs pa = phys_args(s_m, s_0, s_p, u_m, u_0, u_p, R, R + NL, R + 2 * NL, R + 3 * NL);
+        pa.clamp_z = 1;
+        if (int rc = launch_phys<true, false, false>(c, g, pa, st, npl)) return rc;
+    }
+    // time-t output adjoint A_t of the slab's points
+    GradArgs ga{};
+    if (int rc = grad_args_common(c, g, w, t, dt, ga, st)) return rc;
+    ga.z_begin = s.z_begin; ga.z_end = s.z_end; ga.z_origin = zlo;
+    ga.wrap_z = whole ? ga.periodic : 0;
+    ga.cstride = NL;
+    ga.s0 = s_0; ga.u0 = u_0;
+    for (int k = 0; k < 4; ++k) ga.R[k] = R + k * NL;
+    float4* adj = reinterpret_cast<float4*>(f + 16 * NL);
+    CU(cudaError_t(adjoint_launch(ga, adj, st)));
+    c->launches++;
+    // back-propagation through every layer, then the block-order reduction
+    const long long npts = (long long)pln * (s.z_end - s.z_begin);
+    const int blocks = deep_grad_blocks(H, npts, c->sm_count);
+    const size_t ck = size_t(blocks) * deep_grad_ckpt_floats(H, L);
+    if (ck > c->dckpt_cap) {
+        if (c->dckpt) CU(cudaFree(c->dckpt));
+        c->dckpt = nullptr; c->dckpt_cap = 0;
+        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
+        c->dckpt_cap = ck;
+    }
+    if (int rc = ensure_grad_partials(c, size_t(blocks) * (P + 2))) return rc;
+    DeepGradArgs a{};
+    a.nx = g->nx; a.ny = g->ny; a.nz = g->nz;
+    a.z_begin = s.z_begin; a.z_end = s.z_end; a.z_origin = zlo;
+    a.hidden_layers = L;
+    a.cxs = ga.cxs; a.cys = ga.cys; a.czs = ga.czs;
+    a.W1 = c->dW1; a.b1 = c->db1; a.W2 = c->dW2;
+    for (int k = 0; k < 3; ++k) a.tc[k] = ga.tc[k];
+    a.wh = c->d_wh; a.bh = c->d_bh;
+    for (int k = 0; k < 4; ++k) a.R[k] = ga.R[k];
+    a.adj = adj;
+    a.scale_s = ga.scale_s; a.scale_u = ga.scale_u; a.inv2dt = ga.inv2dt;
+    a.ckpt = c->dckpt;
+    a.partials = c->gpart;
+    CU(cudaError_t(deep_grad_launch(H, a, blocks, grad, whole ? nullptr : acc, st)));
+    c->launches += 2;
+    return 0;
+}
+
+int physad_deep_loss_grad_host(physad_ctx* c, const physad_grid* g, const physad_phys_weights* w, float t, float dt,
+                               float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dWh, float* dbh, float* dW2,
+                               float* db2) {
+    if (!c || !w) return fail(PHYSAD_E_INVALID, "deep_loss_grad: null argument");
+    if (int rc = check_grid(g)) return rc;
+    if (int rc = deep_ready(c, "deep_loss_grad")) return rc;
+    DeviceGuard dg(c->device);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (P + 2 > c->dgrad_cap) {
+        if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
+        if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
+        c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
+        CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
+        CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
+        c->dgrad_cap = P + 2;
+    }
+    if (int rc = physad_deep_loss_grad_dev(c, g, nullptr, w, t, dt, c->d_dgrad, c->d_dgrad + 2, c->stream)) return rc;
+    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 2) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    physad_finalize_loss(c->h_dgrad, w, size_t(g->nx) * g->ny * g->nz, loss_sigma, loss_u);
+    const double* gd = c->h_dgrad + 2;
+    const size_t nl = size_t(L - 1), hh = size_t(H);
+    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
+    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
+    for (int k = 0; k < 6; ++k) {
+        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
+        gd += len[k];
+    }
     return 0;
 }
 

@@ -38,6 +38,7 @@ class Context:
         self._h = C.c_void_p()
         check(self._lib.physad_ctx_create(C.byref(self._h), C.c_int(-1 if device is None else device)), "ctx_create")
         self.cfg: Optional[MLPConfig] = None
+        self.hidden_layers: Optional[int] = None   # L of the network set by set_weights_deep
         self._peers = None  # (rank, world) once connect_peers() has mapped the peers' exchange buffers
 
     def close(self):
@@ -126,6 +127,7 @@ class Context:
         c = cfg.c()
         check(self._lib.physad_set_weights(self._h, C.byref(c), ptr(W1), ptr(b1), ptr(W2), ptr(b2)), "set_weights")
         self.cfg = cfg
+        self.hidden_layers = None   # a plain set_weights replaces any deep network
 
     # -- helpers -------------------------------------------------------------------------------
     @staticmethod
@@ -210,6 +212,7 @@ class Context:
                                                 ptr(Wh) if Wh.size else None, ptr(bh) if bh.size else None, ptr(W2), ptr(b2)),
               "set_weights_deep")
         self.cfg = cfg
+        self.hidden_layers = hidden_layers
 
     def deep_loss(self, g: Grid, pw: PhysWeights, t: float, dt: float):
         """(L_sigma, L_u) of the deep network set by set_weights_deep, in one call (fields stay in context scratch)."""
@@ -218,6 +221,46 @@ class Context:
         check(self._lib.physad_deep_loss_host(self._h, C.byref(cg), C.byref(cw), C.c_float(t), C.c_float(dt), C.byref(ls),
                                               C.byref(lu)), "deep_loss")
         return np.float32(ls.value), np.float32(lu.value)
+
+    # -- closed loop of deeper networks (additive) -------------------------------------------------------------
+    def deep_grad_len(self) -> int:
+        """P(H, L) = 9H + 4 + (L-1)(H^2 + H): the gradient length of the network set by set_weights_deep."""
+        return int(self._lib.physad_deep_grad_len(C.c_int(self.cfg.H), C.c_int(self.hidden_layers or 1)))
+
+    def deep_loss_grad_acc(self, g: Grid, pw: PhysWeights, t: float, dt: float, slab=None, out=None):
+        """Device form: a float64 device tensor [acc_sigma, acc_u, grad(P)] of the slab (None = whole grid) for the deep
+        network; grad = dW1 | db1 | dWh | dbh | dW2 | db2, scaled by 2w/N of the whole grid, so the slabs' tensors add up."""
+        import torch
+        out = out if out is not None else self._empty(self.deep_grad_len() + 2, torch.float64)
+        cs, _ = self._slab(g, slab)
+        cg, cw = g.c(), pw.c()
+        check(self._lib.physad_deep_loss_grad_dev(self._h, C.byref(cg), C.byref(cs), C.byref(cw), C.c_float(t), C.c_float(dt),
+                                                  ptr(out), ptr(out[2:]), self._stream()), "deep_loss_grad")
+        return out
+
+    def deep_loss_grad(self, g: Grid, pw: PhysWeights, t: float, dt: float, group=None):
+        """(L_sigma, L_u, grad float64 ndarray[P]) of the deep network.  With torch.distributed initialised each rank
+        differentiates its z-slab (field planes two around it recomputed locally) and ONE all-reduce of P+2 doubles
+        combines them."""
+        import torch.distributed as dist
+        world, rank = (dist.get_world_size(group), dist.get_rank(group)) if dist.is_initialized() else (1, 0)
+        buf = self.deep_loss_grad_acc(g, pw, t, dt, slab_for_rank(g.nz, rank, world))
+        if world > 1:
+            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+        h = buf.cpu().numpy()
+        ls, lu = self.finalize(h[:2], pw, g.N)
+        return ls, lu, h[2:].copy()
+
+    def deep_loss_grad_host(self, g: Grid, pw: PhysWeights, t: float, dt: float):
+        """Host-buffer form with the context's deep weights: (L_sigma, L_u, dW1, db1, dWh, dbh, dW2, db2), float32."""
+        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
+        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        ls, lu = C.c_float(), C.c_float()
+        cg, cw = g.c(), pw.c()
+        check(self._lib.physad_deep_loss_grad_host(self._h, C.byref(cg), C.byref(cw), C.c_float(t), C.c_float(dt), C.byref(ls),
+                                                   C.byref(lu), *[ptr(x) if x.size else None for x in d]),
+              "deep_loss_grad_host")
+        return (np.float32(ls.value), np.float32(lu.value), *d)
 
     def set_deep_mode(self, mode: int) -> None:
         """0: strict fp32 (bit-exact, default); 1: hidden layers on the tensor cores with three-term bf16 operands (~1e-6)."""
@@ -705,6 +748,14 @@ def mlp_phys_loss_tangent_cuda(g: Grid, cfg: MLPConfig, w, pw: PhysWeights, t: f
 def mlp_phys_loss_grad_cuda(g: Grid, cfg: MLPConfig, w, pw: PhysWeights, t: float, dt: float):
     """Closed loop (additive): losses and d(L_sigma + L_u)/d(W1, b1, W2, b2)."""
     return default_context().fused_loss_grad_host(g, cfg, *w, pw, t, dt)
+
+
+def mlp_phys_loss_deep_grad_cuda(g: Grid, cfg: MLPConfig, L: int, w, pw: PhysWeights, t: float, dt: float):
+    """Closed loop of a deep network (additive): w = (W1, b1, Wh, bh, W2, b2) ->
+    (L_sigma, L_u, dW1, db1, dWh, dbh, dW2, db2)."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.deep_loss_grad_host(g, pw, t, dt)
 
 
 def mlp_phys_loss_tangent_grad_cuda(g: Grid, cfg: MLPConfig, w, pw: PhysWeights, t: float):

@@ -2,9 +2,13 @@
 step (fields, residuals + sums, stencil adjoint, MLP backward [+ the all-reduce of 9H+6 doubles under torchrun]).
 --loss tangent times the closed loop of the analytic loss instead (one kernel, physad_tangent_loss_grad_dev) and reports,
 from the same process, the analytic forward alone, the finite-difference step, the counted flops and the GPU it ran on.
-  python tools/bench_grad.py [--loss fd|tangent] [--n 256] [--hidden 64] [--steps 20]
+--loss deep times the closed loop of a deep network (physad_deep_loss_grad_dev) for every --hidden x --layers pair, in
+alternation with the strict deep fields alone (generate_fields_deep) and the one-hidden-layer step; one JSON line per pair.
+  python tools/bench_grad.py [--loss fd|tangent|deep] [--n 256] [--hidden 64] [--layers 3] [--steps 20]
+  python tools/bench_grad.py --loss deep --hidden 32,64,128 --layers 2,3,5
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/bench_grad.py   (z-slab per rank)"""
 import argparse
+import ctypes as C
 import json
 import subprocess
 import sys, os
@@ -18,10 +22,14 @@ from phys_autodiff_b200 import Grid, MLPConfig, PhysWeights, ops
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--n", type=int, default=256)
-    ap.add_argument("--hidden", type=int, default=64)
+    ap.add_argument("--hidden", default="64", help="width; --loss deep takes a comma-separated list")
+    ap.add_argument("--layers", default="3", help="--loss deep: hidden layers, a comma-separated list")
     ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--loss", choices=("fd", "tangent"), default="fd")
+    ap.add_argument("--loss", choices=("fd", "tangent", "deep"), default="fd")
     a = ap.parse_args()
+    if a.loss == "deep":
+        return deep(a, Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True))
+    a.hidden = int(a.hidden)
     g = Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True)
     if "RANK" in os.environ and int(os.environ.get("WORLD_SIZE", "1")) > 1:
         return distributed(a, g)
@@ -111,6 +119,56 @@ def tangent(a, g):
                       "fd_loss_grad_ms": fd[len(fd) // 2], "flops_per_point": flops_pt,
                       "counted_tflops": flops_pt * g.N / (med * 1e-3) / 1e12, "gpu": name, "power_limit_w": plim,
                       "grad_norm": float(abs(h[2:]).max()), "acc": h[:2].tolist()}))
+
+
+# counted work of one deep closed-loop step per row (a row = one point and time slice; 3 rows per point), 2 flops per
+# multiply-add: the strict fields (hidden layers 2(L-1)H^2, layer 1 and output 16H), the recompute in k_deep_grad
+# (2(L-1)H^2 + 8H), W^T delta_z and dW of every hidden layer (4(L-1)H^2), output layer and layer 1 backward (24H)
+def deep_flops_per_point(H, L):
+    return 3 * (8 * (L - 1) * H * H + 48 * H)
+
+
+def deep(a, g):
+    import numpy as np
+    ctx = ops.Context()
+    pw = PhysWeights(1, 1)
+    name, plim = _gpu()
+    for H in (int(x) for x in a.hidden.split(",")):
+        w1 = ops.mlp_random_init(H, 777, 0.25)
+        for L in (int(x) for x in a.layers.split(",")):
+            rng = np.random.default_rng(L)
+            Wh = rng.uniform(-0.2, 0.2, (L - 1) * H * H).astype(np.float32)
+            bh = rng.uniform(-0.2, 0.2, (L - 1) * H).astype(np.float32)
+            ctx.set_weights(MLPConfig(4, H, 4, True), *w1)
+            acc, grad = ctx.fused_loss_grad_acc(g, pw, 0.25, 2e-3)
+            ctx.set_weights_deep(MLPConfig(4, H, 4, True), L, w1[0], w1[1], Wh, bh, w1[2], w1[3])
+            out = ctx.deep_loss_grad_acc(g, pw, 0.25, 2e-3)
+            f = ctx.mlp_generate_fields_deep(g, 0.25, 2e-3)
+            gen = lambda: ctx._lib.physad_mlp_generate_fields_deep_dev(ctx._h, C.byref(cg), None, C.c_float(0.25), C.c_float(2e-3),
+                                                                       *[ops.ptr(x) for x in f], ctx._stream())
+            cg = g.c()
+            for _ in range(2):
+                ctx.deep_loss_grad_acc(g, pw, 0.25, 2e-3, out=out)
+                assert gen() == 0
+            torch.cuda.synchronize()
+            # the three are timed in alternation, so that they share whatever else the GPU is doing; the one-hidden-layer
+            # step runs through the same context after set_weights (the deep weights are restored before the next deep call)
+            dg, fw, fd = [], [], []
+            for _ in range(a.steps):
+                dg += _times(lambda: ctx.deep_loss_grad_acc(g, pw, 0.25, 2e-3, out=out), 1)
+                fw += _times(gen, 1)
+            ctx.set_weights(MLPConfig(4, H, 4, True), *w1)
+            for _ in range(a.steps):
+                fd += _times(lambda: ctx.fused_loss_grad_acc(g, pw, 0.25, 2e-3, acc, grad), 1)
+            dg.sort(); fw.sort(); fd.sort()
+            med = dg[len(dg) // 2]
+            fl = deep_flops_per_point(H, L)
+            h = out.cpu().numpy()
+            print(json.dumps({"workload": f"{a.n}^3 H={H} L={L} deep loss+grad", "ms_median": med, "ms_min": dg[0],
+                              "fields_deep_ms": fw[len(fw) // 2], "ratio_to_fields": med / fw[len(fw) // 2],
+                              "fd_one_layer_loss_grad_ms": fd[len(fd) // 2], "flops_per_point": fl,
+                              "counted_tflops": fl * g.N / (med * 1e-3) / 1e12, "gpu": name, "power_limit_w": plim,
+                              "grad_absmax": float(abs(h[2:]).max()), "acc": h[:2].tolist()}), flush=True)
 
 
 def distributed(a, g):
