@@ -9,8 +9,9 @@ gives every rank the same losses and gradient, and every rank applies the same A
 580 (H=64) parameters -- no parameter broadcast is needed.  --loss tangent trains on the analytic loss instead
 (derivatives propagated through the MLP, physad_tangent_loss_grad_dev): same slabs, same single all-reduce.  --layers L > 1
 trains a deep network (4 -> H -> ... -> H -> 4, L hidden layers; hidden weights drawn uniform in +-0.2) on the
-finite-difference loss through physad_deep_loss_grad_dev, again with one all-reduce of P+2 doubles.  Prints one JSON
-line per 20 steps and a summary."""
+finite-difference loss through physad_deep_loss_grad_dev, or with --loss tangent on the analytic loss through
+physad_deep_tangent_loss_grad_dev, again with one all-reduce of P+2 doubles.  Prints one JSON line per 20 steps and a
+summary."""
 import argparse
 import json
 import os
@@ -31,10 +32,8 @@ def main():
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--lr", type=float, default=3e-3)
     ap.add_argument("--loss", choices=("fd", "tangent"), default="fd")
-    ap.add_argument("--layers", type=int, default=1, help="hidden layers (> 1: a deep network, finite-difference loss only)")
+    ap.add_argument("--layers", type=int, default=1, help="hidden layers (> 1: a deep network)")
     a = ap.parse_args()
-    if a.layers > 1 and a.loss != "fd":
-        ap.error("--layers > 1 trains on the finite-difference loss only")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank, local = int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
@@ -58,7 +57,10 @@ def main():
     t0 = time.perf_counter()
     for k in range(1, a.steps + 1):
         w = np.split(th.astype(np.float32), cuts)
-        if L > 1:
+        if L > 1 and a.loss == "tangent":
+            ctx.set_weights_deep(cfg, L, *w)
+            ls, lu, grad = ctx.deep_tangent_loss_grad(g, pw, 0.25)   # slab per rank + all-reduce when world > 1
+        elif L > 1:
             ctx.set_weights_deep(cfg, L, *w)
             ls, lu, grad = ctx.deep_loss_grad(g, pw, 0.25, 2e-3)     # slab per rank + all-reduce when world > 1
         elif a.loss == "tangent":

@@ -60,6 +60,15 @@ void mlp_phys_loss_tangent_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg
 void mlp_phys_loss_deep_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
                                   float t, float dt, float* out_loss_sigma, float* out_loss_u, DeepMLPWeights& grad);
 
+// The analytic loss of a deep network: the derivatives of mlp_phys_loss_tangent_cuda propagated in forward mode through every
+// layer of the DeepMLPWeights network (value row in the strict fp32 order of the deep forward, tangent rows with FMA), and its
+// closed loop, d(L_sigma + L_u) with respect to every layer's weights.  `grad` is resized to the shapes of `w`.
+void mlp_phys_loss_deep_tangent_cuda(const GridSpec& g, const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
+                                     float t, float* out_loss_sigma, float* out_loss_u);
+void mlp_phys_loss_deep_tangent_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const DeepMLPWeights& w,
+                                          const PhysWeights& pw, float t, float* out_loss_sigma, float* out_loss_u,
+                                          DeepMLPWeights& grad);
+
 }  // namespace phys
 
 #endif  // PHYS_AUTODIFF_PHYS_B200_H

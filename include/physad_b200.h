@@ -370,6 +370,34 @@ int physad_deep_loss_grad_host(physad_ctx* ctx, const physad_grid* g, const phys
                                float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dWh, float* dbh, float* dW2,
                                float* db2);
 
+/* ---- analytic loss of deeper networks and its closed loop (ADDITIVE, no reference counterpart) ---------------------------
+ * The analytic loss of physad_tangent_loss_dev for the network set by physad_set_weights_deep: per point the network runs
+ * on the value row and the four tangent rows d/dc_k (k = x, y, z, t), the value row in the strict fp32 order of
+ * physad_mlp_grid_infer_deep (so the ReLU masks are that network's at time t), the tangent rows with fused multiply-adds
+ * (inputs ascending); residuals and sums as physad_tangent_loss_dev.  One persistent kernel plus a block-order reduction
+ * (bitwise repeatable); points are independent, so a slab needs no window and no halo.
+ * physad_deep_tangent_loss_dev: acc = 2 device doubles (sum R_sigma^2, sum |R_u|^2 over the slab); R_* (all set or all
+ *   null): slab-local residuals.
+ * physad_deep_tangent_loss_grad_dev: the same acc (bit for bit) AND the gradient of L_sigma + L_u (weights w included,
+ *   mean over the GLOBAL N) with respect to every layer, P = physad_deep_grad_len(H, L) device doubles in the layout of
+ *   physad_deep_loss_grad_dev, the slab's share already scaled by 2w/N of the whole grid -- so an all-reduce(sum) of the
+ *   P+2 doubles over the ranks' slabs gives the whole-grid result.  Reverse mode over the forward, in the same kernel:
+ *   per-block activation checkpoints (L x 80 KB per SM), no per-point workspace.
+ * slab NULL = whole grid; an empty slab gives zeros.  L = 1 is physad_tangent_loss_dev / physad_tangent_loss_grad_dev,
+ * bit for bit.  The advection switch does not apply.
+ * Errors: no deep weights (or a physad_set_weights after them): PHYSAD_E_NOWEIGHTS; physad_set_deep_mode(1):
+ * PHYSAD_E_UNSUPPORTED; bad slab, null pointer or residual pointers not all set or all null: PHYSAD_E_INVALID; a grid of
+ * 2^31 points or more (hence any such slab): PHYSAD_E_UNSUPPORTED. */
+int physad_deep_tangent_loss_dev(physad_ctx* ctx, const physad_grid* g, const physad_slab* slab, float t, double* acc,
+                                 float* R_sigma, float* R_ux, float* R_uy, float* R_uz, void* stream);
+int physad_deep_tangent_loss_grad_dev(physad_ctx* ctx, const physad_grid* g, const physad_slab* slab, const physad_phys_weights* w,
+                                      float t, double* acc, double* grad, void* stream);
+/* Host-buffer form on the whole grid with the context's deep weights: the two losses and the gradient out, split into the
+ * six arrays of physad_set_weights_deep's layouts (any output pointer may be null). */
+int physad_deep_tangent_loss_grad_host(physad_ctx* ctx, const physad_grid* g, const physad_phys_weights* w, float t,
+                                       float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dWh, float* dbh,
+                                       float* dW2, float* db2);
+
 /* Host-only: the work partition the fused kernel is launched with.  The sequence of tiles x planes
  * tile-planes (tile-major) is cut into at most `slots` contiguous ranges of equal cost, a range paying
  * ~0.9 plane-equivalents for every z-segment it starts (its recomputed halo planes).  Writes the

@@ -96,6 +96,7 @@ EXPORTS = [
     "physad_mlp_generate_fields_lp_dev", "physad_phys_loss_lp_dev", "physad_tangent_loss_dev", "physad_tangent_loss_host",
     "physad_tangent_loss_grad_dev", "physad_tangent_loss_grad_host",
     "physad_deep_grad_len", "physad_deep_loss_grad_dev", "physad_deep_loss_grad_host",
+    "physad_deep_tangent_loss_dev", "physad_deep_tangent_loss_grad_dev", "physad_deep_tangent_loss_grad_host",
 ]
 
 

@@ -4,6 +4,7 @@
 #include "../../include/physad_b200.h"
 #include "deep_grad_kernels.cuh"
 #include "deep_kernels.cuh"
+#include "deep_tangent_kernels.cuh"
 #include "deep_tc_kernels.cuh"
 #include "dense_kernels.cuh"
 #include "grad_kernels.cuh"
@@ -1814,6 +1815,135 @@ int physad_deep_loss_grad_host(physad_ctx* c, const physad_grid* g, const physad
         c->dgrad_cap = P + 2;
     }
     if (int rc = physad_deep_loss_grad_dev(c, g, nullptr, w, t, dt, c->d_dgrad, c->d_dgrad + 2, c->stream)) return rc;
+    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 2) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    physad_finalize_loss(c->h_dgrad, w, size_t(g->nx) * g->ny * g->nz, loss_sigma, loss_u);
+    const double* gd = c->h_dgrad + 2;
+    const size_t nl = size_t(L - 1), hh = size_t(H);
+    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
+    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
+    for (int k = 0; k < 6; ++k) {
+        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
+        gd += len[k];
+    }
+    return 0;
+}
+
+// ---- analytic loss of deeper networks and its closed loop (deep_tangent_kernels.cuh) ---------------------------------
+}  // extern "C"  (helpers below)
+namespace {
+// checks and arguments shared by the loss and the loss + gradient call; *npts = 0 for an empty slab
+int deep_tangent_args(physad_ctx* c, const physad_grid* g, const physad_slab* slab, float t, const char* what,
+                      DeepTangentArgs& a, long long* npts, cudaStream_t st) {
+    if (int rc = check_grid(g)) return rc;
+    if (int rc = deep_ready(c, what)) return rc;
+    if (c->deep_mode != 0)
+        return fail(PHYSAD_E_UNSUPPORTED, std::string(what) + ": the analytic deep loss is that of the strict fp32 network (set_deep_mode(0))");
+    physad_slab s;
+    if (int rc = check_slab(g, slab, &s)) return rc;
+    const size_t n = size_t(s.z_end - s.z_begin) * g->ny * g->nx;   // < 2^31: check_grid bounds the whole grid
+    *npts = (long long)n;
+    if (n == 0) return 0;
+    if (int rc = upload_weights_if_stale(c, st)) return rc;
+    if (int rc = ensure_coord_tables(c, g, st)) return rc;
+    a.nx = g->nx; a.ny = g->ny; a.nz = g->nz; a.z_begin = s.z_begin; a.z_end = s.z_end;
+    a.hidden_layers = c->deep_layers;
+    a.cxs = c->tab.dev; a.cys = a.cxs + g->nx; a.czs = a.cys + g->ny;
+    a.W1 = c->dW1; a.b1 = c->db1; a.W2 = c->dW2; a.b2 = c->db2;
+    a.wh = c->d_wh; a.bh = c->d_bh;
+    a.tc = time_coord(t, c->cfg.norm);
+    // dc/dx exactly as physad_tangent_loss_dev forms it (0 for an extent of 1)
+    const double f = c->cfg.norm == 1 ? 2.0 : 1.0;
+    a.sx = g->nx > 1 ? float(f / (double(g->nx - 1) * double(g->hx))) : 0.f;
+    a.sy = g->ny > 1 ? float(f / (double(g->ny - 1) * double(g->hy))) : 0.f;
+    a.sz = g->nz > 1 ? float(f / (double(g->nz - 1) * double(g->hz))) : 0.f;
+    return 0;
+}
+}  // namespace
+extern "C" {
+
+int physad_deep_tangent_loss_dev(physad_ctx* c, const physad_grid* g, const physad_slab* slab, float t, double* acc,
+                                 float* Rs, float* Rx, float* Ry, float* Rz, void* stream) {
+    if (!c || !acc) return fail(PHYSAD_E_INVALID, "deep_tangent_loss: null argument");
+    const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
+    if (any && !all) return fail(PHYSAD_E_INVALID, "deep_tangent_loss: residual outputs must be all set or all null");
+    if (int rc = check_grid(g)) return rc;
+    if (int rc = deep_ready(c, "deep_tangent_loss")) return rc;
+    // one hidden layer: the one-hidden-layer analytic loss (its Jacobian products are precomputed on the host)
+    if (c->deep_layers == 1 && c->deep_mode == 0) return physad_tangent_loss_dev(c, g, slab, t, acc, Rs, Rx, Ry, Rz, stream);
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    DeepTangentArgs a{};
+    long long npts = 0;
+    if (int rc = deep_tangent_args(c, g, slab, t, "deep_tangent_loss", a, &npts, st)) return rc;
+    if (npts == 0) {
+        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
+        return 0;
+    }
+    a.R[0] = Rs; a.R[1] = Rx; a.R[2] = Ry; a.R[3] = Rz;
+    const int H = c->cfg.H;
+    const int blocks = deep_tangent_blocks(H, npts, c->sm_count);
+    if (int rc = ensure_grad_partials(c, size_t(blocks) * 2)) return rc;
+    a.partials = c->gpart;
+    CU(cudaError_t(deep_tangent_launch(H, false, a, blocks, acc, nullptr, st)));
+    c->launches += 2;
+    return 0;
+}
+
+int physad_deep_tangent_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad_slab* slab, const physad_phys_weights* w,
+                                      float t, double* acc, double* grad, void* stream) {
+    if (!c || !w || !acc || !grad) return fail(PHYSAD_E_INVALID, "deep_tangent_loss_grad: null argument");
+    if (int rc = check_grid(g)) return rc;
+    if (int rc = deep_ready(c, "deep_tangent_loss_grad")) return rc;
+    // one hidden layer: the one-hidden-layer closed loop, whose gradient layout is the same
+    if (c->deep_layers == 1 && c->deep_mode == 0) return physad_tangent_loss_grad_dev(c, g, slab, w, t, acc, grad, stream);
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    DeepTangentArgs a{};
+    long long npts = 0;
+    if (int rc = deep_tangent_args(c, g, slab, t, "deep_tangent_loss_grad", a, &npts, st)) return rc;
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (npts == 0) {
+        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
+        CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
+        return 0;
+    }
+    vjp_scales(g, w, &a.scale_s, &a.scale_u);   // 2 w / float(N) of the whole grid: slab results add up to the grid's
+    const int blocks = deep_tangent_blocks(H, npts, c->sm_count);
+    const size_t ck = size_t(blocks) * deep_tangent_ckpt_floats(L);
+    if (ck > c->dckpt_cap) {
+        if (c->dckpt) CU(cudaFree(c->dckpt));
+        c->dckpt = nullptr; c->dckpt_cap = 0;
+        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
+        c->dckpt_cap = ck;
+    }
+    if (int rc = ensure_grad_partials(c, size_t(blocks) * (P + 2))) return rc;
+    a.ckpt = c->dckpt;
+    a.partials = c->gpart;
+    CU(cudaError_t(deep_tangent_launch(H, true, a, blocks, acc, grad, st)));
+    c->launches += 2;
+    return 0;
+}
+
+int physad_deep_tangent_loss_grad_host(physad_ctx* c, const physad_grid* g, const physad_phys_weights* w, float t,
+                                       float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dWh, float* dbh,
+                                       float* dW2, float* db2) {
+    if (!c || !w) return fail(PHYSAD_E_INVALID, "deep_tangent_loss_grad: null argument");
+    if (int rc = check_grid(g)) return rc;
+    if (int rc = deep_ready(c, "deep_tangent_loss_grad")) return rc;
+    DeviceGuard dg(c->device);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (P + 2 > c->dgrad_cap) {
+        if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
+        if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
+        c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
+        CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
+        CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
+        c->dgrad_cap = P + 2;
+    }
+    if (int rc = physad_deep_tangent_loss_grad_dev(c, g, nullptr, w, t, c->d_dgrad, c->d_dgrad + 2, c->stream)) return rc;
     CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 2) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     physad_finalize_loss(c->h_dgrad, w, size_t(g->nx) * g->ny * g->nz, loss_sigma, loss_u);

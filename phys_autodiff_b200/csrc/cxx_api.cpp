@@ -350,6 +350,51 @@ void mlp_phys_loss_deep_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, c
     if (rc) die("mlp_phys_loss_deep_grad_cuda", rc);
 }
 
+namespace {
+int set_deep(physad_ctx* c, const MLPGridConfig& cfg, const DeepMLPWeights& w) {
+    const physad_mlp_config mc{int(cfg.dims.In), int(cfg.dims.H), int(cfg.dims.Out), norm_of(cfg.norm)};
+    return physad_set_weights_deep(c, &mc, w.hidden_layers, w.W1.data(), w.b1.data(), w.Wh.empty() ? nullptr : w.Wh.data(),
+                                   w.bh.empty() ? nullptr : w.bh.data(), w.W2.data(), w.b2.data());
+}
+}  // namespace
+
+void mlp_phys_loss_deep_tangent_cuda(const GridSpec& g, const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
+                                     float t, float* out_loss_sigma, float* out_loss_u) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    const physad_grid cg = to_c(g);
+    const physad_phys_weights cw = to_c(pw);
+    physad_ctx* c = ctx();
+    static double* d_acc = nullptr;   // the two device sums; lives as long as the process's context
+    int rc = set_deep(c, cfg, w);
+    if (!rc && !d_acc) rc = int(cudaMalloc(&d_acc, 2 * sizeof(double)));
+    if (!rc) rc = physad_deep_tangent_loss_dev(c, &cg, nullptr, t, d_acc, nullptr, nullptr, nullptr, nullptr, nullptr);
+    double h_acc[2] = {0.0, 0.0};
+    if (!rc) rc = int(cudaMemcpy(h_acc, d_acc, sizeof(h_acc), cudaMemcpyDeviceToHost));
+    if (rc) die("mlp_phys_loss_deep_tangent_cuda", rc);
+    physad_finalize_loss(h_acc, &cw, size_t(g.nx) * g.ny * g.nz, out_loss_sigma, out_loss_u);
+}
+
+void mlp_phys_loss_deep_tangent_grad_cuda(const GridSpec& g, const MLPGridConfig& cfg, const DeepMLPWeights& w,
+                                          const PhysWeights& pw, float t, float* out_loss_sigma, float* out_loss_u,
+                                          DeepMLPWeights& grad) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    const physad_grid cg = to_c(g);
+    const physad_phys_weights cw = to_c(pw);
+    physad_ctx* c = ctx();
+    grad.hidden_layers = w.hidden_layers;
+    grad.W1.resize(w.W1.size());
+    grad.b1.resize(w.b1.size());
+    grad.Wh.resize(w.Wh.size());
+    grad.bh.resize(w.bh.size());
+    grad.W2.resize(w.W2.size());
+    grad.b2.resize(w.b2.size());
+    int rc = set_deep(c, cfg, w);
+    if (!rc) rc = physad_deep_tangent_loss_grad_host(c, &cg, &cw, t, out_loss_sigma, out_loss_u, grad.W1.data(), grad.b1.data(),
+                                                     grad.Wh.empty() ? nullptr : grad.Wh.data(),
+                                                     grad.bh.empty() ? nullptr : grad.bh.data(), grad.W2.data(), grad.b2.data());
+    if (rc) die("mlp_phys_loss_deep_tangent_grad_cuda", rc);
+}
+
 }  // namespace phys
 
 // C-ABI access to the weight generator for non-C++ hosts (bench.py, tests): see include/physad_b200.h.

@@ -262,6 +262,56 @@ class Context:
               "deep_loss_grad_host")
         return (np.float32(ls.value), np.float32(lu.value), *d)
 
+    # -- analytic loss of deeper networks and its closed loop (additive) ---------------------------------------
+    def deep_tangent_loss_acc(self, g: Grid, t: float, slab=None, acc=None, residuals=None):
+        """Analytic (forward-mode) loss of the deep network set by set_weights_deep: the device sums
+        {sum Rs^2, sum |Ru|^2} of the slab (None = whole grid); residuals: four slab-sized float32 device tensors or None."""
+        import torch
+        cs, _ = self._slab(g, slab)
+        if acc is None:
+            acc = self._empty(2, torch.float64)
+        R = residuals if residuals is not None else [None] * 4
+        cg = g.c()
+        check(self._lib.physad_deep_tangent_loss_dev(self._h, C.byref(cg), C.byref(cs), C.c_float(t), ptr(acc),
+                                                     *[ptr(r) for r in R], self._stream()), "deep_tangent_loss")
+        return acc
+
+    def deep_tangent_loss_grad_acc(self, g: Grid, pw: PhysWeights, t: float, slab=None, out=None):
+        """Device form: a float64 device tensor [acc_sigma, acc_u, grad(P)] of the analytic loss of the deep network for
+        the slab (None = whole grid); grad = dW1 | db1 | dWh | dbh | dW2 | db2, scaled by 2w/N of the whole grid, so the
+        slabs' tensors add up."""
+        import torch
+        out = out if out is not None else self._empty(self.deep_grad_len() + 2, torch.float64)
+        cs, _ = self._slab(g, slab)
+        cg, cw = g.c(), pw.c()
+        check(self._lib.physad_deep_tangent_loss_grad_dev(self._h, C.byref(cg), C.byref(cs), C.byref(cw), C.c_float(t),
+                                                          ptr(out), ptr(out[2:]), self._stream()), "deep_tangent_loss_grad")
+        return out
+
+    def deep_tangent_loss_grad(self, g: Grid, pw: PhysWeights, t: float, group=None):
+        """(L_sigma, L_u, grad float64 ndarray[P]) of the analytic loss of the deep network.  With torch.distributed
+        initialised each rank differentiates its z-slab and ONE all-reduce of P+2 doubles combines them."""
+        import torch.distributed as dist
+        world, rank = (dist.get_world_size(group), dist.get_rank(group)) if dist.is_initialized() else (1, 0)
+        buf = self.deep_tangent_loss_grad_acc(g, pw, t, slab_for_rank(g.nz, rank, world))
+        if world > 1:
+            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+        h = buf.cpu().numpy()
+        ls, lu = self.finalize(h[:2], pw, g.N)
+        return ls, lu, h[2:].copy()
+
+    def deep_tangent_loss_grad_host(self, g: Grid, pw: PhysWeights, t: float):
+        """Host-buffer form with the context's deep weights: (L_sigma, L_u, dW1, db1, dWh, dbh, dW2, db2) of the analytic
+        loss, float32."""
+        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
+        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        ls, lu = C.c_float(), C.c_float()
+        cg, cw = g.c(), pw.c()
+        check(self._lib.physad_deep_tangent_loss_grad_host(self._h, C.byref(cg), C.byref(cw), C.c_float(t), C.byref(ls),
+                                                           C.byref(lu), *[ptr(x) if x.size else None for x in d]),
+              "deep_tangent_loss_grad_host")
+        return (np.float32(ls.value), np.float32(lu.value), *d)
+
     def set_deep_mode(self, mode: int) -> None:
         """0: strict fp32 (bit-exact, default); 1: hidden layers on the tensor cores with three-term bf16 operands (~1e-6)."""
         check(self._lib.physad_set_deep_mode(self._h, C.c_int(mode)), "set_deep_mode")
@@ -761,3 +811,11 @@ def mlp_phys_loss_deep_grad_cuda(g: Grid, cfg: MLPConfig, L: int, w, pw: PhysWei
 def mlp_phys_loss_tangent_grad_cuda(g: Grid, cfg: MLPConfig, w, pw: PhysWeights, t: float):
     """Closed loop of the analytic loss (additive): (L_sigma, L_u, dW1, db1, dW2, db2)."""
     return default_context().tangent_loss_grad_host(g, cfg, *w, pw, t)
+
+
+def mlp_phys_loss_deep_tangent_grad_cuda(g: Grid, cfg: MLPConfig, L: int, w, pw: PhysWeights, t: float):
+    """Closed loop of the analytic loss of a deep network (additive): w = (W1, b1, Wh, bh, W2, b2) ->
+    (L_sigma, L_u, dW1, db1, dWh, dbh, dW2, db2)."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.deep_tangent_loss_grad_host(g, pw, t)

@@ -4,7 +4,10 @@ step (fields, residuals + sums, stencil adjoint, MLP backward [+ the all-reduce 
 from the same process, the analytic forward alone, the finite-difference step, the counted flops and the GPU it ran on.
 --loss deep times the closed loop of a deep network (physad_deep_loss_grad_dev) for every --hidden x --layers pair, in
 alternation with the strict deep fields alone (generate_fields_deep) and the one-hidden-layer step; one JSON line per pair.
-  python tools/bench_grad.py [--loss fd|tangent|deep] [--n 256] [--hidden 64] [--layers 3] [--steps 20]
+--loss deep-tangent times the analytic loss of a deep network (physad_deep_tangent_loss_dev) and its closed loop
+(physad_deep_tangent_loss_grad_dev) for every --hidden x --layers pair, in alternation with the strict deep fields pass and
+the finite-difference deep step (physad_deep_loss_grad_dev); one JSON line per pair.
+  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent] [--n 256] [--hidden 64] [--layers 3] [--steps 20]
   python tools/bench_grad.py --loss deep --hidden 32,64,128 --layers 2,3,5
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/bench_grad.py   (z-slab per rank)"""
 import argparse
@@ -25,10 +28,12 @@ def main():
     ap.add_argument("--hidden", default="64", help="width; --loss deep takes a comma-separated list")
     ap.add_argument("--layers", default="3", help="--loss deep: hidden layers, a comma-separated list")
     ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--loss", choices=("fd", "tangent", "deep"), default="fd")
+    ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent"), default="fd")
     a = ap.parse_args()
     if a.loss == "deep":
         return deep(a, Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True))
+    if a.loss == "deep-tangent":
+        return deep_tangent(a, Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True))
     a.hidden = int(a.hidden)
     g = Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True)
     if "RANK" in os.environ and int(os.environ.get("WORLD_SIZE", "1")) > 1:
@@ -169,6 +174,71 @@ def deep(a, g):
                               "fd_one_layer_loss_grad_ms": fd[len(fd) // 2], "flops_per_point": fl,
                               "counted_tflops": fl * g.N / (med * 1e-3) / 1e12, "gpu": name, "power_limit_w": plim,
                               "grad_absmax": float(abs(h[2:]).max()), "acc": h[:2].tolist()}), flush=True)
+
+
+# counted work of the analytic deep loss per point (5 rows: value + 4 tangents), 2 flops per multiply-add: layer 1 value
+# row 8H; every hidden layer 5 rows x 2H^2; output layer 8H (y) + 32H (J).  The closed loop adds, per point: dW2 and
+# W2^T seed over 5 rows (80H), dW and W^T delta of every hidden layer over 5 rows (20(L-1)H^2), dW1 over 5 rows (40H).
+# The strict fields pass does 3 rows per point of 2(L-1)H^2 + 16H.
+def deep_tangent_flops_per_point(H, L, grad):
+    fwd = 10 * (L - 1) * H * H + 48 * H
+    return fwd + (20 * (L - 1) * H * H + 120 * H if grad else 0)
+
+
+def deep_fields_flops_per_point(H, L):
+    return 3 * (2 * (L - 1) * H * H + 16 * H)
+
+
+def deep_tangent(a, g):
+    import numpy as np
+    ctx = ops.Context()
+    pw = PhysWeights(1, 1)
+    name, plim = _gpu()
+    cg = g.c()
+    for H in (int(x) for x in a.hidden.split(",")):
+        w1 = ops.mlp_random_init(H, 777, 0.25)
+        for L in (int(x) for x in a.layers.split(",")):
+            rng = np.random.default_rng(L)
+            Wh = rng.uniform(-0.2, 0.2, (L - 1) * H * H).astype(np.float32)
+            bh = rng.uniform(-0.2, 0.2, (L - 1) * H).astype(np.float32)
+            ctx.set_weights_deep(MLPConfig(4, H, 4, True), L, w1[0], w1[1], Wh, bh, w1[2], w1[3])
+            acc = ctx.deep_tangent_loss_acc(g, 0.25)
+            out = ctx.deep_tangent_loss_grad_acc(g, pw, 0.25)
+            fdo = ctx.deep_loss_grad_acc(g, pw, 0.25, 2e-3)
+            f = ctx.mlp_generate_fields_deep(g, 0.25, 2e-3)
+            gen = lambda: ctx._lib.physad_mlp_generate_fields_deep_dev(ctx._h, C.byref(cg), None, C.c_float(0.25), C.c_float(2e-3),
+                                                                       *[ops.ptr(x) for x in f], ctx._stream())
+            loss = lambda: ctx.deep_tangent_loss_acc(g, 0.25, acc=acc)
+            step = lambda: ctx.deep_tangent_loss_grad_acc(g, pw, 0.25, out=out)
+            fdstep = lambda: ctx.deep_loss_grad_acc(g, pw, 0.25, 2e-3, out=fdo)
+            for _ in range(2):
+                loss(); step(); fdstep()
+                assert gen() == 0
+            torch.cuda.synchronize()
+            # the four are timed in alternation, so that they share whatever else the GPU is doing
+            tl, tg, fw, fd = [], [], [], []
+            for _ in range(a.steps):
+                tl += _times(loss, 1)
+                tg += _times(step, 1)
+                fw += _times(gen, 1)
+                fd += _times(fdstep, 1)
+            for x in (tl, tg, fw, fd):
+                x.sort()
+            ml, mg, mf, md = (x[len(x) // 2] for x in (tl, tg, fw, fd))
+            fl, fg = deep_tangent_flops_per_point(H, L, False), deep_tangent_flops_per_point(H, L, True)
+            ff, fdf = deep_fields_flops_per_point(H, L), deep_flops_per_point(H, L)
+            h = out.cpu().numpy()
+            print(json.dumps({"workload": f"{a.n}^3 H={H} L={L} deep analytic loss / loss+grad",
+                              "loss_ms": ml, "loss_grad_ms": mg, "fields_deep_ms": mf, "fd_deep_loss_grad_ms": md,
+                              "loss_ratio_to_fields": ml / mf, "loss_gpts_per_s": g.N / ml / 1e6, "loss_grad_gpts_per_s": g.N / mg / 1e6,
+                              "loss_flops_per_point": fl, "loss_grad_flops_per_point": fg,
+                              "loss_counted_tflops": fl * g.N / (ml * 1e-3) / 1e12,
+                              "loss_grad_counted_tflops": fg * g.N / (mg * 1e-3) / 1e12,
+                              "fields_counted_tflops": ff * g.N / (mf * 1e-3) / 1e12,
+                              "fd_deep_loss_grad_counted_tflops": fdf * g.N / (md * 1e-3) / 1e12,
+                              "gpu": name, "power_limit_w": plim,
+                              "grad_absmax": float(abs(h[2:]).max()), "acc": h[:2].tolist(),
+                              "acc_loss_call_equal": bool((acc.cpu().numpy() == h[:2]).all())}), flush=True)
 
 
 def distributed(a, g):
