@@ -128,6 +128,11 @@ int physad_mlp_generate_fields_host(physad_ctx* ctx, const physad_grid* g, float
  * ReLU).  There is no reference implementation for hidden_layers > 1 (parity is against oracle/oracle.c's
  * restatement only); hidden_layers == 1 is bit-identical to the one-hidden-layer entry points.
  * Wh: (hidden_layers-1) matrices [H x H] row-major [g][h]; bh: (hidden_layers-1) x H.  HOST pointers.
+ * While the context holds a network of hidden_layers > 1, every entry point that evaluates the one-hidden-layer network
+ * (physad_mlp_forward_*, physad_mlp_backward_*, physad_mlp_grid_infer_*, physad_mlp_generate_fields_*, physad_fused_loss_*,
+ * physad_tangent_loss_*, physad_fused_loss_grad_*, physad_tangent_loss_grad_*) returns PHYSAD_E_UNSUPPORTED and writes
+ * nothing; the host forms that take new weights (cfg != NULL) replace the network first and run.  Use the *_deep_* and
+ * deep_* counterparts.  hidden_layers == 1 is accepted everywhere.  A refused call leaves the previous network in place.
  * A later physad_set_weights() switches the context back to a one-hidden-layer network. */
 int physad_set_weights_deep(physad_ctx* ctx, const physad_mlp_config* cfg, int hidden_layers, const float* W1,
                             const float* b1, const float* Wh, const float* bh, const float* W2, const float* b2);
@@ -334,7 +339,7 @@ int physad_fused_loss_grad_host(physad_ctx* ctx, const physad_grid* g, const phy
  * grad: 9H+4 device doubles  dW1[H*4] | db1[H] | dW2[4*H] | db2[4]  (the reference's layouts), the slab's share already
  * scaled by 2w/N of the whole grid -- so an all-reduce(sum) of the 9H+6 doubles over the ranks' slabs gives the
  * whole-grid result.  slab NULL = whole grid; an empty slab gives zeros.  Requires In = Out = 4, H <= 128 and a
- * one-hidden-layer network (physad_set_weights_deep with L > 1: PHYSAD_E_UNSUPPORTED).  Bitwise repeatable. */
+ * one-hidden-layer network (see physad_set_weights_deep).  Bitwise repeatable. */
 int physad_tangent_loss_grad_dev(physad_ctx* ctx, const physad_grid* g, const physad_slab* slab, const physad_phys_weights* w,
                                  float t, double* acc, double* grad, void* stream);
 /* Host-buffer form on the whole grid: (optionally) new weights in, the two losses and the gradient out (any output

@@ -189,8 +189,20 @@ void fill_const(const physad_ctx* c, const float tcoord[3], MlpConst<H>& k) {
 // 4th MLP input for a time value (reference src/mlp_grid.cpp:38)
 float time_coord(float t, int norm) { return norm == 1 ? t : (t + 0.5f); }
 
-int need_4x4(const physad_ctx* c, const char* what) {
+// The one-hidden-layer entry points read only the first and the last layer of the context's weights.  After
+// physad_set_weights_deep with L > 1 that pair is not the network the caller set, so they refuse it instead of
+// evaluating 4 -> H -> 4 with the hidden -> hidden layers dropped.
+int need_one_layer(const physad_ctx* c, const char* what, const char* deep_twin) {
+    if (c->deep_layers <= 1) return 0;
+    std::string msg = std::string(what) + ": one-hidden-layer entry point, but the context holds a network of " +
+                      std::to_string(c->deep_layers) + " hidden layers (physad_set_weights_deep)";
+    if (deep_twin) msg += std::string("; use ") + deep_twin;
+    return fail(PHYSAD_E_UNSUPPORTED, msg);
+}
+
+int need_4x4(const physad_ctx* c, const char* what, const char* deep_twin) {
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, std::string(what) + ": no weights set");
+    if (int rc = need_one_layer(c, what, deep_twin)) return rc;
     if (c->cfg.In != 4 || c->cfg.Out != 4)
         return fail(PHYSAD_E_UNSUPPORTED, std::string(what) + ": grid paths need In = Out = 4 (src/mlp_grid.cpp:69-80)");
     if (template_h(c->cfg.H) == 0) return fail(PHYSAD_E_UNSUPPORTED, std::string(what) + ": H > 128 not built");
@@ -779,6 +791,7 @@ GemmArgs gemm_out(const physad_ctx* c, const float* act, float* out, size_t B, c
 int physad_mlp_forward_dev(physad_ctx* c, const float* x, float* y, size_t B, void* stream) {
     if (!c || (B && (!x || !y))) return fail(PHYSAD_E_INVALID, "mlp_forward: null argument");
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, "mlp_forward: no weights set");
+    if (int rc = need_one_layer(c, "mlp_forward", nullptr)) return rc;
     if (B == 0) return 0;
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
@@ -807,6 +820,7 @@ int physad_mlp_forward_dev(physad_ctx* c, const float* x, float* y, size_t B, vo
 int physad_mlp_forward_host(physad_ctx* c, const float* x, float* y, size_t B) {
     if (!c || (B && (!x || !y))) return fail(PHYSAD_E_INVALID, "mlp_forward: null argument");
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, "mlp_forward: no weights set");
+    if (int rc = need_one_layer(c, "mlp_forward", nullptr)) return rc;
     if (B == 0) return 0;
     DeviceGuard dg(c->device);
     const size_t nx = B * size_t(c->cfg.In) * sizeof(float), ny = B * size_t(c->cfg.Out) * sizeof(float);
@@ -825,7 +839,9 @@ int physad_mlp_backward_dev(physad_ctx* c, const float* x, const float* y_target
                             float* db2, size_t B, void* stream) {
     if (!c || !x || !y_target || !dW1 || !db1 || !dW2 || !db2) return fail(PHYSAD_E_INVALID, "mlp_backward: null argument");
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, "mlp_backward: no weights set");
+    if (int rc = need_one_layer(c, "mlp_backward", nullptr)) return rc;
     if (B == 0) return fail(PHYSAD_E_INVALID, "mlp_backward: empty batch (the reference divides by B*Out)");
+    if (B > size_t(65535) * 64) return fail(PHYSAD_E_UNSUPPORTED, "mlp_backward: more than 4 194 240 rows per call");
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
     if (int rc = upload_weights_if_stale(c, st)) return rc;
@@ -834,7 +850,6 @@ int physad_mlp_backward_dev(physad_ctx* c, const float* x, const float* y_target
     CU(cudaMallocAsync(&act, B * size_t(H) * sizeof(float), st));
     CU(cudaMallocAsync(&gz1, B * size_t(H) * sizeof(float), st));
     CU(cudaMallocAsync(&gz2, B * size_t(Out) * sizeof(float), st));
-    if (B > size_t(65535) * 64) return fail(PHYSAD_E_UNSUPPORTED, "mlp_backward: more than 4 194 240 rows per call");
     const float scale = 2.f / float(B * size_t(Out));  // src/mlp_cpu.cpp:58
     // five strict contractions (dense_kernels.cuh); every gradient entry is the reference's sequential fp32 sum over the
     // batch, i ascending -- which is also why the batch cannot be split over blocks: partial sums would round differently
@@ -864,6 +879,7 @@ int physad_mlp_backward_host(physad_ctx* c, const float* x, const float* y_targe
                              float* db2, size_t B) {
     if (!c || !x || !y_target || !dW1 || !db1 || !dW2 || !db2) return fail(PHYSAD_E_INVALID, "mlp_backward: null argument");
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, "mlp_backward: no weights set");
+    if (int rc = need_one_layer(c, "mlp_backward", nullptr)) return rc;
     DeviceGuard dg(c->device);
     const size_t In = c->cfg.In, H = c->cfg.H, Out = c->cfg.Out;
     const size_t n[6] = {B * In, B * Out, H * In, H, Out * H, Out};
@@ -886,7 +902,7 @@ int physad_mlp_grid_infer_dev(physad_ctx* c, const physad_grid* g, const physad_
                               void* stream) {
     if (!c || !out) return fail(PHYSAD_E_INVALID, "mlp_grid_infer: null argument");
     if (int rc = check_grid(g)) return rc;
-    if (int rc = need_4x4(c, "mlp_grid_infer")) return rc;
+    if (int rc = need_4x4(c, "mlp_grid_infer", "physad_mlp_grid_infer_deep_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
     if (uintptr_t(out) % 16) return fail(PHYSAD_E_INVALID, "mlp_grid_infer: out must be 16-byte aligned");
@@ -914,7 +930,7 @@ int physad_mlp_generate_fields_dev(physad_ctx* c, const physad_grid* g, const ph
                                    float* s_m, float* s_0, float* s_p, float* u_m, float* u_0, float* u_p, void* stream) {
     if (!c || !s_m || !s_0 || !s_p || !u_m || !u_0 || !u_p) return fail(PHYSAD_E_INVALID, "generate_fields: null argument");
     if (int rc = check_grid(g)) return rc;
-    if (int rc = need_4x4(c, "generate_fields")) return rc;
+    if (int rc = need_4x4(c, "generate_fields", "physad_mlp_generate_fields_deep_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
     DeviceGuard dg(c->device);
@@ -1120,7 +1136,7 @@ int physad_mlp_generate_fields_lp_dev(physad_ctx* c, const physad_grid* g, const
     if (!c || !s_m || !s_0 || !s_p || !u_m || !u_0 || !u_p) return fail(PHYSAD_E_INVALID, "generate_fields_lp: null argument");
     if (dtype != PHYSAD_F16 && dtype != PHYSAD_BF16) return fail(PHYSAD_E_INVALID, "generate_fields_lp: dtype must be PHYSAD_F16 or PHYSAD_BF16");
     if (int rc = check_grid(g)) return rc;
-    if (int rc = need_4x4(c, "generate_fields_lp")) return rc;
+    if (int rc = need_4x4(c, "generate_fields_lp", nullptr)) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
     DeviceGuard dg(c->device);
@@ -1327,7 +1343,7 @@ int physad_fused_loss_dev(physad_ctx* c, const physad_grid* g, const physad_slab
                           float* Rs, float* Rx, float* Ry, float* Rz, void* stream) {
     if (!c || !acc) return fail(PHYSAD_E_INVALID, "fused_loss: null argument");
     if (int rc = check_grid(g)) return rc;
-    if (int rc = need_4x4(c, "fused_loss")) return rc;
+    if (int rc = need_4x4(c, "fused_loss", "physad_deep_loss_host or physad_deep_loss_grad_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
     const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
@@ -1341,7 +1357,7 @@ int physad_fused_loss_allreduce_dev(physad_ctx* c, const physad_grid* g, const p
                                     double* acc, float* Rs, float* Rx, float* Ry, float* Rz, void* stream) {
     if (!c || !acc) return fail(PHYSAD_E_INVALID, "fused_loss_allreduce: null argument");
     if (int rc = check_grid(g)) return rc;
-    if (int rc = need_4x4(c, "fused_loss_allreduce")) return rc;
+    if (int rc = need_4x4(c, "fused_loss_allreduce", "physad_deep_loss_grad_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
     const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
@@ -1387,7 +1403,7 @@ int physad_tangent_loss_dev(physad_ctx* c, const physad_grid* g, const physad_sl
                             float* Rx, float* Ry, float* Rz, void* stream) {
     if (!c || !acc) return fail(PHYSAD_E_INVALID, "tangent_loss: null argument");
     if (int rc = check_grid(g)) return rc;
-    if (int rc = need_4x4(c, "tangent_loss")) return rc;
+    if (int rc = need_4x4(c, "tangent_loss", "physad_deep_tangent_loss_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
     const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
@@ -1474,7 +1490,7 @@ int physad_fused_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad
                                double* acc, double* grad, void* stream) {
     if (!c || !w || !acc || !grad) return fail(PHYSAD_E_INVALID, "fused_loss_grad: null argument");
     if (int rc = check_grid(g)) return rc;
-    if (int rc = need_4x4(c, "fused_loss_grad")) return rc;
+    if (int rc = need_4x4(c, "fused_loss_grad", "physad_deep_loss_grad_dev")) return rc;
     if (c->advection != 0) return fail(PHYSAD_E_UNSUPPORTED, "fused_loss_grad: the stencil adjoint is that of the central scheme");
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
@@ -1501,7 +1517,7 @@ int physad_fused_loss_grad_slab_dev(physad_ctx* c, const physad_grid* g, const p
                                     const physad_phys_weights* w, float t, float dt, double* acc, double* grad, void* stream) {
     if (!c || !w || !acc || !grad || !slab) return fail(PHYSAD_E_INVALID, "fused_loss_grad_slab: null argument");
     if (int rc = check_grid(g)) return rc;
-    if (int rc = need_4x4(c, "fused_loss_grad_slab")) return rc;
+    if (int rc = need_4x4(c, "fused_loss_grad_slab", "physad_deep_loss_grad_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
     if (s.z_begin == 0 && s.z_end == g->nz) return physad_fused_loss_grad_dev(c, g, w, t, dt, acc, grad, stream);
@@ -1565,7 +1581,7 @@ int physad_fused_loss_grad_host(physad_ctx* c, const physad_grid* g, const physa
     if (cfg) {
         if (int rc = physad_set_weights(c, cfg, W1, b1, W2, b2)) return rc;
     }
-    if (int rc = need_4x4(c, "fused_loss_grad")) return rc;
+    if (int rc = need_4x4(c, "fused_loss_grad", "physad_deep_loss_grad_dev")) return rc;
     DeviceGuard dg(c->device);
     constexpr size_t cap = 9 * 128 + 4;
     if (!c->d_grad) CU(cudaMalloc(&c->d_grad, cap * sizeof(double)));
@@ -1620,9 +1636,7 @@ int physad_tangent_loss_grad_dev(physad_ctx* c, const physad_grid* g, const phys
                                  float t, double* acc, double* grad, void* stream) {
     if (!c || !w || !acc || !grad) return fail(PHYSAD_E_INVALID, "tangent_loss_grad: null argument");
     if (int rc = check_grid(g)) return rc;
-    if (int rc = need_4x4(c, "tangent_loss_grad")) return rc;
-    if (c->deep_layers > 1)
-        return fail(PHYSAD_E_UNSUPPORTED, "tangent_loss_grad: the gradient is of the one-hidden-layer network (set_weights_deep L > 1)");
+    if (int rc = need_4x4(c, "tangent_loss_grad", "physad_deep_tangent_loss_grad_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
     DeviceGuard dg(c->device);
@@ -1666,7 +1680,7 @@ int physad_tangent_loss_grad_host(physad_ctx* c, const physad_grid* g, const phy
     if (cfg) {
         if (int rc = physad_set_weights(c, cfg, W1, b1, W2, b2)) return rc;
     }
-    if (int rc = need_4x4(c, "tangent_loss_grad")) return rc;
+    if (int rc = need_4x4(c, "tangent_loss_grad", "physad_deep_tangent_loss_grad_dev")) return rc;
     DeviceGuard dg(c->device);
     constexpr size_t cap = 9 * 128 + 4;
     if (!c->d_grad) CU(cudaMalloc(&c->d_grad, cap * sizeof(double)));
