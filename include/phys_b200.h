@@ -69,6 +69,18 @@ void mlp_phys_loss_deep_tangent_grad_cuda(const GridSpec& g, const MLPGridConfig
                                           const PhysWeights& pw, float t, float* out_loss_sigma, float* out_loss_u,
                                           DeepMLPWeights& grad);
 
+// A deep network at arbitrary points: coords holds N inputs (x, y, z, t), already normalised like mlp_infer_cuda's; out is
+// resized to N*4, AoS per point.  Strict fp32 in the arithmetic of the grid kernels (bit-identical to them at grid
+// coordinates and to mlp_infer_cuda for hidden_layers = 1).  Every vector of `w` is checked against cfg and hidden_layers.
+void mlp_infer_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const std::vector<float>& coords, std::vector<float>& out);
+
+// Data-fit loss of a deep network and its gradient with respect to every layer's weights: x and target hold B points of 4
+// floats, lam 4 non-negative output weights or nullptr for 1/4 each (the mean((y - target)^2) of mlp_backward);
+// *out_loss = (1/B) sum_i sum_o lam[o] (y_io - target_io)^2.  `grad` is resized to the shapes of `w` and adds directly to
+// the physics gradient of mlp_phys_loss_deep_grad_cuda / mlp_phys_loss_deep_tangent_grad_cuda.  B = 0 gives zeros.
+void mlp_data_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* target,
+                                  std::size_t B, const float* lam, float* out_loss, DeepMLPWeights& grad);
+
 }  // namespace phys
 
 #endif  // PHYS_AUTODIFF_PHYS_B200_H

@@ -132,7 +132,9 @@ int physad_mlp_generate_fields_host(physad_ctx* ctx, const physad_grid* g, float
  * (physad_mlp_forward_*, physad_mlp_backward_*, physad_mlp_grid_infer_*, physad_mlp_generate_fields_*, physad_fused_loss_*,
  * physad_tangent_loss_*, physad_fused_loss_grad_*, physad_tangent_loss_grad_*) returns PHYSAD_E_UNSUPPORTED and writes
  * nothing; the host forms that take new weights (cfg != NULL) replace the network first and run.  Use the *_deep_* and
- * deep_* counterparts.  hidden_layers == 1 is accepted everywhere.  A refused call leaves the previous network in place.
+ * deep_* counterparts: physad_mlp_forward_deep_* for physad_mlp_forward_*, physad_deep_data_loss_grad_* for
+ * physad_mlp_backward_*, physad_mlp_grid_infer_deep_dev, physad_mlp_generate_fields_deep_dev, physad_deep_loss_host,
+ * physad_deep_loss_grad_* and physad_deep_tangent_loss_*.  hidden_layers == 1 is accepted everywhere.  A refused call leaves the previous network in place.
  * A later physad_set_weights() switches the context back to a one-hidden-layer network. */
 int physad_set_weights_deep(physad_ctx* ctx, const physad_mlp_config* cfg, int hidden_layers, const float* W1,
                             const float* b1, const float* Wh, const float* bh, const float* W2, const float* b2);
@@ -402,6 +404,35 @@ int physad_deep_tangent_loss_grad_dev(physad_ctx* ctx, const physad_grid* g, con
 int physad_deep_tangent_loss_grad_host(physad_ctx* ctx, const physad_grid* g, const physad_phys_weights* w, float t,
                                        float* loss_sigma, float* loss_u, float* dW1, float* db1, float* dWh, float* dbh,
                                        float* dW2, float* db2);
+
+/* ---- deeper networks at arbitrary points (ADDITIVE, no reference counterpart) ----------------------------------------
+ * The network set by physad_set_weights_deep (any hidden_layers >= 1) evaluated at caller-supplied inputs, and a data-fit
+ * loss with its gradient with respect to every layer: the term that anchors a physics-informed fit to initial conditions,
+ * boundary values or observations (the physics residual alone is zero for every constant field).  Strict fp32 on the CUDA
+ * cores (deep mode 0).
+ * physad_mlp_forward_deep_*: y[B][4] = MLP(x[B][4]), x = the network's inputs (x, y, z, t) already normalised, like
+ *   physad_mlp_forward's x.  The arithmetic of physad_mlp_grid_infer_deep (layer 1 from b1, + W1[h,k] x_k for k ascending,
+ *   each product rounded; hidden and output layers from the bias, h ascending), so the outputs equal the CPU restatement
+ *   oracle_mlp_forward_deep bit for bit, equal physad_mlp_grid_infer_deep's at the grid's own coordinates, and at
+ *   hidden_layers == 1 equal physad_mlp_forward_*'s.  _dev: x and y DEVICE pointers, 16-byte aligned; no limit on B.
+ * physad_deep_data_loss_grad_dev: L_d = (1/n_norm) sum_i sum_o lam[o] (y_io - target_io)^2 with y = MLP(x).
+ *   lam: 4 HOST floats (finite, >= 0), or NULL for 1/4 each -- the mean((y - target)^2) of physad_mlp_backward.
+ *   acc: 1 device double, the un-normalised weighted sum sum_i sum_o lam[o] (y_io - target_io)^2.
+ *   grad: P = physad_deep_grad_len(H, L) device doubles in the layout of physad_deep_loss_grad_dev
+ *   (dW1 | db1 | dWh | dbh | dW2 | db2), already scaled by 2 lam[o] / n_norm: with n_norm = the points of ALL shards, the
+ *   shards' acc and grad add up (all-reduce(sum)), and grad adds directly to the physics gradient.  x, target: [B][4] device,
+ *   16-byte aligned.  B = 0 (an empty shard) writes acc = 0 and a zero gradient.  Bitwise repeatable.
+ * physad_deep_data_loss_grad_host: host arrays, n_norm = B; loss = L_d as float, the gradient split into the six arrays
+ *   of physad_set_weights_deep's layouts (any output pointer may be null); B = 0 gives zeros.
+ * Errors: no deep weights (or a physad_set_weights after them): PHYSAD_E_NOWEIGHTS; physad_set_deep_mode(1):
+ * PHYSAD_E_UNSUPPORTED; n_norm == 0, a negative or non-finite lam, a null or misaligned pointer with B > 0 (acc and grad
+ * always): PHYSAD_E_INVALID.  A refused call writes nothing. */
+int physad_mlp_forward_deep_dev(physad_ctx* ctx, const float* x, float* y, size_t B, void* stream);
+int physad_mlp_forward_deep_host(physad_ctx* ctx, const float* x, float* y, size_t B);
+int physad_deep_data_loss_grad_dev(physad_ctx* ctx, const float* x, const float* target, size_t B, const float* lam,
+                                   size_t n_norm, double* acc, double* grad, void* stream);
+int physad_deep_data_loss_grad_host(physad_ctx* ctx, const float* x, const float* target, size_t B, const float* lam,
+                                    float* loss, float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2);
 
 /* Host-only: the work partition the fused kernel is launched with.  The sequence of tiles x planes
  * tile-planes (tile-major) is cut into at most `slots` contiguous ranges of equal cost, a range paying

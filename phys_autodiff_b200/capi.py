@@ -97,6 +97,8 @@ EXPORTS = [
     "physad_tangent_loss_grad_dev", "physad_tangent_loss_grad_host",
     "physad_deep_grad_len", "physad_deep_loss_grad_dev", "physad_deep_loss_grad_host",
     "physad_deep_tangent_loss_dev", "physad_deep_tangent_loss_grad_dev", "physad_deep_tangent_loss_grad_host",
+    "physad_mlp_forward_deep_dev", "physad_mlp_forward_deep_host", "physad_deep_data_loss_grad_dev",
+    "physad_deep_data_loss_grad_host",
 ]
 
 

@@ -2,6 +2,7 @@
 // the host-pointer staging wrappers.  All arithmetic lives in the kernels (*.cuh); this file only
 // decides shapes, fills the kernel-parameter weight block and moves bytes.
 #include "../../include/physad_b200.h"
+#include "deep_data_kernels.cuh"
 #include "deep_grad_kernels.cuh"
 #include "deep_kernels.cuh"
 #include "deep_tangent_kernels.cuh"
@@ -13,6 +14,7 @@
 #include "tangent_kernels.cuh"
 
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -791,7 +793,7 @@ GemmArgs gemm_out(const physad_ctx* c, const float* act, float* out, size_t B, c
 int physad_mlp_forward_dev(physad_ctx* c, const float* x, float* y, size_t B, void* stream) {
     if (!c || (B && (!x || !y))) return fail(PHYSAD_E_INVALID, "mlp_forward: null argument");
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, "mlp_forward: no weights set");
-    if (int rc = need_one_layer(c, "mlp_forward", nullptr)) return rc;
+    if (int rc = need_one_layer(c, "mlp_forward", "physad_mlp_forward_deep_dev")) return rc;
     if (B == 0) return 0;
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
@@ -820,7 +822,7 @@ int physad_mlp_forward_dev(physad_ctx* c, const float* x, float* y, size_t B, vo
 int physad_mlp_forward_host(physad_ctx* c, const float* x, float* y, size_t B) {
     if (!c || (B && (!x || !y))) return fail(PHYSAD_E_INVALID, "mlp_forward: null argument");
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, "mlp_forward: no weights set");
-    if (int rc = need_one_layer(c, "mlp_forward", nullptr)) return rc;
+    if (int rc = need_one_layer(c, "mlp_forward", "physad_mlp_forward_deep_dev")) return rc;
     if (B == 0) return 0;
     DeviceGuard dg(c->device);
     const size_t nx = B * size_t(c->cfg.In) * sizeof(float), ny = B * size_t(c->cfg.Out) * sizeof(float);
@@ -839,7 +841,7 @@ int physad_mlp_backward_dev(physad_ctx* c, const float* x, const float* y_target
                             float* db2, size_t B, void* stream) {
     if (!c || !x || !y_target || !dW1 || !db1 || !dW2 || !db2) return fail(PHYSAD_E_INVALID, "mlp_backward: null argument");
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, "mlp_backward: no weights set");
-    if (int rc = need_one_layer(c, "mlp_backward", nullptr)) return rc;
+    if (int rc = need_one_layer(c, "mlp_backward", "physad_deep_data_loss_grad_dev")) return rc;
     if (B == 0) return fail(PHYSAD_E_INVALID, "mlp_backward: empty batch (the reference divides by B*Out)");
     if (B > size_t(65535) * 64) return fail(PHYSAD_E_UNSUPPORTED, "mlp_backward: more than 4 194 240 rows per call");
     DeviceGuard dg(c->device);
@@ -879,7 +881,7 @@ int physad_mlp_backward_host(physad_ctx* c, const float* x, const float* y_targe
                              float* db2, size_t B) {
     if (!c || !x || !y_target || !dW1 || !db1 || !dW2 || !db2) return fail(PHYSAD_E_INVALID, "mlp_backward: null argument");
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, "mlp_backward: no weights set");
-    if (int rc = need_one_layer(c, "mlp_backward", nullptr)) return rc;
+    if (int rc = need_one_layer(c, "mlp_backward", "physad_deep_data_loss_grad_dev")) return rc;
     DeviceGuard dg(c->device);
     const size_t In = c->cfg.In, H = c->cfg.H, Out = c->cfg.Out;
     const size_t n[6] = {B * In, B * Out, H * In, H, Out * H, Out};
@@ -1962,6 +1964,176 @@ int physad_deep_tangent_loss_grad_host(physad_ctx* c, const physad_grid* g, cons
     CU(cudaStreamSynchronize(c->stream));
     physad_finalize_loss(c->h_dgrad, w, size_t(g->nx) * g->ny * g->nz, loss_sigma, loss_u);
     const double* gd = c->h_dgrad + 2;
+    const size_t nl = size_t(L - 1), hh = size_t(H);
+    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
+    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
+    for (int k = 0; k < 6; ++k) {
+        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
+        gd += len[k];
+    }
+    return 0;
+}
+
+// ---- deeper networks at caller-supplied points: forward and data-fit loss + gradient (deep_data_kernels.cuh) --------
+}  // extern "C"  (helpers below)
+namespace {
+template <int H>
+int launch_deep_points(physad_ctx* c, const DeepArgs& a, cudaStream_t st) {
+    MlpConst<H> k;
+    const float no_t[3] = {0.f, 0.f, 0.f};   // points mode forms W1[h,3] * t per row; the pre-rounded products are unused
+    fill_const<H>(c, no_t, k);
+    CU(cudaError_t(deep_points_launch(H, &k, a, c->sm_count, st)));
+    c->launches++;
+    return 0;
+}
+
+template <int H>
+int launch_deep_data(physad_ctx* c, const DeepDataArgs& a, int blocks, double* grad, double* acc, cudaStream_t st) {
+    MlpConst<H> k;
+    const float no_t[3] = {0.f, 0.f, 0.f};   // only the output pairs w2 / b2 are read
+    fill_const<H>(c, no_t, k);
+    CU(cudaError_t(deep_data_launch(H, &k, a, blocks, grad, acc, st)));
+    c->launches += 2;
+    return 0;
+}
+
+// checks shared by the forward and the data loss at points: deep weights, strict mode
+int deep_points_ready(const physad_ctx* c, const char* what) {
+    if (int rc = deep_ready(c, what)) return rc;
+    if (c->deep_mode != 0)
+        return fail(PHYSAD_E_UNSUPPORTED, std::string(what) + ": strict fp32 only (set_deep_mode(0))");
+    return 0;
+}
+
+bool misaligned16(const void* p) { return uintptr_t(p) % 16 != 0; }
+}  // namespace
+extern "C" {
+
+int physad_mlp_forward_deep_dev(physad_ctx* c, const float* x, float* y, size_t B, void* stream) {
+    if (!c) return fail(PHYSAD_E_INVALID, "mlp_forward_deep: null context");
+    if (int rc = deep_points_ready(c, "mlp_forward_deep")) return rc;
+    if (B && (!x || !y)) return fail(PHYSAD_E_INVALID, "mlp_forward_deep: null argument");
+    if (B && (misaligned16(x) || misaligned16(y))) return fail(PHYSAD_E_INVALID, "mlp_forward_deep: x and y must be 16-byte aligned");
+    if (B == 0) return 0;
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    if (int rc = upload_weights_if_stale(c, st)) return rc;
+    DeepArgs a{};
+    a.hidden_layers = c->deep_layers;
+    a.W1 = c->dW1; a.b1 = c->db1; a.wh = c->d_wh; a.bh = c->d_bh;
+    a.pts = reinterpret_cast<const float4*>(x);
+    a.n_points = (long long)B;
+    a.out_aos = reinterpret_cast<float4*>(y);
+    switch (c->cfg.H) {
+        case 32: return launch_deep_points<32>(c, a, st);
+        case 64: return launch_deep_points<64>(c, a, st);
+        default: return launch_deep_points<128>(c, a, st);
+    }
+}
+
+int physad_mlp_forward_deep_host(physad_ctx* c, const float* x, float* y, size_t B) {
+    if (!c) return fail(PHYSAD_E_INVALID, "mlp_forward_deep: null context");
+    if (int rc = deep_points_ready(c, "mlp_forward_deep")) return rc;
+    if (B && (!x || !y)) return fail(PHYSAD_E_INVALID, "mlp_forward_deep: null argument");
+    if (B == 0) return 0;
+    DeviceGuard dg(c->device);
+    const size_t bytes = B * 4 * sizeof(float), off_y = (bytes + 255) & ~size_t(255);
+    if (int rc = ensure_scratch(c, off_y + bytes)) return rc;
+    float* dx = reinterpret_cast<float*>(c->scratch);
+    float* dy = reinterpret_cast<float*>(c->scratch + off_y);
+    CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
+    if (int rc = physad_mlp_forward_deep_dev(c, dx, dy, B, c->stream)) return rc;
+    CU(cudaMemcpyAsync(y, dy, bytes, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int physad_deep_data_loss_grad_dev(physad_ctx* c, const float* x, const float* target, size_t B, const float* lam,
+                                   size_t n_norm, double* acc, double* grad, void* stream) {
+    if (!c) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: null context");
+    if (int rc = deep_points_ready(c, "deep_data_loss_grad")) return rc;
+    if (!acc || !grad || (B && (!x || !target))) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: null argument");
+    if (B && (misaligned16(x) || misaligned16(target)))
+        return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: x and target must be 16-byte aligned");
+    if (uintptr_t(acc) % 8 || uintptr_t(grad) % 8) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: acc and grad must be 8-byte aligned");
+    if (n_norm == 0) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: n_norm must be positive");
+    float lw[4] = {0.25f, 0.25f, 0.25f, 0.25f};   // NULL: the mean over the four outputs
+    if (lam) {
+        for (int o = 0; o < 4; ++o) {
+            if (!std::isfinite(lam[o]) || lam[o] < 0.f)
+                return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: lam must be finite and non-negative");
+            lw[o] = lam[o];
+        }
+    }
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (B == 0) {   // an empty shard: zero sum, zero gradient
+        CU(cudaMemsetAsync(acc, 0, sizeof(double), st));
+        CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
+        return 0;
+    }
+    if (int rc = upload_weights_if_stale(c, st)) return rc;
+    const int blocks = deep_data_blocks(H, (long long)B, c->sm_count);
+    const size_t ck = size_t(blocks) * deep_data_ckpt_floats(H, L);
+    if (ck > c->dckpt_cap) {
+        if (c->dckpt) CU(cudaFree(c->dckpt));
+        c->dckpt = nullptr; c->dckpt_cap = 0;
+        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
+        c->dckpt_cap = ck;
+    }
+    if (int rc = ensure_grad_partials(c, size_t(blocks) * (P + 1))) return rc;
+    DeepDataArgs a{};
+    a.hidden_layers = L;
+    a.n = (long long)B;
+    a.x = reinterpret_cast<const float4*>(x);
+    a.target = reinterpret_cast<const float4*>(target);
+    a.W1 = c->dW1; a.b1 = c->db1; a.W2 = c->dW2;
+    a.wh = c->d_wh; a.bh = c->d_bh;
+    for (int o = 0; o < 4; ++o) {
+        a.coef[o] = float(2.0 * double(lw[o]) / double(n_norm));
+        a.lam[o] = double(lw[o]);
+    }
+    a.ckpt = c->dckpt;
+    a.partials = c->gpart;
+    switch (H) {
+        case 32: return launch_deep_data<32>(c, a, blocks, grad, acc, st);
+        case 64: return launch_deep_data<64>(c, a, blocks, grad, acc, st);
+        default: return launch_deep_data<128>(c, a, blocks, grad, acc, st);
+    }
+}
+
+int physad_deep_data_loss_grad_host(physad_ctx* c, const float* x, const float* target, size_t B, const float* lam,
+                                    float* loss, float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2) {
+    if (!c) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: null context");
+    if (int rc = deep_points_ready(c, "deep_data_loss_grad")) return rc;
+    if (B && (!x || !target)) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: null argument");
+    DeviceGuard dg(c->device);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (P + 2 > c->dgrad_cap) {
+        if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
+        if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
+        c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
+        CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
+        CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
+        c->dgrad_cap = P + 2;
+    }
+    const size_t bytes = B * 4 * sizeof(float), off_t = (bytes + 255) & ~size_t(255);
+    if (int rc = ensure_scratch(c, off_t + bytes + 1)) return rc;
+    float* dx = reinterpret_cast<float*>(c->scratch);
+    float* dtg = reinterpret_cast<float*>(c->scratch + off_t);
+    if (B) {
+        CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
+        CU(cudaMemcpyAsync(dtg, target, bytes, cudaMemcpyHostToDevice, c->stream));
+    }
+    // n_norm = B; an empty set (B = 0) gives a zero loss and a zero gradient
+    if (int rc = physad_deep_data_loss_grad_dev(c, dx, dtg, B, lam, B ? B : 1, c->d_dgrad, c->d_dgrad + 1, c->stream)) return rc;
+    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 1) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    if (loss) *loss = float(c->h_dgrad[0] / double(B ? B : 1));
+    const double* gd = c->h_dgrad + 1;
     const size_t nl = size_t(L - 1), hh = size_t(H);
     float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
     const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};

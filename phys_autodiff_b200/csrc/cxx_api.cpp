@@ -395,6 +395,64 @@ void mlp_phys_loss_deep_tangent_grad_cuda(const GridSpec& g, const MLPGridConfig
     if (rc) die("mlp_phys_loss_deep_tangent_grad_cuda", rc);
 }
 
+namespace {
+// Every vector of a DeepMLPWeights against cfg and hidden_layers, before any pointer reaches the C-ABI (which reads
+// exactly these sizes): a mismatch aborts with the offending field instead of reading past a vector.
+void check_deep_shapes(const MLPGridConfig& cfg, const DeepMLPWeights& w, const char* what) {
+    const std::size_t In = cfg.dims.In, H = cfg.dims.H, Out = cfg.dims.Out;
+    const char* bad = nullptr;
+    if (In != 4 || Out != 4 || (H != 32 && H != 64 && H != 128)) bad = "cfg.dims (In = Out = 4, H in {32, 64, 128})";
+    else if (w.hidden_layers < 1 || w.hidden_layers > 16) bad = "hidden_layers (1 .. 16)";
+    else {
+        const std::size_t nl = std::size_t(w.hidden_layers - 1);
+        if (w.W1.size() != H * In) bad = "W1.size() != H * In";
+        else if (w.b1.size() != H) bad = "b1.size() != H";
+        else if (w.Wh.size() != nl * H * H) bad = "Wh.size() != (hidden_layers - 1) * H * H";
+        else if (w.bh.size() != nl * H) bad = "bh.size() != (hidden_layers - 1) * H";
+        else if (w.W2.size() != Out * H) bad = "W2.size() != Out * H";
+        else if (w.b2.size() != Out) bad = "b2.size() != Out";
+    }
+    if (bad) {
+        std::fprintf(stderr, "phys_autodiff_b200: %s: %s\n", what, bad);
+        std::abort();
+    }
+}
+}  // namespace
+
+void mlp_infer_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const std::vector<float>& coords, std::vector<float>& out) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    check_deep_shapes(cfg, w, "mlp_infer_deep_cuda");
+    if (coords.size() % 4) {
+        std::fprintf(stderr, "phys_autodiff_b200: mlp_infer_deep_cuda: coords.size() is not a multiple of 4\n");
+        std::abort();
+    }
+    const std::size_t N = coords.size() / 4;
+    out.resize(N * 4);
+    physad_ctx* c = ctx();
+    int rc = set_deep(c, cfg, w);
+    if (!rc) rc = physad_mlp_forward_deep_host(c, coords.data(), out.data(), N);
+    if (rc) die("mlp_infer_deep_cuda", rc);
+}
+
+void mlp_data_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* target,
+                                  std::size_t B, const float* lam, float* out_loss, DeepMLPWeights& grad) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    check_deep_shapes(cfg, w, "mlp_data_loss_deep_grad_cuda");
+    physad_ctx* c = ctx();
+    grad.hidden_layers = w.hidden_layers;
+    grad.W1.resize(w.W1.size());
+    grad.b1.resize(w.b1.size());
+    grad.Wh.resize(w.Wh.size());
+    grad.bh.resize(w.bh.size());
+    grad.W2.resize(w.W2.size());
+    grad.b2.resize(w.b2.size());
+    int rc = set_deep(c, cfg, w);
+    if (!rc) rc = physad_deep_data_loss_grad_host(c, x, target, B, lam, out_loss, grad.W1.data(), grad.b1.data(),
+                                                  grad.Wh.empty() ? nullptr : grad.Wh.data(),
+                                                  grad.bh.empty() ? nullptr : grad.bh.data(), grad.W2.data(), grad.b2.data());
+    if (rc) die("mlp_data_loss_deep_grad_cuda", rc);
+}
+
 }  // namespace phys
 
 // C-ABI access to the weight generator for non-C++ hosts (bench.py, tests): see include/physad_b200.h.

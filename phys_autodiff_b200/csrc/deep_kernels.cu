@@ -23,6 +23,8 @@
 // Layer 1 (4 -> H) and the output layer (H -> 4) are 1/32 .. 1/8 of one hidden->hidden layer and run as
 // plain strict-fp32 phases on the same shared-memory activations (weights from the kernel-parameter constant
 // bank, MlpConst<H>, exactly as the one-hidden-layer kernels: L = 1 is bit-identical to them).
+// Points mode (POINTS = true, deep_points_launch) is the same kernel with one time slice whose rows are caller-supplied
+// inputs: one float4 load per row instead of the three coordinate-table loads, W1[h,3] * t rounded per row.
 #include "deep_kernels.cuh"
 #include "mlp_eval.cuh"
 
@@ -45,8 +47,10 @@ constexpr int GT = 16;          // outputs per warp
 constexpr int PT = 6;           // rows per lane
 constexpr int ROWS = 32 * PT;   // rows per row-block
 
-template <int H, bool FIELDS, int VAR>
+// POINTS: rows are the caller's points a.pts[0 .. n_points) (AoS {x, y, z, t}, one time slice), outputs to out_aos
+template <int H, bool FIELDS, int VAR, bool POINTS>
 __global__ void __launch_bounds__(DEEP_THREADS, 1) k_mlp_deep(const __grid_constant__ MlpConst<H> w, const __grid_constant__ DeepArgs a) {
+    static_assert(!(POINTS && FIELDS), "points mode writes AoS outputs");
     constexpr int G = H / GT;              // output groups = warps per row-block
     constexpr int RB = 8 / G;              // row-blocks per block
     constexpr int NS = FIELDS ? 3 : 1;     // time slices
@@ -63,7 +67,7 @@ __global__ void __launch_bounds__(DEEP_THREADS, 1) k_mlp_deep(const __grid_const
     const int rb = warp / G, g0 = (warp % G) * GT;
     const int nl = a.hidden_layers - 1;    // hidden->hidden layers
     const bool resident = nl <= 2;         // both buffers hold a layer for good
-    const long long n_slab = (long long)(a.z_end - a.z_begin) * a.ny * a.nx;
+    const long long n_slab = POINTS ? a.n_points : (long long)(a.z_end - a.z_begin) * a.ny * a.nx;
     const long long tiles = (n_slab + PTS_TILE - 1) / PTS_TILE;
     const int plane = a.nx * a.ny;
 
@@ -100,14 +104,19 @@ __global__ void __launch_bounds__(DEEP_THREADS, 1) k_mlp_deep(const __grid_const
     for (long long tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
         // ---- layer 1: this warp's 16 hidden units for its lane's points, all slices -> s_act ------------------
         {
-            float cx[PPL], cy[PPL], cz[PPL];
+            float cx[PPL], cy[PPL], cz[PPL], ct[PPL];
 #pragma unroll
             for (int jp = 0; jp < PPL; ++jp) {
                 long long p = tile * PTS_TILE + rb * PTS_RB + lane * PPL + jp;
                 if (p > n_slab - 1) p = n_slab - 1;   // tail tile: evaluate a valid point, never stored
-                const int zl = int(p / plane), rem = int(p - (long long)zl * plane);
-                const int y = rem / a.nx, x = rem - y * a.nx;
-                cx[jp] = __ldg(a.cxs + x); cy[jp] = __ldg(a.cys + y); cz[jp] = __ldg(a.czs + a.z_begin + zl);
+                if (POINTS) {
+                    const float4 c4 = __ldg(a.pts + p);
+                    cx[jp] = c4.x; cy[jp] = c4.y; cz[jp] = c4.z; ct[jp] = c4.w;
+                } else {
+                    const int zl = int(p / plane), rem = int(p - (long long)zl * plane);
+                    const int y = rem / a.nx, x = rem - y * a.nx;
+                    cx[jp] = __ldg(a.cxs + x); cy[jp] = __ldg(a.cys + y); cz[jp] = __ldg(a.czs + a.z_begin + zl);
+                }
             }
             float* dst = s_act + (rb * H) * ROWS + lane * PT;
 #pragma unroll 2
@@ -127,7 +136,9 @@ __global__ void __launch_bounds__(DEEP_THREADS, 1) k_mlp_deep(const __grid_const
                     const f32x2 sxyz = add2_rn_swapped(sxy, mul2_rn(pack2(w2s), bcast2(cz[jp])));
 #pragma unroll
                     for (int s = 0; s < NS; ++s) {
-                        const float2 pt = NS == 1 ? t0 : (s == 0 ? tm : (s == 1 ? t0 : tp));
+                        // points mode: the row's own t, the product rounded per row
+                        const float2 pt = POINTS ? make_float2(__fmul_rn(w3.x, ct[jp]), __fmul_rn(w3.y, ct[jp]))
+                                                 : (NS == 1 ? t0 : (s == 0 ? tm : (s == 1 ? t0 : tp)));
                         float v0, v1;
                         unpack2(add2_rn(sxyz, pack2(pt)), v0, v1);
                         dst[(2 * qq) * ROWS + jp * NS + s] = relu_ref(v0);
@@ -270,12 +281,12 @@ size_t smem_for(int hidden_layers) {
     return act + wbuf;
 }
 
-template <int H, bool FIELDS, int VAR>
+template <int H, bool FIELDS, int VAR, bool POINTS = false>
 int launch_v(const void* mlp_const, const DeepArgs& a, int grid_blocks, cudaStream_t st) {
     const size_t smem = smem_for<H>(a.hidden_layers);
-    cudaError_t e = cudaFuncSetAttribute(k_mlp_deep<H, FIELDS, VAR>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    cudaError_t e = cudaFuncSetAttribute(k_mlp_deep<H, FIELDS, VAR, POINTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return int(e);
-    k_mlp_deep<H, FIELDS, VAR><<<grid_blocks, DEEP_THREADS, smem, st>>>(*static_cast<const MlpConst<H>*>(mlp_const), a);
+    k_mlp_deep<H, FIELDS, VAR, POINTS><<<grid_blocks, DEEP_THREADS, smem, st>>>(*static_cast<const MlpConst<H>*>(mlp_const), a);
     return int(cudaGetLastError());
 }
 
@@ -298,6 +309,15 @@ int deep_launch(int H, bool fields, const void* mlp_const, const DeepArgs& a, in
         case 32: return fields ? launch_t<32, true>(mlp_const, a, grid_blocks, st) : launch_t<32, false>(mlp_const, a, grid_blocks, st);
         case 64: return fields ? launch_t<64, true>(mlp_const, a, grid_blocks, st) : launch_t<64, false>(mlp_const, a, grid_blocks, st);
         case 128: return fields ? launch_t<128, true>(mlp_const, a, grid_blocks, st) : launch_t<128, false>(mlp_const, a, grid_blocks, st);
+    }
+    return int(cudaErrorInvalidValue);
+}
+
+int deep_points_launch(int H, const void* mlp_const, const DeepArgs& a, int grid_blocks, cudaStream_t st) {
+    switch (H) {   // the unroll-4 variant only (launch_t's default)
+        case 32: return launch_v<32, false, 1, true>(mlp_const, a, grid_blocks, st);
+        case 64: return launch_v<64, false, 1, true>(mlp_const, a, grid_blocks, st);
+        case 128: return launch_v<128, false, 1, true>(mlp_const, a, grid_blocks, st);
     }
     return int(cudaErrorInvalidValue);
 }

@@ -26,11 +26,19 @@ struct DeepArgs {
     float4* out_aos;            // FIELDS = false: [slab points] {sigma, ux, uy, uz}
     float* sigma[3];            // FIELDS = true: t-dt, t, t+dt
     float* u[3];                //   channel-major, channel stride = slab points
+    // points mode (deep_points_launch): the rows are n_points caller-supplied inputs {x, y, z, t}, outputs to out_aos
+    const float4* pts;
+    long long n_points;
 };
 
 // `mlp_const` points to a host MlpConst<H> (mlp_eval.cuh) for the template width H in {32, 64, 128}.
 // Returns a cudaError_t value.  grid_blocks: persistent grid size (normally the SM count).
 int deep_launch(int H, bool fields, const void* mlp_const, const DeepArgs& a, int grid_blocks, cudaStream_t st);
+// The same kernel with its rows taken from a.pts (one float4 load per row) instead of the grid index: the network at
+// a.n_points arbitrary points, out_aos[i] = MLP(pts[i]).  Layer 1 forms W1[h,3] * t per row (the grid modes use the
+// same IEEE product per slice), so at grid coordinates the outputs equal the grid mode's bit for bit.  a.nx .. a.tc,
+// a.sigma and a.u are not read.
+int deep_points_launch(int H, const void* mlp_const, const DeepArgs& a, int grid_blocks, cudaStream_t st);
 // Dynamic shared memory the kernel needs for (H, hidden_layers), for diagnostics / tests.
 size_t deep_smem_bytes(int H, int hidden_layers);
 

@@ -312,6 +312,84 @@ class Context:
               "deep_tangent_loss_grad_host")
         return (np.float32(ls.value), np.float32(lu.value), *d)
 
+    # -- deeper networks at arbitrary points: forward and data-fit loss (additive) -----------------------------------------
+    def mlp_forward_deep(self, x):
+        """y[B, 4] = MLP(x[B, 4]) of the network set by set_weights_deep, on device tensors.  x: float32 CUDA tensor of the
+        network's inputs (x, y, z, t), already normalised like mlp_forward's; any B (strict fp32, bit-identical to
+        mlp_grid_infer_deep at the grid's own coordinates)."""
+        x = x.contiguous()
+        B = x.numel() // 4
+        y = self._empty(B * 4)
+        check(self._lib.physad_mlp_forward_deep_dev(self._h, ptr(x), ptr(y), C.c_size_t(B), self._stream()), "mlp_forward_deep")
+        return y.view(B, 4)
+
+    def mlp_forward_deep_host(self, x) -> np.ndarray:
+        """Host-array form of mlp_forward_deep: x [B, 4] (or flat) -> y float32 [B, 4]."""
+        x = _f32(x)
+        B = x.size // 4
+        y = np.empty((B, 4), np.float32)
+        check(self._lib.physad_mlp_forward_deep_host(self._h, ptr(x), ptr(y), C.c_size_t(B)), "mlp_forward_deep_host")
+        return y
+
+    @staticmethod
+    def _lam(lam):
+        """The C-ABI's lam: 4 host floats, or NULL (None) for 1/4 each."""
+        if lam is None:
+            return None
+        lam = [float(v) for v in lam]
+        assert len(lam) == 4
+        return (C.c_float * 4)(*lam)
+
+    def deep_data_loss_grad_acc(self, x, target, lam=None, n_norm=None, out=None):
+        """Device form of the data-fit loss L_d = (1/n_norm) sum_i sum_o lam[o] (y_io - target_io)^2 of the deep network at
+        the points x (float32 CUDA tensors x, target [B, 4]): a float64 device tensor [acc, grad(P)] with acc the
+        un-normalised weighted sum and grad = dW1 | db1 | dWh | dbh | dW2 | db2 scaled by 2 lam[o] / n_norm, so the tensors
+        of shards with the same n_norm add up and grad adds to the physics gradient.  lam None: 1/4 each (the mean squared
+        error); n_norm None: B (1 for an empty shard)."""
+        import torch
+        x, target = x.contiguous(), target.contiguous()
+        B = x.numel() // 4
+        assert target.numel() == 4 * B
+        out = out if out is not None else self._empty(self.deep_grad_len() + 1, torch.float64)
+        n = max(B, 1) if n_norm is None else int(n_norm)
+        check(self._lib.physad_deep_data_loss_grad_dev(self._h, ptr(x), ptr(target), C.c_size_t(B), self._lam(lam), C.c_size_t(n),
+                                                       ptr(out), ptr(out[1:]), self._stream()), "deep_data_loss_grad")
+        return out
+
+    def deep_data_loss_grad(self, x, target, lam=None, n_global=None, group=None):
+        """(L_d, grad float64 ndarray[P]) of the data-fit loss over the points of every rank.  With torch.distributed
+        initialised each rank passes its own points; n_global (default: the sum of B over ranks, one all-reduce of one
+        integer) normalises, and ONE all-reduce of P+1 doubles combines the ranks."""
+        import torch
+        import torch.distributed as dist
+        world = dist.get_world_size(group) if dist.is_initialized() else 1
+        B = x.numel() // 4
+        if n_global is None:
+            if world > 1:
+                nb = torch.tensor([B], dtype=torch.int64, device=x.device)
+                dist.all_reduce(nb, op=dist.ReduceOp.SUM, group=group)
+                n_global = int(nb.item())
+            else:
+                n_global = B
+        n_global = max(int(n_global), 1)
+        buf = self.deep_data_loss_grad_acc(x, target, lam, n_global)
+        if world > 1:
+            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+        h = buf.cpu().numpy()
+        return float(h[0] / n_global), h[1:].copy()
+
+    def deep_data_loss_grad_host(self, x, target, lam=None):
+        """Host-array form with n_norm = B: (L_d, dW1, db1, dWh, dbh, dW2, db2), float32."""
+        x, target = _f32(x), _f32(target)
+        B = x.size // 4
+        assert target.size == 4 * B
+        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
+        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        loss = C.c_float()
+        check(self._lib.physad_deep_data_loss_grad_host(self._h, ptr(x), ptr(target), C.c_size_t(B), self._lam(lam), C.byref(loss),
+                                                        *[ptr(a) if a.size else None for a in d]), "deep_data_loss_grad_host")
+        return (np.float32(loss.value), *d)
+
     def set_deep_mode(self, mode: int) -> None:
         """0: strict fp32 (bit-exact, default); 1: hidden layers on the tensor cores with three-term bf16 operands (~1e-6)."""
         check(self._lib.physad_set_deep_mode(self._h, C.c_int(mode)), "set_deep_mode")
@@ -819,3 +897,18 @@ def mlp_phys_loss_deep_tangent_grad_cuda(g: Grid, cfg: MLPConfig, L: int, w, pw:
     c = default_context()
     c.set_weights_deep(cfg, L, *w)
     return c.deep_tangent_loss_grad_host(g, pw, t)
+
+
+def mlp_infer_deep_cuda(cfg: MLPConfig, L: int, w, coords: np.ndarray) -> np.ndarray:
+    """A deep network at arbitrary points (additive): w = (W1, b1, Wh, bh, W2, b2), coords [N, 4] -> y float32 [N, 4]."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.mlp_forward_deep_host(coords)
+
+
+def mlp_data_loss_deep_grad_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, target: np.ndarray, lam=None):
+    """Data-fit loss of a deep network and its gradient (additive): w = (W1, b1, Wh, bh, W2, b2) ->
+    (L_d, dW1, db1, dWh, dbh, dW2, db2), L_d = mean over the points of sum_o lam[o] (y_o - target_o)^2 (lam None: 1/4 each)."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.deep_data_loss_grad_host(x, target, lam)

@@ -7,7 +7,11 @@ alternation with the strict deep fields alone (generate_fields_deep) and the one
 --loss deep-tangent times the analytic loss of a deep network (physad_deep_tangent_loss_dev) and its closed loop
 (physad_deep_tangent_loss_grad_dev) for every --hidden x --layers pair, in alternation with the strict deep fields pass and
 the finite-difference deep step (physad_deep_loss_grad_dev); one JSON line per pair.
-  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent] [--n 256] [--hidden 64] [--layers 3] [--steps 20]
+--loss deep-data times the deep network at arbitrary points (physad_mlp_forward_deep_dev) and the data-fit loss + gradient
+step (physad_deep_data_loss_grad_dev) at B = n^3 and B = n^2 random points for every --hidden x --layers pair, in
+alternation with the strict grid forward (mlp_grid_infer_deep at n^3) and the finite-difference deep step; one JSON line per
+pair and B, and with --out the whole run as one JSON document with the GPU's name and power limit.
+  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent|deep-data] [--n 256] [--hidden 64] [--layers 3] [--steps 20]
   python tools/bench_grad.py --loss deep --hidden 32,64,128 --layers 2,3,5
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/bench_grad.py   (z-slab per rank)"""
 import argparse
@@ -28,8 +32,11 @@ def main():
     ap.add_argument("--hidden", default="64", help="width; --loss deep takes a comma-separated list")
     ap.add_argument("--layers", default="3", help="--loss deep: hidden layers, a comma-separated list")
     ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent"), default="fd")
+    ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent", "deep-data"), default="fd")
+    ap.add_argument("--out", default=None, help="--loss deep-data: also write the run as one JSON document here")
     a = ap.parse_args()
+    if a.loss == "deep-data":
+        return deep_data(a, Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True))
     if a.loss == "deep":
         return deep(a, Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True))
     if a.loss == "deep-tangent":
@@ -239,6 +246,89 @@ def deep_tangent(a, g):
                               "gpu": name, "power_limit_w": plim,
                               "grad_absmax": float(abs(h[2:]).max()), "acc": h[:2].tolist(),
                               "acc_loss_call_equal": bool((acc.cpu().numpy() == h[:2]).all())}), flush=True)
+
+
+# counted work per point of the forward at points (one row: hidden layers 2(L-1)H^2, layer 1 and output 16H) and of the data
+# loss + gradient step (the forward, W^T delta and dW of every hidden layer, output layer and layer 1 backward:
+# 8(L-1)H^2 + 48H, the per-row count of deep_flops_per_point)
+def deep_points_flops_per_point(H, L):
+    return 2 * (L - 1) * H * H + 16 * H
+
+
+def deep_data_flops_per_point(H, L):
+    return 8 * (L - 1) * H * H + 48 * H
+
+
+def deep_data(a, g):
+    import numpy as np
+    ctx = ops.Context()
+    pw = PhysWeights(1, 1)
+    name, plim = _gpu()
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=clocks.max.sm", "--format=csv,noheader,nounits",
+                            f"--id={torch.cuda.current_device()}"], capture_output=True, text=True, timeout=30)
+        clk = float(q.stdout.strip().splitlines()[0])
+    except (OSError, ValueError, IndexError, subprocess.TimeoutExpired):
+        clk = None
+    cg = g.c()
+    rng = np.random.default_rng(5)
+    sizes = (g.N, g.nx * g.ny)   # the point count of the grid, and one plane (the overhead regime)
+    xs = {B: torch.from_numpy(rng.uniform(-1, 1, (B, 4)).astype(np.float32)).cuda() for B in sizes}
+    ts = {B: torch.from_numpy(rng.uniform(-1, 1, (B, 4)).astype(np.float32)).cuda() for B in sizes}
+    results = []
+    for H in (int(x) for x in a.hidden.split(",")):
+        w1 = ops.mlp_random_init(H, 777, 0.25)
+        for L in (int(x) for x in a.layers.split(",")):
+            wr = np.random.default_rng(L)
+            Wh = wr.uniform(-0.2, 0.2, (L - 1) * H * H).astype(np.float32)
+            bh = wr.uniform(-0.2, 0.2, (L - 1) * H).astype(np.float32)
+            ctx.set_weights_deep(MLPConfig(4, H, 4, True), L, w1[0], w1[1], Wh, bh, w1[2], w1[3])
+            grid_out = ctx.mlp_grid_infer_deep(g, 0.25)
+            infer = lambda: ctx._lib.physad_mlp_grid_infer_deep_dev(ctx._h, C.byref(cg), None, C.c_float(0.25), ops.ptr(grid_out),
+                                                                    ctx._stream())
+            fdo = ctx.deep_loss_grad_acc(g, pw, 0.25, 2e-3)
+            fdstep = lambda: ctx.deep_loss_grad_acc(g, pw, 0.25, 2e-3, out=fdo)
+            for B in sizes:
+                x, t = xs[B], ts[B]
+                y = ctx.mlp_forward_deep(x)
+                dout = ctx.deep_data_loss_grad_acc(x, t)
+                fwd = lambda: ctx._lib.physad_mlp_forward_deep_dev(ctx._h, ops.ptr(x), ops.ptr(y), C.c_size_t(B), ctx._stream())
+                step = lambda: ctx.deep_data_loss_grad_acc(x, t, out=dout)
+                for _ in range(2):
+                    assert fwd() == 0 and infer() == 0
+                    step(); fdstep()
+                torch.cuda.synchronize()
+                # the four are timed in alternation, so that they share whatever else the GPU is doing
+                tf, ti, td, tfd = [], [], [], []
+                for _ in range(a.steps):
+                    tf += _times(fwd, 1)
+                    ti += _times(infer, 1)
+                    td += _times(step, 1)
+                    tfd += _times(fdstep, 1)
+                for v in (tf, ti, td, tfd):
+                    v.sort()
+                mf, mi, md, mfd = (v[len(v) // 2] for v in (tf, ti, td, tfd))
+                ff, fdd, fdf = deep_points_flops_per_point(H, L), deep_data_flops_per_point(H, L), deep_flops_per_point(H, L)
+                dt_tf, fd_tf = fdd * B / (md * 1e-3) / 1e12, fdf * g.N / (mfd * 1e-3) / 1e12
+                h = dout.cpu().numpy()
+                r = {"workload": f"H={H} L={L} B={B} deep forward at points / data loss+grad", "points": B,
+                     "forward_points_ms": mf, "grid_infer_deep_ms": mi, "data_loss_grad_ms": md, "fd_deep_loss_grad_ms": mfd,
+                     "forward_per_point_ratio_to_grid_infer": (mf / B) / (mi / g.N),
+                     "forward_points_gpts_per_s": B / mf / 1e6, "data_loss_grad_gpts_per_s": B / md / 1e6,
+                     "forward_flops_per_point": ff, "data_flops_per_point": fdd, "fd_deep_flops_per_point": fdf,
+                     "forward_counted_tflops": ff * B / (mf * 1e-3) / 1e12,
+                     "grid_infer_counted_tflops": ff * g.N / (mi * 1e-3) / 1e12,
+                     "data_counted_tflops": dt_tf, "fd_deep_counted_tflops": fd_tf, "data_to_fd_tflops_ratio": dt_tf / fd_tf,
+                     "gpu": name, "power_limit_w": plim, "grad_absmax": float(abs(h[1:]).max()), "acc": float(h[0])}
+                results.append(r)
+                print(json.dumps(r), flush=True)
+    if a.out:
+        with open(a.out, "w") as fh:
+            json.dump({"what": f"tools/bench_grad.py --loss deep-data --hidden {a.hidden} --layers {a.layers} --steps {a.steps} "
+                               f"at {a.n}^3: the forward at B random points, mlp_grid_infer_deep on the grid, the data loss + "
+                               f"gradient step at the same B points and the finite-difference deep step on the grid, timed in "
+                               f"alternation (CUDA events, median of {a.steps}); B = {sizes[0]} and {sizes[1]}",
+                       "gpu": name, "power_limit_w": plim, "clocks_max_sm_mhz": clk, "results": results}, fh, indent=1)
 
 
 def distributed(a, g):
