@@ -1,7 +1,8 @@
 """Closed-loop training of the coordinate MLP against the physics loss (the reference's planned milestone M6,
 REQUIREMENT.md:155-169), on 1..N GPUs:
 
-  python examples/train_closed_loop.py [--loss fd|tangent] [--layers 1] [--data 0] [--n 128] [--hidden 64] [--steps 200]
+  python examples/train_closed_loop.py [--loss fd|tangent] [--layers 1] [--data 0] [--colloc 0] [--t-range 0,0.5] [--n 128]
+                                      [--hidden 64] [--steps 200]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 examples/train_closed_loop.py
 
 Every rank differentiates its z-slab of the grid (physad_fused_loss_grad_slab_dev), one all-reduce of 9H+6 doubles
@@ -13,7 +14,12 @@ finite-difference loss through physad_deep_loss_grad_dev, or with --loss tangent
 physad_deep_tangent_loss_grad_dev, again with one all-reduce of P+2 doubles.  --data N (with --layers L > 1) adds a data
 term: a fixed "teacher" deep network (another seed) gives targets at N random points at t = 0, each rank fits its share of
 the points (physad_deep_data_loss_grad_dev, mean squared error over all N points) and the student trains on
-L_sigma + L_u + L_d.  Prints one JSON line per 20 steps and a summary."""
+L_sigma + L_u + L_d.  --colloc N (with --layers L > 1) replaces the grid's physics term at t = 0.25 by the analytic loss at
+N collocation points drawn fresh every step on the device, uniform in [-1, 1]^3 for space and in the time input of
+--t-range T0,T1 (each rank draws its share from its own seeded generator; physad_deep_tangent_points_loss_grad_dev, mean
+over all N points, the grid's dc/dx from physad_grid_input_scales, one all-reduce of P+2 doubles).  With --data it fits an
+initial condition (the teacher at t = 0) and the dynamics that carry it over [T0, T1].  Prints one JSON line per 20 steps
+and a summary."""
 import argparse
 import json
 import os
@@ -36,9 +42,15 @@ def main():
     ap.add_argument("--loss", choices=("fd", "tangent"), default="fd")
     ap.add_argument("--layers", type=int, default=1, help="hidden layers (> 1: a deep network)")
     ap.add_argument("--data", type=int, default=0, help="teacher points at t = 0 for a data term (needs --layers > 1)")
+    ap.add_argument("--colloc", type=int, default=0,
+                    help="collocation points per step for the physics term instead of the grid at t = 0.25 (needs --layers > 1)")
+    ap.add_argument("--t-range", default="0,0.5", help="T0,T1: the time interval the collocation points cover")
     a = ap.parse_args()
     if a.data and a.layers < 2:
         ap.error("--data needs --layers > 1")
+    if a.colloc and a.layers < 2:
+        ap.error("--colloc needs --layers > 1")
+    t0c, t1c = (float(v) for v in a.t_range.split(","))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank, local = int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
@@ -69,12 +81,24 @@ def main():
         xd = torch.from_numpy(pts[lo:hi]).cuda()
         ctx.set_weights_deep(cfg, L, tW1, tb1, tWh, tbh, tW2, tb2)
         yd = ctx.mlp_forward_deep(xd).clone()
+    if a.colloc:
+        # this rank's share of the N points per step; MinusOneToOne: the network's time input is t itself
+        lo_c, hi_c = (rank * a.colloc) // world, ((rank + 1) * a.colloc) // world
+        gen = torch.Generator(device="cuda")
+        gen.manual_seed(1000 + rank)
+        lo4 = torch.tensor([-1.0, -1.0, -1.0, t0c], device="cuda")
+        span4 = torch.tensor([2.0, 2.0, 2.0, t1c - t0c], device="cuda")
+        dcdx = ops.grid_input_scales(g, cfg.minus_one_to_one)   # the grid's physical domain
     m, v = np.zeros_like(th), np.zeros_like(th)
     first = last = None
     t0 = time.perf_counter()
     for k in range(1, a.steps + 1):
         w = np.split(th.astype(np.float32), cuts)
-        if L > 1 and a.loss == "tangent":
+        if a.colloc:
+            ctx.set_weights_deep(cfg, L, *w)
+            xc = lo4 + span4 * torch.rand((hi_c - lo_c, 4), generator=gen, device="cuda")
+            ls, lu, grad = ctx.deep_tangent_points_loss_grad(xc, dcdx, pw, n_global=a.colloc)   # + all-reduce when world > 1
+        elif L > 1 and a.loss == "tangent":
             ctx.set_weights_deep(cfg, L, *w)
             ls, lu, grad = ctx.deep_tangent_loss_grad(g, pw, 0.25)   # slab per rank + all-reduce when world > 1
         elif L > 1:
@@ -103,7 +127,12 @@ def main():
     dt = time.perf_counter() - t0
     if rank == 0:
         data = f" + data at {a.data} points" if a.data else ""
-        print(json.dumps({"summary": f"{a.n}^3 H={H} L={L} {a.loss} loss{data} on {world} GPU(s)", "steps": a.steps, "loss_first": first,
+        summary = f"{a.n}^3 H={H} L={L} {a.loss} loss{data} on {world} GPU(s)"
+        if a.colloc:
+            what = " (initial condition + dynamics)" if a.data else ""
+            summary = (f"H={H} L={L} analytic loss at {a.colloc} collocation points per step over t in [{t0c:g}, {t1c:g}] of the "
+                       f"{a.n}^3 domain{data}{what} on {world} GPU(s)")
+        print(json.dumps({"summary": summary, "steps": a.steps, "loss_first": first,
                           "loss_last": last, "reduction_pct": 100 * (1 - last / first),
                           "wall_ms_per_step_incl_host_adam": 1e3 * dt / a.steps}))
     if world > 1:

@@ -81,6 +81,19 @@ void mlp_infer_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, cons
 void mlp_data_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* target,
                                   std::size_t B, const float* lam, float* out_loss, DeepMLPWeights& grad);
 
+// The analytic loss of a deep network at arbitrary space-time points (collocation points) instead of the grid at one time:
+// x holds B host points of 4 floats (x, y, z, t), the network inputs already normalised (the fourth is the grid's time input:
+// t for MinusOneToOne, t + 0.5 for ZeroToOne); dcdx the 3 dc/dx of the space inputs (physad_grid_input_scales gives the
+// grid's).  *out_loss_* = (w / B) sum R^2; opt_R, if given, receives B x 4 residuals {R_sigma, R_ux, R_uy, R_uz} per point.
+// The _grad form also returns d(L_sigma + L_u) with respect to every layer's weights; `grad` is resized to the shapes of `w`
+// and adds directly to mlp_data_loss_deep_grad_cuda's.  B = 0 gives zeros.  Every vector of `w` is checked against cfg.
+void mlp_phys_loss_deep_tangent_points_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
+                                            const float* x, std::size_t B, const float dcdx[3], float* out_loss_sigma,
+                                            float* out_loss_u, float* opt_R = nullptr);
+void mlp_phys_loss_deep_tangent_points_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
+                                                 const float* x, std::size_t B, const float dcdx[3], float* out_loss_sigma,
+                                                 float* out_loss_u, DeepMLPWeights& grad);
+
 }  // namespace phys
 
 #endif  // PHYS_AUTODIFF_PHYS_B200_H

@@ -134,7 +134,8 @@ int physad_mlp_generate_fields_host(physad_ctx* ctx, const physad_grid* g, float
  * nothing; the host forms that take new weights (cfg != NULL) replace the network first and run.  Use the *_deep_* and
  * deep_* counterparts: physad_mlp_forward_deep_* for physad_mlp_forward_*, physad_deep_data_loss_grad_* for
  * physad_mlp_backward_*, physad_mlp_grid_infer_deep_dev, physad_mlp_generate_fields_deep_dev, physad_deep_loss_host,
- * physad_deep_loss_grad_* and physad_deep_tangent_loss_*.  hidden_layers == 1 is accepted everywhere.  A refused call leaves the previous network in place.
+ * physad_deep_loss_grad_*, physad_deep_tangent_loss_* and, at arbitrary points, physad_deep_tangent_points_loss_*.
+ * hidden_layers == 1 is accepted everywhere.  A refused call leaves the previous network in place.
  * A later physad_set_weights() switches the context back to a one-hidden-layer network. */
 int physad_set_weights_deep(physad_ctx* ctx, const physad_mlp_config* cfg, int hidden_layers, const float* W1,
                             const float* b1, const float* Wh, const float* bh, const float* W2, const float* b2);
@@ -433,6 +434,41 @@ int physad_deep_data_loss_grad_dev(physad_ctx* ctx, const float* x, const float*
                                    size_t n_norm, double* acc, double* grad, void* stream);
 int physad_deep_data_loss_grad_host(physad_ctx* ctx, const float* x, const float* target, size_t B, const float* lam,
                                     float* loss, float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2);
+
+/* ---- analytic loss of deeper networks at arbitrary points (ADDITIVE, no reference counterpart) ---------------------------
+ * The physics loss of physad_deep_tangent_loss_* at caller-supplied collocation points (x, y, z, t) spread over the whole
+ * space-time domain instead of the grid's points at one time: the term that makes a fit learn the dynamics between the
+ * times where data anchor it.  The same kernel body as physad_deep_tangent_loss_* (strict fp32 value row, FMA tangent
+ * rows, residuals, seeds and reverse mode), with one float4 load per point for the inputs and W1[h,3] t rounded per point;
+ * so with x = the grid's points (in linear order) and dcdx = physad_grid_input_scales, the sums, residuals and gradient
+ * equal the grid calls' bit for bit.  Any hidden_layers >= 1 (one hidden layer runs the same kernel).
+ * physad_grid_input_scales: dc/dx of the three space inputs exactly as the grid's analytic calls form them
+ *   (f / ((n-1) h), f = 2 for MinusOneToOne (norm 1), 1 for ZeroToOne (norm 0), 0 for an extent of 1).  Host-only, no GPU.
+ * x: [B][4] DEVICE floats, 16-byte aligned: the network inputs, already normalised; the fourth is the grid calls' time input
+ *   (t for MinusOneToOne, t + 0.5 for ZeroToOne), and d/dt is taken with respect to it (factor 1).
+ * dcdx: 3 finite HOST floats, dc/dx of the three space inputs (the residual's d/dx_j = dcdx[j] d/dc_j).
+ * physad_deep_tangent_points_loss_dev: acc = 2 device doubles (sum R_sigma^2, sum |R_u|^2 over the B points, not
+ *   normalised); R: null or [B][4] device floats, 16-byte aligned, {R_sigma, R_ux, R_uy, R_uz} per point.
+ * physad_deep_tangent_points_loss_grad_dev: the same acc (bit for bit) AND the gradient of L_sigma + L_u with
+ *   L = (w / n_norm) sum R^2, P = physad_deep_grad_len(H, L) device doubles in the layout of physad_deep_loss_grad_dev,
+ *   scaled by 2.f * w / float(n_norm): with n_norm = the points of ALL shards, the shards' P+2 doubles add up under one
+ *   all-reduce(sum), and grad adds directly to physad_deep_data_loss_grad_dev's and to the grid calls' gradients.
+ * physad_deep_tangent_points_loss_grad_host: x a host array, n_norm = B; the losses (physad_finalize_loss(acc, w, B)) and the
+ *   gradient split into the six arrays of physad_set_weights_deep's layouts (any output pointer may be null).
+ * B = 0 (an empty shard) writes zero sums and a zero gradient.  Bitwise repeatable.
+ * Errors: no deep weights (or a physad_set_weights after them): PHYSAD_E_NOWEIGHTS; physad_set_deep_mode(1):
+ * PHYSAD_E_UNSUPPORTED; a null pointer (x only with B > 0), a misaligned x or R (16 bytes) or acc or grad (8 bytes), a
+ * non-finite dcdx, n_norm == 0, or (physad_grid_input_scales) a non-positive extent or a norm other than 0 or 1:
+ * PHYSAD_E_INVALID.  A refused call writes nothing. */
+int physad_grid_input_scales(const physad_grid* g, int norm, float dcdx[3]);
+int physad_deep_tangent_points_loss_dev(physad_ctx* ctx, const float* x, size_t B, const float* dcdx, double* acc,
+                                        float* R, void* stream);
+int physad_deep_tangent_points_loss_grad_dev(physad_ctx* ctx, const float* x, size_t B, const float* dcdx,
+                                             const physad_phys_weights* w, size_t n_norm, double* acc, double* grad,
+                                             void* stream);
+int physad_deep_tangent_points_loss_grad_host(physad_ctx* ctx, const float* x, size_t B, const float* dcdx,
+                                              const physad_phys_weights* w, float* loss_sigma, float* loss_u, float* dW1,
+                                              float* db1, float* dWh, float* dbh, float* dW2, float* db2);
 
 /* Host-only: the work partition the fused kernel is launched with.  The sequence of tiles x planes
  * tile-planes (tile-major) is cut into at most `slots` contiguous ranges of equal cost, a range paying

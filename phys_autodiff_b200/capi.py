@@ -98,7 +98,8 @@ EXPORTS = [
     "physad_deep_grad_len", "physad_deep_loss_grad_dev", "physad_deep_loss_grad_host",
     "physad_deep_tangent_loss_dev", "physad_deep_tangent_loss_grad_dev", "physad_deep_tangent_loss_grad_host",
     "physad_mlp_forward_deep_dev", "physad_mlp_forward_deep_host", "physad_deep_data_loss_grad_dev",
-    "physad_deep_data_loss_grad_host",
+    "physad_deep_data_loss_grad_host", "physad_grid_input_scales", "physad_deep_tangent_points_loss_dev",
+    "physad_deep_tangent_points_loss_grad_dev", "physad_deep_tangent_points_loss_grad_host",
 ]
 
 

@@ -1848,6 +1848,15 @@ int physad_deep_loss_grad_host(physad_ctx* c, const physad_grid* g, const physad
 // ---- analytic loss of deeper networks and its closed loop (deep_tangent_kernels.cuh) ---------------------------------
 }  // extern "C"  (helpers below)
 namespace {
+// dc/dx of the three space inputs as physad_tangent_loss_dev forms them: f / ((n-1) h), f = 2 for MinusOneToOne (norm 1),
+// 1 for ZeroToOne, 0 for an extent of 1
+void input_scales(const physad_grid* g, int norm, float s[3]) {
+    const double f = norm == 1 ? 2.0 : 1.0;
+    s[0] = g->nx > 1 ? float(f / (double(g->nx - 1) * double(g->hx))) : 0.f;
+    s[1] = g->ny > 1 ? float(f / (double(g->ny - 1) * double(g->hy))) : 0.f;
+    s[2] = g->nz > 1 ? float(f / (double(g->nz - 1) * double(g->hz))) : 0.f;
+}
+
 // checks and arguments shared by the loss and the loss + gradient call; *npts = 0 for an empty slab
 int deep_tangent_args(physad_ctx* c, const physad_grid* g, const physad_slab* slab, float t, const char* what,
                       DeepTangentArgs& a, long long* npts, cudaStream_t st) {
@@ -1868,11 +1877,9 @@ int deep_tangent_args(physad_ctx* c, const physad_grid* g, const physad_slab* sl
     a.W1 = c->dW1; a.b1 = c->db1; a.W2 = c->dW2; a.b2 = c->db2;
     a.wh = c->d_wh; a.bh = c->d_bh;
     a.tc = time_coord(t, c->cfg.norm);
-    // dc/dx exactly as physad_tangent_loss_dev forms it (0 for an extent of 1)
-    const double f = c->cfg.norm == 1 ? 2.0 : 1.0;
-    a.sx = g->nx > 1 ? float(f / (double(g->nx - 1) * double(g->hx))) : 0.f;
-    a.sy = g->ny > 1 ? float(f / (double(g->ny - 1) * double(g->hy))) : 0.f;
-    a.sz = g->nz > 1 ? float(f / (double(g->nz - 1) * double(g->hz))) : 0.f;
+    float s3[3];
+    input_scales(g, c->cfg.norm, s3);
+    a.sx = s3[0]; a.sy = s3[1]; a.sz = s3[2];
     return 0;
 }
 }  // namespace
@@ -2134,6 +2141,144 @@ int physad_deep_data_loss_grad_host(physad_ctx* c, const float* x, const float* 
     CU(cudaStreamSynchronize(c->stream));
     if (loss) *loss = float(c->h_dgrad[0] / double(B ? B : 1));
     const double* gd = c->h_dgrad + 1;
+    const size_t nl = size_t(L - 1), hh = size_t(H);
+    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
+    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
+    for (int k = 0; k < 6; ++k) {
+        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
+        gd += len[k];
+    }
+    return 0;
+}
+
+// ---- analytic loss of deeper networks at caller-supplied points (collocation points; deep_tangent_kernels.cuh) ---------
+int physad_grid_input_scales(const physad_grid* g, int norm, float dcdx[3]) {
+    if (!g || !dcdx) return fail(PHYSAD_E_INVALID, "grid_input_scales: null argument");
+    if (g->nx <= 0 || g->ny <= 0 || g->nz <= 0) return fail(PHYSAD_E_INVALID, "grid_input_scales: grid extents must be positive");
+    if (norm != 0 && norm != 1) return fail(PHYSAD_E_INVALID, "grid_input_scales: norm must be 0 (ZeroToOne) or 1 (MinusOneToOne)");
+    input_scales(g, norm, dcdx);
+    return 0;
+}
+
+}  // extern "C"  (helpers below)
+namespace {
+// checks shared by the points loss and the points loss + gradient call
+int colloc_check(const float* x, size_t B, const float* dcdx, const char* what) {
+    if (B && !x) return fail(PHYSAD_E_INVALID, std::string(what) + ": null argument");
+    if (B && misaligned16(x)) return fail(PHYSAD_E_INVALID, std::string(what) + ": x must be 16-byte aligned");
+    for (int k = 0; k < 3; ++k)
+        if (!std::isfinite(dcdx[k])) return fail(PHYSAD_E_INVALID, std::string(what) + ": dcdx must be finite");
+    return 0;
+}
+
+// the kernel arguments of B > 0 points; uploads the context's weights first (that may move the device buffers)
+int colloc_args(physad_ctx* c, const float* x, size_t B, const float* dcdx, DeepTangentArgs& a, cudaStream_t st) {
+    if (int rc = upload_weights_if_stale(c, st)) return rc;
+    a.hidden_layers = c->deep_layers;
+    a.W1 = c->dW1; a.b1 = c->db1; a.W2 = c->dW2; a.b2 = c->db2;
+    a.wh = c->d_wh; a.bh = c->d_bh;
+    a.sx = dcdx[0]; a.sy = dcdx[1]; a.sz = dcdx[2];
+    a.pts = reinterpret_cast<const float4*>(x);
+    a.n_points = (long long)B;
+    return 0;
+}
+}  // namespace
+extern "C" {
+
+int physad_deep_tangent_points_loss_dev(physad_ctx* c, const float* x, size_t B, const float* dcdx, double* acc, float* R,
+                                        void* stream) {
+    if (!c) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss: null context");
+    if (int rc = deep_points_ready(c, "deep_tangent_points_loss")) return rc;
+    if (!acc || !dcdx) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss: null argument");
+    if (uintptr_t(acc) % 8) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss: acc must be 8-byte aligned");
+    if (R && misaligned16(R)) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss: R must be 16-byte aligned");
+    if (int rc = colloc_check(x, B, dcdx, "deep_tangent_points_loss")) return rc;
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    if (B == 0) {
+        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
+        return 0;
+    }
+    DeepTangentArgs a{};
+    if (int rc = colloc_args(c, x, B, dcdx, a, st)) return rc;
+    a.R_pts = reinterpret_cast<float4*>(R);
+    const int H = c->cfg.H;
+    const int blocks = deep_tangent_blocks(H, (long long)B, c->sm_count);
+    if (int rc = ensure_grad_partials(c, size_t(blocks) * 2)) return rc;
+    a.partials = c->gpart;
+    CU(cudaError_t(colloc_tangent_launch(H, false, a, blocks, acc, nullptr, st)));
+    c->launches += 2;
+    return 0;
+}
+
+int physad_deep_tangent_points_loss_grad_dev(physad_ctx* c, const float* x, size_t B, const float* dcdx,
+                                             const physad_phys_weights* w, size_t n_norm, double* acc, double* grad,
+                                             void* stream) {
+    if (!c) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss_grad: null context");
+    if (int rc = deep_points_ready(c, "deep_tangent_points_loss_grad")) return rc;
+    if (!w || !acc || !grad || !dcdx) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss_grad: null argument");
+    if (uintptr_t(acc) % 8 || uintptr_t(grad) % 8)
+        return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss_grad: acc and grad must be 8-byte aligned");
+    if (n_norm == 0) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss_grad: n_norm must be positive");
+    if (int rc = colloc_check(x, B, dcdx, "deep_tangent_points_loss_grad")) return rc;
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (B == 0) {   // an empty shard: zero sums, zero gradient
+        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
+        CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
+        return 0;
+    }
+    DeepTangentArgs a{};
+    if (int rc = colloc_args(c, x, B, dcdx, a, st)) return rc;
+    // vjp_scales' formula with n_norm for N: shards with the same n_norm add up to the whole set's gradient
+    a.scale_s = 2.f * w->w_sigma / float(n_norm);
+    a.scale_u = 2.f * w->w_u / float(n_norm);
+    const int blocks = deep_tangent_blocks(H, (long long)B, c->sm_count);
+    const size_t ck = size_t(blocks) * deep_tangent_ckpt_floats(L);
+    if (ck > c->dckpt_cap) {
+        if (c->dckpt) CU(cudaFree(c->dckpt));
+        c->dckpt = nullptr; c->dckpt_cap = 0;
+        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
+        c->dckpt_cap = ck;
+    }
+    if (int rc = ensure_grad_partials(c, size_t(blocks) * (P + 2))) return rc;
+    a.ckpt = c->dckpt;
+    a.partials = c->gpart;
+    CU(cudaError_t(colloc_tangent_launch(H, true, a, blocks, acc, grad, st)));
+    c->launches += 2;
+    return 0;
+}
+
+int physad_deep_tangent_points_loss_grad_host(physad_ctx* c, const float* x, size_t B, const float* dcdx,
+                                              const physad_phys_weights* w, float* loss_sigma, float* loss_u, float* dW1,
+                                              float* db1, float* dWh, float* dbh, float* dW2, float* db2) {
+    if (!c) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss_grad: null context");
+    if (int rc = deep_points_ready(c, "deep_tangent_points_loss_grad")) return rc;
+    if (!w || !dcdx || (B && !x)) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss_grad: null argument");
+    DeviceGuard dg(c->device);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (P + 2 > c->dgrad_cap) {
+        if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
+        if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
+        c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
+        CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
+        CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
+        c->dgrad_cap = P + 2;
+    }
+    const size_t bytes = B * 4 * sizeof(float);
+    if (int rc = ensure_scratch(c, bytes + 1)) return rc;
+    float* dx = reinterpret_cast<float*>(c->scratch);
+    if (B) CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
+    // n_norm = B; an empty set (B = 0) gives zero losses and a zero gradient
+    const size_t n = B ? B : 1;
+    if (int rc = physad_deep_tangent_points_loss_grad_dev(c, dx, B, dcdx, w, n, c->d_dgrad, c->d_dgrad + 2, c->stream)) return rc;
+    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 2) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    physad_finalize_loss(c->h_dgrad, w, n, loss_sigma, loss_u);
+    const double* gd = c->h_dgrad + 2;
     const size_t nl = size_t(L - 1), hh = size_t(H);
     float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
     const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};

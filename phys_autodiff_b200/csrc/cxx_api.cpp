@@ -453,6 +453,54 @@ void mlp_data_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights
     if (rc) die("mlp_data_loss_deep_grad_cuda", rc);
 }
 
+void mlp_phys_loss_deep_tangent_points_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
+                                            const float* x, std::size_t B, const float dcdx[3], float* out_loss_sigma,
+                                            float* out_loss_u, float* opt_R) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    check_deep_shapes(cfg, w, "mlp_phys_loss_deep_tangent_points_cuda");
+    const physad_phys_weights cw = to_c(pw);
+    physad_ctx* c = ctx();
+    const std::size_t bytes = B * 4 * sizeof(float);
+    float *d_x = nullptr, *d_R = nullptr;
+    double* d_acc = nullptr;
+    double h_acc[2] = {0.0, 0.0};
+    int rc = set_deep(c, cfg, w);
+    if (!rc) rc = int(cudaMalloc(&d_acc, 2 * sizeof(double)));
+    if (!rc && B) rc = int(cudaMalloc(&d_x, bytes));
+    if (!rc && B && opt_R) rc = int(cudaMalloc(&d_R, bytes));
+    if (!rc && B) rc = int(cudaMemcpy(d_x, x, bytes, cudaMemcpyHostToDevice));
+    if (!rc) rc = physad_deep_tangent_points_loss_dev(c, d_x, B, dcdx, d_acc, d_R, nullptr);
+    if (!rc) rc = int(cudaMemcpy(h_acc, d_acc, sizeof(h_acc), cudaMemcpyDeviceToHost));
+    if (!rc && d_R) rc = int(cudaMemcpy(opt_R, d_R, bytes, cudaMemcpyDeviceToHost));
+    cudaFree(d_x);
+    cudaFree(d_R);
+    cudaFree(d_acc);
+    if (rc) die("mlp_phys_loss_deep_tangent_points_cuda", rc);
+    physad_finalize_loss(h_acc, &cw, B ? B : 1, out_loss_sigma, out_loss_u);
+}
+
+void mlp_phys_loss_deep_tangent_points_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
+                                                 const float* x, std::size_t B, const float dcdx[3], float* out_loss_sigma,
+                                                 float* out_loss_u, DeepMLPWeights& grad) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    check_deep_shapes(cfg, w, "mlp_phys_loss_deep_tangent_points_grad_cuda");
+    const physad_phys_weights cw = to_c(pw);
+    physad_ctx* c = ctx();
+    grad.hidden_layers = w.hidden_layers;
+    grad.W1.resize(w.W1.size());
+    grad.b1.resize(w.b1.size());
+    grad.Wh.resize(w.Wh.size());
+    grad.bh.resize(w.bh.size());
+    grad.W2.resize(w.W2.size());
+    grad.b2.resize(w.b2.size());
+    int rc = set_deep(c, cfg, w);
+    if (!rc) rc = physad_deep_tangent_points_loss_grad_host(c, x, B, dcdx, &cw, out_loss_sigma, out_loss_u, grad.W1.data(),
+                                                            grad.b1.data(), grad.Wh.empty() ? nullptr : grad.Wh.data(),
+                                                            grad.bh.empty() ? nullptr : grad.bh.data(), grad.W2.data(),
+                                                            grad.b2.data());
+    if (rc) die("mlp_phys_loss_deep_tangent_points_grad_cuda", rc);
+}
+
 }  // namespace phys
 
 // C-ABI access to the weight generator for non-C++ hosts (bench.py, tests): see include/physad_b200.h.

@@ -390,6 +390,80 @@ class Context:
                                                         *[ptr(a) if a.size else None for a in d]), "deep_data_loss_grad_host")
         return (np.float32(loss.value), *d)
 
+    # -- analytic loss of deeper networks at arbitrary points (collocation points; additive) -------------------------------
+    @staticmethod
+    def _dcdx(dcdx):
+        """The C-ABI's dcdx: 3 host floats, dc/dx of the three space inputs (grid_input_scales gives a grid's)."""
+        d = [float(v) for v in dcdx]
+        assert len(d) == 3
+        return (C.c_float * 3)(*d)
+
+    def deep_tangent_points_loss_acc(self, x, dcdx, acc=None, residuals=None):
+        """Analytic loss of the deep network set by set_weights_deep at the points x (float32 CUDA tensor [B, 4] of network
+        inputs (x, y, z, t), already normalised; the fourth is the grid calls' time input): the device sums
+        {sum Rs^2, sum |Ru|^2} over the points; residuals: a float32 CUDA tensor [B, 4] (R_sigma, R_ux, R_uy, R_uz per
+        point) or None."""
+        import torch
+        x = x.contiguous()
+        B = x.numel() // 4
+        acc = acc if acc is not None else self._empty(2, torch.float64)
+        if residuals is not None:
+            assert residuals.is_contiguous() and residuals.numel() == 4 * B
+        check(self._lib.physad_deep_tangent_points_loss_dev(self._h, ptr(x), C.c_size_t(B), self._dcdx(dcdx), ptr(acc),
+                                                            ptr(residuals), self._stream()), "deep_tangent_points_loss")
+        return acc
+
+    def deep_tangent_points_loss_grad_acc(self, x, dcdx, pw: PhysWeights, n_norm=None, out=None):
+        """Device form: a float64 device tensor [acc_sigma, acc_u, grad(P)] of the analytic loss at the points x, with
+        grad = dW1 | db1 | dWh | dbh | dW2 | db2 scaled by 2w/n_norm, so the tensors of shards with the same n_norm add up and
+        grad adds to the data-fit and grid gradients.  n_norm None: B (1 for an empty shard)."""
+        import torch
+        x = x.contiguous()
+        B = x.numel() // 4
+        out = out if out is not None else self._empty(self.deep_grad_len() + 2, torch.float64)
+        n = max(B, 1) if n_norm is None else int(n_norm)
+        cw = pw.c()
+        check(self._lib.physad_deep_tangent_points_loss_grad_dev(self._h, ptr(x), C.c_size_t(B), self._dcdx(dcdx), C.byref(cw),
+                                                                 C.c_size_t(n), ptr(out), ptr(out[2:]), self._stream()),
+              "deep_tangent_points_loss_grad")
+        return out
+
+    def deep_tangent_points_loss_grad(self, x, dcdx, pw: PhysWeights, n_global=None, group=None):
+        """(L_sigma, L_u, grad float64 ndarray[P]) of the analytic loss over the points of every rank.  With
+        torch.distributed initialised each rank passes its own points; n_global (default: the sum of B over ranks, one
+        all-reduce of one integer) normalises, and ONE all-reduce of P+2 doubles combines the ranks."""
+        import torch
+        import torch.distributed as dist
+        world = dist.get_world_size(group) if dist.is_initialized() else 1
+        B = x.numel() // 4
+        if n_global is None:
+            if world > 1:
+                nb = torch.tensor([B], dtype=torch.int64, device=x.device)
+                dist.all_reduce(nb, op=dist.ReduceOp.SUM, group=group)
+                n_global = int(nb.item())
+            else:
+                n_global = B
+        n_global = max(int(n_global), 1)
+        buf = self.deep_tangent_points_loss_grad_acc(x, dcdx, pw, n_global)
+        if world > 1:
+            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+        h = buf.cpu().numpy()
+        ls, lu = self.finalize(h[:2], pw, n_global)
+        return ls, lu, h[2:].copy()
+
+    def deep_tangent_points_loss_grad_host(self, x, dcdx, pw: PhysWeights):
+        """Host-array form with n_norm = B: x [B, 4] (or flat) -> (L_sigma, L_u, dW1, db1, dWh, dbh, dW2, db2), float32."""
+        x = _f32(x)
+        B = x.size // 4
+        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
+        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        ls, lu = C.c_float(), C.c_float()
+        cw = pw.c()
+        check(self._lib.physad_deep_tangent_points_loss_grad_host(self._h, ptr(x), C.c_size_t(B), self._dcdx(dcdx), C.byref(cw),
+                                                                  C.byref(ls), C.byref(lu), *[ptr(a) if a.size else None for a in d]),
+              "deep_tangent_points_loss_grad_host")
+        return (np.float32(ls.value), np.float32(lu.value), *d)
+
     def set_deep_mode(self, mode: int) -> None:
         """0: strict fp32 (bit-exact, default); 1: hidden layers on the tensor cores with three-term bf16 operands (~1e-6)."""
         check(self._lib.physad_set_deep_mode(self._h, C.c_int(mode)), "set_deep_mode")
@@ -801,6 +875,16 @@ def mlp_random_init(H: int, seed: int = 42, scale: float = 0.5, In: int = 4, Out
     return W1, b1, W2, b2
 
 
+def grid_input_scales(g: Grid, norm) -> np.ndarray:
+    """dc/dx of the three space inputs (float32 [3]) exactly as the grid's analytic calls form them: the dcdx with which
+    points of the grid's domain give the grid's physics.  norm: 1 / True = MinusOneToOne, 0 / False = ZeroToOne.
+    Host-only, no GPU."""
+    out = np.empty(3, np.float32)
+    cg = g.c()
+    check(capi.lib().physad_grid_input_scales(C.byref(cg), C.c_int(int(norm)), ptr(out)), "grid_input_scales")
+    return out
+
+
 # ---- reference-named host functions (one shared context, like the C++ layer) -----------------------
 _CTX: Optional[Context] = None
 
@@ -912,3 +996,11 @@ def mlp_data_loss_deep_grad_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, targe
     c = default_context()
     c.set_weights_deep(cfg, L, *w)
     return c.deep_data_loss_grad_host(x, target, lam)
+
+
+def mlp_phys_loss_deep_tangent_points_grad_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, dcdx, pw: PhysWeights):
+    """Analytic loss of a deep network at arbitrary points and its gradient (additive): w = (W1, b1, Wh, bh, W2, b2),
+    x [B, 4] network inputs -> (L_sigma, L_u, dW1, db1, dWh, dbh, dW2, db2), the losses the mean over the points."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.deep_tangent_points_loss_grad_host(x, dcdx, pw)

@@ -11,7 +11,12 @@ the finite-difference deep step (physad_deep_loss_grad_dev); one JSON line per p
 step (physad_deep_data_loss_grad_dev) at B = n^3 and B = n^2 random points for every --hidden x --layers pair, in
 alternation with the strict grid forward (mlp_grid_infer_deep at n^3) and the finite-difference deep step; one JSON line per
 pair and B, and with --out the whole run as one JSON document with the GPU's name and power limit.
-  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent|deep-data] [--n 256] [--hidden 64] [--layers 3] [--steps 20]
+--loss deep-tangent-points times the analytic deep loss at B uniform random space-time points
+(physad_deep_tangent_points_loss_dev) and its loss + gradient step (physad_deep_tangent_points_loss_grad_dev) at B = n^3
+and B = n^2, in alternation with the grid's analytic loss and loss + gradient step at n^3 (physad_deep_tangent_loss_dev /
+_grad_dev); one JSON line per pair and B, and with --out the whole run as one JSON document.
+  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent|deep-data|deep-tangent-points] [--n 256] [--hidden 64]
+                             [--layers 3] [--steps 20]
   python tools/bench_grad.py --loss deep --hidden 32,64,128 --layers 2,3,5
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/bench_grad.py   (z-slab per rank)"""
 import argparse
@@ -32,9 +37,11 @@ def main():
     ap.add_argument("--hidden", default="64", help="width; --loss deep takes a comma-separated list")
     ap.add_argument("--layers", default="3", help="--loss deep: hidden layers, a comma-separated list")
     ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent", "deep-data"), default="fd")
-    ap.add_argument("--out", default=None, help="--loss deep-data: also write the run as one JSON document here")
+    ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent", "deep-data", "deep-tangent-points"), default="fd")
+    ap.add_argument("--out", default=None, help="--loss deep-data / deep-tangent-points: also write the run as one JSON document here")
     a = ap.parse_args()
+    if a.loss == "deep-tangent-points":
+        return deep_tangent_points(a, Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True))
     if a.loss == "deep-data":
         return deep_data(a, Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True))
     if a.loss == "deep":
@@ -328,6 +335,79 @@ def deep_data(a, g):
                                f"at {a.n}^3: the forward at B random points, mlp_grid_infer_deep on the grid, the data loss + "
                                f"gradient step at the same B points and the finite-difference deep step on the grid, timed in "
                                f"alternation (CUDA events, median of {a.steps}); B = {sizes[0]} and {sizes[1]}",
+                       "gpu": name, "power_limit_w": plim, "clocks_max_sm_mhz": clk, "results": results}, fh, indent=1)
+
+
+def deep_tangent_points(a, g):
+    import numpy as np
+    ctx = ops.Context()
+    pw = PhysWeights(1, 1)
+    name, plim = _gpu()
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=clocks.max.sm", "--format=csv,noheader,nounits",
+                            f"--id={torch.cuda.current_device()}"], capture_output=True, text=True, timeout=30)
+        clk = float(q.stdout.strip().splitlines()[0])
+    except (OSError, ValueError, IndexError, subprocess.TimeoutExpired):
+        clk = None
+    dcdx = ops.grid_input_scales(g, True)
+    rng = np.random.default_rng(5)
+    sizes = (g.N, g.nx * g.ny)   # the grid's point count, and one plane (the overhead regime)
+    # uniform random space-time points: space in [-1, 1]^3, the time input (MinusOneToOne: t) in [0, 0.5]
+    xs = {}
+    for B in sizes:
+        x = rng.uniform(-1, 1, (B, 4)).astype(np.float32)
+        x[:, 3] = rng.uniform(0.0, 0.5, B).astype(np.float32)
+        xs[B] = torch.from_numpy(x).cuda()
+    results = []
+    for H in (int(v) for v in a.hidden.split(",")):
+        w1 = ops.mlp_random_init(H, 777, 0.25)
+        for L in (int(v) for v in a.layers.split(",")):
+            wr = np.random.default_rng(L)
+            Wh = wr.uniform(-0.2, 0.2, (L - 1) * H * H).astype(np.float32)
+            bh = wr.uniform(-0.2, 0.2, (L - 1) * H).astype(np.float32)
+            ctx.set_weights_deep(MLPConfig(4, H, 4, True), L, w1[0], w1[1], Wh, bh, w1[2], w1[3])
+            gacc = ctx.deep_tangent_loss_acc(g, 0.25)
+            gout = ctx.deep_tangent_loss_grad_acc(g, pw, 0.25)
+            calls = {"grid_loss": lambda: ctx.deep_tangent_loss_acc(g, 0.25, acc=gacc),
+                     "grid_loss_grad": lambda: ctx.deep_tangent_loss_grad_acc(g, pw, 0.25, out=gout)}
+            outs = {}
+            for B in sizes:
+                pacc = ctx.deep_tangent_points_loss_acc(xs[B], dcdx)
+                pout = ctx.deep_tangent_points_loss_grad_acc(xs[B], dcdx, pw)
+                outs[B] = pout
+                calls[f"points_loss_{B}"] = lambda x=xs[B], o=pacc: ctx.deep_tangent_points_loss_acc(x, dcdx, acc=o)
+                calls[f"points_loss_grad_{B}"] = lambda x=xs[B], o=pout: ctx.deep_tangent_points_loss_grad_acc(x, dcdx, pw, out=o)
+            for _ in range(2):
+                for fn in calls.values():
+                    fn()
+            torch.cuda.synchronize()
+            # every call is timed in alternation with the others, so that they share whatever else the GPU is doing
+            ts = {k: [] for k in calls}
+            for _ in range(a.steps):
+                for k, fn in calls.items():
+                    ts[k] += _times(fn, 1)
+            med = {k: sorted(v)[len(v) // 2] for k, v in ts.items()}
+            ml, mg = med["grid_loss"], med["grid_loss_grad"]
+            for B in sizes:
+                pl, pg = med[f"points_loss_{B}"], med[f"points_loss_grad_{B}"]
+                h = outs[B].cpu().numpy()
+                r = {"workload": f"H={H} L={L} B={B} deep analytic loss / loss+grad at points vs the grid at {a.n}^3", "points": B,
+                     "points_loss_ms": pl, "points_loss_grad_ms": pg, "grid_loss_ms": ml, "grid_loss_grad_ms": mg,
+                     "loss_per_point_ratio_to_grid": (pl / B) / (ml / g.N),
+                     "loss_grad_per_point_ratio_to_grid": (pg / B) / (mg / g.N),
+                     "points_loss_gpts_per_s": B / pl / 1e6, "points_loss_grad_gpts_per_s": B / pg / 1e6,
+                     "loss_counted_tflops": deep_tangent_flops_per_point(H, L, False) * B / (pl * 1e-3) / 1e12,
+                     "loss_grad_counted_tflops": deep_tangent_flops_per_point(H, L, True) * B / (pg * 1e-3) / 1e12,
+                     "gpu": name, "power_limit_w": plim, "grad_absmax": float(abs(h[2:]).max()), "acc": h[:2].tolist()}
+                results.append(r)
+                print(json.dumps(r), flush=True)
+    if a.out:
+        with open(a.out, "w") as fh:
+            json.dump({"what": f"tools/bench_grad.py --loss deep-tangent-points --hidden {a.hidden} --layers {a.layers} "
+                               f"--steps {a.steps} at {a.n}^3: the analytic deep loss and its loss + gradient step at B uniform "
+                               f"random space-time points (space in [-1, 1]^3, t in [0, 0.5], dc/dx of the grid) and the same two "
+                               f"calls on the grid, timed in alternation (CUDA events, median of {a.steps}); B = {sizes[0]} and "
+                               f"{sizes[1]}; the ratios are per point (B = n^3: the same point count as the grid)",
                        "gpu": name, "power_limit_w": plim, "clocks_max_sm_mhz": clk, "results": results}, fh, indent=1)
 
 
