@@ -25,6 +25,44 @@ def bits_equal(a, b):
     return a.shape == b.shape and bool(np.array_equal(a.view(np.uint32), b.view(np.uint32)))
 
 
+def grad_segments(H, L):
+    """Named slices of the weight-gradient layout dW1 | db1 | dWh1 .. dWh{L-1} | dbh1 .. dbh{L-1} | dW2 | db2 (the
+    argument order of physad_set_weights_deep; with L = 1 the one-hidden-layer layout dW1 | db1 | dW2 | db2)."""
+    sizes = [("dW1", 4 * H), ("db1", H)] + [(f"dWh{l}", H * H) for l in range(1, L)] + \
+            [(f"dbh{l}", H) for l in range(1, L)] + [("dW2", 4 * H), ("db2", 4)]
+    out, o = [], 0
+    for name, n in sizes:
+        out.append((name, slice(o, o + n)))
+        o += n
+    return out
+
+
+def grad_error_ratios(got, want, H, L, floor=1e-3, floors=None):
+    """Per tensor s: max|got_s - want_s| / max(max|want_s|, floor_s * max|want|), floor_s = floors.get(s, floor)."""
+    got = np.asarray(got, np.float64).ravel(); want = np.asarray(want, np.float64).ravel()
+    segs = grad_segments(H, L)
+    assert got.shape == want.shape == (segs[-1][1].stop,), (got.shape, want.shape, segs[-1][1].stop)
+    gmax = np.abs(want).max()
+    out = {}
+    for name, s in segs:
+        err = np.abs(got[s] - want[s]).max()
+        ref = max(np.abs(want[s]).max(), (floors or {}).get(name, floor) * gmax)
+        out[name] = err / ref if ref > 0 else (0.0 if err == 0 else np.inf)
+    return out
+
+
+def assert_grad_close(got, want, H, L, tol=1e-4, floor=1e-3, floors=None):
+    """Every tensor of the gradient on its own scale: max|got_s - want_s| <= tol * max(max|want_s|, floor * max|want|).
+    One norm over the whole vector barely checks a tensor much smaller than the largest one.  floors = {tensor: floor}
+    raises the floor of named tensors only, where a measured fp32 rounding error needs it.  Returns the largest ratio
+    max|got_s - want_s| / max(...) over the tensors."""
+    r = grad_error_ratios(got, want, H, L, floor, floors)
+    bad = {k: v for k, v in r.items() if not v <= tol}
+    assert not bad, "gradient tensors off by more than %g of their own scale: %s" % (
+        tol, ", ".join(f"{k} ({v:.3g})" for k, v in bad.items()))
+    return max(r.values())
+
+
 def manufactured_fields(g, t, kx=1, ky=1, kz=1, const_u=True):
     """sigma = sin(kx x + ky y + kz z - t) on a 2*pi-periodic box, u = (1,1,1) or
     (sin z, cos x, sin y): the fields of test/test_phys_cpu_ref.cpp:32-48 and

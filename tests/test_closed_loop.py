@@ -9,6 +9,7 @@ The reference has no such function (its backward stops at dL/dR), so the chain i
 import numpy as np
 import pytest
 
+from helpers import assert_grad_close
 from oracle import Grid as OGrid
 
 TOL_GRAD = 1e-4   # max |d| / max |grad|: fp32 adjoint arithmetic + fp32 batch sums vs the double checker
@@ -95,8 +96,7 @@ def test_gradient_vs_checker(ctx, port, shape, H, per, m1p1, h, dt):
     want = port.phys_loss_grad(og, w, 0.25, dt, 1.3, 0.7, m1p1, all_double=False)
     ls, lu, dW1, db1, dW2, db2 = ctx.fused_loss_grad_host(_g(og), MLPConfig(4, H, 4, m1p1), *w, PhysWeights(1.3, 0.7), 0.25, dt)
     got = np.concatenate([dW1, db1, dW2, db2]).astype(np.float64)
-    gmax = np.abs(want["grad"]).max()
-    assert np.abs(got - want["grad"]).max() <= TOL_GRAD * gmax + 1e-30, (np.abs(got - want["grad"]).max(), gmax)
+    assert_grad_close(got, want["grad"], H, 1, TOL_GRAD)
     assert abs(ls - want["loss_sigma"]) <= TOL_LOSS * abs(want["loss_sigma"]) + 1e-30
     assert abs(lu - want["loss_u"]) <= TOL_LOSS * abs(want["loss_u"]) + 1e-30
     # the losses are the fused forward kernel's
@@ -116,8 +116,7 @@ def test_gradient_with_slice_offset_different_from_grid_dt(ctx, port, shape, H, 
     want = port.phys_loss_grad(og, w, 0.25, dt, 1.3, 0.7, True, all_double=False)
     ls, lu, dW1, db1, dW2, db2 = ctx.fused_loss_grad_host(_g(og), MLPConfig(4, H, 4, True), *w, PhysWeights(1.3, 0.7), 0.25, dt)
     got = np.concatenate([dW1, db1, dW2, db2]).astype(np.float64)
-    gmax = np.abs(want["grad"]).max()
-    assert np.abs(got - want["grad"]).max() <= TOL_GRAD * gmax, (np.abs(got - want["grad"]).max(), gmax)
+    assert_grad_close(got, want["grad"], H, 1, TOL_GRAD)
     assert abs(ls - want["loss_sigma"]) <= TOL_LOSS * abs(want["loss_sigma"])
     assert abs(lu - want["loss_u"]) <= TOL_LOSS * abs(want["loss_u"])
     # the slab form shares grad_args_common
@@ -126,7 +125,7 @@ def test_gradient_with_slice_offset_different_from_grid_dt(ctx, port, shape, H, 
     tot = np.zeros(9 * H + 6)
     for r in range(3):
         tot += ctx.fused_loss_grad_slab_acc(_g(og), PhysWeights(1.3, 0.7), 0.25, dt, slab_for_rank(og.nz, r, 3)).cpu().numpy()
-    assert np.abs(tot[2:] - want["grad"]).max() <= TOL_GRAD * gmax
+    assert_grad_close(tot[2:], want["grad"], H, 1, TOL_GRAD)
 
 
 @pytest.mark.gpu

@@ -18,6 +18,7 @@ import sys
 import numpy as np
 import pytest
 
+from helpers import assert_grad_close
 from oracle import Grid as OGrid
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -271,9 +272,7 @@ def test_gradient_vs_checker(ctx, port, chk, H, L, B, lam, n_norm):
     out = ctx.deep_data_loss_grad_acc(_dev(x), _dev(tgt), lam, n).cpu().numpy()
     assert out.shape == (_plen(H, L) + 1,)
     assert abs(out[0] - acc) <= 1e-6 * abs(acc)
-    gmax = np.abs(want).max()
-    err = np.abs(out[1:] - want).max()
-    assert err <= TOL_GRAD * gmax + 1e-30, (err, gmax)
+    assert_grad_close(out[1:], want, H, L, TOL_GRAD)
 
 
 @pytest.mark.gpu
@@ -290,7 +289,7 @@ def test_one_hidden_layer_matches_mlp_backward(ctx, port, H):
     ctx.set_weights_deep(MLPConfig(4, H, 4, True), 1, W1, b1, None, None, W2, b2)
     got = ctx.deep_data_loss_grad_acc(_dev(x), _dev(tgt)).cpu().numpy()[1:]
     # layouts: mlp_backward gives dW1 | db1 | dW2 | db2; with L = 1 the deep layout is the same
-    assert np.abs(got - ref).max() <= TOL_GRAD * np.abs(ref).max()
+    assert_grad_close(got, ref, H, 1, TOL_GRAD)
 
 
 @pytest.mark.gpu

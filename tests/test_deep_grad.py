@@ -16,6 +16,7 @@ import sys
 import numpy as np
 import pytest
 
+from helpers import assert_grad_close
 from oracle import Grid as OGrid
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -227,6 +228,13 @@ GPU_CASES = [
     ((96, 8, 3), 128, 3, False, False, (1, 1, 1)),
 ]
 
+# Per-tensor floors where fp32 rounding is measured to dominate.  (1, 4, 3), H = 32, L = 5: twelve points of a nearly
+# constant network, so the residuals are mostly rounding of nearly equal outputs; the checker's fp32-faithful gradient
+# differs from its all-double one by 0.6 - 2.6e-3 of every tensor's own scale.  dbh2 - dbh4 are 0.2 - 0.5 % of the largest
+# entry, and the kernel's fp32 adjoint puts them 1.0e-3, 2.5e-3 and 1.0e-3 of their own scale (at most 7e-6 of the largest
+# entry) from the faithful checker on a B200.
+FP32_FLOORS = {((1, 4, 3), 32, 5): {"dbh2": 0.1, "dbh3": 0.1, "dbh4": 0.1}}
+
 
 def _g(og):
     from phys_autodiff_b200 import Grid
@@ -249,9 +257,7 @@ def test_gradient_vs_checker(ctx, port, deep, shape, H, L, per, m1p1, h):
     pw = PhysWeights(1.3, 0.7)
     out = ctx.deep_loss_grad_acc(_g(og), pw, 0.25, 2e-3).cpu().numpy()
     assert out.shape == (_plen(H, L) + 2,)
-    gmax = np.abs(want["grad"]).max()
-    err = np.abs(out[2:] - want["grad"]).max()
-    assert err <= TOL_GRAD * gmax + 1e-30, (err, gmax)
+    assert_grad_close(out[2:], want["grad"], H, L, TOL_GRAD, floors=FP32_FLOORS.get((shape, H, L)))
     # the losses are physad_deep_loss_host's: same fields, same residual kernel, same sums
     ls, lu = ctx.finalize(out[:2], pw, og.N)
     assert (ls, lu) == ctx.deep_loss(_g(og), pw, 0.25, 2e-3)
@@ -266,7 +272,7 @@ def test_gradient_vs_checker_when_dt_differs_from_the_grid_step(ctx, port, deep)
     want = deep.phys_loss_grad_deep(og, 64, 3, w, 0.3, 5e-3, 1.0, 1.0, True, all_double=False)["grad"]
     _set(ctx, 64, 3, w)
     out = ctx.deep_loss_grad_acc(_g(og), PhysWeights(1.0, 1.0), 0.3, 5e-3).cpu().numpy()
-    assert np.abs(out[2:] - want).max() <= TOL_GRAD * np.abs(want).max()
+    assert_grad_close(out[2:], want, 64, 3, TOL_GRAD)
 
 
 @pytest.mark.gpu

@@ -17,6 +17,7 @@ import sys
 import numpy as np
 import pytest
 
+from helpers import assert_grad_close
 from oracle import Grid as OGrid
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -259,9 +260,7 @@ def test_loss_and_gradient_vs_checker(ctx, port, chk, shape, H, L, m1p1, h):
     out = ctx.deep_tangent_loss_grad_acc(g, PhysWeights(1.3, 0.7), 0.25).cpu().numpy()
     assert out.shape == (_plen(H, L) + 2,)
     assert np.array_equal(out[:2].view(np.uint64), acc.view(np.uint64))   # the grad call's sums are the loss call's
-    gmax = np.abs(want["grad"]).max()
-    err = np.abs(out[2:] - want["grad"]).max()
-    assert err <= TOL_GRAD * gmax + 1e-30, (err, gmax)
+    assert_grad_close(out[2:], want["grad"], H, L, TOL_GRAD)
 
 
 @pytest.mark.gpu

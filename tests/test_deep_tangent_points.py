@@ -18,6 +18,7 @@ import sys
 import numpy as np
 import pytest
 
+from helpers import assert_grad_close
 from oracle import Grid as OGrid
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -265,8 +266,7 @@ def test_points_loss_and_gradient_vs_checker(ctx, port, chk, H, L, B):
     out = ctx.deep_tangent_points_loss_grad_acc(xd, DCDX, PhysWeights(1.3, 0.7)).cpu().numpy()
     assert out.shape == (_plen(H, L) + 2,)
     assert np.array_equal(out[:2].view(np.uint64), acc.view(np.uint64))   # the grad call's sums are the loss call's
-    gmax = np.abs(want["grad"]).max()
-    assert np.abs(out[2:] - want["grad"]).max() <= 1e-4 * gmax + 1e-30
+    assert_grad_close(out[2:], want["grad"], H, L, 1e-4)
 
 
 @pytest.mark.gpu
