@@ -1,8 +1,8 @@
 """Closed-loop training of the coordinate MLP against the physics loss (the reference's planned milestone M6,
 REQUIREMENT.md:155-169), on 1..N GPUs:
 
-  python examples/train_closed_loop.py [--loss fd|tangent] [--layers 1] [--data 0] [--colloc 0] [--t-range 0,0.5] [--n 128]
-                                      [--hidden 64] [--steps 200]
+  python examples/train_closed_loop.py [--loss fd|tangent] [--layers 1] [--data 0] [--colloc 0] [--periodic 0]
+                                      [--t-range 0,0.5] [--n 128] [--hidden 64] [--steps 200]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 examples/train_closed_loop.py
 
 Every rank differentiates its z-slab of the grid (physad_fused_loss_grad_slab_dev), one all-reduce of 9H+6 doubles
@@ -18,8 +18,12 @@ L_sigma + L_u + L_d.  --colloc N (with --layers L > 1) replaces the grid's physi
 N collocation points drawn fresh every step on the device, uniform in [-1, 1]^3 for space and in the time input of
 --t-range T0,T1 (each rank draws its share from its own seeded generator; physad_deep_tangent_points_loss_grad_dev, mean
 over all N points, the grid's dc/dx from physad_grid_input_scales, one all-reduce of P+2 doubles).  With --data it fits an
-initial condition (the teacher at t = 0) and the dynamics that carry it over [T0, T1].  Prints one JSON line per 20 steps
-and a summary."""
+initial condition (the teacher at t = 0) and the dynamics that carry it over [T0, T1].  --periodic N (with --colloc) adds
+the periodic boundary condition of the grid's domain, which the analytic loss has no stencil to impose: N pairs drawn fresh
+every step on the device, a third per space axis a, p on the face p_a = -1 (the other two space inputs uniform in [-1, 1],
+the time input in [T0, T1]) and q = p + T_a e_a one period on (ops.grid_periods), fitted with the pair loss
+(physad_deep_pair_loss_grad_dev, lam = 1/4 each, mean over all N pairs, one all-reduce of P+1 doubles).  Prints one JSON
+line per 20 steps and a summary."""
 import argparse
 import json
 import os
@@ -44,12 +48,16 @@ def main():
     ap.add_argument("--data", type=int, default=0, help="teacher points at t = 0 for a data term (needs --layers > 1)")
     ap.add_argument("--colloc", type=int, default=0,
                     help="collocation points per step for the physics term instead of the grid at t = 0.25 (needs --layers > 1)")
+    ap.add_argument("--periodic", type=int, default=0,
+                    help="pairs per step for the periodic boundary condition of the grid's domain (needs --colloc)")
     ap.add_argument("--t-range", default="0,0.5", help="T0,T1: the time interval the collocation points cover")
     a = ap.parse_args()
     if a.data and a.layers < 2:
         ap.error("--data needs --layers > 1")
     if a.colloc and a.layers < 2:
         ap.error("--colloc needs --layers > 1")
+    if a.periodic and not a.colloc:
+        ap.error("--periodic needs --colloc")
     t0c, t1c = (float(v) for v in a.t_range.split(","))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank, local = int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0"))
@@ -89,6 +97,14 @@ def main():
         lo4 = torch.tensor([-1.0, -1.0, -1.0, t0c], device="cuda")
         span4 = torch.tensor([2.0, 2.0, 2.0, t1c - t0c], device="cuda")
         dcdx = ops.grid_input_scales(g, cfg.minus_one_to_one)   # the grid's physical domain
+    if a.periodic:
+        # this rank's share of the N pairs per step; pair i lies across the faces of space axis i % 3
+        lo_p, hi_p = (rank * a.periodic) // world, ((rank + 1) * a.periodic) // world
+        pgen = torch.Generator(device="cuda")
+        pgen.manual_seed(2000 + rank)
+        period = torch.from_numpy(ops.grid_periods(g, cfg.minus_one_to_one)).cuda()
+        rows = torch.arange(hi_p - lo_p, device="cuda")
+        axis = (rows + lo_p) % 3
     m, v = np.zeros_like(th), np.zeros_like(th)
     first = last = None
     t0 = time.perf_counter()
@@ -110,11 +126,19 @@ def main():
         else:
             ctx.set_weights(cfg, *w)
             ls, lu, grad = ctx.fused_loss_grad(g, pw, 0.25, 2e-3)
+        lp = None
+        if a.periodic:   # the network set above
+            p = lo4 + span4 * torch.rand((hi_p - lo_p, 4), generator=pgen, device="cuda")
+            p[rows, axis] = -1.0
+            q = p.clone()
+            q[rows, axis] += period[axis]
+            lp, gp = ctx.deep_pair_loss_grad(torch.stack([p, q], 1), n_global=a.periodic)
+            grad = grad + gp
         ld = None
         if a.data:   # the network set above; all ranks' points, one all-reduce of P+1 doubles
             ld, gd = ctx.deep_data_loss_grad(xd, yd, n_global=a.data)
             grad = grad + gd
-        last = float(ls) + float(lu) + (ld or 0.0)
+        last = float(ls) + float(lu) + (ld or 0.0) + (lp or 0.0)
         first = last if first is None else first
         m = 0.9 * m + 0.1 * grad
         v = 0.999 * v + 0.001 * grad * grad
@@ -123,6 +147,8 @@ def main():
             rec = {"step": k, "loss_sigma": float(ls), "loss_u": float(lu)}
             if ld is not None:
                 rec["loss_data"] = ld
+            if lp is not None:
+                rec["loss_periodic"] = lp
             print(json.dumps(rec), flush=True)
     dt = time.perf_counter() - t0
     if rank == 0:
@@ -130,6 +156,7 @@ def main():
         summary = f"{a.n}^3 H={H} L={L} {a.loss} loss{data} on {world} GPU(s)"
         if a.colloc:
             what = " (initial condition + dynamics)" if a.data else ""
+            what += f" + periodic boundaries at {a.periodic} pairs per step" if a.periodic else ""
             summary = (f"H={H} L={L} analytic loss at {a.colloc} collocation points per step over t in [{t0c:g}, {t1c:g}] of the "
                        f"{a.n}^3 domain{data}{what} on {world} GPU(s)")
         print(json.dumps({"summary": summary, "steps": a.steps, "loss_first": first,

@@ -81,6 +81,14 @@ void mlp_infer_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, cons
 void mlp_data_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* target,
                                   std::size_t B, const float* lam, float* out_loss, DeepMLPWeights& grad);
 
+// Periodic-pair loss of a deep network and its gradient with respect to every layer's weights: x holds B host pairs of two
+// points of 4 floats, (p_i, q_i) (e.g. p on a face and q = p + T_a e_a one period on, T_a = f n_a / (n_a - 1)); lam as in
+// mlp_data_loss_deep_grad_cuda; *out_loss = (1/B) sum_i sum_o lam[o] (y(p_i)_o - y(q_i)_o)^2.  `grad` is resized to the
+// shapes of `w` and adds directly to mlp_data_loss_deep_grad_cuda's.  B = 0 gives zeros.  Every vector of `w` is checked
+// against cfg.
+void mlp_pair_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, std::size_t B,
+                                  const float* lam, float* out_loss, DeepMLPWeights& grad);
+
 // The analytic loss of a deep network at arbitrary space-time points (collocation points) instead of the grid at one time:
 // x holds B host points of 4 floats (x, y, z, t), the network inputs already normalised (the fourth is the grid's time input:
 // t for MinusOneToOne, t + 0.5 for ZeroToOne); dcdx the 3 dc/dx of the space inputs (physad_grid_input_scales gives the

@@ -134,7 +134,8 @@ int physad_mlp_generate_fields_host(physad_ctx* ctx, const physad_grid* g, float
  * nothing; the host forms that take new weights (cfg != NULL) replace the network first and run.  Use the *_deep_* and
  * deep_* counterparts: physad_mlp_forward_deep_* for physad_mlp_forward_*, physad_deep_data_loss_grad_* for
  * physad_mlp_backward_*, physad_mlp_grid_infer_deep_dev, physad_mlp_generate_fields_deep_dev, physad_deep_loss_host,
- * physad_deep_loss_grad_*, physad_deep_tangent_loss_* and, at arbitrary points, physad_deep_tangent_points_loss_*.
+ * physad_deep_loss_grad_*, physad_deep_tangent_loss_* and, at arbitrary points, physad_deep_tangent_points_loss_* and
+ * physad_deep_pair_loss_grad_*.
  * hidden_layers == 1 is accepted everywhere.  A refused call leaves the previous network in place.
  * A later physad_set_weights() switches the context back to a one-hidden-layer network. */
 int physad_set_weights_deep(physad_ctx* ctx, const physad_mlp_config* cfg, int hidden_layers, const float* W1,
@@ -434,6 +435,34 @@ int physad_deep_data_loss_grad_dev(physad_ctx* ctx, const float* x, const float*
                                    size_t n_norm, double* acc, double* grad, void* stream);
 int physad_deep_data_loss_grad_host(physad_ctx* ctx, const float* x, const float* target, size_t B, const float* lam,
                                     float* loss, float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2);
+
+/* ---- periodic boundaries at arbitrary points: a matched-pair loss of deeper networks (ADDITIVE, no reference counterpart)
+ * L_p = (1/n_norm) sum_i sum_o lam[o] (y(p_i)_o - y(q_i)_o)^2 over B pairs of network inputs (p_i, q_i), with its gradient
+ * with respect to every layer of the network set by physad_set_weights_deep (any hidden_layers >= 1, deep mode 0).  The
+ * analytic calls have no stencil and so no boundary rule; this term states one.  For periodicity along space axis a, take
+ * p on the face (p_a = -1 for MinusOneToOne, 0 for ZeroToOne) and q = p + T_a e_a with the period in network coordinates
+ *   T_a = f n_a / (n_a - 1)   (f = 2 for MinusOneToOne, 1 for ZeroToOne; computed in double and rounded once to float),
+ * the coordinate of the virtual index n_a that the grid's periodic stencil identifies with index 0.  The call itself takes
+ * any pairs (any axis, or t).
+ * x: [B][2][4] DEVICE floats, 16-byte aligned: row 2i is p_i, row 2i + 1 is q_i.  lam: 4 HOST floats (finite, >= 0) or NULL
+ *   for 1/4 each.  The outputs are physad_mlp_forward_deep_dev's bit for bit; the seeds are
+ *   y_bar(p_i)_o = fp32(2 lam[o] / n_norm) * fp32(y(p_i)_o - y(q_i)_o) and y_bar(q_i) = -y_bar(p_i) (exact in fp32).
+ * physad_deep_pair_loss_grad_dev: acc = 1 device double, the un-normalised sum_i sum_o lam[o] (y(p_i)_o - y(q_i)_o)^2 (each
+ *   pair counted once); grad = P = physad_deep_grad_len(H, L) device doubles in the layout of physad_deep_loss_grad_dev,
+ *   already scaled by 2 lam[o] / n_norm: with n_norm = the pairs of ALL shards, the shards' acc and grad add up under one
+ *   all-reduce(sum), and grad adds directly to physad_deep_data_loss_grad_dev's and the physics calls' gradients.  db2 is
+ *   exactly zero (the two seeds of a pair cancel).  B = 0 (an empty shard) writes acc = 0 and a zero gradient.  Bitwise
+ *   repeatable.
+ * physad_deep_pair_loss_grad_host: x a host array, n_norm = B; loss = L_p as float, the gradient split into the six arrays
+ *   of physad_set_weights_deep's layouts (any output pointer may be null); B = 0 gives zeros.
+ * Errors: those of physad_deep_data_loss_grad_*: no deep weights (or a physad_set_weights after them): PHYSAD_E_NOWEIGHTS;
+ * physad_set_deep_mode(1): PHYSAD_E_UNSUPPORTED; n_norm == 0, a negative or non-finite lam, a null or misaligned x with
+ * B > 0, a null or misaligned acc or grad: PHYSAD_E_INVALID.  The same checkpoint and partials scratch as the data loss.
+ * A refused call writes nothing. */
+int physad_deep_pair_loss_grad_dev(physad_ctx* ctx, const float* x, size_t B, const float* lam, size_t n_norm,
+                                   double* acc, double* grad, void* stream);
+int physad_deep_pair_loss_grad_host(physad_ctx* ctx, const float* x, size_t B, const float* lam, float* loss,
+                                    float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2);
 
 /* ---- analytic loss of deeper networks at arbitrary points (ADDITIVE, no reference counterpart) ---------------------------
  * The physics loss of physad_deep_tangent_loss_* at caller-supplied collocation points (x, y, z, t) spread over the whole

@@ -1995,11 +1995,11 @@ int launch_deep_points(physad_ctx* c, const DeepArgs& a, cudaStream_t st) {
 }
 
 template <int H>
-int launch_deep_data(physad_ctx* c, const DeepDataArgs& a, int blocks, double* grad, double* acc, cudaStream_t st) {
+int launch_deep_data(physad_ctx* c, bool pairs, const DeepDataArgs& a, int blocks, double* grad, double* acc, cudaStream_t st) {
     MlpConst<H> k;
     const float no_t[3] = {0.f, 0.f, 0.f};   // only the output pairs w2 / b2 are read
     fill_const<H>(c, no_t, k);
-    CU(cudaError_t(deep_data_launch(H, &k, a, blocks, grad, acc, st)));
+    CU(cudaError_t(pairs ? deep_pair_launch(H, &k, a, blocks, grad, acc, st) : deep_data_launch(H, &k, a, blocks, grad, acc, st)));
     c->launches += 2;
     return 0;
 }
@@ -2055,20 +2055,25 @@ int physad_mlp_forward_deep_host(physad_ctx* c, const float* x, float* y, size_t
     return 0;
 }
 
-int physad_deep_data_loss_grad_dev(physad_ctx* c, const float* x, const float* target, size_t B, const float* lam,
-                                   size_t n_norm, double* acc, double* grad, void* stream) {
-    if (!c) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: null context");
-    if (int rc = deep_points_ready(c, "deep_data_loss_grad")) return rc;
-    if (!acc || !grad || (B && (!x || !target))) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: null argument");
-    if (B && (misaligned16(x) || misaligned16(target)))
-        return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: x and target must be 16-byte aligned");
-    if (uintptr_t(acc) % 8 || uintptr_t(grad) % 8) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: acc and grad must be 8-byte aligned");
-    if (n_norm == 0) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: n_norm must be positive");
+}  // extern "C"  (helpers below)
+namespace {
+// The data loss (B points and their targets) and the pair loss (B pairs = 2B rows of x, no target) share everything but
+// the kernel: the checks, the scratch, the arguments and the reduction.  `what` names the caller in error messages.
+int deep_fit_dev(physad_ctx* c, const char* what, bool pairs, const float* x, const float* target, size_t B, const float* lam,
+                 size_t n_norm, double* acc, double* grad, void* stream) {
+    const std::string w(what);
+    if (!c) return fail(PHYSAD_E_INVALID, w + ": null context");
+    if (int rc = deep_points_ready(c, what)) return rc;
+    if (!acc || !grad || (B && (!x || (!pairs && !target)))) return fail(PHYSAD_E_INVALID, w + ": null argument");
+    if (B && (misaligned16(x) || (!pairs && misaligned16(target))))
+        return fail(PHYSAD_E_INVALID, w + (pairs ? ": x must be 16-byte aligned" : ": x and target must be 16-byte aligned"));
+    if (uintptr_t(acc) % 8 || uintptr_t(grad) % 8) return fail(PHYSAD_E_INVALID, w + ": acc and grad must be 8-byte aligned");
+    if (n_norm == 0) return fail(PHYSAD_E_INVALID, w + ": n_norm must be positive");
     float lw[4] = {0.25f, 0.25f, 0.25f, 0.25f};   // NULL: the mean over the four outputs
     if (lam) {
         for (int o = 0; o < 4; ++o) {
             if (!std::isfinite(lam[o]) || lam[o] < 0.f)
-                return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: lam must be finite and non-negative");
+                return fail(PHYSAD_E_INVALID, w + ": lam must be finite and non-negative");
             lw[o] = lam[o];
         }
     }
@@ -2082,7 +2087,8 @@ int physad_deep_data_loss_grad_dev(physad_ctx* c, const float* x, const float* t
         return 0;
     }
     if (int rc = upload_weights_if_stale(c, st)) return rc;
-    const int blocks = deep_data_blocks(H, (long long)B, c->sm_count);
+    const size_t rows = pairs ? 2 * B : B;
+    const int blocks = deep_data_blocks(H, (long long)rows, c->sm_count);
     const size_t ck = size_t(blocks) * deep_data_ckpt_floats(H, L);
     if (ck > c->dckpt_cap) {
         if (c->dckpt) CU(cudaFree(c->dckpt));
@@ -2093,7 +2099,7 @@ int physad_deep_data_loss_grad_dev(physad_ctx* c, const float* x, const float* t
     if (int rc = ensure_grad_partials(c, size_t(blocks) * (P + 1))) return rc;
     DeepDataArgs a{};
     a.hidden_layers = L;
-    a.n = (long long)B;
+    a.n = (long long)rows;
     a.x = reinterpret_cast<const float4*>(x);
     a.target = reinterpret_cast<const float4*>(target);
     a.W1 = c->dW1; a.b1 = c->db1; a.W2 = c->dW2;
@@ -2105,17 +2111,18 @@ int physad_deep_data_loss_grad_dev(physad_ctx* c, const float* x, const float* t
     a.ckpt = c->dckpt;
     a.partials = c->gpart;
     switch (H) {
-        case 32: return launch_deep_data<32>(c, a, blocks, grad, acc, st);
-        case 64: return launch_deep_data<64>(c, a, blocks, grad, acc, st);
-        default: return launch_deep_data<128>(c, a, blocks, grad, acc, st);
+        case 32: return launch_deep_data<32>(c, pairs, a, blocks, grad, acc, st);
+        case 64: return launch_deep_data<64>(c, pairs, a, blocks, grad, acc, st);
+        default: return launch_deep_data<128>(c, pairs, a, blocks, grad, acc, st);
     }
 }
 
-int physad_deep_data_loss_grad_host(physad_ctx* c, const float* x, const float* target, size_t B, const float* lam,
-                                    float* loss, float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2) {
-    if (!c) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: null context");
-    if (int rc = deep_points_ready(c, "deep_data_loss_grad")) return rc;
-    if (B && (!x || !target)) return fail(PHYSAD_E_INVALID, "deep_data_loss_grad: null argument");
+// The host forms: x (and target) uploaded, n_norm = B, the gradient split into set_weights_deep's six arrays.
+int deep_fit_host(physad_ctx* c, const char* what, bool pairs, const float* x, const float* target, size_t B, const float* lam,
+                  float* loss, float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2) {
+    if (!c) return fail(PHYSAD_E_INVALID, std::string(what) + ": null context");
+    if (int rc = deep_points_ready(c, what)) return rc;
+    if (B && (!x || (!pairs && !target))) return fail(PHYSAD_E_INVALID, std::string(what) + ": null argument");
     DeviceGuard dg(c->device);
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
@@ -2127,16 +2134,16 @@ int physad_deep_data_loss_grad_host(physad_ctx* c, const float* x, const float* 
         CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
         c->dgrad_cap = P + 2;
     }
-    const size_t bytes = B * 4 * sizeof(float), off_t = (bytes + 255) & ~size_t(255);
-    if (int rc = ensure_scratch(c, off_t + bytes + 1)) return rc;
+    const size_t bytes = B * (pairs ? 8 : 4) * sizeof(float), off_t = (bytes + 255) & ~size_t(255);
+    if (int rc = ensure_scratch(c, off_t + (pairs ? 0 : bytes) + 1)) return rc;
     float* dx = reinterpret_cast<float*>(c->scratch);
-    float* dtg = reinterpret_cast<float*>(c->scratch + off_t);
+    float* dtg = pairs ? nullptr : reinterpret_cast<float*>(c->scratch + off_t);
     if (B) {
         CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
-        CU(cudaMemcpyAsync(dtg, target, bytes, cudaMemcpyHostToDevice, c->stream));
+        if (!pairs) CU(cudaMemcpyAsync(dtg, target, bytes, cudaMemcpyHostToDevice, c->stream));
     }
     // n_norm = B; an empty set (B = 0) gives a zero loss and a zero gradient
-    if (int rc = physad_deep_data_loss_grad_dev(c, dx, dtg, B, lam, B ? B : 1, c->d_dgrad, c->d_dgrad + 1, c->stream)) return rc;
+    if (int rc = deep_fit_dev(c, what, pairs, dx, dtg, B, lam, B ? B : 1, c->d_dgrad, c->d_dgrad + 1, c->stream)) return rc;
     CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 1) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     if (loss) *loss = float(c->h_dgrad[0] / double(B ? B : 1));
@@ -2149,6 +2156,29 @@ int physad_deep_data_loss_grad_host(physad_ctx* c, const float* x, const float* 
         gd += len[k];
     }
     return 0;
+}
+}  // namespace
+extern "C" {
+
+int physad_deep_data_loss_grad_dev(physad_ctx* c, const float* x, const float* target, size_t B, const float* lam,
+                                   size_t n_norm, double* acc, double* grad, void* stream) {
+    return deep_fit_dev(c, "deep_data_loss_grad", false, x, target, B, lam, n_norm, acc, grad, stream);
+}
+
+int physad_deep_data_loss_grad_host(physad_ctx* c, const float* x, const float* target, size_t B, const float* lam,
+                                    float* loss, float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2) {
+    return deep_fit_host(c, "deep_data_loss_grad", false, x, target, B, lam, loss, dW1, db1, dWh, dbh, dW2, db2);
+}
+
+// ---- periodic boundaries at points: the matched-pair loss of deeper networks (deep_data_kernels.cuh) -------------------
+int physad_deep_pair_loss_grad_dev(physad_ctx* c, const float* x, size_t B, const float* lam, size_t n_norm, double* acc,
+                                   double* grad, void* stream) {
+    return deep_fit_dev(c, "deep_pair_loss_grad", true, x, nullptr, B, lam, n_norm, acc, grad, stream);
+}
+
+int physad_deep_pair_loss_grad_host(physad_ctx* c, const float* x, size_t B, const float* lam, float* loss, float* dW1,
+                                    float* db1, float* dWh, float* dbh, float* dW2, float* db2) {
+    return deep_fit_host(c, "deep_pair_loss_grad", true, x, nullptr, B, lam, loss, dW1, db1, dWh, dbh, dW2, db2);
 }
 
 // ---- analytic loss of deeper networks at caller-supplied points (collocation points; deep_tangent_kernels.cuh) ---------

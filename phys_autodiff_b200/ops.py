@@ -390,6 +390,58 @@ class Context:
                                                         *[ptr(a) if a.size else None for a in d]), "deep_data_loss_grad_host")
         return (np.float32(loss.value), *d)
 
+    # -- periodic boundaries at arbitrary points: the matched-pair loss of deeper networks (additive) ---------------------
+    def deep_pair_loss_grad_acc(self, x, lam=None, n_norm=None, out=None):
+        """Device form of the pair loss L_p = (1/n_norm) sum_i sum_o lam[o] (y(p_i)_o - y(q_i)_o)^2 of the deep network: x a
+        float32 CUDA tensor [B, 2, 4] of pairs (p_i, q_i) of network inputs (x, y, z, t), already normalised (for periodicity
+        along axis a: q = p + grid_periods(g, norm)[a] e_a).  Returns a float64 device tensor [acc, grad(P)] with acc the
+        un-normalised weighted sum (each pair once) and grad = dW1 | db1 | dWh | dbh | dW2 | db2 scaled by 2 lam[o] / n_norm,
+        so the tensors of shards with the same n_norm add up and grad adds to the data and physics gradients.  lam None: 1/4
+        each; n_norm None: B (1 for an empty shard)."""
+        import torch
+        x = x.contiguous()
+        B = x.numel() // 8
+        assert x.numel() == 8 * B
+        out = out if out is not None else self._empty(self.deep_grad_len() + 1, torch.float64)
+        n = max(B, 1) if n_norm is None else int(n_norm)
+        check(self._lib.physad_deep_pair_loss_grad_dev(self._h, ptr(x), C.c_size_t(B), self._lam(lam), C.c_size_t(n), ptr(out),
+                                                       ptr(out[1:]), self._stream()), "deep_pair_loss_grad")
+        return out
+
+    def deep_pair_loss_grad(self, x, lam=None, n_global=None, group=None):
+        """(L_p, grad float64 ndarray[P]) of the pair loss over the pairs of every rank.  With torch.distributed initialised
+        each rank passes its own pairs; n_global (default: the sum of B over ranks, one all-reduce of one integer)
+        normalises, and ONE all-reduce of P+1 doubles combines the ranks."""
+        import torch
+        import torch.distributed as dist
+        world = dist.get_world_size(group) if dist.is_initialized() else 1
+        B = x.numel() // 8
+        if n_global is None:
+            if world > 1:
+                nb = torch.tensor([B], dtype=torch.int64, device=x.device)
+                dist.all_reduce(nb, op=dist.ReduceOp.SUM, group=group)
+                n_global = int(nb.item())
+            else:
+                n_global = B
+        n_global = max(int(n_global), 1)
+        buf = self.deep_pair_loss_grad_acc(x, lam, n_global)
+        if world > 1:
+            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+        h = buf.cpu().numpy()
+        return float(h[0] / n_global), h[1:].copy()
+
+    def deep_pair_loss_grad_host(self, x, lam=None):
+        """Host-array form with n_norm = B: x [B, 2, 4] -> (L_p, dW1, db1, dWh, dbh, dW2, db2), float32."""
+        x = _f32(x)
+        B = x.size // 8
+        assert x.size == 8 * B
+        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
+        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        loss = C.c_float()
+        check(self._lib.physad_deep_pair_loss_grad_host(self._h, ptr(x), C.c_size_t(B), self._lam(lam), C.byref(loss),
+                                                        *[ptr(a) if a.size else None for a in d]), "deep_pair_loss_grad_host")
+        return (np.float32(loss.value), *d)
+
     # -- analytic loss of deeper networks at arbitrary points (collocation points; additive) -------------------------------
     @staticmethod
     def _dcdx(dcdx):
@@ -885,6 +937,15 @@ def grid_input_scales(g: Grid, norm) -> np.ndarray:
     return out
 
 
+def grid_periods(g: Grid, norm) -> np.ndarray:
+    """The period of each space axis in network coordinates (float32 [3]): T = f n / (n - 1), f = 2 for MinusOneToOne (norm
+    1 / True) and 1 for ZeroToOne (0 / False), computed in double and rounded once; 0 for an extent of 1.  It is the
+    coordinate offset of the virtual index n, which the grid's periodic stencil identifies with index 0, so a point p on
+    the face and p + T e_a are the two ends of one period.  Host-only, no GPU."""
+    f = 2.0 if int(norm) == 1 else 1.0
+    return np.array([f * n / (n - 1) if n > 1 else 0.0 for n in (g.nx, g.ny, g.nz)], np.float32)
+
+
 # ---- reference-named host functions (one shared context, like the C++ layer) -----------------------
 _CTX: Optional[Context] = None
 
@@ -996,6 +1057,14 @@ def mlp_data_loss_deep_grad_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, targe
     c = default_context()
     c.set_weights_deep(cfg, L, *w)
     return c.deep_data_loss_grad_host(x, target, lam)
+
+
+def mlp_pair_loss_deep_grad_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, lam=None):
+    """Pair loss of a deep network and its gradient (additive): w = (W1, b1, Wh, bh, W2, b2), x [B, 2, 4] pairs ->
+    (L_p, dW1, db1, dWh, dbh, dW2, db2), L_p = mean over the pairs of sum_o lam[o] (y(p)_o - y(q)_o)^2 (lam None: 1/4 each)."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.deep_pair_loss_grad_host(x, lam)
 
 
 def mlp_phys_loss_deep_tangent_points_grad_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, dcdx, pw: PhysWeights):

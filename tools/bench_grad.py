@@ -15,7 +15,11 @@ pair and B, and with --out the whole run as one JSON document with the GPU's nam
 (physad_deep_tangent_points_loss_dev) and its loss + gradient step (physad_deep_tangent_points_loss_grad_dev) at B = n^3
 and B = n^2, in alternation with the grid's analytic loss and loss + gradient step at n^3 (physad_deep_tangent_loss_dev /
 _grad_dev); one JSON line per pair and B, and with --out the whole run as one JSON document.
-  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent|deep-data|deep-tangent-points] [--n 256] [--hidden 64]
+--loss deep-pair times the periodic-pair loss + gradient step (physad_deep_pair_loss_grad_dev) at B = 2^23 and 32 768 pairs
+for every --hidden x --layers pair, in alternation with the data loss + gradient step at the same 2B rows and with the
+composition a caller could write without it (two forwards at points and two data steps of B points, each point's target
+its partner's output); one JSON line per pair and B, and with --out the whole run as one JSON document.
+  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent|deep-data|deep-tangent-points|deep-pair] [--n 256] [--hidden 64]
                              [--layers 3] [--steps 20]
   python tools/bench_grad.py --loss deep --hidden 32,64,128 --layers 2,3,5
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/bench_grad.py   (z-slab per rank)"""
@@ -37,9 +41,13 @@ def main():
     ap.add_argument("--hidden", default="64", help="width; --loss deep takes a comma-separated list")
     ap.add_argument("--layers", default="3", help="--loss deep: hidden layers, a comma-separated list")
     ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent", "deep-data", "deep-tangent-points"), default="fd")
-    ap.add_argument("--out", default=None, help="--loss deep-data / deep-tangent-points: also write the run as one JSON document here")
+    ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent", "deep-data", "deep-tangent-points", "deep-pair"),
+                    default="fd")
+    ap.add_argument("--out", default=None,
+                    help="--loss deep-data / deep-tangent-points / deep-pair: also write the run as one JSON document here")
     a = ap.parse_args()
+    if a.loss == "deep-pair":
+        return deep_pair(a)
     if a.loss == "deep-tangent-points":
         return deep_tangent_points(a, Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True))
     if a.loss == "deep-data":
@@ -336,6 +344,75 @@ def deep_data(a, g):
                                f"gradient step at the same B points and the finite-difference deep step on the grid, timed in "
                                f"alternation (CUDA events, median of {a.steps}); B = {sizes[0]} and {sizes[1]}",
                        "gpu": name, "power_limit_w": plim, "clocks_max_sm_mhz": clk, "results": results}, fh, indent=1)
+
+
+def deep_pair(a):
+    import numpy as np
+    ctx = ops.Context()
+    name, plim = _gpu()
+    rng = np.random.default_rng(5)
+    sizes = (1 << 23, 32768)   # pairs: 2^24 rows (well past L2), and the overhead regime
+    # pairs across the x faces of a periodic domain: p uniform with p_x = -1, q = p + T e_x (T of a 256-point axis)
+    T = float(ops.grid_periods(Grid(256, 256, 256), True)[0])
+    xs = {}
+    for B in sizes:
+        x = rng.uniform(-1, 1, (B, 2, 4)).astype(np.float32)
+        x[:, 0, 0] = -1.0
+        x[:, 1] = x[:, 0]
+        x[:, 1, 0] += np.float32(T)
+        xs[B] = torch.from_numpy(x).cuda()
+    results = []
+    for H in (int(v) for v in a.hidden.split(",")):
+        w1 = ops.mlp_random_init(H, 777, 0.25)
+        for L in (int(v) for v in a.layers.split(",")):
+            wr = np.random.default_rng(L)
+            Wh = wr.uniform(-0.2, 0.2, (L - 1) * H * H).astype(np.float32)
+            bh = wr.uniform(-0.2, 0.2, (L - 1) * H).astype(np.float32)
+            ctx.set_weights_deep(MLPConfig(4, H, 4, True), L, w1[0], w1[1], Wh, bh, w1[2], w1[3])
+            for B in sizes:
+                x = xs[B]
+                rows = x.view(2 * B, 4)
+                p, q = x[:, 0].contiguous(), x[:, 1].contiguous()
+                pout = ctx.deep_pair_loss_grad_acc(x)
+                dout = ctx.deep_data_loss_grad_acc(rows, rows)
+                cout = [ctx.deep_data_loss_grad_acc(p, p, n_norm=B) for _ in range(2)]
+                yp, yq = ctx.mlp_forward_deep(p), ctx.mlp_forward_deep(q)
+
+                def compose():
+                    assert ctx._lib.physad_mlp_forward_deep_dev(ctx._h, ops.ptr(p), ops.ptr(yp), C.c_size_t(B), ctx._stream()) == 0
+                    assert ctx._lib.physad_mlp_forward_deep_dev(ctx._h, ops.ptr(q), ops.ptr(yq), C.c_size_t(B), ctx._stream()) == 0
+                    ctx.deep_data_loss_grad_acc(p, yq, n_norm=B, out=cout[0])
+                    ctx.deep_data_loss_grad_acc(q, yp, n_norm=B, out=cout[1])
+                calls = {"pair_loss_grad": lambda: ctx.deep_pair_loss_grad_acc(x, out=pout),
+                         "data_loss_grad_2B": lambda: ctx.deep_data_loss_grad_acc(rows, rows, out=dout),
+                         "composition": compose}
+                for _ in range(2):
+                    for fn in calls.values():
+                        fn()
+                torch.cuda.synchronize()
+                ts = {k: [] for k in calls}
+                for _ in range(a.steps):   # in alternation, so that they share whatever else the GPU is doing
+                    for k, fn in calls.items():
+                        ts[k] += _times(fn, 1)
+                med = {k: sorted(v)[len(v) // 2] for k, v in ts.items()}
+                hp, hc = pout.cpu().numpy(), (cout[0] + cout[1]).cpu().numpy()
+                r = {"workload": f"H={H} L={L} B={B} pairs: pair loss+grad vs data loss+grad at 2B rows vs composition",
+                     "pairs": B, "rows": 2 * B, **{k + "_ms": v for k, v in med.items()},
+                     "pair_to_data_ratio": med["pair_loss_grad"] / med["data_loss_grad_2B"],
+                     "pair_to_composition_ratio": med["pair_loss_grad"] / med["composition"],
+                     "pair_gpts_per_s": 2 * B / med["pair_loss_grad"] / 1e6,
+                     "grad_maxdiff_vs_composition": float(abs(hp[1:] - hc[1:]).max() / abs(hc[1:]).max()),
+                     "db2": [float(v) for v in hp[-4:]], "acc": float(hp[0]), "gpu": name, "power_limit_w": plim}
+                results.append(r)
+                print(json.dumps(r), flush=True)
+    if a.out:
+        with open(a.out, "w") as fh:
+            json.dump({"what": f"tools/bench_grad.py --loss deep-pair --hidden {a.hidden} --layers {a.layers} --steps {a.steps}: "
+                               f"the pair loss + gradient step at B pairs (p on the x = -1 face, q one period on), the data loss + "
+                               f"gradient step at the same 2B rows, and two forwards at points + two data steps of B points "
+                               f"(the composition), timed in alternation (CUDA events, median of {a.steps}); B = {sizes[0]} "
+                               f"and {sizes[1]}",
+                       "gpu": name, "power_limit_w": plim, "results": results}, fh, indent=1)
 
 
 def deep_tangent_points(a, g):
