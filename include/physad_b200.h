@@ -44,7 +44,14 @@ enum {
     PHYSAD_E_PEER_TIMEOUT = -4 /* in-kernel multi-GPU exchange: a peer rank never arrived */
 };
 
-/* phys::GridSpec, include/phys.h:8-13 (bool widened to int for C). */
+/* phys::GridSpec, include/phys.h:8-13 (bool widened to int for C).
+ * Limits: every call refuses a grid of N = nx*ny*nz >= 2^31 points with PHYSAD_E_UNSUPPORTED (the reference indexes with
+ * int).  Below that, the launch geometry adds these, each refused with PHYSAD_E_UNSUPPORTED before anything is written:
+ *   - MLP over the grid (mlp_grid_infer, generate_fields and its _lp form, with one hidden layer also the _deep forms, and
+ *     the fields of fused_loss_grad*): ny <= 2097120.  Any nz: more than 65535 planes go out in several launches.
+ *   - physics on supplied fields (phys_residuals, phys_loss*, phys_backward_from_fields, the forward of
+ *     fused_loss_grad* and deep_loss_host): ny <= 524280; with 16-bit fields (phys_loss_lp) ny <= 131070.
+ *     Any nz. */
 typedef struct physad_grid {
     int nx, ny, nz;
     float hx, hy, hz;

@@ -438,17 +438,37 @@ int launch_grid_t(physad_ctx* c, const physad_grid* g, const physad_slab& s, con
                   cudaStream_t st, int dtype = PHYSAD_F32) {
     const int nzl = s.z_end - s.z_begin;
     if (nzl == 0) return 0;
-    if (nzl > 65535) return fail(PHYSAD_E_UNSUPPORTED, "grid MLP kernels: more than 65535 planes per call");
+    // a block covers 32 rows: gridDim.y caps ny at 65535 * 32
+    if ((g->ny + 31) / 32 > 65535) return fail(PHYSAD_E_UNSUPPORTED, "grid MLP kernels: ny > 2097120");
     if (int rc = ensure_coord_tables(c, g, st)) return rc;
     a.cxs = c->tab.dev; a.cys = a.cxs + g->nx; a.czs = a.cys + g->ny;
     MlpConst<H> k;
     fill_const<H>(c, tc, k);
-    const dim3 grid(unsigned((g->nx + 31) / 32), unsigned((g->ny + 31) / 32), unsigned(nzl));
-    if (FIELDS && dtype == PHYSAD_F16) k_mlp_grid<H, FIELDS, 2, __half><<<grid, 256, 0, st>>>(k, a);
-    else if (FIELDS && dtype == PHYSAD_BF16) k_mlp_grid<H, FIELDS, 2, __nv_bfloat16><<<grid, 256, 0, st>>>(k, a);
-    else k_mlp_grid<H, FIELDS, 2><<<grid, 256, 0, st>>>(k, a);
-    c->launches++;
-    CU(cudaGetLastError());
+    // one plane per blockIdx.z, so more than 65535 planes go out in bands; the kernel indexes its outputs from the
+    // band's first plane, and the u arrays keep the channel stride of the whole slab
+    const size_t pln = size_t(g->nx) * g->ny;
+    const size_t esz = (FIELDS && dtype != PHYSAD_F32) ? 2 : sizeof(float);   // bytes per stored field element
+    if (a.cstride == 0) a.cstride = size_t(nzl) * pln;
+    for (int z0 = s.z_begin; z0 < s.z_end; z0 += 65535) {
+        const int nb = std::min(65535, s.z_end - z0);
+        const size_t off = size_t(z0 - s.z_begin) * pln;
+        GridInferArgs b = a;
+        b.z_begin = z0; b.z_end = z0 + nb;
+        if (FIELDS) {
+            for (int q = 0; q < 3; ++q) {
+                b.sigma[q] = reinterpret_cast<float*>(reinterpret_cast<char*>(a.sigma[q]) + off * esz);
+                b.u[q] = reinterpret_cast<float*>(reinterpret_cast<char*>(a.u[q]) + off * esz);
+            }
+        } else {
+            b.out_aos = a.out_aos + off;
+        }
+        const dim3 grid(unsigned((g->nx + 31) / 32), unsigned((g->ny + 31) / 32), unsigned(nb));
+        if (FIELDS && dtype == PHYSAD_F16) k_mlp_grid<H, FIELDS, 2, __half><<<grid, 256, 0, st>>>(k, b);
+        else if (FIELDS && dtype == PHYSAD_BF16) k_mlp_grid<H, FIELDS, 2, __nv_bfloat16><<<grid, 256, 0, st>>>(k, b);
+        else k_mlp_grid<H, FIELDS, 2><<<grid, 256, 0, st>>>(k, b);
+        c->launches++;
+        CU(cudaGetLastError());
+    }
     return 0;
 }
 
@@ -489,11 +509,14 @@ int launch_phys(physad_ctx* c, const physad_grid* g_in, PhysArgs a, cudaStream_t
     const void* ptrs[12] = {a.s_m, a.s_0, a.s_p, a.u_m, a.u_0, a.u_p, a.R[0], a.R[1], a.R[2], a.R[3], a.halo_lo, a.halo_hi};
     for (int k = 0; k < 12; ++k) v4 = v4 && (uintptr_t(ptrs[k]) % ((dtype != PHYSAD_F32 && (k < 6 || k >= 10)) ? 8 : 16) == 0);
     v4 = v4 && (size_t(g->nx) * g->ny * g->nz) % 4 == 0;  // channel stride of the u arrays
+    // the v4 grid has one block row per 2 rows (gridDim.y <= 65535): fp32 fields beyond that take the scalar kernel
+    const bool v4_rows = (g->ny + V4_THREADS / 64 - 1) / (V4_THREADS / 64) <= 65535;
+    if (dtype == PHYSAD_F32) v4 = v4 && v4_rows;
     if (dtype != PHYSAD_F32 && (!v4 || SCALE || c->exact_residuals))
         return fail(PHYSAD_E_UNSUPPORTED, "16-bit fields: need nx % 4 == 0, 8-byte aligned arrays, the central scheme and fp32 residual arithmetic");
     if (v4) {
         const unsigned tx = unsigned((g->nx + 255) / 256), ty = unsigned((g->ny + V4_THREADS / 64 - 1) / (V4_THREADS / 64));
-        if (ty > 65535u) return fail(PHYSAD_E_UNSUPPORTED, "phys kernels: ny > 131070");
+        if (ty > 65535u) return fail(PHYSAD_E_UNSUPPORTED, "phys kernels: 16-bit fields need ny <= 131070");
         const long long want = (long long)c->sm_count * 8;
         long long nch = std::max(1LL, std::min<long long>(g->nz, (want + (long long)tx * ty - 1) / ((long long)tx * ty)));
         a.zc = int((g->nz + nch - 1) / nch);
