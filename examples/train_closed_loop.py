@@ -2,7 +2,7 @@
 REQUIREMENT.md:155-169), on 1..N GPUs:
 
   python examples/train_closed_loop.py [--loss fd|tangent] [--layers 1] [--data 0] [--colloc 0] [--periodic 0]
-                                      [--t-range 0,0.5] [--n 128] [--hidden 64] [--steps 200]
+                                      [--neumann 0] [--t-range 0,0.5] [--n 128] [--hidden 64] [--steps 200]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 examples/train_closed_loop.py
 
 Every rank differentiates its z-slab of the grid (physad_fused_loss_grad_slab_dev), one all-reduce of 9H+6 doubles
@@ -22,8 +22,14 @@ initial condition (the teacher at t = 0) and the dynamics that carry it over [T0
 the periodic boundary condition of the grid's domain, which the analytic loss has no stencil to impose: N pairs drawn fresh
 every step on the device, a third per space axis a, p on the face p_a = -1 (the other two space inputs uniform in [-1, 1],
 the time input in [T0, T1]) and q = p + T_a e_a one period on (ops.grid_periods), fitted with the pair loss
-(physad_deep_pair_loss_grad_dev, lam = 1/4 each, mean over all N pairs, one all-reduce of P+1 doubles).  Prints one JSON
-line per 20 steps and a summary."""
+(physad_deep_pair_loss_grad_dev, lam = 1/4 each, mean over all N pairs, one all-reduce of P+1 doubles).  --neumann M (with
+--colloc, not with --periodic) makes the domain clamped instead: the grid is non-periodic, and the condition its clamped
+stencil states, a zero normal derivative at the faces, is fitted at M face points drawn fresh every step on the device, a
+third per space axis a alternating the faces c_a = -1 and +1 (the other space inputs uniform in [-1, 1], the time input in
+[T0, T1]), with the derivative-fit loss (physad_deep_deriv_loss_grad_dev, direction dc_a/dx_a e_a, target 0, lam = 1/4
+each, mean over all M points, one all-reduce of P+1 doubles).  The summary then reports the final mean squared normal
+derivative at 4 096 fixed held-out face points (physad_mlp_jacobian_deep_dev).  Prints one JSON line per 20 steps and a
+summary."""
 import argparse
 import json
 import os
@@ -50,6 +56,8 @@ def main():
                     help="collocation points per step for the physics term instead of the grid at t = 0.25 (needs --layers > 1)")
     ap.add_argument("--periodic", type=int, default=0,
                     help="pairs per step for the periodic boundary condition of the grid's domain (needs --colloc)")
+    ap.add_argument("--neumann", type=int, default=0,
+                    help="face points per step for a zero normal derivative on a clamped domain (needs --colloc)")
     ap.add_argument("--t-range", default="0,0.5", help="T0,T1: the time interval the collocation points cover")
     a = ap.parse_args()
     if a.data and a.layers < 2:
@@ -58,6 +66,10 @@ def main():
         ap.error("--colloc needs --layers > 1")
     if a.periodic and not a.colloc:
         ap.error("--periodic needs --colloc")
+    if a.neumann and not a.colloc:
+        ap.error("--neumann needs --colloc")
+    if a.neumann and a.periodic:
+        ap.error("--neumann and --periodic exclude each other: a domain is either periodic or clamped")
     t0c, t1c = (float(v) for v in a.t_range.split(","))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank, local = int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0"))
@@ -66,7 +78,7 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     H = a.hidden
-    g = Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, True)
+    g = Grid(a.n, a.n, a.n, 1, 1, 1, 2e-3, not a.neumann)
     cfg, pw = MLPConfig(4, H, 4, True), PhysWeights(1, 1)
     ctx = ops.Context(local)
     W1, b1, W2, b2 = ops.mlp_random_init(H, 777, 0.25)
@@ -105,6 +117,18 @@ def main():
         period = torch.from_numpy(ops.grid_periods(g, cfg.minus_one_to_one)).cuda()
         rows = torch.arange(hi_p - lo_p, device="cuda")
         axis = (rows + lo_p) % 3
+    if a.neumann:
+        # this rank's share of the M face points per step: point i on face c_a = -1 or +1 (alternating) of axis a = i % 3,
+        # direction dc_a/dx_a e_a (the physical normal derivative), target 0
+        lo_n, hi_n = (rank * a.neumann) // world, ((rank + 1) * a.neumann) // world
+        ngen = torch.Generator(device="cuda")
+        ngen.manual_seed(3000 + rank)
+        idx = torch.arange(lo_n, hi_n, device="cuda")
+        nrows, naxis = idx - lo_n, idx % 3
+        nface = torch.where((idx // 3) % 2 == 0, -1.0, 1.0).to(torch.float32)
+        ndir = torch.zeros((hi_n - lo_n, 4), device="cuda")
+        ndir[nrows, naxis] = torch.from_numpy(dcdx).cuda()[naxis]
+        nzero = torch.zeros_like(ndir)
     m, v = np.zeros_like(th), np.zeros_like(th)
     first = last = None
     t0 = time.perf_counter()
@@ -134,11 +158,17 @@ def main():
             q[rows, axis] += period[axis]
             lp, gp = ctx.deep_pair_loss_grad(torch.stack([p, q], 1), n_global=a.periodic)
             grad = grad + gp
+        ln = None
+        if a.neumann:   # the network set above
+            xn = lo4 + span4 * torch.rand((hi_n - lo_n, 4), generator=ngen, device="cuda")
+            xn[nrows, naxis] = nface
+            ln, gn = ctx.deep_deriv_loss_grad(xn, ndir, nzero, n_global=a.neumann)
+            grad = grad + gn
         ld = None
         if a.data:   # the network set above; all ranks' points, one all-reduce of P+1 doubles
             ld, gd = ctx.deep_data_loss_grad(xd, yd, n_global=a.data)
             grad = grad + gd
-        last = float(ls) + float(lu) + (ld or 0.0) + (lp or 0.0)
+        last = float(ls) + float(lu) + (ld or 0.0) + (lp or 0.0) + (ln or 0.0)
         first = last if first is None else first
         m = 0.9 * m + 0.1 * grad
         v = 0.999 * v + 0.001 * grad * grad
@@ -149,19 +179,36 @@ def main():
                 rec["loss_data"] = ld
             if lp is not None:
                 rec["loss_periodic"] = lp
+            if ln is not None:
+                rec["loss_neumann"] = ln
             print(json.dumps(rec), flush=True)
     dt = time.perf_counter() - t0
+    held_dn2 = None
+    if a.neumann and rank == 0:
+        # the final network's mean squared normal derivative (over points and outputs) at 4 096 fixed face points
+        hrng = np.random.default_rng(5)
+        hx = hrng.uniform(-1, 1, (4096, 4)).astype(np.float32)
+        hx[:, 3] = hrng.uniform(t0c, t1c, 4096).astype(np.float32)
+        hax = np.arange(4096) % 3
+        hx[np.arange(4096), hax] = np.where((np.arange(4096) // 3) % 2 == 0, -1.0, 1.0)
+        ctx.set_weights_deep(cfg, L, *np.split(th.astype(np.float32), cuts))
+        _, J = ctx.mlp_jacobian_deep(torch.from_numpy(hx).cuda())
+        dn = J.cpu().numpy().astype(np.float64)[np.arange(4096), :, hax] * dcdx.astype(np.float64)[hax][:, None]
+        held_dn2 = float(np.mean(dn * dn))
     if rank == 0:
         data = f" + data at {a.data} points" if a.data else ""
         summary = f"{a.n}^3 H={H} L={L} {a.loss} loss{data} on {world} GPU(s)"
         if a.colloc:
             what = " (initial condition + dynamics)" if a.data else ""
             what += f" + periodic boundaries at {a.periodic} pairs per step" if a.periodic else ""
+            what += f" + Neumann boundaries at {a.neumann} face points per step" if a.neumann else ""
             summary = (f"H={H} L={L} analytic loss at {a.colloc} collocation points per step over t in [{t0c:g}, {t1c:g}] of the "
                        f"{a.n}^3 domain{data}{what} on {world} GPU(s)")
-        print(json.dumps({"summary": summary, "steps": a.steps, "loss_first": first,
-                          "loss_last": last, "reduction_pct": 100 * (1 - last / first),
-                          "wall_ms_per_step_incl_host_adam": 1e3 * dt / a.steps}))
+        out = {"summary": summary, "steps": a.steps, "loss_first": first, "loss_last": last,
+               "reduction_pct": 100 * (1 - last / first), "wall_ms_per_step_incl_host_adam": 1e3 * dt / a.steps}
+        if held_dn2 is not None:
+            out["heldout_mean_sq_normal_derivative"] = held_dn2
+        print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
 

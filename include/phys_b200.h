@@ -89,6 +89,20 @@ void mlp_data_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights
 void mlp_pair_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, std::size_t B,
                                   const float* lam, float* out_loss, DeepMLPWeights& grad);
 
+// The Jacobian of a deep network at arbitrary points: x holds B host points of 4 floats (network inputs, already
+// normalised); y[B][4] gets the outputs (mlp_infer_deep_cuda's bit for bit) and J[B][4][4] the derivatives
+// J[i][o][k] = dy_o / dc_k, formed exactly by forward-mode tangent rows.  B = 0 writes nothing.
+void mlp_jacobian_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, std::size_t B, float* y,
+                            float* J);
+
+// Derivative-fit loss of a deep network and its gradient with respect to every layer's weights (Neumann boundaries at
+// points): x, dir and target hold B host rows of 4 floats; D_io = sum_k dir[i][k] J[i][o][k] and
+// *out_loss = (1/B) sum_i sum_o lam[o] (D_io - target[i][o])^2 (lam as in mlp_data_loss_deep_grad_cuda).  For a zero
+// normal derivative along space axis a, dir = dcdx[a] e_a and target = 0.  `grad` is resized to the shapes of `w` and
+// adds directly to the data, pair and physics gradients; its b2 part is exactly zero.  B = 0 gives zeros.
+void mlp_deriv_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* dir,
+                                   const float* target, std::size_t B, const float* lam, float* out_loss, DeepMLPWeights& grad);
+
 // The analytic loss of a deep network at arbitrary space-time points (collocation points) instead of the grid at one time:
 // x holds B host points of 4 floats (x, y, z, t), the network inputs already normalised (the fourth is the grid's time input:
 // t for MinusOneToOne, t + 0.5 for ZeroToOne); dcdx the 3 dc/dx of the space inputs (physad_grid_input_scales gives the

@@ -141,8 +141,8 @@ int physad_mlp_generate_fields_host(physad_ctx* ctx, const physad_grid* g, float
  * nothing; the host forms that take new weights (cfg != NULL) replace the network first and run.  Use the *_deep_* and
  * deep_* counterparts: physad_mlp_forward_deep_* for physad_mlp_forward_*, physad_deep_data_loss_grad_* for
  * physad_mlp_backward_*, physad_mlp_grid_infer_deep_dev, physad_mlp_generate_fields_deep_dev, physad_deep_loss_host,
- * physad_deep_loss_grad_*, physad_deep_tangent_loss_* and, at arbitrary points, physad_deep_tangent_points_loss_* and
- * physad_deep_pair_loss_grad_*.
+ * physad_deep_loss_grad_*, physad_deep_tangent_loss_* and, at arbitrary points, physad_deep_tangent_points_loss_*,
+ * physad_deep_pair_loss_grad_*, physad_mlp_jacobian_deep_* and physad_deep_deriv_loss_grad_*.
  * hidden_layers == 1 is accepted everywhere.  A refused call leaves the previous network in place.
  * A later physad_set_weights() switches the context back to a one-hidden-layer network. */
 int physad_set_weights_deep(physad_ctx* ctx, const physad_mlp_config* cfg, int hidden_layers, const float* W1,
@@ -470,6 +470,42 @@ int physad_deep_pair_loss_grad_dev(physad_ctx* ctx, const float* x, size_t B, co
                                    double* acc, double* grad, void* stream);
 int physad_deep_pair_loss_grad_host(physad_ctx* ctx, const float* x, size_t B, const float* lam, float* loss,
                                     float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2);
+
+/* ---- Neumann boundaries at arbitrary points: the Jacobian of deeper networks and a derivative-fit loss (ADDITIVE, no
+ * reference counterpart).  Both take the network set by physad_set_weights_deep (any hidden_layers >= 1, deep mode 0) and
+ * network inputs x[B][4] = (c_x, c_y, c_z, c_t), already normalised as for physad_deep_tangent_points_loss_dev; d/dc_t is
+ * with respect to the time input itself.
+ * physad_mlp_jacobian_deep_dev: y[B][4] and J[B][4][4], J[i][o][k] = dy_o / dc_k at x_i; DEVICE pointers, 16-byte
+ *   aligned.  y is physad_mlp_forward_deep_dev's output bit for bit; J is formed by forward-mode tangent rows (scalar
+ *   fma.rn from +0, inputs ascending, then J = W2 a_dot by fma.rn from +0, h ascending).  Exact at any point, unlike
+ *   finite differences of the forward near a ReLU kink.  B = 0 writes nothing.
+ * physad_mlp_jacobian_deep_host: the same with host arrays.
+ * physad_deep_deriv_loss_grad_dev: the loss
+ *   L_g = (1/n_norm) sum_i sum_o lam[o] (D_io - g_io)^2,   D_io = sum_k d_ik J[i][o][k],
+ *   with d_i = dir[i] a direction in network coordinates and g_i = target[i] (both [B][4] DEVICE floats, 16-byte aligned,
+ *   like x).  For the normal derivative along space axis a, pass d = dcdx[a] e_a (physad_grid_input_scales); for a
+ *   homogeneous Neumann condition dy/dn = 0 (the clamped grid's edge rule, ghost f[-1] = f[0]), pass zero targets.
+ *   lam: 4 HOST floats (finite, >= 0) or NULL for 1/4 each.  In fp32: D_o = ((d_x J[o][0] + d_y J[o][1]) + d_z J[o][2])
+ *   + d_t J[o][3] with every product and sum rounded, e_o = D_o - g_o, seeds y_bar = 0 and
+ *   J_bar[o][k] = (fp32(2 lam[o] / n_norm) * e_o) * d_k.
+ *   acc = 1 device double, the un-normalised sum_i sum_o lam[o] (D_io - g_io)^2 (in double from the fp32 D and g); grad =
+ *   P = physad_deep_grad_len(H, L) device doubles in the layout of physad_deep_loss_grad_dev, already scaled: with n_norm =
+ *   the points of ALL shards, the shards' acc and grad add up under one all-reduce(sum), and grad adds directly to the
+ *   data, pair and physics gradients.  db2 is exactly +0 (every value-row seed is zero).  B = 0 (an empty shard) writes
+ *   acc = 0 and a zero gradient.  Bitwise repeatable.  The same checkpoint and partials scratch as
+ *   physad_deep_tangent_points_loss_grad_dev.
+ * physad_deep_deriv_loss_grad_host: host arrays, n_norm = B; loss = L_g as float, the gradient split into the six arrays of
+ *   physad_set_weights_deep's layouts (any output pointer may be null); B = 0 gives zeros.
+ * Errors: no deep weights (or a physad_set_weights after them): PHYSAD_E_NOWEIGHTS; physad_set_deep_mode(1):
+ * PHYSAD_E_UNSUPPORTED; n_norm == 0, a negative or non-finite lam, a null or misaligned x, dir, target, y or J with B > 0,
+ * a null or misaligned (8 bytes) acc or grad: PHYSAD_E_INVALID.  A refused call writes nothing. */
+int physad_mlp_jacobian_deep_dev(physad_ctx* ctx, const float* x, float* y, float* J, size_t B, void* stream);
+int physad_mlp_jacobian_deep_host(physad_ctx* ctx, const float* x, float* y, float* J, size_t B);
+int physad_deep_deriv_loss_grad_dev(physad_ctx* ctx, const float* x, const float* dir, const float* target, size_t B,
+                                    const float* lam, size_t n_norm, double* acc, double* grad, void* stream);
+int physad_deep_deriv_loss_grad_host(physad_ctx* ctx, const float* x, const float* dir, const float* target, size_t B,
+                                     const float* lam, float* loss, float* dW1, float* db1, float* dWh, float* dbh,
+                                     float* dW2, float* db2);
 
 /* ---- analytic loss of deeper networks at arbitrary points (ADDITIVE, no reference counterpart) ---------------------------
  * The physics loss of physad_deep_tangent_loss_* at caller-supplied collocation points (x, y, z, t) spread over the whole

@@ -101,6 +101,8 @@ EXPORTS = [
     "physad_deep_data_loss_grad_host", "physad_grid_input_scales", "physad_deep_tangent_points_loss_dev",
     "physad_deep_tangent_points_loss_grad_dev", "physad_deep_tangent_points_loss_grad_host",
     "physad_deep_pair_loss_grad_dev", "physad_deep_pair_loss_grad_host",
+    "physad_mlp_jacobian_deep_dev", "physad_mlp_jacobian_deep_host", "physad_deep_deriv_loss_grad_dev",
+    "physad_deep_deriv_loss_grad_host",
 ]
 
 

@@ -2080,6 +2080,42 @@ int physad_mlp_forward_deep_host(physad_ctx* c, const float* x, float* y, size_t
 
 }  // extern "C"  (helpers below)
 namespace {
+// lam[4] of the fit losses (data, pair, derivative): NULL gives 1/4 each (the mean over the four outputs); each must be
+// finite and non-negative
+int read_lam(const float* lam, float lw[4], const std::string& what) {
+    for (int o = 0; o < 4; ++o) lw[o] = 0.25f;
+    if (lam) {
+        for (int o = 0; o < 4; ++o) {
+            if (!std::isfinite(lam[o]) || lam[o] < 0.f) return fail(PHYSAD_E_INVALID, what + ": lam must be finite and non-negative");
+            lw[o] = lam[o];
+        }
+    }
+    return 0;
+}
+
+// The host forms of the deep gradients: the context's device result buffer [P + 2] and its pinned host copy ...
+int ensure_host_grad(physad_ctx* c, size_t P) {
+    if (P + 2 <= c->dgrad_cap) return 0;
+    if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
+    if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
+    c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
+    CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
+    CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
+    c->dgrad_cap = P + 2;
+    return 0;
+}
+
+// ... and the gradient gd[P] split into physad_set_weights_deep's six arrays (a null array is skipped)
+void split_deep_grad(const double* gd, int H, int L, float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2) {
+    const size_t nl = size_t(L - 1), hh = size_t(H);
+    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
+    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
+    for (int k = 0; k < 6; ++k) {
+        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
+        gd += len[k];
+    }
+}
+
 // The data loss (B points and their targets) and the pair loss (B pairs = 2B rows of x, no target) share everything but
 // the kernel: the checks, the scratch, the arguments and the reduction.  `what` names the caller in error messages.
 int deep_fit_dev(physad_ctx* c, const char* what, bool pairs, const float* x, const float* target, size_t B, const float* lam,
@@ -2092,14 +2128,8 @@ int deep_fit_dev(physad_ctx* c, const char* what, bool pairs, const float* x, co
         return fail(PHYSAD_E_INVALID, w + (pairs ? ": x must be 16-byte aligned" : ": x and target must be 16-byte aligned"));
     if (uintptr_t(acc) % 8 || uintptr_t(grad) % 8) return fail(PHYSAD_E_INVALID, w + ": acc and grad must be 8-byte aligned");
     if (n_norm == 0) return fail(PHYSAD_E_INVALID, w + ": n_norm must be positive");
-    float lw[4] = {0.25f, 0.25f, 0.25f, 0.25f};   // NULL: the mean over the four outputs
-    if (lam) {
-        for (int o = 0; o < 4; ++o) {
-            if (!std::isfinite(lam[o]) || lam[o] < 0.f)
-                return fail(PHYSAD_E_INVALID, w + ": lam must be finite and non-negative");
-            lw[o] = lam[o];
-        }
-    }
+    float lw[4];
+    if (int rc = read_lam(lam, lw, w)) return rc;
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
     const int H = c->cfg.H, L = c->deep_layers;
@@ -2149,14 +2179,7 @@ int deep_fit_host(physad_ctx* c, const char* what, bool pairs, const float* x, c
     DeviceGuard dg(c->device);
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
-    if (P + 2 > c->dgrad_cap) {
-        if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
-        if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
-        c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
-        CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
-        CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
-        c->dgrad_cap = P + 2;
-    }
+    if (int rc = ensure_host_grad(c, P)) return rc;
     const size_t bytes = B * (pairs ? 8 : 4) * sizeof(float), off_t = (bytes + 255) & ~size_t(255);
     if (int rc = ensure_scratch(c, off_t + (pairs ? 0 : bytes) + 1)) return rc;
     float* dx = reinterpret_cast<float*>(c->scratch);
@@ -2170,14 +2193,7 @@ int deep_fit_host(physad_ctx* c, const char* what, bool pairs, const float* x, c
     CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 1) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     if (loss) *loss = float(c->h_dgrad[0] / double(B ? B : 1));
-    const double* gd = c->h_dgrad + 1;
-    const size_t nl = size_t(L - 1), hh = size_t(H);
-    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
-    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
-    for (int k = 0; k < 6; ++k) {
-        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
-        gd += len[k];
-    }
+    split_deep_grad(c->h_dgrad + 1, H, L, dW1, db1, dWh, dbh, dW2, db2);
     return 0;
 }
 }  // namespace
@@ -2224,15 +2240,45 @@ int colloc_check(const float* x, size_t B, const float* dcdx, const char* what) 
     return 0;
 }
 
-// the kernel arguments of B > 0 points; uploads the context's weights first (that may move the device buffers)
+// the kernel arguments of B > 0 points; uploads the context's weights first (that may move the device buffers).  dcdx
+// null: the derivative calls, which read no space scales
 int colloc_args(physad_ctx* c, const float* x, size_t B, const float* dcdx, DeepTangentArgs& a, cudaStream_t st) {
     if (int rc = upload_weights_if_stale(c, st)) return rc;
     a.hidden_layers = c->deep_layers;
     a.W1 = c->dW1; a.b1 = c->db1; a.W2 = c->dW2; a.b2 = c->db2;
     a.wh = c->d_wh; a.bh = c->d_bh;
-    a.sx = dcdx[0]; a.sy = dcdx[1]; a.sz = dcdx[2];
+    if (dcdx) { a.sx = dcdx[0]; a.sy = dcdx[1]; a.sz = dcdx[2]; }
     a.pts = reinterpret_cast<const float4*>(x);
     a.n_points = (long long)B;
+    return 0;
+}
+
+// The gradient launch at B > 0 points, shared by the physics loss (k_colloc_tangent) and the derivative-fit loss
+// (k_deriv_tangent): one kernel body, so one scratch, L x 80 KB of checkpoint and P + 2 partials per block.  The physics
+// loss returns both sums in acc[2]; the derivative loss one, so its reduction writes {acc, 0} to two doubles after the
+// partials and acc is copied out from there.
+int colloc_grad_launch(physad_ctx* c, bool deriv, DeepTangentArgs& a, double* acc, double* grad, cudaStream_t st) {
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    const int blocks = deep_tangent_blocks(H, a.n_points, c->sm_count);
+    const size_t ck = size_t(blocks) * deep_tangent_ckpt_floats(L);
+    if (ck > c->dckpt_cap) {
+        if (c->dckpt) CU(cudaFree(c->dckpt));
+        c->dckpt = nullptr; c->dckpt_cap = 0;
+        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
+        c->dckpt_cap = ck;
+    }
+    const size_t np = size_t(blocks) * (P + 2);
+    if (int rc = ensure_grad_partials(c, np + (deriv ? 2 : 0))) return rc;
+    a.ckpt = c->dckpt;
+    a.partials = c->gpart;
+    if (deriv) {
+        CU(cudaError_t(deriv_tangent_launch(H, true, a, blocks, c->gpart + np, grad, st)));
+        CU(cudaMemcpyAsync(acc, c->gpart + np, sizeof(double), cudaMemcpyDeviceToDevice, st));
+    } else {
+        CU(cudaError_t(colloc_tangent_launch(H, true, a, blocks, acc, grad, st)));
+    }
+    c->launches += 2;
     return 0;
 }
 }  // namespace
@@ -2288,20 +2334,7 @@ int physad_deep_tangent_points_loss_grad_dev(physad_ctx* c, const float* x, size
     // vjp_scales' formula with n_norm for N: shards with the same n_norm add up to the whole set's gradient
     a.scale_s = 2.f * w->w_sigma / float(n_norm);
     a.scale_u = 2.f * w->w_u / float(n_norm);
-    const int blocks = deep_tangent_blocks(H, (long long)B, c->sm_count);
-    const size_t ck = size_t(blocks) * deep_tangent_ckpt_floats(L);
-    if (ck > c->dckpt_cap) {
-        if (c->dckpt) CU(cudaFree(c->dckpt));
-        c->dckpt = nullptr; c->dckpt_cap = 0;
-        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
-        c->dckpt_cap = ck;
-    }
-    if (int rc = ensure_grad_partials(c, size_t(blocks) * (P + 2))) return rc;
-    a.ckpt = c->dckpt;
-    a.partials = c->gpart;
-    CU(cudaError_t(colloc_tangent_launch(H, true, a, blocks, acc, grad, st)));
-    c->launches += 2;
-    return 0;
+    return colloc_grad_launch(c, false, a, acc, grad, st);
 }
 
 int physad_deep_tangent_points_loss_grad_host(physad_ctx* c, const float* x, size_t B, const float* dcdx,
@@ -2313,14 +2346,7 @@ int physad_deep_tangent_points_loss_grad_host(physad_ctx* c, const float* x, siz
     DeviceGuard dg(c->device);
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
-    if (P + 2 > c->dgrad_cap) {
-        if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
-        if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
-        c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
-        CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
-        CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
-        c->dgrad_cap = P + 2;
-    }
+    if (int rc = ensure_host_grad(c, P)) return rc;
     const size_t bytes = B * 4 * sizeof(float);
     if (int rc = ensure_scratch(c, bytes + 1)) return rc;
     float* dx = reinterpret_cast<float*>(c->scratch);
@@ -2331,14 +2357,103 @@ int physad_deep_tangent_points_loss_grad_host(physad_ctx* c, const float* x, siz
     CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 2) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     physad_finalize_loss(c->h_dgrad, w, n, loss_sigma, loss_u);
-    const double* gd = c->h_dgrad + 2;
-    const size_t nl = size_t(L - 1), hh = size_t(H);
-    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
-    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
-    for (int k = 0; k < 6; ++k) {
-        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
-        gd += len[k];
+    split_deep_grad(c->h_dgrad + 2, H, L, dW1, db1, dWh, dbh, dW2, db2);
+    return 0;
+}
+
+// ---- Neumann boundaries at points: the Jacobian of deeper networks and the derivative-fit loss (deep_tangent_kernels.cuh)
+int physad_mlp_jacobian_deep_dev(physad_ctx* c, const float* x, float* y, float* J, size_t B, void* stream) {
+    if (!c) return fail(PHYSAD_E_INVALID, "mlp_jacobian_deep: null context");
+    if (int rc = deep_points_ready(c, "mlp_jacobian_deep")) return rc;
+    if (B && (!x || !y || !J)) return fail(PHYSAD_E_INVALID, "mlp_jacobian_deep: null argument");
+    if (B && (misaligned16(x) || misaligned16(y) || misaligned16(J)))
+        return fail(PHYSAD_E_INVALID, "mlp_jacobian_deep: x, y and J must be 16-byte aligned");
+    if (B == 0) return 0;
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    DeepTangentArgs a{};
+    if (int rc = colloc_args(c, x, B, nullptr, a, st)) return rc;
+    a.y_pts = reinterpret_cast<float4*>(y);
+    a.J_pts = reinterpret_cast<float4*>(J);
+    const int H = c->cfg.H;
+    CU(cudaError_t(deriv_tangent_launch(H, false, a, deep_tangent_blocks(H, (long long)B, c->sm_count), nullptr, nullptr, st)));
+    c->launches++;
+    return 0;
+}
+
+int physad_mlp_jacobian_deep_host(physad_ctx* c, const float* x, float* y, float* J, size_t B) {
+    if (!c) return fail(PHYSAD_E_INVALID, "mlp_jacobian_deep: null context");
+    if (int rc = deep_points_ready(c, "mlp_jacobian_deep")) return rc;
+    if (B && (!x || !y || !J)) return fail(PHYSAD_E_INVALID, "mlp_jacobian_deep: null argument");
+    if (B == 0) return 0;
+    DeviceGuard dg(c->device);
+    const size_t bytes = B * 4 * sizeof(float), off = (bytes + 255) & ~size_t(255);
+    if (int rc = ensure_scratch(c, 2 * off + 4 * bytes)) return rc;
+    float* dx = reinterpret_cast<float*>(c->scratch);
+    float* dy = reinterpret_cast<float*>(c->scratch + off);
+    float* dJ = reinterpret_cast<float*>(c->scratch + 2 * off);
+    CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
+    if (int rc = physad_mlp_jacobian_deep_dev(c, dx, dy, dJ, B, c->stream)) return rc;
+    CU(cudaMemcpyAsync(y, dy, bytes, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(J, dJ, 4 * bytes, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int physad_deep_deriv_loss_grad_dev(physad_ctx* c, const float* x, const float* dir, const float* target, size_t B,
+                                    const float* lam, size_t n_norm, double* acc, double* grad, void* stream) {
+    const std::string w("deep_deriv_loss_grad");
+    if (!c) return fail(PHYSAD_E_INVALID, w + ": null context");
+    if (int rc = deep_points_ready(c, w.c_str())) return rc;
+    if (!acc || !grad || (B && (!x || !dir || !target))) return fail(PHYSAD_E_INVALID, w + ": null argument");
+    if (B && (misaligned16(x) || misaligned16(dir) || misaligned16(target)))
+        return fail(PHYSAD_E_INVALID, w + ": x, dir and target must be 16-byte aligned");
+    if (uintptr_t(acc) % 8 || uintptr_t(grad) % 8) return fail(PHYSAD_E_INVALID, w + ": acc and grad must be 8-byte aligned");
+    if (n_norm == 0) return fail(PHYSAD_E_INVALID, w + ": n_norm must be positive");
+    float lw[4];
+    if (int rc = read_lam(lam, lw, w)) return rc;
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    if (B == 0) {   // an empty shard: zero sum, zero gradient
+        CU(cudaMemsetAsync(acc, 0, sizeof(double), st));
+        CU(cudaMemsetAsync(grad, 0, deep_grad_len(c->cfg.H, c->deep_layers) * sizeof(double), st));
+        return 0;
     }
+    DeepTangentArgs a{};
+    if (int rc = colloc_args(c, x, B, nullptr, a, st)) return rc;
+    a.dirs = reinterpret_cast<const float4*>(dir);
+    a.targets = reinterpret_cast<const float4*>(target);
+    for (int o = 0; o < 4; ++o) {   // deep_fit_dev's coefficients: shards with the same n_norm add up
+        a.coef[o] = float(2.0 * double(lw[o]) / double(n_norm));
+        a.lam[o] = double(lw[o]);
+    }
+    return colloc_grad_launch(c, true, a, acc, grad, st);
+}
+
+int physad_deep_deriv_loss_grad_host(physad_ctx* c, const float* x, const float* dir, const float* target, size_t B,
+                                     const float* lam, float* loss, float* dW1, float* db1, float* dWh, float* dbh, float* dW2,
+                                     float* db2) {
+    if (!c) return fail(PHYSAD_E_INVALID, "deep_deriv_loss_grad: null context");
+    if (int rc = deep_points_ready(c, "deep_deriv_loss_grad")) return rc;
+    if (B && (!x || !dir || !target)) return fail(PHYSAD_E_INVALID, "deep_deriv_loss_grad: null argument");
+    DeviceGuard dg(c->device);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (int rc = ensure_host_grad(c, P)) return rc;
+    const size_t bytes = B * 4 * sizeof(float), off = (bytes + 255) & ~size_t(255);
+    if (int rc = ensure_scratch(c, 2 * off + bytes + 1)) return rc;
+    float* d[3] = {reinterpret_cast<float*>(c->scratch), reinterpret_cast<float*>(c->scratch + off),
+                   reinterpret_cast<float*>(c->scratch + 2 * off)};
+    const float* h[3] = {x, dir, target};
+    if (B)
+        for (int k = 0; k < 3; ++k) CU(cudaMemcpyAsync(d[k], h[k], bytes, cudaMemcpyHostToDevice, c->stream));
+    // n_norm = B; an empty set (B = 0) gives a zero loss and a zero gradient
+    const size_t n = B ? B : 1;
+    if (int rc = physad_deep_deriv_loss_grad_dev(c, d[0], d[1], d[2], B, lam, n, c->d_dgrad, c->d_dgrad + 1, c->stream)) return rc;
+    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 1) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    if (loss) *loss = float(c->h_dgrad[0] / double(n));
+    split_deep_grad(c->h_dgrad + 1, H, L, dW1, db1, dWh, dbh, dW2, db2);
     return 0;
 }
 

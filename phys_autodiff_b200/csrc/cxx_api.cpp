@@ -472,6 +472,35 @@ void mlp_pair_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights
     if (rc) die("mlp_pair_loss_deep_grad_cuda", rc);
 }
 
+void mlp_jacobian_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, std::size_t B, float* y,
+                            float* J) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    check_deep_shapes(cfg, w, "mlp_jacobian_deep_cuda");
+    physad_ctx* c = ctx();
+    int rc = set_deep(c, cfg, w);
+    if (!rc) rc = physad_mlp_jacobian_deep_host(c, x, y, J, B);
+    if (rc) die("mlp_jacobian_deep_cuda", rc);
+}
+
+void mlp_deriv_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* dir,
+                                   const float* target, std::size_t B, const float* lam, float* out_loss, DeepMLPWeights& grad) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    check_deep_shapes(cfg, w, "mlp_deriv_loss_deep_grad_cuda");
+    physad_ctx* c = ctx();
+    grad.hidden_layers = w.hidden_layers;
+    grad.W1.resize(w.W1.size());
+    grad.b1.resize(w.b1.size());
+    grad.Wh.resize(w.Wh.size());
+    grad.bh.resize(w.bh.size());
+    grad.W2.resize(w.W2.size());
+    grad.b2.resize(w.b2.size());
+    int rc = set_deep(c, cfg, w);
+    if (!rc) rc = physad_deep_deriv_loss_grad_host(c, x, dir, target, B, lam, out_loss, grad.W1.data(), grad.b1.data(),
+                                                   grad.Wh.empty() ? nullptr : grad.Wh.data(),
+                                                   grad.bh.empty() ? nullptr : grad.bh.data(), grad.W2.data(), grad.b2.data());
+    if (rc) die("mlp_deriv_loss_deep_grad_cuda", rc);
+}
+
 void mlp_phys_loss_deep_tangent_points_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
                                             const float* x, std::size_t B, const float dcdx[3], float* out_loss_sigma,
                                             float* out_loss_u, float* opt_R) {

@@ -1,10 +1,15 @@
-// The kernel behind k_deep_tangent (deep_tangent_kernels.cu) and k_colloc_tangent (colloc_tangent_kernels.cu); see
-// deep_tangent_kernels.cuh for what they compute.  The two differ only in where a point's inputs come from.  Each of the
-// two files includes this one once, after defining
+// The kernel behind k_deep_tangent (deep_tangent_kernels.cu), k_colloc_tangent (colloc_tangent_kernels.cu) and
+// k_deriv_tangent (deriv_tangent_kernels.cu); see deep_tangent_kernels.cuh for what they compute.  The first two differ
+// only in where a point's inputs come from, the third from the second only in its last stage.  Each of the three files
+// includes this one once, after defining
 //   DEEP_TANGENT_KERNEL   the kernel's name;
 //   DEEP_TANGENT_POINTS   its row source: false, the slab's grid points in linear order (coordinates from the axis tables,
 //                         one time input a.tc); true, the caller's points a.pts[0 .. a.n_points) (one float4 per point,
 //                         its own time input).
+//   DEEP_TANGENT_DERIV    optional, default false; true (with POINTS) makes k_deriv_tangent (deriv_tangent_kernels.cu):
+//                         only the stage after the output layer differs.  GRAD = false writes y and J of each point
+//                         (a.y_pts, a.J_pts) instead of residuals and sums; GRAD = true reads a.dirs / a.targets and seeds
+//                         the tangent rows with the derivative-fit loss of DESIGN section 4.13 (value-row seeds zero).
 // The body is the kernel itself, not a __device__ function both kernels inline: inlined, it loses the thread-index range
 // that __launch_bounds__ gives the kernel, and k_deep_tangent<128, *> compiles to different code.
 //
@@ -26,6 +31,9 @@
 // No FFMA2 and no tcgen05: the value row keeps k_mlp_deep's FMUL2 / FADD2, everything else is scalar FFMA.
 #if !defined(DEEP_TANGENT_KERNEL) || !defined(DEEP_TANGENT_POINTS)
 #error "define DEEP_TANGENT_KERNEL and DEEP_TANGENT_POINTS before including deep_tangent_body.cuh"
+#endif
+#ifndef DEEP_TANGENT_DERIV
+#define DEEP_TANGENT_DERIV false
 #endif
 #include "deep_tangent_kernels.cuh"
 #include "mlp_eval.cuh"
@@ -79,7 +87,8 @@ __host__ __device__ constexpr size_t grad_len(int H, int L) {
 
 template <int H, bool GRAD>
 __global__ void __launch_bounds__(NT, 1) DEEP_TANGENT_KERNEL(const __grid_constant__ DeepTangentArgs a) {
-    constexpr bool POINTS = DEEP_TANGENT_POINTS;
+    constexpr bool POINTS = DEEP_TANGENT_POINTS, DERIV = DEEP_TANGENT_DERIV;
+    static_assert(POINTS || !DERIV, "the derivative stage reads per-point directions");
     using Q = Geo<H, GRAD>;
     constexpr int G = Q::G, RB = Q::RB, NROW = Q::NROW, PTS_TILE = Q::PTS_TILE, ACT = Q::ACT;
     extern __shared__ __align__(16) float smem[];
@@ -270,7 +279,32 @@ __global__ void __launch_bounds__(NT, 1) DEEP_TANGENT_KERNEL(const __grid_consta
             float4 seed[PT];
 #pragma unroll
             for (int j = 0; j < PT; ++j) seed[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (p < n_slab) {
+            if (DERIV && !GRAD && p < n_slab) {   // the Jacobian query: y and J as they are
+                a.y_pts[p] = make_float4(y[0], y[1], y[2], y[3]);
+#pragma unroll
+                for (int o = 0; o < 4; ++o) a.J_pts[4 * p + o] = make_float4(J[o][0], J[o][1], J[o][2], J[o][3]);
+            }
+            if (DERIV && GRAD && p < n_slab) {
+                // DESIGN section 4.13: D_o = sum_k d_k J[o][k] (products and sums rounded separately, k ascending),
+                // e_o = D_o - g_o;  y_bar = 0,  J_bar[o][k] = (coef_o e_o) d_k;  acc += lam_o (D_o - g_o)^2 in double
+                const float4 d4 = __ldg(a.dirs + p), g4 = __ldg(a.targets + p);
+                const float d[4] = {d4.x, d4.y, d4.z, d4.w}, tg[4] = {g4.x, g4.y, g4.z, g4.w};
+                float Jb[4][4];
+#pragma unroll
+                for (int o = 0; o < 4; ++o) {
+                    const float D = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(d[0], J[o][0]), __fmul_rn(d[1], J[o][1])),
+                                                        __fmul_rn(d[2], J[o][2])),
+                                              __fmul_rn(d[3], J[o][3]));
+                    const float ce = __fmul_rn(a.coef[o], __fsub_rn(D, tg[o]));
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) Jb[o][k] = __fmul_rn(ce, d[k]);
+                    const double dd = double(D) - double(tg[o]);
+                    red[4] += a.lam[o] * (dd * dd);
+                }
+#pragma unroll
+                for (int k = 0; k < 4; ++k) seed[1 + k] = make_float4(Jb[0][k], Jb[1][k], Jb[2][k], Jb[3][k]);
+            }
+            if (!DERIV && p < n_slab) {
                 const float s[3] = {a.sx, a.sy, a.sz};
                 float g[4][3];   // d y_o / d x_j
 #pragma unroll
@@ -492,7 +526,7 @@ __global__ void __launch_bounds__(NT, 1) DEEP_TANGENT_KERNEL(const __grid_consta
         if (lane == 0) s_red[warp][o] = v;
     }
     __syncthreads();
-    if (threadIdx.x < 6 && (GRAD || threadIdx.x >= 4)) {
+    if (threadIdx.x < 6 && (GRAD || threadIdx.x >= 4) && (GRAD || !DERIV)) {   // the Jacobian query has no partials
         double s = 0.0;
         for (int w = 0; w < NT / 32; ++w) s += s_red[w][threadIdx.x];
         part[threadIdx.x < 4 ? ob2 + threadIdx.x : P + (threadIdx.x - 4)] = s;

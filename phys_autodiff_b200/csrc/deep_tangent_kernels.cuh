@@ -21,6 +21,8 @@
 //                            every layer.  Weight gradients in fp32 within a tile, then added to block-owned double partials.
 //   k_colloc_tangent<H, GRAD>  the same at caller-supplied points (x, y, z, t) instead of the grid (collocation points):
 //                            one float4 per point, its own time input; residuals (optional) AoS per point.
+//   k_deriv_tangent<H, GRAD>  the points kernel with another last stage (deriv_tangent_kernels.cu): GRAD = false writes
+//                            y and J per point; GRAD = true the derivative-fit loss of DESIGN section 4.13 and its gradient.
 //   k_deep_tangent_reduce    sums the block partials in block order (bitwise repeatable): grad[P] and the two sums.
 // Gradient layout: that of deep_grad_kernels.cuh,  dW1 | db1 | dWh | dbh | dW2 | db2  (P = 9H + 4 + (L-1)(H^2 + H)).
 #pragma once
@@ -52,6 +54,14 @@ struct DeepTangentArgs {
     const float4* pts;
     long long n_points;
     float4* R_pts;              // [n_points] {R_sigma, R_ux, R_uy, R_uz} or null (loss only)
+    // derivative mode (deriv_tangent_launch), at the end so that no earlier field's offset moves; sx .. scale_u and R_pts
+    // are not read
+    const float4* dirs;         // [n_points] direction d_i in network coordinates (GRAD)
+    const float4* targets;      // [n_points] target g_i of the four directional derivatives (GRAD)
+    float coef[4];              // float(2 lam_o / n_norm) (GRAD)
+    double lam[4];              // lam_o of the un-normalised sum (GRAD)
+    float4* y_pts;              // [n_points] outputs y (not GRAD)
+    float4* J_pts;              // [n_points][4] rows J[o][0..3] = dy_o / dc_k (not GRAD)
 };
 
 constexpr int DEEP_TANGENT_THREADS = 256;
@@ -67,6 +77,11 @@ int deep_tangent_launch(int H, bool grad, const DeepTangentArgs& a, int blocks, 
 // k_colloc_tangent<H, grad> (colloc_tangent_kernels.cu), then the same reduction: at the grid's own coordinates the
 // sums, residuals and gradient equal deep_tangent_launch's bit for bit.  Any hidden_layers >= 1.
 int colloc_tangent_launch(int H, bool grad, const DeepTangentArgs& a, int blocks, double* acc, double* grad_out, cudaStream_t st);
+// The same body at a.pts as k_deriv_tangent<H, grad> (deriv_tangent_kernels.cu), any hidden_layers >= 1.  grad = false:
+// the Jacobian query, y and J of every point into a.y_pts / a.J_pts, no partials and no reduction (acc and grad_out
+// unused).  grad = true: the derivative-fit loss of DESIGN section 4.13 and its gradient, then deep_tangent_reduce, whose
+// acc[2] is {sum_i sum_o lam_o (D_io - g_io)^2, 0}.
+int deriv_tangent_launch(int H, bool grad, const DeepTangentArgs& a, int blocks, double* acc, double* grad_out, cudaStream_t st);
 // k_deep_tangent_reduce: the block partials [blocks][P + 2] summed in block order into grad[P] and acc[2].
 int deep_tangent_reduce(const double* partials, int blocks, size_t P, double* acc, double* grad, cudaStream_t st);
 

@@ -340,6 +340,28 @@ class Context:
         assert len(lam) == 4
         return (C.c_float * 4)(*lam)
 
+    @staticmethod
+    def _fit_allreduce(B, device, n_global, group, acc):
+        """(loss, grad float64 ndarray[P]) of a fit loss over every rank: n_global (default: the sum of B over ranks, one
+        all-reduce of one integer) normalises, acc(n_global) is the rank's device [acc, grad(P)], and ONE all-reduce of P+1
+        doubles combines the ranks."""
+        import torch
+        import torch.distributed as dist
+        world = dist.get_world_size(group) if dist.is_initialized() else 1
+        if n_global is None:
+            if world > 1:
+                nb = torch.tensor([B], dtype=torch.int64, device=device)
+                dist.all_reduce(nb, op=dist.ReduceOp.SUM, group=group)
+                n_global = int(nb.item())
+            else:
+                n_global = B
+        n_global = max(int(n_global), 1)
+        buf = acc(n_global)
+        if world > 1:
+            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+        h = buf.cpu().numpy()
+        return float(h[0] / n_global), h[1:].copy()
+
     def deep_data_loss_grad_acc(self, x, target, lam=None, n_norm=None, out=None):
         """Device form of the data-fit loss L_d = (1/n_norm) sum_i sum_o lam[o] (y_io - target_io)^2 of the deep network at
         the points x (float32 CUDA tensors x, target [B, 4]): a float64 device tensor [acc, grad(P)] with acc the
@@ -360,23 +382,8 @@ class Context:
         """(L_d, grad float64 ndarray[P]) of the data-fit loss over the points of every rank.  With torch.distributed
         initialised each rank passes its own points; n_global (default: the sum of B over ranks, one all-reduce of one
         integer) normalises, and ONE all-reduce of P+1 doubles combines the ranks."""
-        import torch
-        import torch.distributed as dist
-        world = dist.get_world_size(group) if dist.is_initialized() else 1
-        B = x.numel() // 4
-        if n_global is None:
-            if world > 1:
-                nb = torch.tensor([B], dtype=torch.int64, device=x.device)
-                dist.all_reduce(nb, op=dist.ReduceOp.SUM, group=group)
-                n_global = int(nb.item())
-            else:
-                n_global = B
-        n_global = max(int(n_global), 1)
-        buf = self.deep_data_loss_grad_acc(x, target, lam, n_global)
-        if world > 1:
-            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
-        h = buf.cpu().numpy()
-        return float(h[0] / n_global), h[1:].copy()
+        return self._fit_allreduce(x.numel() // 4, x.device, n_global, group,
+                                   lambda n: self.deep_data_loss_grad_acc(x, target, lam, n))
 
     def deep_data_loss_grad_host(self, x, target, lam=None):
         """Host-array form with n_norm = B: (L_d, dW1, db1, dWh, dbh, dW2, db2), float32."""
@@ -412,23 +419,7 @@ class Context:
         """(L_p, grad float64 ndarray[P]) of the pair loss over the pairs of every rank.  With torch.distributed initialised
         each rank passes its own pairs; n_global (default: the sum of B over ranks, one all-reduce of one integer)
         normalises, and ONE all-reduce of P+1 doubles combines the ranks."""
-        import torch
-        import torch.distributed as dist
-        world = dist.get_world_size(group) if dist.is_initialized() else 1
-        B = x.numel() // 8
-        if n_global is None:
-            if world > 1:
-                nb = torch.tensor([B], dtype=torch.int64, device=x.device)
-                dist.all_reduce(nb, op=dist.ReduceOp.SUM, group=group)
-                n_global = int(nb.item())
-            else:
-                n_global = B
-        n_global = max(int(n_global), 1)
-        buf = self.deep_pair_loss_grad_acc(x, lam, n_global)
-        if world > 1:
-            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
-        h = buf.cpu().numpy()
-        return float(h[0] / n_global), h[1:].copy()
+        return self._fit_allreduce(x.numel() // 8, x.device, n_global, group, lambda n: self.deep_pair_loss_grad_acc(x, lam, n))
 
     def deep_pair_loss_grad_host(self, x, lam=None):
         """Host-array form with n_norm = B: x [B, 2, 4] -> (L_p, dW1, db1, dWh, dbh, dW2, db2), float32."""
@@ -441,6 +432,67 @@ class Context:
         check(self._lib.physad_deep_pair_loss_grad_host(self._h, ptr(x), C.c_size_t(B), self._lam(lam), C.byref(loss),
                                                         *[ptr(a) if a.size else None for a in d]), "deep_pair_loss_grad_host")
         return (np.float32(loss.value), *d)
+
+    # -- Neumann boundaries at arbitrary points: the Jacobian and the derivative-fit loss of deeper networks (additive) -----
+    def mlp_jacobian_deep(self, x):
+        """(y [B, 4], J [B, 4, 4]) of the network set by set_weights_deep at the points x (float32 CUDA tensor [B, 4] of
+        network inputs (x, y, z, t), already normalised), on the device: J[i, o, k] = dy_o / dc_k, exact (forward-mode
+        tangents, no finite differences).  y is mlp_forward_deep's bit for bit.  The derivative in physical units along
+        space axis a is J[:, :, a] * grid_input_scales(g, norm)[a]."""
+        x = x.contiguous()
+        B = x.numel() // 4
+        assert x.numel() == 4 * B
+        y, J = self._empty(B * 4), self._empty(B * 16)
+        check(self._lib.physad_mlp_jacobian_deep_dev(self._h, ptr(x), ptr(y), ptr(J), C.c_size_t(B), self._stream()),
+              "mlp_jacobian_deep")
+        return y.view(B, 4), J.view(B, 4, 4)
+
+    def mlp_jacobian_deep_host(self, x):
+        """Host-array form of mlp_jacobian_deep: x [B, 4] -> (y float32 [B, 4], J float32 [B, 4, 4])."""
+        x = _f32(x)
+        B = x.size // 4
+        assert x.size == 4 * B
+        y, J = np.empty((B, 4), np.float32), np.empty((B, 4, 4), np.float32)
+        check(self._lib.physad_mlp_jacobian_deep_host(self._h, ptr(x), ptr(y), ptr(J), C.c_size_t(B)), "mlp_jacobian_deep_host")
+        return y, J
+
+    def deep_deriv_loss_grad_acc(self, x, d, target, lam=None, n_norm=None, out=None):
+        """Device form of the derivative-fit loss L_g = (1/n_norm) sum_i sum_o lam[o] (D_io - target_io)^2 with
+        D_io = sum_k d_ik J[i, o, k], at the points x (float32 CUDA tensors x, d, target [B, 4]; d a direction in network
+        coordinates, e.g. grid_input_scales(g, norm)[a] e_a for the normal derivative along space axis a; target zeros for a
+        homogeneous Neumann condition).  Returns a float64 device tensor [acc, grad(P)] as deep_data_loss_grad_acc does
+        (db2 exactly zero), so shards with the same n_norm add up and grad adds to the data, pair and physics gradients.
+        lam None: 1/4 each; n_norm None: B (1 for an empty shard)."""
+        import torch
+        x, d, target = x.contiguous(), d.contiguous(), target.contiguous()
+        B = x.numel() // 4
+        assert x.numel() == 4 * B and d.numel() == 4 * B and target.numel() == 4 * B
+        out = out if out is not None else self._empty(self.deep_grad_len() + 1, torch.float64)
+        n = max(B, 1) if n_norm is None else int(n_norm)
+        check(self._lib.physad_deep_deriv_loss_grad_dev(self._h, ptr(x), ptr(d), ptr(target), C.c_size_t(B), self._lam(lam),
+                                                        C.c_size_t(n), ptr(out), ptr(out[1:]), self._stream()),
+              "deep_deriv_loss_grad")
+        return out
+
+    def deep_deriv_loss_grad(self, x, d, target, lam=None, n_global=None, group=None):
+        """(L_g, grad float64 ndarray[P]) of the derivative-fit loss over the points of every rank.  With torch.distributed
+        initialised each rank passes its own points; n_global (default: the sum of B over ranks, one all-reduce of one
+        integer) normalises, and ONE all-reduce of P+1 doubles combines the ranks."""
+        return self._fit_allreduce(x.numel() // 4, x.device, n_global, group,
+                                   lambda n: self.deep_deriv_loss_grad_acc(x, d, target, lam, n))
+
+    def deep_deriv_loss_grad_host(self, x, d, target, lam=None):
+        """Host-array form with n_norm = B: x, d, target [B, 4] -> (L_g, dW1, db1, dWh, dbh, dW2, db2), float32."""
+        x, d, target = _f32(x), _f32(d), _f32(target)
+        B = x.size // 4
+        assert x.size == 4 * B and d.size == 4 * B and target.size == 4 * B
+        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
+        g = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        loss = C.c_float()
+        check(self._lib.physad_deep_deriv_loss_grad_host(self._h, ptr(x), ptr(d), ptr(target), C.c_size_t(B), self._lam(lam),
+                                                         C.byref(loss), *[ptr(a) if a.size else None for a in g]),
+              "deep_deriv_loss_grad_host")
+        return (np.float32(loss.value), *g)
 
     # -- analytic loss of deeper networks at arbitrary points (collocation points; additive) -------------------------------
     @staticmethod
@@ -1065,6 +1117,23 @@ def mlp_pair_loss_deep_grad_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, lam=N
     c = default_context()
     c.set_weights_deep(cfg, L, *w)
     return c.deep_pair_loss_grad_host(x, lam)
+
+
+def mlp_jacobian_deep_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray):
+    """Jacobian of a deep network at arbitrary points (additive): w = (W1, b1, Wh, bh, W2, b2), x [B, 4] network inputs ->
+    (y [B, 4], J [B, 4, 4]), J[i, o, k] = dy_o / dc_k."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.mlp_jacobian_deep_host(x)
+
+
+def mlp_deriv_loss_deep_grad_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, d: np.ndarray, target: np.ndarray, lam=None):
+    """Derivative-fit loss of a deep network and its gradient (additive): w = (W1, b1, Wh, bh, W2, b2), x, d, target [B, 4]
+    -> (L_g, dW1, db1, dWh, dbh, dW2, db2), L_g = mean over the points of sum_o lam[o] (sum_k d_k dy_o/dc_k - target_o)^2
+    (lam None: 1/4 each)."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.deep_deriv_loss_grad_host(x, d, target, lam)
 
 
 def mlp_phys_loss_deep_tangent_points_grad_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, dcdx, pw: PhysWeights):

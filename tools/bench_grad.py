@@ -19,7 +19,13 @@ _grad_dev); one JSON line per pair and B, and with --out the whole run as one JS
 for every --hidden x --layers pair, in alternation with the data loss + gradient step at the same 2B rows and with the
 composition a caller could write without it (two forwards at points and two data steps of B points, each point's target
 its partner's output); one JSON line per pair and B, and with --out the whole run as one JSON document.
-  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent|deep-data|deep-tangent-points|deep-pair] [--n 256] [--hidden 64]
+--loss deep-deriv times the derivative-fit loss + gradient step (physad_deep_deriv_loss_grad_dev) and the Jacobian query
+(physad_mlp_jacobian_deep_dev) at B = 2^24 and 65 536 points for every --hidden x --layers pair, in alternation with the
+points physics loss + gradient step and loss (physad_deep_tangent_points_loss_grad_dev / _dev) at the same points and the
+forward at points (physad_mlp_forward_deep_dev); one JSON line per pair and B, and with --out the whole run as one JSON
+document.
+  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent|deep-data|deep-tangent-points|deep-pair|deep-deriv]
+                             [--n 256] [--hidden 64]
                              [--layers 3] [--steps 20]
   python tools/bench_grad.py --loss deep --hidden 32,64,128 --layers 2,3,5
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/bench_grad.py   (z-slab per rank)"""
@@ -41,11 +47,14 @@ def main():
     ap.add_argument("--hidden", default="64", help="width; --loss deep takes a comma-separated list")
     ap.add_argument("--layers", default="3", help="--loss deep: hidden layers, a comma-separated list")
     ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent", "deep-data", "deep-tangent-points", "deep-pair"),
-                    default="fd")
+    ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent", "deep-data", "deep-tangent-points", "deep-pair",
+                                       "deep-deriv"), default="fd")
     ap.add_argument("--out", default=None,
-                    help="--loss deep-data / deep-tangent-points / deep-pair: also write the run as one JSON document here")
+                    help="--loss deep-data / deep-tangent-points / deep-pair / deep-deriv: also write the run as one JSON "
+                         "document here")
     a = ap.parse_args()
+    if a.loss == "deep-deriv":
+        return deep_deriv(a)
     if a.loss == "deep-pair":
         return deep_pair(a)
     if a.loss == "deep-tangent-points":
@@ -412,6 +421,81 @@ def deep_pair(a):
                                f"gradient step at the same 2B rows, and two forwards at points + two data steps of B points "
                                f"(the composition), timed in alternation (CUDA events, median of {a.steps}); B = {sizes[0]} "
                                f"and {sizes[1]}",
+                       "gpu": name, "power_limit_w": plim, "results": results}, fh, indent=1)
+
+
+def deep_deriv(a):
+    import numpy as np
+    ctx = ops.Context()
+    pw = PhysWeights(1, 1)
+    name, plim = _gpu()
+    dcdx = ops.grid_input_scales(Grid(256, 256, 256), True)
+    rng = np.random.default_rng(5)
+    sizes = (1 << 24, 65536)   # 2^24 points (well past L2), and the overhead regime
+    # uniform random space-time points (space in [-1, 1]^3, t in [0, 0.5]); the direction of point i is the physical normal
+    # of space axis i % 3 (dc/dx e_a), the target zero: the Neumann term of a clamped domain
+    pts = {}
+    for B in sizes:
+        x = rng.uniform(-1, 1, (B, 4)).astype(np.float32)
+        x[:, 3] = rng.uniform(0.0, 0.5, B).astype(np.float32)
+        d = np.zeros((B, 4), np.float32)
+        ax = np.arange(B) % 3
+        d[np.arange(B), ax] = dcdx[ax]
+        pts[B] = tuple(torch.from_numpy(v).cuda() for v in (x, d, np.zeros((B, 4), np.float32)))
+    results = []
+    for H in (int(v) for v in a.hidden.split(",")):
+        w1 = ops.mlp_random_init(H, 777, 0.25)
+        for L in (int(v) for v in a.layers.split(",")):
+            wr = np.random.default_rng(L)
+            Wh = wr.uniform(-0.2, 0.2, (L - 1) * H * H).astype(np.float32)
+            bh = wr.uniform(-0.2, 0.2, (L - 1) * H).astype(np.float32)
+            ctx.set_weights_deep(MLPConfig(4, H, 4, True), L, w1[0], w1[1], Wh, bh, w1[2], w1[3])
+            for B in sizes:
+                x, d, tg = pts[B]
+                dout = ctx.deep_deriv_loss_grad_acc(x, d, tg)
+                pout = ctx.deep_tangent_points_loss_grad_acc(x, dcdx, pw)
+                pacc = ctx.deep_tangent_points_loss_acc(x, dcdx)
+                y, J = ctx.mlp_jacobian_deep(x)
+                yf = ctx.mlp_forward_deep(x)
+
+                def jac():
+                    assert ctx._lib.physad_mlp_jacobian_deep_dev(ctx._h, ops.ptr(x), ops.ptr(y), ops.ptr(J), C.c_size_t(B),
+                                                                 ctx._stream()) == 0
+
+                def fwd():
+                    assert ctx._lib.physad_mlp_forward_deep_dev(ctx._h, ops.ptr(x), ops.ptr(yf), C.c_size_t(B), ctx._stream()) == 0
+                calls = {"deriv_loss_grad": lambda: ctx.deep_deriv_loss_grad_acc(x, d, tg, out=dout),
+                         "points_loss_grad": lambda: ctx.deep_tangent_points_loss_grad_acc(x, dcdx, pw, out=pout),
+                         "jacobian": jac,
+                         "points_loss": lambda: ctx.deep_tangent_points_loss_acc(x, dcdx, acc=pacc),
+                         "forward": fwd}
+                for _ in range(2):
+                    for fn in calls.values():
+                        fn()
+                torch.cuda.synchronize()
+                ts = {k: [] for k in calls}
+                for _ in range(a.steps):   # in alternation, so that they share whatever else the GPU is doing
+                    for k, fn in calls.items():
+                        ts[k] += _times(fn, 1)
+                med = {k: sorted(v)[len(v) // 2] for k, v in ts.items()}
+                h = dout.cpu().numpy()
+                r = {"workload": f"H={H} L={L} B={B} points: derivative loss+grad vs physics loss+grad, Jacobian vs physics loss "
+                                 f"vs forward", "points": B, **{k + "_ms": v for k, v in med.items()},
+                     "deriv_to_points_loss_grad_ratio": med["deriv_loss_grad"] / med["points_loss_grad"],
+                     "jacobian_to_points_loss_ratio": med["jacobian"] / med["points_loss"],
+                     "jacobian_to_forward_ratio": med["jacobian"] / med["forward"],
+                     "deriv_gpts_per_s": B / med["deriv_loss_grad"] / 1e6,
+                     "jacobian_gbytes_written_per_s": 80 * B / med["jacobian"] / 1e6,
+                     "db2": [float(v) for v in h[-4:]], "acc": float(h[0]), "gpu": name, "power_limit_w": plim}
+                results.append(r)
+                print(json.dumps(r), flush=True)
+    if a.out:
+        with open(a.out, "w") as fh:
+            json.dump({"what": f"tools/bench_grad.py --loss deep-deriv --hidden {a.hidden} --layers {a.layers} --steps {a.steps}: "
+                               f"the derivative-fit loss + gradient step (direction dc/dx e_a of axis i % 3, target 0) and the "
+                               f"physics loss + gradient step at the same B uniform random space-time points, the Jacobian "
+                               f"query, the physics loss and the forward at those points, timed in alternation (CUDA events, "
+                               f"median of {a.steps}); B = {sizes[0]} and {sizes[1]}",
                        "gpu": name, "power_limit_w": plim, "results": results}, fh, indent=1)
 
 
