@@ -28,8 +28,13 @@ stencil states, a zero normal derivative at the faces, is fitted at M face point
 third per space axis a alternating the faces c_a = -1 and +1 (the other space inputs uniform in [-1, 1], the time input in
 [T0, T1]), with the derivative-fit loss (physad_deep_deriv_loss_grad_dev, direction dc_a/dx_a e_a, target 0, lam = 1/4
 each, mean over all M points, one all-reduce of P+1 doubles).  The summary then reports the final mean squared normal
-derivative at 4 096 fixed held-out face points (physad_mlp_jacobian_deep_dev).  Prints one JSON line per 20 steps and a
-summary."""
+derivative at 4 096 fixed held-out face points (physad_mlp_jacobian_deep_dev).  --torch (with --layers > 1 and --colloc)
+trains the same objective through phys_autodiff_b200.autograd.DeepMLP and torch.optim.Adam instead: the residuals, the
+data, pair and Neumann terms are written in PyTorch from the module's (y, J) (the library's forward and Jacobian), and
+.backward() runs the library's vector-Jacobian products; with several ranks every rank back-propagates its share and the
+parameters' .grad are all-reduced.  The same points are drawn in the same order, so step 1's losses are the fused run's.
+--grad-out FILE writes step 1's gradient (float64, the flat layout of the deep gradients) in either mode.  Prints one JSON
+line per 20 steps and a summary."""
 import argparse
 import json
 import os
@@ -59,7 +64,13 @@ def main():
     ap.add_argument("--neumann", type=int, default=0,
                     help="face points per step for a zero normal derivative on a clamped domain (needs --colloc)")
     ap.add_argument("--t-range", default="0,0.5", help="T0,T1: the time interval the collocation points cover")
+    ap.add_argument("--torch", action="store_true",
+                    help="losses written in PyTorch on DeepMLP, torch.optim.Adam (needs --layers > 1 and --colloc)")
+    ap.add_argument("--grad-out", default=None, help="write step 1's gradient (float64) to this file")
     a = ap.parse_args()
+    if a.torch and (a.layers < 2 or not a.colloc):
+        ap.error("--torch needs --layers > 1 and --colloc: the one-hidden-layer and grid (finite-difference) objectives "
+                 "have no PyTorch form here")
     if a.data and a.layers < 2:
         ap.error("--data needs --layers > 1")
     if a.colloc and a.layers < 2:
@@ -129,60 +140,65 @@ def main():
         ndir = torch.zeros((hi_n - lo_n, 4), device="cuda")
         ndir[nrows, naxis] = torch.from_numpy(dcdx).cuda()[naxis]
         nzero = torch.zeros_like(ndir)
-    m, v = np.zeros_like(th), np.zeros_like(th)
-    first = last = None
-    t0 = time.perf_counter()
-    for k in range(1, a.steps + 1):
-        w = np.split(th.astype(np.float32), cuts)
-        if a.colloc:
-            ctx.set_weights_deep(cfg, L, *w)
-            xc = lo4 + span4 * torch.rand((hi_c - lo_c, 4), generator=gen, device="cuda")
-            ls, lu, grad = ctx.deep_tangent_points_loss_grad(xc, dcdx, pw, n_global=a.colloc)   # + all-reduce when world > 1
-        elif L > 1 and a.loss == "tangent":
-            ctx.set_weights_deep(cfg, L, *w)
-            ls, lu, grad = ctx.deep_tangent_loss_grad(g, pw, 0.25)   # slab per rank + all-reduce when world > 1
-        elif L > 1:
-            ctx.set_weights_deep(cfg, L, *w)
-            ls, lu, grad = ctx.deep_loss_grad(g, pw, 0.25, 2e-3)     # slab per rank + all-reduce when world > 1
-        elif a.loss == "tangent":
-            ctx.set_weights(cfg, *w)
-            ls, lu, grad = ctx.tangent_loss_grad(g, pw, 0.25)      # slab per rank + all-reduce when world > 1
-        else:
-            ctx.set_weights(cfg, *w)
-            ls, lu, grad = ctx.fused_loss_grad(g, pw, 0.25, 2e-3)
-        lp = None
-        if a.periodic:   # the network set above
-            p = lo4 + span4 * torch.rand((hi_p - lo_p, 4), generator=pgen, device="cuda")
-            p[rows, axis] = -1.0
-            q = p.clone()
-            q[rows, axis] += period[axis]
-            lp, gp = ctx.deep_pair_loss_grad(torch.stack([p, q], 1), n_global=a.periodic)
-            grad = grad + gp
-        ln = None
-        if a.neumann:   # the network set above
-            xn = lo4 + span4 * torch.rand((hi_n - lo_n, 4), generator=ngen, device="cuda")
-            xn[nrows, naxis] = nface
-            ln, gn = ctx.deep_deriv_loss_grad(xn, ndir, nzero, n_global=a.neumann)
-            grad = grad + gn
-        ld = None
-        if a.data:   # the network set above; all ranks' points, one all-reduce of P+1 doubles
-            ld, gd = ctx.deep_data_loss_grad(xd, yd, n_global=a.data)
-            grad = grad + gd
-        last = float(ls) + float(lu) + (ld or 0.0) + (lp or 0.0) + (ln or 0.0)
-        first = last if first is None else first
-        m = 0.9 * m + 0.1 * grad
-        v = 0.999 * v + 0.001 * grad * grad
-        th = th - a.lr * (m / (1 - 0.9 ** k)) / (np.sqrt(v / (1 - 0.999 ** k)) + 1e-8)
-        if rank == 0 and (k == 1 or k % 20 == 0):
-            rec = {"step": k, "loss_sigma": float(ls), "loss_u": float(lu)}
-            if ld is not None:
-                rec["loss_data"] = ld
-            if lp is not None:
-                rec["loss_periodic"] = lp
-            if ln is not None:
-                rec["loss_neumann"] = ln
-            print(json.dumps(rec), flush=True)
-    dt = time.perf_counter() - t0
+    if a.torch:
+        first, last, dt, th = _train_torch(a, ctx, cfg, pw, L, th, cuts, world, locals())
+    else:
+        m, v = np.zeros_like(th), np.zeros_like(th)
+        first = last = None
+        t0 = time.perf_counter()
+        for k in range(1, a.steps + 1):
+            w = np.split(th.astype(np.float32), cuts)
+            if a.colloc:
+                ctx.set_weights_deep(cfg, L, *w)
+                xc = lo4 + span4 * torch.rand((hi_c - lo_c, 4), generator=gen, device="cuda")
+                ls, lu, grad = ctx.deep_tangent_points_loss_grad(xc, dcdx, pw, n_global=a.colloc)   # + all-reduce when world > 1
+            elif L > 1 and a.loss == "tangent":
+                ctx.set_weights_deep(cfg, L, *w)
+                ls, lu, grad = ctx.deep_tangent_loss_grad(g, pw, 0.25)   # slab per rank + all-reduce when world > 1
+            elif L > 1:
+                ctx.set_weights_deep(cfg, L, *w)
+                ls, lu, grad = ctx.deep_loss_grad(g, pw, 0.25, 2e-3)     # slab per rank + all-reduce when world > 1
+            elif a.loss == "tangent":
+                ctx.set_weights(cfg, *w)
+                ls, lu, grad = ctx.tangent_loss_grad(g, pw, 0.25)      # slab per rank + all-reduce when world > 1
+            else:
+                ctx.set_weights(cfg, *w)
+                ls, lu, grad = ctx.fused_loss_grad(g, pw, 0.25, 2e-3)
+            lp = None
+            if a.periodic:   # the network set above
+                p = lo4 + span4 * torch.rand((hi_p - lo_p, 4), generator=pgen, device="cuda")
+                p[rows, axis] = -1.0
+                q = p.clone()
+                q[rows, axis] += period[axis]
+                lp, gp = ctx.deep_pair_loss_grad(torch.stack([p, q], 1), n_global=a.periodic)
+                grad = grad + gp
+            ln = None
+            if a.neumann:   # the network set above
+                xn = lo4 + span4 * torch.rand((hi_n - lo_n, 4), generator=ngen, device="cuda")
+                xn[nrows, naxis] = nface
+                ln, gn = ctx.deep_deriv_loss_grad(xn, ndir, nzero, n_global=a.neumann)
+                grad = grad + gn
+            ld = None
+            if a.data:   # the network set above; all ranks' points, one all-reduce of P+1 doubles
+                ld, gd = ctx.deep_data_loss_grad(xd, yd, n_global=a.data)
+                grad = grad + gd
+            last = float(ls) + float(lu) + (ld or 0.0) + (lp or 0.0) + (ln or 0.0)
+            first = last if first is None else first
+            if k == 1 and a.grad_out and rank == 0:
+                np.asarray(grad, np.float64).tofile(a.grad_out)
+            m = 0.9 * m + 0.1 * grad
+            v = 0.999 * v + 0.001 * grad * grad
+            th = th - a.lr * (m / (1 - 0.9 ** k)) / (np.sqrt(v / (1 - 0.999 ** k)) + 1e-8)
+            if rank == 0 and (k == 1 or k % 20 == 0):
+                rec = {"step": k, "loss_sigma": float(ls), "loss_u": float(lu)}
+                if ld is not None:
+                    rec["loss_data"] = ld
+                if lp is not None:
+                    rec["loss_periodic"] = lp
+                if ln is not None:
+                    rec["loss_neumann"] = ln
+                print(json.dumps(rec), flush=True)
+        dt = time.perf_counter() - t0
     held_dn2 = None
     if a.neumann and rank == 0:
         # the final network's mean squared normal derivative (over points and outputs) at 4 096 fixed face points
@@ -198,12 +214,13 @@ def main():
     if rank == 0:
         data = f" + data at {a.data} points" if a.data else ""
         summary = f"{a.n}^3 H={H} L={L} {a.loss} loss{data} on {world} GPU(s)"
+        via = " (losses in PyTorch through DeepMLP, torch.optim.Adam)" if a.torch else ""
         if a.colloc:
             what = " (initial condition + dynamics)" if a.data else ""
             what += f" + periodic boundaries at {a.periodic} pairs per step" if a.periodic else ""
             what += f" + Neumann boundaries at {a.neumann} face points per step" if a.neumann else ""
             summary = (f"H={H} L={L} analytic loss at {a.colloc} collocation points per step over t in [{t0c:g}, {t1c:g}] of the "
-                       f"{a.n}^3 domain{data}{what} on {world} GPU(s)")
+                       f"{a.n}^3 domain{data}{what} on {world} GPU(s){via}")
         out = {"summary": summary, "steps": a.steps, "loss_first": first, "loss_last": last,
                "reduction_pct": 100 * (1 - last / first), "wall_ms_per_step_incl_host_adam": 1e3 * dt / a.steps}
         if held_dn2 is not None:
@@ -211,6 +228,74 @@ def main():
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
+
+
+def torch_objective(model, dcdx, pw, xc, n_colloc, xd=None, yd=None, n_data=1, pq=None, n_pairs=1, xn=None, ndir=None,
+                    n_neumann=1):
+    """The fused calls' objective written in PyTorch on DeepMLP's (y, J): the analytic residuals of k_tangent_loss at the
+    collocation points xc (w / n_colloc) sum R^2), and the data, pair and Neumann terms with lam = 1/4 each.  Each term is
+    this rank's share of a mean over all ranks' points.  -> (total, {name: term})."""
+    y, J = model(xc, jacobian=True)
+    s = torch.as_tensor(np.asarray(dcdx, np.float32), device=xc.device)
+    gr = J[:, :, :3] * s                                   # d y_o / d x_j
+    div = (gr[:, 1, 0] + gr[:, 2, 1]) + gr[:, 3, 2]
+    R = J[:, :, 3] + ((y[:, 1:2] * gr[:, :, 0] + y[:, 2:3] * gr[:, :, 1]) + y[:, 3:4] * gr[:, :, 2])
+    Rs = R[:, 0] + y[:, 0] * div
+    terms = {"loss_sigma": pw.w_sigma * (Rs * Rs).sum() / n_colloc,
+             "loss_u": pw.w_u * (R[:, 1:] * R[:, 1:]).sum() / n_colloc}
+    if xd is not None:
+        terms["loss_data"] = 0.25 * ((model(xd) - yd) ** 2).sum() / n_data
+    if pq is not None:
+        ypq = model(pq.reshape(-1, 4)).reshape(-1, 2, 4)
+        terms["loss_periodic"] = 0.25 * ((ypq[:, 0] - ypq[:, 1]) ** 2).sum() / n_pairs
+    if xn is not None:
+        _, Jn = model(xn, jacobian=True)
+        D = (Jn * ndir[:, None, :]).sum(-1)
+        terms["loss_neumann"] = 0.25 * (D * D).sum() / n_neumann
+    return sum(terms.values()), terms
+
+
+def _train_torch(a, ctx, cfg, pw, L, th, cuts, world, env):
+    """--torch: the loop of main() with DeepMLP and torch.optim.Adam; the same point draws in the same order."""
+    from phys_autodiff_b200.autograd import DeepMLP
+    rank = int(os.environ.get("RANK", "0"))
+    model = DeepMLP(ctx, cfg.H, L, np.split(th.astype(np.float32), cuts), cfg.minus_one_to_one)
+    opt = torch.optim.Adam(model.parameters(), lr=a.lr, betas=(0.9, 0.999), eps=1e-8)
+    first = last = None
+    t0 = time.perf_counter()
+    for k in range(1, a.steps + 1):
+        xc = env["lo4"] + env["span4"] * torch.rand((env["hi_c"] - env["lo_c"], 4), generator=env["gen"], device="cuda")
+        pq = xn = None
+        if a.periodic:
+            p = env["lo4"] + env["span4"] * torch.rand((env["hi_p"] - env["lo_p"], 4), generator=env["pgen"], device="cuda")
+            p[env["rows"], env["axis"]] = -1.0
+            q = p.clone()
+            q[env["rows"], env["axis"]] += env["period"][env["axis"]]
+            pq = torch.stack([p, q], 1)
+        if a.neumann:
+            xn = env["lo4"] + env["span4"] * torch.rand((env["hi_n"] - env["lo_n"], 4), generator=env["ngen"], device="cuda")
+            xn[env["nrows"], env["naxis"]] = env["nface"]
+        opt.zero_grad(set_to_none=True)
+        total, terms = torch_objective(model, env["dcdx"], pw, xc, a.colloc, env.get("xd"), env.get("yd"), a.data or 1, pq,
+                                       a.periodic or 1, xn, env.get("ndir"), a.neumann or 1)
+        total.backward()
+        vals = torch.stack([t.detach().double() for t in terms.values()])
+        if world > 1:
+            import torch.distributed as dist
+            dist.all_reduce(vals)
+            for p_ in model.parameters():
+                dist.all_reduce(p_.grad)
+        vals = dict(zip(terms, vals.tolist()))
+        last = sum(vals.values())
+        first = last if first is None else first
+        if k == 1 and a.grad_out and rank == 0:
+            np.concatenate([p_.grad.detach().double().cpu().numpy().ravel() for p_ in model._params()]).tofile(a.grad_out)
+        opt.step()
+        if rank == 0 and (k == 1 or k % 20 == 0):
+            print(json.dumps({"step": k, **vals}), flush=True)
+    torch.cuda.synchronize()
+    dt = time.perf_counter() - t0
+    return first, last, dt, model.flat_parameters().astype(np.float64)
 
 
 if __name__ == "__main__":

@@ -103,6 +103,16 @@ void mlp_jacobian_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, c
 void mlp_deriv_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* dir,
                                    const float* target, std::size_t B, const float* lam, float* out_loss, DeepMLPWeights& grad);
 
+// Vector-Jacobian products of a deep network at arbitrary points: the gradient with respect to every layer's weights of any
+// loss whose derivatives with respect to the outputs and the Jacobian are given.  x and ybar hold B host rows of 4 floats,
+// Jbar B host blocks of 4 x 4 in mlp_jacobian_deep_cuda's J layout (Jbar[i][o][k] pairs with dy_o / dc_k).
+// grad = sum_i ybar_i . dy_i/dtheta (+ sum_i Jbar_i : dJ_i/dtheta), the plain sum over the points with no scale; it adds
+// directly to the other deep gradients.  `grad` is resized to the shapes of `w`.  B = 0 gives zeros.
+void mlp_vjp_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* ybar, std::size_t B,
+                       DeepMLPWeights& grad);
+void mlp_jacobian_vjp_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* ybar,
+                                const float* Jbar, std::size_t B, DeepMLPWeights& grad);
+
 // The analytic loss of a deep network at arbitrary space-time points (collocation points) instead of the grid at one time:
 // x holds B host points of 4 floats (x, y, z, t), the network inputs already normalised (the fourth is the grid's time input:
 // t for MinusOneToOne, t + 0.5 for ZeroToOne); dcdx the 3 dc/dx of the space inputs (physad_grid_input_scales gives the

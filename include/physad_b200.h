@@ -507,6 +507,35 @@ int physad_deep_deriv_loss_grad_host(physad_ctx* ctx, const float* x, const floa
                                      const float* lam, float* loss, float* dW1, float* db1, float* dWh, float* dbh,
                                      float* dW2, float* db2);
 
+/* ---- vector-Jacobian products of deeper networks at arbitrary points (ADDITIVE, no reference counterpart) ---------------
+ * The gradient of ANY loss of the outputs y and the Jacobian J at points, given its cotangents: the primitive under which a
+ * loss written by the caller (in PyTorch, say) trains the network, whose forward is physad_mlp_forward_deep_dev or
+ * physad_mlp_jacobian_deep_dev.  The network set by physad_set_weights_deep (any hidden_layers >= 1, deep mode 0); x[B][4]
+ * network inputs as for physad_mlp_jacobian_deep_dev.
+ * physad_mlp_vjp_deep_dev: grad = sum_i sum_o ybar[i][o] dy_io / dtheta, ybar [B][4] DEVICE floats (16-byte aligned, like
+ *   x).  The kernel is the data loss's with ybar as its seeds: with ybar = fp32(2 lam[o] / n_norm) * (y - target) formed in
+ *   fp32 from physad_mlp_forward_deep_dev's y, grad equals physad_deep_data_loss_grad_dev's bit for bit.
+ * physad_mlp_jacobian_vjp_deep_dev: grad = sum_i (sum_o ybar[i][o] dy_io / dtheta + sum_o sum_k Jbar[i][o][k]
+ *   dJ[i][o][k] / dtheta), Jbar [B][4][4] DEVICE floats in the layout of physad_mlp_jacobian_deep_dev's J (Jbar[i][o][k]
+ *   pairs with dy_o / dc_k).  ybar is required: pass zeros for a loss on J only.  The kernel is the derivative-fit loss's with
+ *   the seeds read: ybar on the value row, the column Jbar[i][.][k] on tangent row k.
+ * grad = P = physad_deep_grad_len(H, L) DEVICE doubles (8-byte aligned) in the layout of physad_deep_loss_grad_dev, the
+ *   plain sum over the points with no scale (the cotangents carry every weight and normalisation): the shards' grad add up
+ *   under one all-reduce(sum), and grad adds to every other deep gradient.  B = 0 writes a zero gradient.  Bitwise
+ *   repeatable.  The same checkpoint and partials scratch as the data loss and the points physics loss.
+ * The _host forms take host arrays and split the gradient into the six arrays of physad_set_weights_deep's layouts (any
+ *   output pointer may be null).
+ * Errors: no deep weights (or a physad_set_weights after them): PHYSAD_E_NOWEIGHTS; physad_set_deep_mode(1):
+ * PHYSAD_E_UNSUPPORTED; a null or misaligned x, ybar or Jbar with B > 0, a null or misaligned (8 bytes) grad:
+ * PHYSAD_E_INVALID.  A refused call writes nothing. */
+int physad_mlp_vjp_deep_dev(physad_ctx* ctx, const float* x, const float* ybar, size_t B, double* grad, void* stream);
+int physad_mlp_vjp_deep_host(physad_ctx* ctx, const float* x, const float* ybar, size_t B, float* dW1, float* db1,
+                             float* dWh, float* dbh, float* dW2, float* db2);
+int physad_mlp_jacobian_vjp_deep_dev(physad_ctx* ctx, const float* x, const float* ybar, const float* Jbar, size_t B,
+                                     double* grad, void* stream);
+int physad_mlp_jacobian_vjp_deep_host(physad_ctx* ctx, const float* x, const float* ybar, const float* Jbar, size_t B,
+                                      float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2);
+
 /* ---- analytic loss of deeper networks at arbitrary points (ADDITIVE, no reference counterpart) ---------------------------
  * The physics loss of physad_deep_tangent_loss_* at caller-supplied collocation points (x, y, z, t) spread over the whole
  * space-time domain instead of the grid's points at one time: the term that makes a fit learn the dynamics between the

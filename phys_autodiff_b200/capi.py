@@ -102,7 +102,8 @@ EXPORTS = [
     "physad_deep_tangent_points_loss_grad_dev", "physad_deep_tangent_points_loss_grad_host",
     "physad_deep_pair_loss_grad_dev", "physad_deep_pair_loss_grad_host",
     "physad_mlp_jacobian_deep_dev", "physad_mlp_jacobian_deep_host", "physad_deep_deriv_loss_grad_dev",
-    "physad_deep_deriv_loss_grad_host",
+    "physad_deep_deriv_loss_grad_host", "physad_mlp_vjp_deep_dev", "physad_mlp_vjp_deep_host",
+    "physad_mlp_jacobian_vjp_deep_dev", "physad_mlp_jacobian_vjp_deep_host",
 ]
 
 

@@ -2017,12 +2017,17 @@ int launch_deep_points(physad_ctx* c, const DeepArgs& a, cudaStream_t st) {
     return 0;
 }
 
+// how the kernel of deep_data_body.cuh forms its seeds: data fit, matched pairs, or the caller's cotangents (the VJP)
+enum class DataSeeds { data, pairs, vjp };
+
 template <int H>
-int launch_deep_data(physad_ctx* c, bool pairs, const DeepDataArgs& a, int blocks, double* grad, double* acc, cudaStream_t st) {
+int launch_deep_data(physad_ctx* c, DataSeeds seeds, const DeepDataArgs& a, int blocks, double* grad, double* acc, cudaStream_t st) {
     MlpConst<H> k;
     const float no_t[3] = {0.f, 0.f, 0.f};   // only the output pairs w2 / b2 are read
     fill_const<H>(c, no_t, k);
-    CU(cudaError_t(pairs ? deep_pair_launch(H, &k, a, blocks, grad, acc, st) : deep_data_launch(H, &k, a, blocks, grad, acc, st)));
+    CU(cudaError_t(seeds == DataSeeds::pairs ? deep_pair_launch(H, &k, a, blocks, grad, acc, st)
+                   : seeds == DataSeeds::vjp ? vjp_points_launch(H, &k, a, blocks, grad, acc, st)
+                                             : deep_data_launch(H, &k, a, blocks, grad, acc, st)));
     c->launches += 2;
     return 0;
 }
@@ -2116,6 +2121,36 @@ void split_deep_grad(const double* gd, int H, int L, float* dW1, float* db1, flo
     }
 }
 
+// The launch shared by the data loss, the pair loss and the VJP at a.n > 0 rows: the weights, the grid, the checkpoint, the
+// partials, the kernel and the reduction.  `a` brings the rows and the seed inputs; the network's fields are filled here.
+// acc null (the VJP): the reduction's (zero) loss sum goes to a slot after the partials.
+int deep_data_run(physad_ctx* c, DataSeeds seeds, DeepDataArgs& a, double* grad, double* acc, cudaStream_t st) {
+    if (int rc = upload_weights_if_stale(c, st)) return rc;
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    const int blocks = deep_data_blocks(H, a.n, c->sm_count);
+    const size_t ck = size_t(blocks) * deep_data_ckpt_floats(H, L);
+    if (ck > c->dckpt_cap) {
+        if (c->dckpt) CU(cudaFree(c->dckpt));
+        c->dckpt = nullptr; c->dckpt_cap = 0;
+        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
+        c->dckpt_cap = ck;
+    }
+    const size_t np = size_t(blocks) * (P + 1);
+    if (int rc = ensure_grad_partials(c, np + (acc ? 0 : 1))) return rc;
+    a.hidden_layers = L;
+    a.W1 = c->dW1; a.b1 = c->db1; a.W2 = c->dW2;
+    a.wh = c->d_wh; a.bh = c->d_bh;
+    a.ckpt = c->dckpt;
+    a.partials = c->gpart;
+    if (!acc) acc = c->gpart + np;
+    switch (H) {
+        case 32: return launch_deep_data<32>(c, seeds, a, blocks, grad, acc, st);
+        case 64: return launch_deep_data<64>(c, seeds, a, blocks, grad, acc, st);
+        default: return launch_deep_data<128>(c, seeds, a, blocks, grad, acc, st);
+    }
+}
+
 // The data loss (B points and their targets) and the pair loss (B pairs = 2B rows of x, no target) share everything but
 // the kernel: the checks, the scratch, the arguments and the reduction.  `what` names the caller in error messages.
 int deep_fit_dev(physad_ctx* c, const char* what, bool pairs, const float* x, const float* target, size_t B, const float* lam,
@@ -2139,35 +2174,15 @@ int deep_fit_dev(physad_ctx* c, const char* what, bool pairs, const float* x, co
         CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
         return 0;
     }
-    if (int rc = upload_weights_if_stale(c, st)) return rc;
-    const size_t rows = pairs ? 2 * B : B;
-    const int blocks = deep_data_blocks(H, (long long)rows, c->sm_count);
-    const size_t ck = size_t(blocks) * deep_data_ckpt_floats(H, L);
-    if (ck > c->dckpt_cap) {
-        if (c->dckpt) CU(cudaFree(c->dckpt));
-        c->dckpt = nullptr; c->dckpt_cap = 0;
-        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
-        c->dckpt_cap = ck;
-    }
-    if (int rc = ensure_grad_partials(c, size_t(blocks) * (P + 1))) return rc;
     DeepDataArgs a{};
-    a.hidden_layers = L;
-    a.n = (long long)rows;
+    a.n = (long long)(pairs ? 2 * B : B);
     a.x = reinterpret_cast<const float4*>(x);
     a.target = reinterpret_cast<const float4*>(target);
-    a.W1 = c->dW1; a.b1 = c->db1; a.W2 = c->dW2;
-    a.wh = c->d_wh; a.bh = c->d_bh;
     for (int o = 0; o < 4; ++o) {
         a.coef[o] = float(2.0 * double(lw[o]) / double(n_norm));
         a.lam[o] = double(lw[o]);
     }
-    a.ckpt = c->dckpt;
-    a.partials = c->gpart;
-    switch (H) {
-        case 32: return launch_deep_data<32>(c, pairs, a, blocks, grad, acc, st);
-        case 64: return launch_deep_data<64>(c, pairs, a, blocks, grad, acc, st);
-        default: return launch_deep_data<128>(c, pairs, a, blocks, grad, acc, st);
-    }
+    return deep_data_run(c, pairs ? DataSeeds::pairs : DataSeeds::data, a, grad, acc, st);
 }
 
 // The host forms: x (and target) uploaded, n_norm = B, the gradient split into set_weights_deep's six arrays.
@@ -2253,11 +2268,15 @@ int colloc_args(physad_ctx* c, const float* x, size_t B, const float* dcdx, Deep
     return 0;
 }
 
-// The gradient launch at B > 0 points, shared by the physics loss (k_colloc_tangent) and the derivative-fit loss
-// (k_deriv_tangent): one kernel body, so one scratch, L x 80 KB of checkpoint and P + 2 partials per block.  The physics
-// loss returns both sums in acc[2]; the derivative loss one, so its reduction writes {acc, 0} to two doubles after the
-// partials and acc is copied out from there.
-int colloc_grad_launch(physad_ctx* c, bool deriv, DeepTangentArgs& a, double* acc, double* grad, cudaStream_t st) {
+// how the points kernel of deep_tangent_body.cuh forms its seeds: physics residuals, derivative fit, or the caller's
+// cotangents (the VJP)
+enum class TangentSeeds { physics, deriv, vjp };
+
+// The gradient launch at B > 0 points, shared by the physics loss (k_colloc_tangent), the derivative-fit loss
+// (k_deriv_tangent) and the VJP (k_vjp_tangent): one kernel body, so one scratch, L x 80 KB of checkpoint and P + 2
+// partials per block.  The physics loss returns both sums in acc[2]; the derivative loss one and the VJP none, so their
+// reductions write two doubles after the partials and acc (if any) is copied out from there.
+int colloc_grad_launch(physad_ctx* c, TangentSeeds seeds, DeepTangentArgs& a, double* acc, double* grad, cudaStream_t st) {
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
     const int blocks = deep_tangent_blocks(H, a.n_points, c->sm_count);
@@ -2269,14 +2288,16 @@ int colloc_grad_launch(physad_ctx* c, bool deriv, DeepTangentArgs& a, double* ac
         c->dckpt_cap = ck;
     }
     const size_t np = size_t(blocks) * (P + 2);
-    if (int rc = ensure_grad_partials(c, np + (deriv ? 2 : 0))) return rc;
+    const bool physics = seeds == TangentSeeds::physics;
+    if (int rc = ensure_grad_partials(c, np + (physics ? 0 : 2))) return rc;
     a.ckpt = c->dckpt;
     a.partials = c->gpart;
-    if (deriv) {
-        CU(cudaError_t(deriv_tangent_launch(H, true, a, blocks, c->gpart + np, grad, st)));
-        CU(cudaMemcpyAsync(acc, c->gpart + np, sizeof(double), cudaMemcpyDeviceToDevice, st));
-    } else {
+    if (physics) {
         CU(cudaError_t(colloc_tangent_launch(H, true, a, blocks, acc, grad, st)));
+    } else {
+        CU(cudaError_t(seeds == TangentSeeds::deriv ? deriv_tangent_launch(H, true, a, blocks, c->gpart + np, grad, st)
+                                                    : vjp_tangent_launch(H, a, blocks, c->gpart + np, grad, st)));
+        if (acc) CU(cudaMemcpyAsync(acc, c->gpart + np, sizeof(double), cudaMemcpyDeviceToDevice, st));
     }
     c->launches += 2;
     return 0;
@@ -2334,7 +2355,7 @@ int physad_deep_tangent_points_loss_grad_dev(physad_ctx* c, const float* x, size
     // vjp_scales' formula with n_norm for N: shards with the same n_norm add up to the whole set's gradient
     a.scale_s = 2.f * w->w_sigma / float(n_norm);
     a.scale_u = 2.f * w->w_u / float(n_norm);
-    return colloc_grad_launch(c, false, a, acc, grad, st);
+    return colloc_grad_launch(c, TangentSeeds::physics, a, acc, grad, st);
 }
 
 int physad_deep_tangent_points_loss_grad_host(physad_ctx* c, const float* x, size_t B, const float* dcdx,
@@ -2427,7 +2448,7 @@ int physad_deep_deriv_loss_grad_dev(physad_ctx* c, const float* x, const float* 
         a.coef[o] = float(2.0 * double(lw[o]) / double(n_norm));
         a.lam[o] = double(lw[o]);
     }
-    return colloc_grad_launch(c, true, a, acc, grad, st);
+    return colloc_grad_launch(c, TangentSeeds::deriv, a, acc, grad, st);
 }
 
 int physad_deep_deriv_loss_grad_host(physad_ctx* c, const float* x, const float* dir, const float* target, size_t B,
@@ -2454,6 +2475,99 @@ int physad_deep_deriv_loss_grad_host(physad_ctx* c, const float* x, const float*
     CU(cudaStreamSynchronize(c->stream));
     if (loss) *loss = float(c->h_dgrad[0] / double(n));
     split_deep_grad(c->h_dgrad + 1, H, L, dW1, db1, dWh, dbh, dW2, db2);
+    return 0;
+}
+
+// ---- vector-Jacobian products of deeper networks at points (deep_data_kernels.cuh, deep_tangent_kernels.cuh) ----------
+int physad_mlp_vjp_deep_dev(physad_ctx* c, const float* x, const float* ybar, size_t B, double* grad, void* stream) {
+    const std::string w("mlp_vjp_deep");
+    if (!c) return fail(PHYSAD_E_INVALID, w + ": null context");
+    if (int rc = deep_points_ready(c, w.c_str())) return rc;
+    if (!grad || (B && (!x || !ybar))) return fail(PHYSAD_E_INVALID, w + ": null argument");
+    if (B && (misaligned16(x) || misaligned16(ybar))) return fail(PHYSAD_E_INVALID, w + ": x and ybar must be 16-byte aligned");
+    if (uintptr_t(grad) % 8) return fail(PHYSAD_E_INVALID, w + ": grad must be 8-byte aligned");
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    if (B == 0) {   // an empty shard: zero gradient
+        CU(cudaMemsetAsync(grad, 0, deep_grad_len(c->cfg.H, c->deep_layers) * sizeof(double), st));
+        return 0;
+    }
+    DeepDataArgs a{};
+    a.n = (long long)B;
+    a.x = reinterpret_cast<const float4*>(x);
+    a.ybar = reinterpret_cast<const float4*>(ybar);
+    return deep_data_run(c, DataSeeds::vjp, a, grad, nullptr, st);
+}
+
+int physad_mlp_vjp_deep_host(physad_ctx* c, const float* x, const float* ybar, size_t B, float* dW1, float* db1, float* dWh,
+                             float* dbh, float* dW2, float* db2) {
+    if (!c) return fail(PHYSAD_E_INVALID, "mlp_vjp_deep: null context");
+    if (int rc = deep_points_ready(c, "mlp_vjp_deep")) return rc;
+    if (B && (!x || !ybar)) return fail(PHYSAD_E_INVALID, "mlp_vjp_deep: null argument");
+    DeviceGuard dg(c->device);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (int rc = ensure_host_grad(c, P)) return rc;
+    const size_t bytes = B * 4 * sizeof(float), off = (bytes + 255) & ~size_t(255);
+    if (int rc = ensure_scratch(c, off + bytes + 1)) return rc;
+    float* dx = reinterpret_cast<float*>(c->scratch);
+    float* dyb = reinterpret_cast<float*>(c->scratch + off);
+    if (B) {
+        CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
+        CU(cudaMemcpyAsync(dyb, ybar, bytes, cudaMemcpyHostToDevice, c->stream));
+    }
+    if (int rc = physad_mlp_vjp_deep_dev(c, dx, dyb, B, c->d_dgrad, c->stream)) return rc;
+    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, P * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    split_deep_grad(c->h_dgrad, H, L, dW1, db1, dWh, dbh, dW2, db2);
+    return 0;
+}
+
+int physad_mlp_jacobian_vjp_deep_dev(physad_ctx* c, const float* x, const float* ybar, const float* Jbar, size_t B, double* grad,
+                                     void* stream) {
+    const std::string w("mlp_jacobian_vjp_deep");
+    if (!c) return fail(PHYSAD_E_INVALID, w + ": null context");
+    if (int rc = deep_points_ready(c, w.c_str())) return rc;
+    if (!grad || (B && (!x || !ybar || !Jbar))) return fail(PHYSAD_E_INVALID, w + ": null argument");
+    if (B && (misaligned16(x) || misaligned16(ybar) || misaligned16(Jbar)))
+        return fail(PHYSAD_E_INVALID, w + ": x, ybar and Jbar must be 16-byte aligned");
+    if (uintptr_t(grad) % 8) return fail(PHYSAD_E_INVALID, w + ": grad must be 8-byte aligned");
+    DeviceGuard dg(c->device);
+    cudaStream_t st = cudaStream_t(stream);
+    if (B == 0) {   // an empty shard: zero gradient
+        CU(cudaMemsetAsync(grad, 0, deep_grad_len(c->cfg.H, c->deep_layers) * sizeof(double), st));
+        return 0;
+    }
+    DeepTangentArgs a{};
+    if (int rc = colloc_args(c, x, B, nullptr, a, st)) return rc;
+    a.ybar = reinterpret_cast<const float4*>(ybar);
+    a.Jbar = reinterpret_cast<const float4*>(Jbar);
+    return colloc_grad_launch(c, TangentSeeds::vjp, a, nullptr, grad, st);
+}
+
+int physad_mlp_jacobian_vjp_deep_host(physad_ctx* c, const float* x, const float* ybar, const float* Jbar, size_t B, float* dW1,
+                                      float* db1, float* dWh, float* dbh, float* dW2, float* db2) {
+    if (!c) return fail(PHYSAD_E_INVALID, "mlp_jacobian_vjp_deep: null context");
+    if (int rc = deep_points_ready(c, "mlp_jacobian_vjp_deep")) return rc;
+    if (B && (!x || !ybar || !Jbar)) return fail(PHYSAD_E_INVALID, "mlp_jacobian_vjp_deep: null argument");
+    DeviceGuard dg(c->device);
+    const int H = c->cfg.H, L = c->deep_layers;
+    const size_t P = deep_grad_len(H, L);
+    if (int rc = ensure_host_grad(c, P)) return rc;
+    const size_t bytes = B * 4 * sizeof(float), off = (bytes + 255) & ~size_t(255);
+    if (int rc = ensure_scratch(c, 2 * off + 4 * bytes + 1)) return rc;
+    float* dx = reinterpret_cast<float*>(c->scratch);
+    float* dyb = reinterpret_cast<float*>(c->scratch + off);
+    float* dJb = reinterpret_cast<float*>(c->scratch + 2 * off);
+    if (B) {
+        CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
+        CU(cudaMemcpyAsync(dyb, ybar, bytes, cudaMemcpyHostToDevice, c->stream));
+        CU(cudaMemcpyAsync(dJb, Jbar, 4 * bytes, cudaMemcpyHostToDevice, c->stream));
+    }
+    if (int rc = physad_mlp_jacobian_vjp_deep_dev(c, dx, dyb, dJb, B, c->d_dgrad, c->stream)) return rc;
+    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, P * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    split_deep_grad(c->h_dgrad, H, L, dW1, db1, dWh, dbh, dW2, db2);
     return 0;
 }
 

@@ -501,6 +501,40 @@ void mlp_deriv_loss_deep_grad_cuda(const MLPGridConfig& cfg, const DeepMLPWeight
     if (rc) die("mlp_deriv_loss_deep_grad_cuda", rc);
 }
 
+namespace {
+// the two VJPs share everything but the call: jacobian = false ignores Jbar
+void vjp_deep(const char* what, bool jacobian, const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x,
+              const float* ybar, const float* Jbar, std::size_t B, DeepMLPWeights& grad) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    check_deep_shapes(cfg, w, what);
+    physad_ctx* c = ctx();
+    grad.hidden_layers = w.hidden_layers;
+    grad.W1.resize(w.W1.size());
+    grad.b1.resize(w.b1.size());
+    grad.Wh.resize(w.Wh.size());
+    grad.bh.resize(w.bh.size());
+    grad.W2.resize(w.W2.size());
+    grad.b2.resize(w.b2.size());
+    float* out[6] = {grad.W1.data(), grad.b1.data(), grad.Wh.empty() ? nullptr : grad.Wh.data(),
+                     grad.bh.empty() ? nullptr : grad.bh.data(), grad.W2.data(), grad.b2.data()};
+    int rc = set_deep(c, cfg, w);
+    if (!rc)
+        rc = jacobian ? physad_mlp_jacobian_vjp_deep_host(c, x, ybar, Jbar, B, out[0], out[1], out[2], out[3], out[4], out[5])
+                      : physad_mlp_vjp_deep_host(c, x, ybar, B, out[0], out[1], out[2], out[3], out[4], out[5]);
+    if (rc) die(what, rc);
+}
+}  // namespace
+
+void mlp_vjp_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* ybar, std::size_t B,
+                       DeepMLPWeights& grad) {
+    vjp_deep("mlp_vjp_deep_cuda", false, cfg, w, x, ybar, nullptr, B, grad);
+}
+
+void mlp_jacobian_vjp_deep_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const float* x, const float* ybar,
+                                const float* Jbar, std::size_t B, DeepMLPWeights& grad) {
+    vjp_deep("mlp_jacobian_vjp_deep_cuda", true, cfg, w, x, ybar, Jbar, B, grad);
+}
+
 void mlp_phys_loss_deep_tangent_points_cuda(const MLPGridConfig& cfg, const DeepMLPWeights& w, const PhysWeights& pw,
                                             const float* x, std::size_t B, const float dcdx[3], float* out_loss_sigma,
                                             float* out_loss_u, float* opt_R) {

@@ -1,10 +1,13 @@
-// The kernel behind k_deep_data_grad (deep_data_kernels.cu) and k_deep_pair_grad (deep_pair_kernels.cu); see
-// deep_data_kernels.cuh for what they compute.  The two differ only in how a row's seeds are formed.  Each of the two files
-// includes this one once, after defining
+// The kernel behind k_deep_data_grad (deep_data_kernels.cu), k_deep_pair_grad (deep_pair_kernels.cu) and k_vjp_points
+// (vjp_points_kernels.cu); see deep_data_kernels.cuh for what they compute.  The three differ only in how a row's seeds
+// are formed.  Each of the three files includes this one once, after defining
 //   DEEP_DATA_KERNEL   the kernel's name;
 //   DEEP_DATA_PAIRS    its seeds: false, y_bar = coef (y - target) against the caller's targets; true, rows 2i and 2i+1 are
 //                      the two points of pair i and each row's target is its partner's output, y_bar = coef (y - y_partner)
-//                      (so the two rows' seeds are exact negatives), the loss summed once per pair (on the even row).
+//                      (so the two rows' seeds are exact negatives), the loss summed once per pair (on the even row);
+//   DEEP_DATA_VJP      optional, default false; true (with PAIRS false) makes k_vjp_points: y_bar is the caller's
+//                      cotangent a.ybar[p] as it is, and there is no loss sum.  The output layer's values are then unused
+//                      and the compiler drops that stage.
 // As in deep_tangent_body.cuh, the body is the kernel itself rather than a __device__ function both kernels inline, so
 // k_deep_data_grad compiles to exactly the code it had as a kernel of its own.
 //
@@ -20,6 +23,9 @@
 // No FFMA2 anywhere: the forward keeps k_mlp_deep's un-contracted FMUL2 / FADD2, the backward uses scalar FFMA.
 #if !defined(DEEP_DATA_KERNEL) || !defined(DEEP_DATA_PAIRS)
 #error "define DEEP_DATA_KERNEL and DEEP_DATA_PAIRS before including deep_data_body.cuh"
+#endif
+#ifndef DEEP_DATA_VJP
+#define DEEP_DATA_VJP false
 #endif
 #include "deep_data_kernels.cuh"
 #include "mlp_eval.cuh"
@@ -70,7 +76,8 @@ __host__ __device__ constexpr size_t grad_len(int H, int L) {
 
 template <int H>
 __global__ void __launch_bounds__(NT, 1) DEEP_DATA_KERNEL(const __grid_constant__ MlpConst<H> w, const __grid_constant__ DeepDataArgs a) {
-    constexpr bool PAIRS = DEEP_DATA_PAIRS;
+    constexpr bool PAIRS = DEEP_DATA_PAIRS, VJP = DEEP_DATA_VJP;
+    static_assert(!(PAIRS && VJP), "the VJP reads one cotangent per row");
     using Q = Geo<H>;
     constexpr int G = Q::G, RB = Q::RB, NROW = Q::NROW, PTS_TILE = NROW, ACT = Q::ACT;
     extern __shared__ __align__(16) float smem[];
@@ -241,7 +248,11 @@ __global__ void __launch_bounds__(NT, 1) DEEP_DATA_KERNEL(const __grid_constant_
                 const long long p = tile * PTS_TILE + r;
                 if (r_raw < NROW) {
                     float4 yb = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (p < n) {   // pairs: n is even, so both rows of a pair are in range or neither
+                    if (VJP && p < n) {   // the caller's cotangent, as it is; tail rows keep zero
+                        yb = __ldg(a.ybar + p);
+                        red[0] += double(yb.x); red[1] += double(yb.y); red[2] += double(yb.z); red[3] += double(yb.w);
+                    }
+                    if (!VJP && p < n) {   // pairs: n is even, so both rows of a pair are in range or neither
                         float4 t4;
                         if constexpr (PAIRS) t4 = make_float4(yp[0], yp[1], yp[2], yp[3]);
                         else t4 = __ldg(a.target + p);

@@ -21,6 +21,11 @@
 // x[B][2] (row 2i = p_i, row 2i + 1 = q_i) with the partner row's outputs as the target: seeds
 // y_bar(p_i) = coef (y(p_i) - y(q_i)) and y_bar(q_i) = -y_bar(p_i) exactly, the double sum counted once per pair; then
 // k_deep_data_reduce.  The grid size, checkpoint area and partials are the data kernel's for 2B points.
+// Vector-Jacobian product (vjp_points_kernels.cu): for caller-supplied cotangents y_bar[n][4],
+//   grad = sum_i J_theta(y_i)^T y_bar_i,   the plain sum over the points (no scale: y_bar carries every weight),
+// the gradient of any loss whose derivative with respect to y_i is y_bar_i.  k_vjp_points<H> is k_deep_data_grad's body
+// with y_bar read from a.ybar (zero on tail rows) and no loss sum; then k_deep_data_reduce (acc[1] = 0).  With
+// y_bar = coef (y - target) formed in fp32 it is k_deep_data_grad's gradient bit for bit.
 // Gradient layout: that of physad_deep_loss_grad_dev (P = 9H + 4 + (L-1)(H^2 + H) doubles):
 //   dW1 [H x 4] | db1 [H] | dWh [(L-1) x H x H, row-major [out][in]] | dbh [(L-1) x H] | dW2 [4 x H] | db2 [4]
 #pragma once
@@ -44,6 +49,8 @@ struct DeepDataArgs {
     double lam[4];              // loss weights of the double sum
     float* ckpt;                // [blocks][L][rows x H] activations of the current tile
     double* partials;           // [blocks][P + 1]
+    // the VJP (vjp_points_launch), at the end so that no earlier field's offset moves; target, coef and lam are not read
+    const float4* ybar;         // [n] cotangents of the outputs
 };
 
 constexpr int DEEP_DATA_THREADS = 256;
@@ -57,6 +64,8 @@ int deep_data_blocks(int H, long long n_points, int max_blocks);
 int deep_data_launch(int H, const void* mlp_const, const DeepDataArgs& a, int blocks, double* grad, double* acc, cudaStream_t st);
 // k_deep_pair_grad<H> on `blocks` blocks (a.n = 2B rows, a.target unused), then the same reduction.
 int deep_pair_launch(int H, const void* mlp_const, const DeepDataArgs& a, int blocks, double* grad, double* acc, cudaStream_t st);
+// k_vjp_points<H> on `blocks` blocks (a.ybar the seeds, a.target unused), then the same reduction (acc[1] = 0).
+int vjp_points_launch(int H, const void* mlp_const, const DeepDataArgs& a, int blocks, double* grad, double* acc, cudaStream_t st);
 // k_deep_data_reduce: partials [blocks][P + 1] summed in block order into grad[P] and acc[1].
 int deep_data_reduce(const double* partials, int blocks, size_t P, double* grad, double* acc, cudaStream_t st);
 

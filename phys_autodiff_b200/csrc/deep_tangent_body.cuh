@@ -1,7 +1,7 @@
-// The kernel behind k_deep_tangent (deep_tangent_kernels.cu), k_colloc_tangent (colloc_tangent_kernels.cu) and
-// k_deriv_tangent (deriv_tangent_kernels.cu); see deep_tangent_kernels.cuh for what they compute.  The first two differ
-// only in where a point's inputs come from, the third from the second only in its last stage.  Each of the three files
-// includes this one once, after defining
+// The kernel behind k_deep_tangent (deep_tangent_kernels.cu), k_colloc_tangent (colloc_tangent_kernels.cu),
+// k_deriv_tangent (deriv_tangent_kernels.cu) and k_vjp_tangent (vjp_tangent_kernels.cu); see deep_tangent_kernels.cuh for
+// what they compute.  The first two differ only in where a point's inputs come from, the last two from the second only in
+// their last stages.  Each of the four files includes this one once, after defining
 //   DEEP_TANGENT_KERNEL   the kernel's name;
 //   DEEP_TANGENT_POINTS   its row source: false, the slab's grid points in linear order (coordinates from the axis tables,
 //                         one time input a.tc); true, the caller's points a.pts[0 .. a.n_points) (one float4 per point,
@@ -10,6 +10,9 @@
 //                         only the stage after the output layer differs.  GRAD = false writes y and J of each point
 //                         (a.y_pts, a.J_pts) instead of residuals and sums; GRAD = true reads a.dirs / a.targets and seeds
 //                         the tangent rows with the derivative-fit loss of DESIGN section 4.13 (value-row seeds zero).
+//   DEEP_TANGENT_VJP      optional, default false; true (with POINTS, GRAD only) makes k_vjp_tangent: the seeds are the
+//                         caller's cotangents, value row a.ybar[p], tangent row k the column a.Jbar[p][:][k]; no sums.  The
+//                         output layer's values are not needed, so that stage is skipped.
 // The body is the kernel itself, not a __device__ function both kernels inline: inlined, it loses the thread-index range
 // that __launch_bounds__ gives the kernel, and k_deep_tangent<128, *> compiles to different code.
 //
@@ -34,6 +37,9 @@
 #endif
 #ifndef DEEP_TANGENT_DERIV
 #define DEEP_TANGENT_DERIV false
+#endif
+#ifndef DEEP_TANGENT_VJP
+#define DEEP_TANGENT_VJP false
 #endif
 #include "deep_tangent_kernels.cuh"
 #include "mlp_eval.cuh"
@@ -87,8 +93,9 @@ __host__ __device__ constexpr size_t grad_len(int H, int L) {
 
 template <int H, bool GRAD>
 __global__ void __launch_bounds__(NT, 1) DEEP_TANGENT_KERNEL(const __grid_constant__ DeepTangentArgs a) {
-    constexpr bool POINTS = DEEP_TANGENT_POINTS, DERIV = DEEP_TANGENT_DERIV;
+    constexpr bool POINTS = DEEP_TANGENT_POINTS, DERIV = DEEP_TANGENT_DERIV, VJP = DEEP_TANGENT_VJP;
     static_assert(POINTS || !DERIV, "the derivative stage reads per-point directions");
+    static_assert(!VJP || (POINTS && !DERIV && GRAD), "the VJP is a gradient at points");
     using Q = Geo<H, GRAD>;
     constexpr int G = Q::G, RB = Q::RB, NROW = Q::NROW, PTS_TILE = Q::PTS_TILE, ACT = Q::ACT;
     extern __shared__ __align__(16) float smem[];
@@ -250,7 +257,7 @@ __global__ void __launch_bounds__(NT, 1) DEEP_TANGENT_KERNEL(const __grid_consta
         }
         __syncthreads();   // s_act = a_L (5 rows per point)
         // ---- output layer: y_o strict (k_mlp_deep's order), J[o][k] with FFMA from +0, h ascending ------------------
-        for (int i = threadIdx.x; i < 4 * PTS_TILE; i += NT) {
+        for (int i = threadIdx.x; i < 4 * PTS_TILE && !VJP; i += NT) {   // the VJP's seeds do not depend on y or J
             const int o = i / PTS_TILE, pt = i - o * PTS_TILE;   // o is warp-uniform: W2 arrives by broadcast loads
             const float* src = s_act + ((pt / 32) * H) * ROWS + (pt % 32) * PT;
             const float* w2 = a.W2 + size_t(o) * H;
@@ -304,7 +311,18 @@ __global__ void __launch_bounds__(NT, 1) DEEP_TANGENT_KERNEL(const __grid_consta
 #pragma unroll
                 for (int k = 0; k < 4; ++k) seed[1 + k] = make_float4(Jb[0][k], Jb[1][k], Jb[2][k], Jb[3][k]);
             }
-            if (!DERIV && p < n_slab) {
+            if (VJP && p < n_slab) {   // the caller's cotangents: y_bar, and J_bar[p][o][k] (row o = one float4) by column
+                seed[0] = __ldg(a.ybar + p);
+                float4 jr[4];
+#pragma unroll
+                for (int o = 0; o < 4; ++o) jr[o] = __ldg(a.Jbar + 4 * p + o);
+                seed[1] = make_float4(jr[0].x, jr[1].x, jr[2].x, jr[3].x);
+                seed[2] = make_float4(jr[0].y, jr[1].y, jr[2].y, jr[3].y);
+                seed[3] = make_float4(jr[0].z, jr[1].z, jr[2].z, jr[3].z);
+                seed[4] = make_float4(jr[0].w, jr[1].w, jr[2].w, jr[3].w);
+                red[0] += double(seed[0].x); red[1] += double(seed[0].y); red[2] += double(seed[0].z); red[3] += double(seed[0].w);
+            }
+            if (!DERIV && !VJP && p < n_slab) {
                 const float s[3] = {a.sx, a.sy, a.sz};
                 float g[4][3];   // d y_o / d x_j
 #pragma unroll

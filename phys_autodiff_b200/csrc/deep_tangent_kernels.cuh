@@ -23,6 +23,9 @@
 //                            one float4 per point, its own time input; residuals (optional) AoS per point.
 //   k_deriv_tangent<H, GRAD>  the points kernel with another last stage (deriv_tangent_kernels.cu): GRAD = false writes
 //                            y and J per point; GRAD = true the derivative-fit loss of DESIGN section 4.13 and its gradient.
+//   k_vjp_tangent<H, true>   the points kernel seeded with the caller's cotangents (vjp_tangent_kernels.cu):
+//                            grad = sum_i (J_theta(y_i)^T y_bar_i + J_theta(J_i)^T : J_bar_i), the plain sum over the
+//                            points; the output layer's values are not computed.
 //   k_deep_tangent_reduce    sums the block partials in block order (bitwise repeatable): grad[P] and the two sums.
 // Gradient layout: that of deep_grad_kernels.cuh,  dW1 | db1 | dWh | dbh | dW2 | db2  (P = 9H + 4 + (L-1)(H^2 + H)).
 #pragma once
@@ -62,6 +65,9 @@ struct DeepTangentArgs {
     double lam[4];              // lam_o of the un-normalised sum (GRAD)
     float4* y_pts;              // [n_points] outputs y (not GRAD)
     float4* J_pts;              // [n_points][4] rows J[o][0..3] = dy_o / dc_k (not GRAD)
+    // VJP mode (vjp_tangent_launch), at the end likewise; sx .. scale_u, R_pts and the derivative fields are not read
+    const float4* ybar;         // [n_points] cotangents of y
+    const float4* Jbar;         // [n_points][4] cotangents of J, row o = {J_bar[o][0..3]} (the layout of J_pts)
 };
 
 constexpr int DEEP_TANGENT_THREADS = 256;
@@ -82,6 +88,9 @@ int colloc_tangent_launch(int H, bool grad, const DeepTangentArgs& a, int blocks
 // unused).  grad = true: the derivative-fit loss of DESIGN section 4.13 and its gradient, then deep_tangent_reduce, whose
 // acc[2] is {sum_i sum_o lam_o (D_io - g_io)^2, 0}.
 int deriv_tangent_launch(int H, bool grad, const DeepTangentArgs& a, int blocks, double* acc, double* grad_out, cudaStream_t st);
+// The same body at a.pts as k_vjp_tangent<H, true> (vjp_tangent_kernels.cu), any hidden_layers >= 1: seeds a.ybar (value
+// row) and a.Jbar (tangent rows), then deep_tangent_reduce, whose acc[2] is {0, 0}.
+int vjp_tangent_launch(int H, const DeepTangentArgs& a, int blocks, double* acc, double* grad_out, cudaStream_t st);
 // k_deep_tangent_reduce: the block partials [blocks][P + 2] summed in block order into grad[P] and acc[2].
 int deep_tangent_reduce(const double* partials, int blocks, size_t P, double* acc, double* grad, cudaStream_t st);
 

@@ -40,6 +40,7 @@ class Context:
         self.cfg: Optional[MLPConfig] = None
         self.hidden_layers: Optional[int] = None   # L of the network set by set_weights_deep
         self._peers = None  # (rank, world) once connect_peers() has mapped the peers' exchange buffers
+        self.weights_owner = None
 
     def close(self):
         if self._h:
@@ -128,6 +129,7 @@ class Context:
         check(self._lib.physad_set_weights(self._h, C.byref(c), ptr(W1), ptr(b1), ptr(W2), ptr(b2)), "set_weights")
         self.cfg = cfg
         self.hidden_layers = None   # a plain set_weights replaces any deep network
+        self.weights_owner = None
 
     # -- helpers -------------------------------------------------------------------------------
     @staticmethod
@@ -213,6 +215,7 @@ class Context:
               "set_weights_deep")
         self.cfg = cfg
         self.hidden_layers = hidden_layers
+        self.weights_owner = None   # autograd.DeepMLP: whose parameters (and which versions) the context holds
 
     def deep_loss(self, g: Grid, pw: PhysWeights, t: float, dt: float):
         """(L_sigma, L_u) of the deep network set by set_weights_deep, in one call (fields stay in context scratch)."""
@@ -493,6 +496,56 @@ class Context:
                                                          C.byref(loss), *[ptr(a) if a.size else None for a in g]),
               "deep_deriv_loss_grad_host")
         return (np.float32(loss.value), *g)
+
+    # -- vector-Jacobian products of deeper networks at arbitrary points (additive) ----------------------------------------
+    def mlp_vjp_deep(self, x, ybar, out=None):
+        """grad = sum_i ybar_i . dy_i / dtheta of the network set by set_weights_deep at the points x: x and ybar float32 CUDA
+        tensors [B, 4].  Returns a float64 device tensor [P] in the layout of the deep gradients (dW1 | db1 | dWh | dbh | dW2 |
+        db2): the plain sum over the points, unscaled, so shards add up and it adds to every other deep gradient.  The
+        backward of mlp_forward_deep (phys_autodiff_b200.autograd.DeepMLP)."""
+        import torch
+        x, ybar = x.contiguous(), ybar.contiguous()
+        B = x.numel() // 4
+        assert x.numel() == 4 * B and ybar.numel() == 4 * B
+        out = out if out is not None else self._empty(self.deep_grad_len(), torch.float64)
+        check(self._lib.physad_mlp_vjp_deep_dev(self._h, ptr(x), ptr(ybar), C.c_size_t(B), ptr(out), self._stream()),
+              "mlp_vjp_deep")
+        return out
+
+    def mlp_jacobian_vjp_deep(self, x, ybar, Jbar, out=None):
+        """grad = sum_i (ybar_i . dy_i / dtheta + Jbar_i : dJ_i / dtheta) at the points x: x, ybar float32 CUDA tensors [B, 4],
+        Jbar [B, 4, 4] in mlp_jacobian_deep's J layout (Jbar[i, o, k] pairs with dy_o / dc_k); ybar zeros for a loss on J
+        only.  Returns a float64 device tensor [P] as mlp_vjp_deep does.  The backward of mlp_jacobian_deep."""
+        import torch
+        x, ybar, Jbar = x.contiguous(), ybar.contiguous(), Jbar.contiguous()
+        B = x.numel() // 4
+        assert x.numel() == 4 * B and ybar.numel() == 4 * B and Jbar.numel() == 16 * B
+        out = out if out is not None else self._empty(self.deep_grad_len(), torch.float64)
+        check(self._lib.physad_mlp_jacobian_vjp_deep_dev(self._h, ptr(x), ptr(ybar), ptr(Jbar), C.c_size_t(B), ptr(out),
+                                                         self._stream()), "mlp_jacobian_vjp_deep")
+        return out
+
+    def mlp_vjp_deep_host(self, x, ybar):
+        """Host-array form of mlp_vjp_deep: x, ybar [B, 4] -> (dW1, db1, dWh, dbh, dW2, db2), float32."""
+        x, ybar = _f32(x), _f32(ybar)
+        B = x.size // 4
+        assert x.size == 4 * B and ybar.size == 4 * B
+        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
+        g = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        check(self._lib.physad_mlp_vjp_deep_host(self._h, ptr(x), ptr(ybar), C.c_size_t(B),
+                                                 *[ptr(a) if a.size else None for a in g]), "mlp_vjp_deep_host")
+        return tuple(g)
+
+    def mlp_jacobian_vjp_deep_host(self, x, ybar, Jbar):
+        """Host-array form of mlp_jacobian_vjp_deep: x, ybar [B, 4], Jbar [B, 4, 4] -> (dW1, db1, dWh, dbh, dW2, db2), float32."""
+        x, ybar, Jbar = _f32(x), _f32(ybar), _f32(Jbar)
+        B = x.size // 4
+        assert x.size == 4 * B and ybar.size == 4 * B and Jbar.size == 16 * B
+        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
+        g = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        check(self._lib.physad_mlp_jacobian_vjp_deep_host(self._h, ptr(x), ptr(ybar), ptr(Jbar), C.c_size_t(B),
+                                                          *[ptr(a) if a.size else None for a in g]), "mlp_jacobian_vjp_deep_host")
+        return tuple(g)
 
     # -- analytic loss of deeper networks at arbitrary points (collocation points; additive) -------------------------------
     @staticmethod
@@ -814,6 +867,7 @@ class Context:
                                                       C.byref(cw), C.c_float(t), C.byref(ls), C.byref(lu),
                                                       *[ptr(x) for x in d]), "tangent_loss_grad_host")
         self.cfg = cfg
+        self.weights_owner = None
         return (np.float32(ls.value), np.float32(lu.value), *d)
 
     # -- closed loop: loss + gradient with respect to the MLP weights (additive) ----------------------------
@@ -865,6 +919,7 @@ class Context:
                                                     C.byref(cw), C.c_float(t), C.c_float(dt), C.byref(ls), C.byref(lu),
                                                     *[ptr(x) for x in d]), "fused_loss_grad_host")
         self.cfg = cfg
+        self.weights_owner = None
         return (np.float32(ls.value), np.float32(lu.value), *d)
 
     # -- host-buffer forms (the reference's contract) -----------------------------------------------------
@@ -878,6 +933,7 @@ class Context:
                                                C.byref(cw), C.c_float(t), C.c_float(dt), C.byref(ls), C.byref(lu),
                                                *[ptr(r) for r in R]), "fused_loss_host")
         self.cfg = cfg
+        self.weights_owner = None
         return (np.float32(ls.value), np.float32(lu.value)) + ((tuple(R),) if want_residuals else ())
 
     def prepare_step_host(self, g: Grid, cfg: MLPConfig, W1, b1, W2, b2, pw: PhysWeights, t: float, dt: float, slab=None):
@@ -892,6 +948,7 @@ class Context:
                 C.c_float(dt), C.c_int(1 if self._peers else 0), C.byref(ls), C.byref(lu))
         keep = (cg, cs, cc, cw, W1, b1, W2, b2)
         self.cfg = cfg
+        self.weights_owner = None
 
         def step(_keep=keep):
             rc = fn(h, *args)
@@ -1067,6 +1124,7 @@ def mlp_phys_loss_tangent_cuda(g: Grid, cfg: MLPConfig, w, pw: PhysWeights, t: f
     check(c._lib.physad_tangent_loss_host(c._h, C.byref(cg), C.byref(cc), ptr(W1), ptr(b1), ptr(W2), ptr(b2), C.byref(cw),
                                           C.c_float(t), C.byref(ls), C.byref(lu)), "tangent_loss_host")
     c.cfg = cfg
+    c.weights_owner = None
     return np.float32(ls.value), np.float32(lu.value)
 
 
@@ -1142,3 +1200,19 @@ def mlp_phys_loss_deep_tangent_points_grad_cuda(cfg: MLPConfig, L: int, w, x: np
     c = default_context()
     c.set_weights_deep(cfg, L, *w)
     return c.deep_tangent_points_loss_grad_host(x, dcdx, pw)
+
+
+def mlp_vjp_deep_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, ybar: np.ndarray):
+    """Vector-Jacobian product of a deep network (additive): w = (W1, b1, Wh, bh, W2, b2), x, ybar [B, 4] ->
+    (dW1, db1, dWh, dbh, dW2, db2) = sum_i ybar_i . dy_i / dtheta, the plain sum over the points."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.mlp_vjp_deep_host(x, ybar)
+
+
+def mlp_jacobian_vjp_deep_cuda(cfg: MLPConfig, L: int, w, x: np.ndarray, ybar: np.ndarray, Jbar: np.ndarray):
+    """Vector-Jacobian product of a deep network and its Jacobian (additive): x, ybar [B, 4], Jbar [B, 4, 4] ->
+    (dW1, db1, dWh, dbh, dW2, db2) = sum_i (ybar_i . dy_i / dtheta + Jbar_i : dJ_i / dtheta)."""
+    c = default_context()
+    c.set_weights_deep(cfg, L, *w)
+    return c.mlp_jacobian_vjp_deep_host(x, ybar, Jbar)

@@ -24,7 +24,12 @@ its partner's output); one JSON line per pair and B, and with --out the whole ru
 points physics loss + gradient step and loss (physad_deep_tangent_points_loss_grad_dev / _dev) at the same points and the
 forward at points (physad_mlp_forward_deep_dev); one JSON line per pair and B, and with --out the whole run as one JSON
 document.
-  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent|deep-data|deep-tangent-points|deep-pair|deep-deriv]
+--loss deep-vjp times the vector-Jacobian products at B = 2^24 and 65 536 points for every --hidden x --layers pair, in
+alternation: physad_mlp_vjp_deep_dev against the data loss + gradient step, physad_mlp_jacobian_vjp_deep_dev against the
+derivative-fit loss + gradient step, and the whole physics step through autograd.DeepMLP (forward with the Jacobian, the
+residual loss in torch, .backward(), with and without the weight upload an optimizer step causes) against the fused points
+physics loss + gradient step; one JSON line per pair and B, and with --out the whole run as one JSON document.
+  python tools/bench_grad.py [--loss fd|tangent|deep|deep-tangent|deep-data|deep-tangent-points|deep-pair|deep-deriv|deep-vjp]
                              [--n 256] [--hidden 64]
                              [--layers 3] [--steps 20]
   python tools/bench_grad.py --loss deep --hidden 32,64,128 --layers 2,3,5
@@ -48,11 +53,13 @@ def main():
     ap.add_argument("--layers", default="3", help="--loss deep: hidden layers, a comma-separated list")
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--loss", choices=("fd", "tangent", "deep", "deep-tangent", "deep-data", "deep-tangent-points", "deep-pair",
-                                       "deep-deriv"), default="fd")
+                                       "deep-deriv", "deep-vjp"), default="fd")
     ap.add_argument("--out", default=None,
-                    help="--loss deep-data / deep-tangent-points / deep-pair / deep-deriv: also write the run as one JSON "
-                         "document here")
+                    help="--loss deep-data / deep-tangent-points / deep-pair / deep-deriv / deep-vjp: also write the run as "
+                         "one JSON document here")
     a = ap.parse_args()
+    if a.loss == "deep-vjp":
+        return deep_vjp(a)
     if a.loss == "deep-deriv":
         return deep_deriv(a)
     if a.loss == "deep-pair":
@@ -496,6 +503,96 @@ def deep_deriv(a):
                                f"physics loss + gradient step at the same B uniform random space-time points, the Jacobian "
                                f"query, the physics loss and the forward at those points, timed in alternation (CUDA events, "
                                f"median of {a.steps}); B = {sizes[0]} and {sizes[1]}",
+                       "gpu": name, "power_limit_w": plim, "results": results}, fh, indent=1)
+
+
+def deep_vjp(a):
+    import numpy as np
+    from phys_autodiff_b200.autograd import DeepMLP
+    ctx = ops.Context()
+    pw = PhysWeights(1, 1)
+    name, plim = _gpu()
+    dcdx = ops.grid_input_scales(Grid(256, 256, 256), True)
+    s = torch.tensor(dcdx, device="cuda")
+    rng = np.random.default_rng(5)
+    sizes = (1 << 24, 65536)   # 2^24 points (well past L2), and the overhead regime
+    pts = {}
+    for B in sizes:
+        x = rng.uniform(-1, 1, (B, 4)).astype(np.float32)
+        x[:, 3] = rng.uniform(0.0, 0.5, B).astype(np.float32)
+        d = np.zeros((B, 4), np.float32)
+        ax = np.arange(B) % 3
+        d[np.arange(B), ax] = dcdx[ax]
+        t = rng.uniform(-0.5, 0.5, (B, 4)).astype(np.float32)
+        pts[B] = tuple(torch.from_numpy(v).cuda() for v in (x, d, t))
+    results = []
+    for H in (int(v) for v in a.hidden.split(",")):
+        w1 = ops.mlp_random_init(H, 777, 0.25)
+        for L in (int(v) for v in a.layers.split(",")):
+            wr = np.random.default_rng(L)
+            Wh = wr.uniform(-0.2, 0.2, (L - 1) * H * H).astype(np.float32)
+            bh = wr.uniform(-0.2, 0.2, (L - 1) * H).astype(np.float32)
+            w = (w1[0], w1[1], Wh, bh, w1[2], w1[3])
+            model = DeepMLP(ctx, H, L, w)
+            for B in sizes:
+                x, d, t = pts[B]
+                ctx.set_weights_deep(MLPConfig(4, H, 4, True), L, *w)
+                yb = (ctx.mlp_forward_deep(x) - t) * (0.5 / B)
+                _, J = ctx.mlp_jacobian_deep(x)
+                Jb = (J * (0.5 / B)).contiguous()
+                gv, gj = ctx.mlp_vjp_deep(x, yb), ctx.mlp_jacobian_vjp_deep(x, yb, Jb)
+                dout = ctx.deep_data_loss_grad_acc(x, t)
+                vout = ctx.deep_deriv_loss_grad_acc(x, d, t)
+                pout = ctx.deep_tangent_points_loss_grad_acc(x, dcdx, pw)
+
+                def bridge(sync):
+                    if sync:   # what an optimizer step does to the parameters: their versions move, the module re-uploads
+                        with torch.no_grad():
+                            for p in model.parameters():
+                                p.add_(0)
+                    for p in model.parameters():
+                        p.grad = None
+                    y, Jm = model(x, jacobian=True)
+                    gr = Jm[:, :, :3] * s
+                    div = (gr[:, 1, 0] + gr[:, 2, 1]) + gr[:, 3, 2]
+                    R = Jm[:, :, 3] + ((y[:, 1:2] * gr[:, :, 0] + y[:, 2:3] * gr[:, :, 1]) + y[:, 3:4] * gr[:, :, 2])
+                    Rs = R[:, 0] + y[:, 0] * div
+                    ((Rs * Rs).sum() / B + (R[:, 1:] * R[:, 1:]).sum() / B).backward()
+                calls = {"vjp": lambda: ctx.mlp_vjp_deep(x, yb, out=gv),
+                         "data_loss_grad": lambda: ctx.deep_data_loss_grad_acc(x, t, out=dout),
+                         "jacobian_vjp": lambda: ctx.mlp_jacobian_vjp_deep(x, yb, Jb, out=gj),
+                         "deriv_loss_grad": lambda: ctx.deep_deriv_loss_grad_acc(x, d, t, out=vout),
+                         "bridge_step": lambda: bridge(True),
+                         "bridge_step_no_upload": lambda: bridge(False),
+                         "points_loss_grad": lambda: (ctx.set_weights_deep(MLPConfig(4, H, 4, True), L, *w),
+                                                      ctx.deep_tangent_points_loss_grad_acc(x, dcdx, pw, out=pout))}
+                for _ in range(2):
+                    for fn in calls.values():
+                        fn()
+                torch.cuda.synchronize()
+                ts = {k: [] for k in calls}
+                for _ in range(a.steps):   # in alternation, so that they share whatever else the GPU is doing
+                    for k, fn in calls.items():
+                        ts[k] += _times(fn, 1)
+                med = {k: sorted(v)[len(v) // 2] for k, v in ts.items()}
+                r = {"workload": f"H={H} L={L} B={B} points: VJPs vs their sibling losses, the DeepMLP physics step vs the "
+                                 f"fused points physics step", "points": B, **{k + "_ms": v for k, v in med.items()},
+                     "vjp_to_data_ratio": med["vjp"] / med["data_loss_grad"],
+                     "jacobian_vjp_to_deriv_ratio": med["jacobian_vjp"] / med["deriv_loss_grad"],
+                     "bridge_to_fused_ratio": med["bridge_step"] / med["points_loss_grad"],
+                     "weight_upload_ms": med["bridge_step"] - med["bridge_step_no_upload"],
+                     "gpu": name, "power_limit_w": plim}
+                results.append(r)
+                print(json.dumps(r), flush=True)
+                ctx.weights_owner = None
+    if a.out:
+        with open(a.out, "w") as fh:
+            json.dump({"what": f"tools/bench_grad.py --loss deep-vjp --hidden {a.hidden} --layers {a.layers} --steps {a.steps}: "
+                               f"mlp_vjp_deep vs deep_data_loss_grad, mlp_jacobian_vjp_deep vs deep_deriv_loss_grad, and the "
+                               f"DeepMLP physics step (Jacobian forward, residuals in torch, backward; with the weight upload "
+                               f"of an optimizer step, and without) vs deep_tangent_points_loss_grad with set_weights_deep, "
+                               f"at the same B uniform random space-time points, timed in alternation (CUDA events, median "
+                               f"of {a.steps}); B = {sizes[0]} and {sizes[1]}",
                        "gpu": name, "power_limit_w": plim, "results": results}, fh, indent=1)
 
 
