@@ -14,6 +14,7 @@
 #include "tangent_kernels.cuh"
 
 #include <algorithm>
+#include <array>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -73,16 +74,14 @@ struct physad_ctx {
     size_t gws_cap = 0;
     double* gpart = nullptr;
     size_t gpart_cap = 0;
-    double* d_grad = nullptr;   // [9 * 128 + 4]
-    double* h_grad = nullptr;   // pinned, same size
     int grad_blocks_per_sm[3] = {0, 0, 0};   // HT = 32, 64, 128 on this device
     int tgrad_blocks_per_sm[3] = {0, 0, 0};  // the same for the tangent-loss gradient (physad_tangent_loss_grad_*)
-    // deep closed loop (physad_deep_loss_grad_*): per-block activation checkpoints, host-form result buffers
+    // deep closed loop (physad_deep_loss_grad_*): per-block activation checkpoints; the host forms' result [acc | grad]
     float* dckpt = nullptr;
     size_t dckpt_cap = 0;
     double* d_dgrad = nullptr;   // [P + 2]
     double* h_dgrad = nullptr;   // pinned, same size
-    size_t dgrad_cap = 0;
+    size_t d_dgrad_cap = 0, h_dgrad_cap = 0;
     uint64_t launches = 0;
     int fused_variant = 0;
     int exact_residuals = 0;  // 1: residual arithmetic in double exactly as the CPU reference; 0: fp32 with FMAs
@@ -122,25 +121,25 @@ struct physad_ctx {
 
 namespace {
 
-int ensure_partials(physad_ctx* c, size_t blocks) {
-    if (blocks <= c->partials_cap) return 0;
-    if (c->partials) CU(cudaFree(c->partials));
-    c->partials = nullptr;
-    c->partials_cap = 0;
-    CU(cudaMalloc(&c->partials, blocks * sizeof(double2)));
-    c->partials_cap = blocks;
+// Grow the context buffer p of cap elements to at least n (device memory, or pinned host memory).  It never shrinks and
+// keeps no contents: every caller refills the buffer.  The old buffer is freed before the new one is allocated, so the peak
+// does not double, and a failed allocation leaves (nullptr, 0) so that the next call tries again.
+template <class T>
+int grow(T*& p, size_t& cap, size_t n, bool pinned = false) {
+    if (n <= cap) return 0;
+    if (p) CU(pinned ? cudaFreeHost(p) : cudaFree(p));
+    p = nullptr;
+    cap = 0;
+    void* q = nullptr;
+    CU(pinned ? cudaMallocHost(&q, n * sizeof(T)) : cudaMalloc(&q, n * sizeof(T)));
+    p = static_cast<T*>(q);
+    cap = n;
     return 0;
 }
 
-int ensure_scratch(physad_ctx* c, size_t bytes) {
-    if (bytes <= c->scratch_cap) return 0;
-    if (c->scratch) CU(cudaFree(c->scratch));
-    c->scratch = nullptr;
-    c->scratch_cap = 0;
-    CU(cudaMalloc(&c->scratch, bytes));
-    c->scratch_cap = bytes;
-    return 0;
-}
+int ensure_partials(physad_ctx* c, size_t blocks) { return grow(c->partials, c->partials_cap, blocks); }
+int ensure_scratch(physad_ctx* c, size_t bytes) { return grow(c->scratch, c->scratch_cap, bytes); }
+int ensure_grad_partials(physad_ctx* c, size_t doubles) { return grow(c->gpart, c->gpart_cap, doubles); }
 
 int check_grid(const physad_grid* g) {
     if (!g) return fail(PHYSAD_E_INVALID, "grid is null");
@@ -233,12 +232,7 @@ int ensure_coord_tables(physad_ctx* c, const physad_grid* g, cudaStream_t st) {
     for (int i = 0; i < g->nx; ++i) host[i] = host_axis_coord(i, g->nx, m1p1);
     for (int i = 0; i < g->ny; ++i) host[g->nx + i] = host_axis_coord(i, g->ny, m1p1);
     for (int i = 0; i < g->nz; ++i) host[g->nx + g->ny + i] = host_axis_coord(i, g->nz, m1p1);
-    if (nf > t.cap) {
-        if (t.dev) CU(cudaFree(t.dev));
-        t.dev = nullptr; t.cap = 0;
-        CU(cudaMalloc(&t.dev, nf * sizeof(float)));
-        t.cap = nf;
-    }
+    if (int rc = grow(t.dev, t.cap, nf)) return rc;
     // rare path: copy on the CONSUMING stream and wait, so the first kernel after a geometry change cannot read
     // stale tables (a NULL-stream copy is not ordered against a cudaStreamNonBlocking stream) and the pageable
     // staging vector may die at the end of this scope
@@ -302,12 +296,7 @@ int build_fused_plan(physad_ctx* c, const physad_grid* g, const physad_slab& s, 
     const long long want = std::min<long long>(slots, (long long)tiles * nzl);
     const std::vector<int> ranges = balanced_ranges(tiles, nzl, want, 0.9);
     const size_t bytes = ranges.size() * sizeof(int);
-    if (bytes > p.cap) {
-        if (p.dev) CU(cudaFree(p.dev));
-        p.dev = nullptr; p.cap = 0;
-        CU(cudaMalloc(&p.dev, bytes));
-        p.cap = bytes;
-    }
+    if (int rc = grow(p.dev, p.cap, bytes)) return rc;
     CU(cudaMemcpyAsync(p.dev, ranges.data(), bytes, cudaMemcpyHostToDevice, st));   // same ordering rule as the coordinate tables
     CU(cudaStreamSynchronize(st));
     p.ranges = reinterpret_cast<const int*>(p.dev);
@@ -576,6 +565,60 @@ void vjp_scales(const physad_grid* g, const physad_phys_weights* w, float* ss, f
     *su = 2.f * w->w_u / float(N);
 }
 
+// dc/dx of the three space inputs of a grid: a coordinate c = norm(i / (n - 1)) sampled at x = i h has dc/dx = f / ((n-1) h),
+// f = 2 for MinusOneToOne (norm 1), 1 for ZeroToOne, and 0 for an extent of 1
+void input_scales(const physad_grid* g, int norm, float s[3]) {
+    const double f = norm == 1 ? 2.0 : 1.0;
+    s[0] = g->nx > 1 ? float(f / (double(g->nx - 1) * double(g->hx))) : 0.f;
+    s[1] = g->ny > 1 ? float(f / (double(g->ny - 1) * double(g->hy))) : 0.f;
+    s[2] = g->nz > 1 ? float(f / (double(g->nz - 1) * double(g->hz))) : 0.f;
+}
+
+int check_residual_outputs(const float* Rs, const float* Rx, const float* Ry, const float* Rz, const char* what) {
+    const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
+    if (any && !all) return fail(PHYSAD_E_INVALID, std::string(what) + ": residual outputs must be all set or all null");
+    return 0;
+}
+
+// The result of an empty slab or shard: nacc zero sums in acc and, if grad is set, a zero gradient of P entries
+int zero_result(double* acc, int nacc, double* grad, size_t P, cudaStream_t st) {
+    if (nacc) CU(cudaMemsetAsync(acc, 0, nacc * sizeof(double), st));
+    if (grad) CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
+    return 0;
+}
+
+// One array of a host-pointer call, staged in the context's scratch: `up` is uploaded before the device call, `down`
+// downloaded after it; either may be null (an input only, an output only, an output the caller did not ask for, or
+// workspace).  `dev` is the array's place in scratch.
+struct Staged {
+    const void* up;
+    void* down;
+    size_t bytes;
+    float* dev = nullptr;
+};
+
+// Lay the arrays out in scratch, each at a 256-byte aligned offset, and upload the inputs on c->stream.
+template <size_t K>
+int stage_in(physad_ctx* c, Staged (&a)[K]) {
+    size_t off[K + 1] = {0};
+    for (size_t k = 0; k < K; ++k) off[k + 1] = off[k] + ((a[k].bytes + 255) & ~size_t(255));
+    if (int rc = grow(c->scratch, c->scratch_cap, off[K])) return rc;
+    for (size_t k = 0; k < K; ++k) {
+        a[k].dev = reinterpret_cast<float*>(c->scratch + off[k]);
+        if (a[k].up && a[k].bytes) CU(cudaMemcpyAsync(a[k].dev, a[k].up, a[k].bytes, cudaMemcpyHostToDevice, c->stream));
+    }
+    return 0;
+}
+
+// After the device call: download the outputs and synchronise c->stream once.
+template <size_t K>
+int stage_out(physad_ctx* c, const Staged (&a)[K]) {
+    for (const Staged& s : a)
+        if (s.down && s.bytes) CU(cudaMemcpyAsync(s.down, s.dev, s.bytes, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
 struct DeviceGuard {
     int prev = -1;
     explicit DeviceGuard(int dev) {
@@ -598,13 +641,7 @@ int launch_grad(physad_ctx* c, int HT, const GradArgs& a, float4* adj, size_t ch
         if (bps < 1) return fail(PHYSAD_E_UNSUPPORTED, "fused_loss_grad: kernel does not fit an SM");
     }
     const size_t blocks = std::max<size_t>(1, std::min<size_t>(chunks, size_t(c->sm_count) * bps));
-    const size_t need = blocks * (GRAD_NACC * HT + 6);
-    if (need > c->gpart_cap) {
-        if (c->gpart) CU(cudaFree(c->gpart));
-        c->gpart = nullptr; c->gpart_cap = 0;
-        CU(cudaMalloc(&c->gpart, need * sizeof(double)));
-        c->gpart_cap = need;
-    }
+    if (int rc = ensure_grad_partials(c, blocks * (GRAD_NACC * HT + 6))) return rc;
     GradArgs k = a;
     k.partials = c->gpart;
     c->launches += 2;
@@ -621,12 +658,7 @@ int upload_weights_if_stale(physad_ctx* c, cudaStream_t st) {
     float** dev[4] = {&c->dW1, &c->db1, &c->dW2, &c->db2};
     for (int k = 0; k < 4; ++k) {
         const size_t n = host[k]->size();
-        if (n > c->dW_cap[k]) {
-            if (*dev[k]) CU(cudaFree(*dev[k]));
-            *dev[k] = nullptr;
-            CU(cudaMalloc(dev[k], n * sizeof(float)));
-            c->dW_cap[k] = n;
-        }
+        if (int rc = grow(*dev[k], c->dW_cap[k], n)) return rc;
         // pageable source: the copy is staged before the call returns, so the host vector may change afterwards
         CU(cudaMemcpyAsync(*dev[k], host[k]->data(), n * sizeof(float), cudaMemcpyHostToDevice, st));
     }
@@ -739,8 +771,7 @@ int physad_ctx_destroy(physad_ctx* c) {
     cudaFree(c->tab.dev);
     cudaFree(c->d_wh); cudaFree(c->d_bh); cudaFree(c->d_wparts);
     cudaFree(c->partials); cudaFree(c->ticket); cudaFree(c->d_acc); cudaFree(c->scratch);
-    cudaFree(c->gws); cudaFree(c->gpart); cudaFree(c->d_grad);
-    if (c->h_grad) cudaFreeHost(c->h_grad);
+    cudaFree(c->gws); cudaFree(c->gpart);
     cudaFree(c->dckpt); cudaFree(c->d_dgrad);
     if (c->h_dgrad) cudaFreeHost(c->h_dgrad);
     if (c->h_acc) cudaFreeHost(c->h_acc);
@@ -848,16 +879,10 @@ int physad_mlp_forward_host(physad_ctx* c, const float* x, float* y, size_t B) {
     if (int rc = need_one_layer(c, "mlp_forward", "physad_mlp_forward_deep_dev")) return rc;
     if (B == 0) return 0;
     DeviceGuard dg(c->device);
-    const size_t nx = B * size_t(c->cfg.In) * sizeof(float), ny = B * size_t(c->cfg.Out) * sizeof(float);
-    const size_t off_y = (nx + 255) & ~size_t(255);
-    if (int rc = ensure_scratch(c, off_y + ny)) return rc;
-    float* dx = reinterpret_cast<float*>(c->scratch);
-    float* dy = reinterpret_cast<float*>(c->scratch + off_y);
-    CU(cudaMemcpyAsync(dx, x, nx, cudaMemcpyHostToDevice, c->stream));
-    if (int rc = physad_mlp_forward_dev(c, dx, dy, B, c->stream)) return rc;
-    CU(cudaMemcpyAsync(y, dy, ny, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
+    Staged a[2] = {{x, nullptr, B * c->cfg.In * sizeof(float)}, {nullptr, y, B * c->cfg.Out * sizeof(float)}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_mlp_forward_dev(c, a[0].dev, a[1].dev, B, c->stream)) return rc;
+    return stage_out(c, a);
 }
 
 int physad_mlp_backward_dev(physad_ctx* c, const float* x, const float* y_target, float* dW1, float* db1, float* dW2,
@@ -906,21 +931,12 @@ int physad_mlp_backward_host(physad_ctx* c, const float* x, const float* y_targe
     if (!c->has_weights) return fail(PHYSAD_E_NOWEIGHTS, "mlp_backward: no weights set");
     if (int rc = need_one_layer(c, "mlp_backward", "physad_deep_data_loss_grad_dev")) return rc;
     DeviceGuard dg(c->device);
-    const size_t In = c->cfg.In, H = c->cfg.H, Out = c->cfg.Out;
-    const size_t n[6] = {B * In, B * Out, H * In, H, Out * H, Out};
-    size_t off[7] = {0};
-    for (int k = 0; k < 6; ++k) off[k + 1] = off[k] + ((n[k] * sizeof(float) + 255) & ~size_t(255));
-    if (int rc = ensure_scratch(c, off[6])) return rc;
-    float* d[6];
-    for (int k = 0; k < 6; ++k) d[k] = reinterpret_cast<float*>(c->scratch + off[k]);
-    CU(cudaMemcpyAsync(d[0], x, n[0] * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    CU(cudaMemcpyAsync(d[1], y_target, n[1] * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    if (int rc = physad_mlp_backward_dev(c, d[0], d[1], d[2], d[3], d[4], d[5], B, c->stream)) return rc;
-    float* dst[4] = {dW1, db1, dW2, db2};
-    for (int k = 0; k < 4; ++k)
-        CU(cudaMemcpyAsync(dst[k], d[2 + k], n[2 + k] * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
+    const size_t In = c->cfg.In, H = c->cfg.H, Out = c->cfg.Out, f = sizeof(float);
+    Staged a[6] = {{x, nullptr, B * In * f}, {y_target, nullptr, B * Out * f}, {nullptr, dW1, H * In * f},
+                   {nullptr, db1, H * f}, {nullptr, dW2, Out * H * f}, {nullptr, db2, Out * f}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_mlp_backward_dev(c, a[0].dev, a[1].dev, a[2].dev, a[3].dev, a[4].dev, a[5].dev, B, c->stream)) return rc;
+    return stage_out(c, a);
 }
 
 int physad_mlp_grid_infer_dev(physad_ctx* c, const physad_grid* g, const physad_slab* slab, float t, float* out,
@@ -943,12 +959,10 @@ int physad_mlp_grid_infer_host(physad_ctx* c, const physad_grid* g, float t, flo
     if (!c || !out) return fail(PHYSAD_E_INVALID, "mlp_grid_infer: null argument");
     if (int rc = check_grid(g)) return rc;
     DeviceGuard dg(c->device);
-    const size_t bytes = size_t(g->nx) * g->ny * g->nz * 4 * sizeof(float);
-    if (int rc = ensure_scratch(c, bytes)) return rc;
-    if (int rc = physad_mlp_grid_infer_dev(c, g, nullptr, t, reinterpret_cast<float*>(c->scratch), c->stream)) return rc;
-    CU(cudaMemcpyAsync(out, c->scratch, bytes, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
+    Staged a[1] = {{nullptr, out, size_t(g->nx) * g->ny * g->nz * 4 * sizeof(float)}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_mlp_grid_infer_dev(c, g, nullptr, t, a[0].dev, c->stream)) return rc;
+    return stage_out(c, a);
 }
 
 int physad_mlp_generate_fields_dev(physad_ctx* c, const physad_grid* g, const physad_slab* slab, float t, float dt,
@@ -970,20 +984,17 @@ int physad_mlp_generate_fields_dev(physad_ctx* c, const physad_grid* g, const ph
 int physad_mlp_generate_fields_host(physad_ctx* c, const physad_grid* g, float t, float dt, float* s_m, float* s_0,
                                     float* s_p, float* u_m, float* u_0, float* u_p) {
     if (!c) return fail(PHYSAD_E_INVALID, "generate_fields: null context");
+    if (!s_m || !s_0 || !s_p || !u_m || !u_0 || !u_p) return fail(PHYSAD_E_INVALID, "generate_fields: null argument");
     if (int rc = check_grid(g)) return rc;
     DeviceGuard dg(c->device);
-    const size_t N = size_t(g->nx) * g->ny * g->nz;
-    if (int rc = ensure_scratch(c, 12 * N * sizeof(float))) return rc;
-    float* d = reinterpret_cast<float*>(c->scratch);
-    if (int rc = physad_mlp_generate_fields_dev(c, g, nullptr, t, dt, d, d + N, d + 2 * N, d + 3 * N, d + 6 * N, d + 9 * N,
+    const size_t n = size_t(g->nx) * g->ny * g->nz * sizeof(float);
+    Staged a[6] = {{nullptr, s_m, n}, {nullptr, s_0, n}, {nullptr, s_p, n},
+                   {nullptr, u_m, 3 * n}, {nullptr, u_0, 3 * n}, {nullptr, u_p, 3 * n}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_mlp_generate_fields_dev(c, g, nullptr, t, dt, a[0].dev, a[1].dev, a[2].dev, a[3].dev, a[4].dev, a[5].dev,
                                                 c->stream))
         return rc;
-    float* dst[6] = {s_m, s_0, s_p, u_m, u_0, u_p};
-    const size_t off[6] = {0, N, 2 * N, 3 * N, 6 * N, 9 * N}, cnt[6] = {N, N, N, 3 * N, 3 * N, 3 * N};
-    for (int k = 0; k < 6; ++k)
-        CU(cudaMemcpyAsync(dst[k], d + off[k], cnt[k] * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
+    return stage_out(c, a);
 }
 
 // ---- deeper MLPs (additive; BASELINE config 5) ------------------------------------------------------
@@ -1004,30 +1015,14 @@ int physad_set_weights_deep(physad_ctx* c, const physad_mlp_config* cfg, int hid
                 wt[(l * H + h) * H + g] = Wh[(l * H + g + 1) * H + h];
                 wt[(l * H + h) * H + g + 1] = Wh[(l * H + g) * H + h];
             }
-    if (wt.size() > c->d_wh_cap) {
-        if (c->d_wh) CU(cudaFree(c->d_wh));
-        c->d_wh = nullptr; c->d_wh_cap = 0;
-        CU(cudaMalloc(&c->d_wh, wt.size() * sizeof(float)));
-        c->d_wh_cap = wt.size();
-    }
-    const size_t nb = std::max<size_t>(1, nl * H);
-    if (nb > c->d_bh_cap) {
-        if (c->d_bh) CU(cudaFree(c->d_bh));
-        c->d_bh = nullptr; c->d_bh_cap = 0;
-        CU(cudaMalloc(&c->d_bh, nb * sizeof(float)));
-        c->d_bh_cap = nb;
-    }
+    if (int rc = grow(c->d_wh, c->d_wh_cap, wt.size())) return rc;
+    if (int rc = grow(c->d_bh, c->d_bh_cap, std::max<size_t>(1, nl * H))) return rc;
     // fast mode (physad_set_deep_mode): every layer as three bf16 terms in the MMA's shared-memory layout
     std::vector<uint8_t> images;
     if (deep_tc_supported(int(H), hidden_layers)) {
         images.resize(nl * deep_tc_layer_bytes(int(H)));
         for (size_t l = 0; l < nl; ++l) deep_tc_pack_layer(int(H), Wh + l * H * H, images.data() + l * deep_tc_layer_bytes(int(H)));
-        if (images.size() > c->d_wparts_cap) {
-            if (c->d_wparts) CU(cudaFree(c->d_wparts));
-            c->d_wparts = nullptr; c->d_wparts_cap = 0;
-            CU(cudaMalloc(&c->d_wparts, images.size()));
-            c->d_wparts_cap = images.size();
-        }
+        if (int rc = grow(c->d_wparts, c->d_wparts_cap, images.size())) return rc;
     }
     CU(cudaDeviceSynchronize());   // kernels of ANY stream may still read the previous layers
     if (nl) {
@@ -1118,13 +1113,15 @@ int physad_deep_loss_host(physad_ctx* c, const physad_grid* g, const physad_phys
     if (int rc = check_grid(g)) return rc;
     if (int rc = deep_ready(c, "deep_loss")) return rc;
     DeviceGuard dg(c->device);
-    const size_t N = size_t(g->nx) * g->ny * g->nz;
-    if (int rc = ensure_scratch(c, 12 * N * sizeof(float))) return rc;
-    float* f = reinterpret_cast<float*>(c->scratch);   // sigma_{-,0,+} (N each) | u_{-,0,+} (3N each)
-    if (int rc = physad_mlp_generate_fields_deep_dev(c, g, nullptr, t, dt, f, f + N, f + 2 * N, f + 3 * N, f + 6 * N, f + 9 * N, c->stream))
+    const size_t N = size_t(g->nx) * g->ny * g->nz, n = N * sizeof(float);
+    Staged f[6] = {{nullptr, nullptr, n}, {nullptr, nullptr, n}, {nullptr, nullptr, n},   // sigma_{-,0,+}, u_{-,0,+}: workspace
+                   {nullptr, nullptr, 3 * n}, {nullptr, nullptr, 3 * n}, {nullptr, nullptr, 3 * n}};
+    if (int rc = stage_in(c, f)) return rc;
+    if (int rc = physad_mlp_generate_fields_deep_dev(c, g, nullptr, t, dt, f[0].dev, f[1].dev, f[2].dev, f[3].dev, f[4].dev, f[5].dev,
+                                                     c->stream))
         return rc;
-    if (int rc = physad_phys_loss_dev(c, g, f, f + N, f + 2 * N, f + 3 * N, f + 6 * N, f + 9 * N, c->d_acc, nullptr, nullptr, nullptr,
-                                      nullptr, c->stream))
+    if (int rc = physad_phys_loss_dev(c, g, f[0].dev, f[1].dev, f[2].dev, f[3].dev, f[4].dev, f[5].dev, c->d_acc, nullptr, nullptr,
+                                      nullptr, nullptr, c->stream))
         return rc;
     CU(cudaMemcpyAsync(c->h_acc, c->d_acc, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
@@ -1179,13 +1176,12 @@ int physad_phys_loss_lp_dev(physad_ctx* c, const physad_grid* g, int dtype, cons
     if (!c || !s_m || !s_0 || !s_p || !u_m || !u_0 || !u_p || !acc) return fail(PHYSAD_E_INVALID, "phys_loss_lp: null argument");
     if (dtype != PHYSAD_F16 && dtype != PHYSAD_BF16) return fail(PHYSAD_E_INVALID, "phys_loss_lp: dtype must be PHYSAD_F16 or PHYSAD_BF16");
     if (int rc = check_grid(g)) return rc;
-    const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
-    if (any && !all) return fail(PHYSAD_E_INVALID, "phys_loss_lp: residual outputs must be all set or all null");
+    if (int rc = check_residual_outputs(Rs, Rx, Ry, Rz, "phys_loss_lp")) return rc;
     DeviceGuard dg(c->device);
     auto f = [](const void* p) { return static_cast<const float*>(p); };   // element type travels in `dtype`
     PhysArgs a = phys_args(f(s_m), f(s_0), f(s_p), f(u_m), f(u_0), f(u_p), Rs, Rx, Ry, Rz);
     a.acc_out = acc;
-    if (any) return launch_phys<true, true, false>(c, g, a, cudaStream_t(stream), -1, dtype);
+    if (Rs) return launch_phys<true, true, false>(c, g, a, cudaStream_t(stream), -1, dtype);
     return launch_phys<false, true, false>(c, g, a, cudaStream_t(stream), -1, dtype);
 }
 
@@ -1246,19 +1242,7 @@ int physad_phys_backward_from_fields_dev(physad_ctx* c, const physad_grid* g, co
 }
 
 // Host-pointer forms: stage 12N floats in, run, stage results out (the reference API's contract,
-// include/phys.h:66, minus its per-call cudaMalloc/cudaFree: scratch is kept by the context).
-namespace {
-int upload_fields(physad_ctx* c, size_t N, const float* const src[6], float** d_out) {
-    if (int rc = ensure_scratch(c, 16 * N * sizeof(float))) return rc;
-    float* d = reinterpret_cast<float*>(c->scratch);
-    const size_t off[6] = {0, N, 2 * N, 3 * N, 6 * N, 9 * N}, cnt[6] = {N, N, N, 3 * N, 3 * N, 3 * N};
-    for (int k = 0; k < 6; ++k)
-        CU(cudaMemcpyAsync(d + off[k], src[k], cnt[k] * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    *d_out = d;
-    return 0;
-}
-}  // namespace
-
+// include/phys.h:66, minus its per-call allocations: scratch is kept by the context).
 int physad_phys_residuals_host(physad_ctx* c, const physad_grid* g, const float* s_m, const float* s_0, const float* s_p,
                                const float* u_m, const float* u_0, const float* u_p, float* Rs, float* Rx, float* Ry,
                                float* Rz, float* kernel_ms) {
@@ -1266,25 +1250,21 @@ int physad_phys_residuals_host(physad_ctx* c, const physad_grid* g, const float*
         return fail(PHYSAD_E_INVALID, "phys_residuals: null argument");
     if (int rc = check_grid(g)) return rc;
     DeviceGuard dg(c->device);
-    const size_t N = size_t(g->nx) * g->ny * g->nz;
-    const float* src[6] = {s_m, s_0, s_p, u_m, u_0, u_p};
-    float* d;
-    if (int rc = upload_fields(c, N, src, &d)) return rc;
-    float* r = d + 12 * N;
+    const size_t n = size_t(g->nx) * g->ny * g->nz * sizeof(float);
+    Staged a[10] = {{s_m, nullptr, n}, {s_0, nullptr, n}, {s_p, nullptr, n}, {u_m, nullptr, 3 * n}, {u_0, nullptr, 3 * n},
+                    {u_p, nullptr, 3 * n}, {nullptr, Rs, n}, {nullptr, Rx, n}, {nullptr, Ry, n}, {nullptr, Rz, n}};
+    if (int rc = stage_in(c, a)) return rc;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     if (kernel_ms) {
         CU(cudaEventCreate(&e0));
         CU(cudaEventCreate(&e1));
         CU(cudaEventRecord(e0, c->stream));
     }
-    if (int rc = physad_phys_residuals_dev(c, g, d, d + N, d + 2 * N, d + 3 * N, d + 6 * N, d + 9 * N, r, r + N, r + 2 * N,
-                                           r + 3 * N, c->stream))
+    if (int rc = physad_phys_residuals_dev(c, g, a[0].dev, a[1].dev, a[2].dev, a[3].dev, a[4].dev, a[5].dev, a[6].dev, a[7].dev,
+                                           a[8].dev, a[9].dev, c->stream))
         return rc;
     if (kernel_ms) CU(cudaEventRecord(e1, c->stream));
-    float* dst[4] = {Rs, Rx, Ry, Rz};
-    for (int k = 0; k < 4; ++k)
-        CU(cudaMemcpyAsync(dst[k], r + k * N, N * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
+    if (int rc = stage_out(c, a)) return rc;
     if (kernel_ms) {
         CU(cudaEventElapsedTime(kernel_ms, e0, e1));
         cudaEventDestroy(e0);
@@ -1299,21 +1279,17 @@ int physad_phys_loss_host(physad_ctx* c, const physad_grid* g, const physad_phys
     if (!c || !w || !s_m || !s_0 || !s_p || !u_m || !u_0 || !u_p) return fail(PHYSAD_E_INVALID, "phys_loss: null argument");
     if (int rc = check_grid(g)) return rc;
     DeviceGuard dg(c->device);
-    const size_t N = size_t(g->nx) * g->ny * g->nz;
-    const float* src[6] = {s_m, s_0, s_p, u_m, u_0, u_p};
-    float* d;
-    if (int rc = upload_fields(c, N, src, &d)) return rc;
-    float* r = d + 12 * N;
-    float* host_r[4] = {Rs, Rx, Ry, Rz};
+    const size_t N = size_t(g->nx) * g->ny * g->nz, n = N * sizeof(float);
+    Staged a[10] = {{s_m, nullptr, n}, {s_0, nullptr, n}, {s_p, nullptr, n}, {u_m, nullptr, 3 * n}, {u_0, nullptr, 3 * n},
+                    {u_p, nullptr, 3 * n}, {nullptr, Rs, n}, {nullptr, Rx, n}, {nullptr, Ry, n}, {nullptr, Rz, n}};
+    if (int rc = stage_in(c, a)) return rc;
     float* dev_r[4];
-    for (int k = 0; k < 4; ++k) dev_r[k] = host_r[k] ? r + k * N : nullptr;
-    if (int rc = physad_phys_loss_dev(c, g, d, d + N, d + 2 * N, d + 3 * N, d + 6 * N, d + 9 * N, c->d_acc, dev_r[0],
+    for (int k = 0; k < 4; ++k) dev_r[k] = a[6 + k].down ? a[6 + k].dev : nullptr;
+    if (int rc = physad_phys_loss_dev(c, g, a[0].dev, a[1].dev, a[2].dev, a[3].dev, a[4].dev, a[5].dev, c->d_acc, dev_r[0],
                                       dev_r[1], dev_r[2], dev_r[3], c->stream))
         return rc;
     CU(cudaMemcpyAsync(c->h_acc, c->d_acc, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    for (int k = 0; k < 4; ++k)
-        if (host_r[k]) CU(cudaMemcpyAsync(host_r[k], dev_r[k], N * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
+    if (int rc = stage_out(c, a)) return rc;
     physad_finalize_loss(c->h_acc, w, N, loss_sigma, loss_u);
     return 0;
 }
@@ -1325,20 +1301,14 @@ int physad_phys_backward_host(physad_ctx* c, const physad_grid* g, const physad_
         return fail(PHYSAD_E_INVALID, "phys_backward: null argument");
     if (int rc = check_grid(g)) return rc;
     DeviceGuard dg(c->device);
-    const size_t N = size_t(g->nx) * g->ny * g->nz;
-    if (int rc = ensure_scratch(c, 8 * N * sizeof(float))) return rc;
-    float* d = reinterpret_cast<float*>(c->scratch);
-    const float* src[4] = {Rs, Rx, Ry, Rz};
-    float* dst[4] = {gs, gx, gy, gz};
-    for (int k = 0; k < 4; ++k)
-        CU(cudaMemcpyAsync(d + k * N, src[k], N * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    float* o = d + 4 * N;
-    if (int rc = physad_phys_backward_dev(c, g, w, d, d + N, d + 2 * N, d + 3 * N, o, o + N, o + 2 * N, o + 3 * N, c->stream))
+    const size_t n = size_t(g->nx) * g->ny * g->nz * sizeof(float);
+    Staged a[8] = {{Rs, nullptr, n}, {Rx, nullptr, n}, {Ry, nullptr, n}, {Rz, nullptr, n},
+                   {nullptr, gs, n}, {nullptr, gx, n}, {nullptr, gy, n}, {nullptr, gz, n}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_phys_backward_dev(c, g, w, a[0].dev, a[1].dev, a[2].dev, a[3].dev, a[4].dev, a[5].dev, a[6].dev, a[7].dev,
+                                          c->stream))
         return rc;
-    for (int k = 0; k < 4; ++k)
-        CU(cudaMemcpyAsync(dst[k], o + k * N, N * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
+    return stage_out(c, a);
 }
 
 int physad_phys_backward_from_fields_host(physad_ctx* c, const physad_grid* g, const physad_phys_weights* w,
@@ -1348,19 +1318,14 @@ int physad_phys_backward_from_fields_host(physad_ctx* c, const physad_grid* g, c
         return fail(PHYSAD_E_INVALID, "phys_backward_from_fields: null argument");
     if (int rc = check_grid(g)) return rc;
     DeviceGuard dg(c->device);
-    const size_t N = size_t(g->nx) * g->ny * g->nz;
-    const float* src[6] = {s_m, s_0, s_p, u_m, u_0, u_p};
-    float* d;
-    if (int rc = upload_fields(c, N, src, &d)) return rc;
-    float* o = d + 12 * N;
-    if (int rc = physad_phys_backward_from_fields_dev(c, g, w, d, d + N, d + 2 * N, d + 3 * N, d + 6 * N, d + 9 * N, o, o + N,
-                                                      o + 2 * N, o + 3 * N, c->stream))
+    const size_t n = size_t(g->nx) * g->ny * g->nz * sizeof(float);
+    Staged a[10] = {{s_m, nullptr, n}, {s_0, nullptr, n}, {s_p, nullptr, n}, {u_m, nullptr, 3 * n}, {u_0, nullptr, 3 * n},
+                    {u_p, nullptr, 3 * n}, {nullptr, gs, n}, {nullptr, gx, n}, {nullptr, gy, n}, {nullptr, gz, n}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_phys_backward_from_fields_dev(c, g, w, a[0].dev, a[1].dev, a[2].dev, a[3].dev, a[4].dev, a[5].dev,
+                                                      a[6].dev, a[7].dev, a[8].dev, a[9].dev, c->stream))
         return rc;
-    float* dst[4] = {gs, gx, gy, gz};
-    for (int k = 0; k < 4; ++k)
-        CU(cudaMemcpyAsync(dst[k], o + k * N, N * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
+    return stage_out(c, a);
 }
 
 // ---- the metric path ---------------------------------------------------------------------------------
@@ -1371,8 +1336,7 @@ int physad_fused_loss_dev(physad_ctx* c, const physad_grid* g, const physad_slab
     if (int rc = need_4x4(c, "fused_loss", "physad_deep_loss_host or physad_deep_loss_grad_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
-    const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
-    if (any && !all) return fail(PHYSAD_E_INVALID, "fused_loss: residual outputs must be all set or all null");
+    if (int rc = check_residual_outputs(Rs, Rx, Ry, Rz, "fused_loss")) return rc;
     DeviceGuard dg(c->device);
     float* R[4] = {Rs, Rx, Ry, Rz};
     return launch_fused(c, g, s, t, dt, acc, R, cudaStream_t(stream));
@@ -1385,8 +1349,7 @@ int physad_fused_loss_allreduce_dev(physad_ctx* c, const physad_grid* g, const p
     if (int rc = need_4x4(c, "fused_loss_allreduce", "physad_deep_loss_grad_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
-    const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
-    if (any && !all) return fail(PHYSAD_E_INVALID, "fused_loss_allreduce: residual outputs must be all set or all null");
+    if (int rc = check_residual_outputs(Rs, Rx, Ry, Rz, "fused_loss_allreduce")) return rc;
     DeviceGuard dg(c->device);
     float* R[4] = {Rs, Rx, Ry, Rz};
     return launch_fused(c, g, s, t, dt, acc, R, cudaStream_t(stream), true);
@@ -1431,23 +1394,17 @@ int physad_tangent_loss_dev(physad_ctx* c, const physad_grid* g, const physad_sl
     if (int rc = need_4x4(c, "tangent_loss", "physad_deep_tangent_loss_dev")) return rc;
     physad_slab s;
     if (int rc = check_slab(g, slab, &s)) return rc;
-    const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
-    if (any && !all) return fail(PHYSAD_E_INVALID, "tangent_loss: residual outputs must be all set or all null");
+    if (int rc = check_residual_outputs(Rs, Rx, Ry, Rz, "tangent_loss")) return rc;
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
-    if (s.z_end == s.z_begin) {
-        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
-        return 0;
-    }
+    if (s.z_end == s.z_begin) return zero_result(acc, 2, nullptr, 0, st);
     if (int rc = ensure_coord_tables(c, g, st)) return rc;
     TangentArgs a{};
     a.nx = g->nx; a.ny = g->ny; a.nz = g->nz; a.z_begin = s.z_begin; a.z_end = s.z_end;
     a.cxs = c->tab.dev; a.cys = a.cxs + g->nx; a.czs = a.cys + g->ny;
-    // dc/dx of a coordinate c = norm(i / (n - 1)) sampled at x = i h:  MinusOneToOne 2 / ((n-1) h), ZeroToOne 1 / ((n-1) h)
-    const double f = c->cfg.norm == 1 ? 2.0 : 1.0;
-    a.sx = g->nx > 1 ? float(f / (double(g->nx - 1) * double(g->hx))) : 0.f;
-    a.sy = g->ny > 1 ? float(f / (double(g->ny - 1) * double(g->hy))) : 0.f;
-    a.sz = g->nz > 1 ? float(f / (double(g->nz - 1) * double(g->hz))) : 0.f;
+    float s3[3];
+    input_scales(g, c->cfg.norm, s3);
+    a.sx = s3[0]; a.sy = s3[1]; a.sz = s3[2];
     const size_t n = size_t(s.z_end - s.z_begin) * g->ny * g->nx;
     const int blocks = int(std::max<size_t>(1, std::min<size_t>(size_t(c->sm_count) * 2, (n + 2 * TANGENT_THREADS - 1) / (2 * TANGENT_THREADS))));
     if (int rc = ensure_partials(c, size_t(blocks))) return rc;
@@ -1481,12 +1438,55 @@ int physad_tangent_loss_host(physad_ctx* c, const physad_grid* g, const physad_m
 // ---- closed loop: loss and its gradient with respect to the MLP weights (additive, grad_kernels.cuh) ----
 
 namespace {
-int ensure_grad_workspace(physad_ctx* c, size_t floats) {
-    if (floats <= c->gws_cap) return 0;
-    if (c->gws) CU(cudaFree(c->gws));
-    c->gws = nullptr; c->gws_cap = 0;
-    CU(cudaMalloc(&c->gws, floats * sizeof(float)));
-    c->gws_cap = floats;
+// The closed loops' workspace for NL points in gws: the six fields sigma_{-,0,+} (NL each) and u_{-,0,+} (3 NL each), the
+// four residuals R[k] = R + k NL, and the time-t output adjoint (4 NL)
+struct LoopWorkspace {
+    float *s_m, *s_0, *s_p, *u_m, *u_0, *u_p, *R;
+    float4* adj;
+};
+
+int loop_workspace(physad_ctx* c, size_t NL, LoopWorkspace& w) {
+    if (int rc = grow(c->gws, c->gws_cap, 20 * NL)) return rc;
+    float* f = c->gws;
+    w = {f, f + NL, f + 2 * NL, f + 3 * NL, f + 6 * NL, f + 9 * NL, f + 12 * NL, reinterpret_cast<float4*>(f + 16 * NL)};
+    return 0;
+}
+
+// The lengths of the gradient's six arrays in physad_set_weights_deep's order dW1, db1, dWh, dbh, dW2, db2 for the context's
+// network; returns their sum P.  With one hidden layer dWh and dbh are empty: the layout dW1 | db1 | dW2 | db2 of any width.
+size_t grad_parts(const physad_ctx* c, size_t len[6]) {
+    const size_t nl = size_t(std::max(1, c->deep_layers) - 1), H = size_t(c->cfg.H);
+    const size_t l[6] = {4 * H, H, nl * H * H, nl * H, 4 * H, 4};
+    std::copy(l, l + 6, len);
+    return 9 * H + 4 + nl * (H * H + H);
+}
+
+// The host forms of the gradients: the context's device result buffer d_dgrad [acc | grad] (at most 2 sums + P) and its
+// pinned host copy h_dgrad ...
+int ensure_host_grad(physad_ctx* c) {
+    size_t len[6];
+    const size_t n = grad_parts(c, len) + 2;
+    if (int rc = grow(c->d_dgrad, c->d_dgrad_cap, n)) return rc;
+    return grow(c->h_dgrad, c->h_dgrad_cap, n, true);
+}
+
+// ... and the way back: one copy of [acc (nacc sums) | grad (P)] into h_dgrad, one stream synchronisation, then the loss
+// -- physad_finalize_loss of the two physics sums over n points (nacc = 2), the fit loss acc / n (nacc = 1), none for the
+// VJPs (nacc = 0) -- and the gradient split into physad_set_weights_deep's six arrays dW1, db1, dWh, dbh, dW2, db2 (a null
+// array is skipped; at one hidden layer dWh and dbh are empty)
+int grad_to_host(physad_ctx* c, int nacc, size_t n, const physad_phys_weights* w, float* loss_a, float* loss_b,
+                 const std::array<float*, 6>& out) {
+    size_t len[6];
+    const size_t P = grad_parts(c, len);
+    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (nacc + P) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    if (nacc == 2) physad_finalize_loss(c->h_dgrad, w, n, loss_a, loss_b);
+    if (nacc == 1 && loss_a) *loss_a = float(c->h_dgrad[0] / double(n));
+    const double* gd = c->h_dgrad + nacc;
+    for (int k = 0; k < 6; ++k) {
+        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
+        gd += len[k];
+    }
     return 0;
 }
 
@@ -1520,22 +1520,23 @@ int physad_fused_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
     const size_t N = size_t(g->nx) * g->ny * g->nz;
-    if (int rc = ensure_grad_workspace(c, 20 * N)) return rc;   // 12 N fields, 4 N residuals, 4 N time-t adjoint
+    LoopWorkspace f;
+    if (int rc = loop_workspace(c, N, f)) return rc;
     // forward, stage-wise on the device: fields of the three slices, then residuals + the two sums
-    float* f = c->gws;
-    float *s_m = f, *s_0 = f + N, *s_p = f + 2 * N, *u_m = f + 3 * N, *u_0 = f + 6 * N, *u_p = f + 9 * N, *R = f + 12 * N;
-    if (int rc = physad_mlp_generate_fields_dev(c, g, nullptr, t, dt, s_m, s_0, s_p, u_m, u_0, u_p, stream)) return rc;
-    if (int rc = physad_phys_loss_dev(c, g, s_m, s_0, s_p, u_m, u_0, u_p, acc, R, R + N, R + 2 * N, R + 3 * N, stream)) return rc;
+    float* R = f.R;
+    if (int rc = physad_mlp_generate_fields_dev(c, g, nullptr, t, dt, f.s_m, f.s_0, f.s_p, f.u_m, f.u_0, f.u_p, stream)) return rc;
+    if (int rc = physad_phys_loss_dev(c, g, f.s_m, f.s_0, f.s_p, f.u_m, f.u_0, f.u_p, acc, R, R + N, R + 2 * N, R + 3 * N, stream))
+        return rc;
     // backward
     GradArgs a{};
     if (int rc = grad_args_common(c, g, w, t, dt, a, st)) return rc;
     a.z_begin = 0; a.z_end = g->nz; a.z_origin = 0;
     a.wrap_z = a.periodic;
     a.cstride = N;
-    a.s0 = s_0; a.u0 = u_0;
+    a.s0 = f.s_0; a.u0 = f.u_0;
     for (int k = 0; k < 4; ++k) a.R[k] = R + k * N;
     a.grad = grad;
-    return launch_grad(c, template_h(c->cfg.H), a, reinterpret_cast<float4*>(f + 16 * N), (N + GRAD_THREADS - 1) / GRAD_THREADS, st);
+    return launch_grad(c, template_h(c->cfg.H), a, f.adj, (N + GRAD_THREADS - 1) / GRAD_THREADS, st);
 }
 
 int physad_fused_loss_grad_slab_dev(physad_ctx* c, const physad_grid* g, const physad_slab* slab,
@@ -1550,11 +1551,7 @@ int physad_fused_loss_grad_slab_dev(physad_ctx* c, const physad_grid* g, const p
     cudaStream_t st = cudaStream_t(stream);
     const int H = c->cfg.H;
     if (c->advection != 0) return fail(PHYSAD_E_UNSUPPORTED, "fused_loss_grad_slab: the stencil adjoint is that of the central scheme");
-    if (s.z_begin == s.z_end) {
-        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
-        CU(cudaMemsetAsync(grad, 0, size_t(9 * H + 4) * sizeof(double), st));
-        return 0;
-    }
+    if (s.z_begin == s.z_end) return zero_result(acc, 2, grad, size_t(9 * H + 4), st);
     // The gradient of the slab's points needs the residuals one plane beyond the slab, hence the fields two planes
     // beyond it: a window of VIRTUAL planes [zlo, zhi) (wrapped on a periodic grid, cut at the faces otherwise) is
     // recomputed locally -- no halo exchange, like the forward path (SURVEY.md 8e).
@@ -1564,9 +1561,9 @@ int physad_fused_loss_grad_slab_dev(physad_ctx* c, const physad_grid* g, const p
     const int npl = zhi - zlo;
     const size_t pln = size_t(g->nx) * g->ny, NL = pln * npl;
     if (NL >= (size_t(1) << 31)) return fail(PHYSAD_E_UNSUPPORTED, "fused_loss_grad_slab: window of 2^31 points or more");
-    if (int rc = ensure_grad_workspace(c, 20 * NL)) return rc;
-    float* f = c->gws;
-    float *s_m = f, *s_0 = f + NL, *s_p = f + 2 * NL, *u_m = f + 3 * NL, *u_0 = f + 6 * NL, *u_p = f + 9 * NL, *R = f + 12 * NL;
+    LoopWorkspace f;
+    if (int rc = loop_workspace(c, NL, f)) return rc;
+    float* R = f.R;
     const float ts[3] = {t - dt, t, t + dt};
     const float tc[3] = {time_coord(ts[0], c->cfg.norm), time_coord(ts[1], c->cfg.norm), time_coord(ts[2], c->cfg.norm)};
     // fields: one launch per run of consecutive global planes inside the window
@@ -1575,15 +1572,15 @@ int physad_fused_loss_grad_slab_dev(physad_ctx* c, const physad_grid* g, const p
         const int run = std::min(zhi - zv, g->nz - ga);
         const size_t off = size_t(zv - zlo) * pln;
         GridInferArgs ga_args{};
-        ga_args.sigma[0] = s_m + off; ga_args.sigma[1] = s_0 + off; ga_args.sigma[2] = s_p + off;
-        ga_args.u[0] = u_m + off; ga_args.u[1] = u_0 + off; ga_args.u[2] = u_p + off;
+        ga_args.sigma[0] = f.s_m + off; ga_args.sigma[1] = f.s_0 + off; ga_args.sigma[2] = f.s_p + off;
+        ga_args.u[0] = f.u_m + off; ga_args.u[1] = f.u_0 + off; ga_args.u[2] = f.u_p + off;
         ga_args.cstride = NL;
         if (int rc = launch_grid<true>(c, g, physad_slab{ga, ga + run}, tc, ga_args, st)) return rc;
         zv += run;
     }
     // residuals of every plane of the window with the z neighbours clamped at its ends: exact wherever both z
     // neighbours are inside the window (or the end is a face of a non-periodic grid); the other planes are not used
-    PhysArgs pa = phys_args(s_m, s_0, s_p, u_m, u_0, u_p, R, R + NL, R + 2 * NL, R + 3 * NL);
+    PhysArgs pa = phys_args(f.s_m, f.s_0, f.s_p, f.u_m, f.u_0, f.u_p, R, R + NL, R + 2 * NL, R + 3 * NL);
     pa.clamp_z = 1;
     if (int rc = launch_phys<true, false, false>(c, g, pa, st, npl)) return rc;
     GradArgs a{};
@@ -1591,11 +1588,11 @@ int physad_fused_loss_grad_slab_dev(physad_ctx* c, const physad_grid* g, const p
     a.z_begin = s.z_begin; a.z_end = s.z_end; a.z_origin = zlo;
     a.wrap_z = 0;
     a.cstride = NL;
-    a.s0 = s_0; a.u0 = u_0;
+    a.s0 = f.s_0; a.u0 = f.u_0;
     for (int k = 0; k < 4; ++k) a.R[k] = R + k * NL;
     a.grad = grad;
     a.acc_out = acc;
-    return launch_grad(c, template_h(H), a, reinterpret_cast<float4*>(f + 16 * NL), (pln * size_t(s.z_end - s.z_begin) + GRAD_THREADS - 1) / GRAD_THREADS, st);
+    return launch_grad(c, template_h(H), a, f.adj, (pln * size_t(s.z_end - s.z_begin) + GRAD_THREADS - 1) / GRAD_THREADS, st);
 }
 
 int physad_fused_loss_grad_host(physad_ctx* c, const physad_grid* g, const physad_mlp_config* cfg, const float* W1,
@@ -1608,35 +1605,14 @@ int physad_fused_loss_grad_host(physad_ctx* c, const physad_grid* g, const physa
     }
     if (int rc = need_4x4(c, "fused_loss_grad", "physad_deep_loss_grad_dev")) return rc;
     DeviceGuard dg(c->device);
-    constexpr size_t cap = 9 * 128 + 4;
-    if (!c->d_grad) CU(cudaMalloc(&c->d_grad, cap * sizeof(double)));
-    if (!c->h_grad) CU(cudaMallocHost(&c->h_grad, cap * sizeof(double)));
-    if (int rc = physad_fused_loss_grad_dev(c, g, w, t, dt, c->d_acc, c->d_grad, c->stream)) return rc;
-    const int H = c->cfg.H;
-    CU(cudaMemcpyAsync(c->h_acc, c->d_acc, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(c->h_grad, c->d_grad, size_t(9 * H + 4) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    physad_finalize_loss(c->h_acc, w, size_t(g->nx) * g->ny * g->nz, loss_sigma, loss_u);
-    const double* gd = c->h_grad;
-    if (dW1) for (int i = 0; i < 4 * H; ++i) dW1[i] = float(gd[i]);
-    if (db1) for (int i = 0; i < H; ++i) db1[i] = float(gd[4 * H + i]);
-    if (dW2) for (int i = 0; i < 4 * H; ++i) dW2[i] = float(gd[5 * H + i]);
-    if (db2) for (int i = 0; i < 4; ++i) db2[i] = float(gd[9 * H + i]);
-    return 0;
+    if (int rc = ensure_host_grad(c)) return rc;
+    if (int rc = physad_fused_loss_grad_dev(c, g, w, t, dt, c->d_dgrad, c->d_dgrad + 2, c->stream)) return rc;
+    return grad_to_host(c, 2, size_t(g->nx) * g->ny * g->nz, w, loss_sigma, loss_u, {dW1, db1, nullptr, nullptr, dW2, db2});
 }
 
 // ---- closed loop of the analytic loss: its gradient with respect to the MLP weights (tangent_grad_kernels.cuh) ----
 }  // extern "C"  (templates below)
 namespace {
-int ensure_grad_partials(physad_ctx* c, size_t doubles) {
-    if (doubles <= c->gpart_cap) return 0;
-    if (c->gpart) CU(cudaFree(c->gpart));
-    c->gpart = nullptr; c->gpart_cap = 0;
-    CU(cudaMalloc(&c->gpart, doubles * sizeof(double)));
-    c->gpart_cap = doubles;
-    return 0;
-}
-
 template <int H>
 int launch_tangent_grad_t(physad_ctx* c, const TangentGradArgs& a, float tcoord, size_t chunks, cudaStream_t st) {
     int& bps = c->tgrad_blocks_per_sm[H == 32 ? 0 : (H == 64 ? 1 : 2)];
@@ -1667,21 +1643,15 @@ int physad_tangent_loss_grad_dev(physad_ctx* c, const physad_grid* g, const phys
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
     const int H = c->cfg.H;
-    if (s.z_end == s.z_begin) {
-        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
-        CU(cudaMemsetAsync(grad, 0, size_t(9 * H + 4) * sizeof(double), st));
-        return 0;
-    }
+    if (s.z_end == s.z_begin) return zero_result(acc, 2, grad, size_t(9 * H + 4), st);
     if (int rc = upload_weights_if_stale(c, st)) return rc;
     if (int rc = ensure_coord_tables(c, g, st)) return rc;
     TangentGradArgs a{};
     a.nx = g->nx; a.ny = g->ny; a.nz = g->nz; a.z_begin = s.z_begin; a.z_end = s.z_end;
     a.cxs = c->tab.dev; a.cys = a.cxs + g->nx; a.czs = a.cys + g->ny;
-    // dc/dx exactly as physad_tangent_loss_dev forms it (0 for an extent of 1)
-    const double f = c->cfg.norm == 1 ? 2.0 : 1.0;
-    a.sx = g->nx > 1 ? float(f / (double(g->nx - 1) * double(g->hx))) : 0.f;
-    a.sy = g->ny > 1 ? float(f / (double(g->ny - 1) * double(g->hy))) : 0.f;
-    a.sz = g->nz > 1 ? float(f / (double(g->nz - 1) * double(g->hz))) : 0.f;
+    float s3[3];
+    input_scales(g, c->cfg.norm, s3);
+    a.sx = s3[0]; a.sy = s3[1]; a.sz = s3[2];
     vjp_scales(g, w, &a.scale_s, &a.scale_u);   // 2 w / float(N) of the whole grid: slab results add up to the grid's
     a.ct = time_coord(t, c->cfg.norm);
     a.W1 = c->dW1; a.W2 = c->dW2;
@@ -1707,21 +1677,9 @@ int physad_tangent_loss_grad_host(physad_ctx* c, const physad_grid* g, const phy
     }
     if (int rc = need_4x4(c, "tangent_loss_grad", "physad_deep_tangent_loss_grad_dev")) return rc;
     DeviceGuard dg(c->device);
-    constexpr size_t cap = 9 * 128 + 4;
-    if (!c->d_grad) CU(cudaMalloc(&c->d_grad, cap * sizeof(double)));
-    if (!c->h_grad) CU(cudaMallocHost(&c->h_grad, cap * sizeof(double)));
-    if (int rc = physad_tangent_loss_grad_dev(c, g, nullptr, w, t, c->d_acc, c->d_grad, c->stream)) return rc;
-    const int H = c->cfg.H;
-    CU(cudaMemcpyAsync(c->h_acc, c->d_acc, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(c->h_grad, c->d_grad, size_t(9 * H + 4) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    physad_finalize_loss(c->h_acc, w, size_t(g->nx) * g->ny * g->nz, loss_sigma, loss_u);
-    const double* gd = c->h_grad;
-    if (dW1) for (int i = 0; i < 4 * H; ++i) dW1[i] = float(gd[i]);
-    if (db1) for (int i = 0; i < H; ++i) db1[i] = float(gd[4 * H + i]);
-    if (dW2) for (int i = 0; i < 4 * H; ++i) dW2[i] = float(gd[5 * H + i]);
-    if (db2) for (int i = 0; i < 4; ++i) db2[i] = float(gd[9 * H + i]);
-    return 0;
+    if (int rc = ensure_host_grad(c)) return rc;
+    if (int rc = physad_tangent_loss_grad_dev(c, g, nullptr, w, t, c->d_dgrad, c->d_dgrad + 2, c->stream)) return rc;
+    return grad_to_host(c, 2, size_t(g->nx) * g->ny * g->nz, w, loss_sigma, loss_u, {dW1, db1, nullptr, nullptr, dW2, db2});
 }
 
 // ---- closed loop of deeper networks (deep_grad_kernels.cuh) ----------------------------------------------------------
@@ -1746,11 +1704,7 @@ int physad_deep_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad_
     cudaStream_t st = cudaStream_t(stream);
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
-    if (s.z_begin == s.z_end) {
-        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
-        CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
-        return 0;
-    }
+    if (s.z_begin == s.z_end) return zero_result(acc, 2, grad, P, st);
     // window of VIRTUAL planes [zlo, zhi) whose fields the slab's gradient needs (as physad_fused_loss_grad_slab_dev)
     const bool per = g->periodic != 0;
     const int zlo = whole ? 0 : (per ? s.z_begin - 2 : std::max(0, s.z_begin - 2));
@@ -1758,13 +1712,15 @@ int physad_deep_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad_
     const int npl = zhi - zlo;
     const size_t pln = size_t(g->nx) * g->ny, NL = pln * npl;
     if (NL >= (size_t(1) << 31)) return fail(PHYSAD_E_UNSUPPORTED, "deep_loss_grad: window of 2^31 points or more");
-    if (int rc = ensure_grad_workspace(c, 20 * NL)) return rc;   // 12 NL fields, 4 NL residuals, 4 NL time-t adjoint
-    float* f = c->gws;
-    float *s_m = f, *s_0 = f + NL, *s_p = f + 2 * NL, *u_m = f + 3 * NL, *u_0 = f + 6 * NL, *u_p = f + 9 * NL, *R = f + 12 * NL;
+    LoopWorkspace f;
+    if (int rc = loop_workspace(c, NL, f)) return rc;
+    float* R = f.R;
     if (whole) {
         // the arithmetic of physad_deep_loss_host: same fields, same residual kernel, same sums
-        if (int rc = physad_mlp_generate_fields_deep_dev(c, g, nullptr, t, dt, s_m, s_0, s_p, u_m, u_0, u_p, stream)) return rc;
-        if (int rc = physad_phys_loss_dev(c, g, s_m, s_0, s_p, u_m, u_0, u_p, acc, R, R + NL, R + 2 * NL, R + 3 * NL, stream))
+        if (int rc = physad_mlp_generate_fields_deep_dev(c, g, nullptr, t, dt, f.s_m, f.s_0, f.s_p, f.u_m, f.u_0, f.u_p, stream))
+            return rc;
+        if (int rc = physad_phys_loss_dev(c, g, f.s_m, f.s_0, f.s_p, f.u_m, f.u_0, f.u_p, acc, R, R + NL, R + 2 * NL, R + 3 * NL,
+                                          stream))
             return rc;
     } else {
         // fields: the deep kernel writes u with the channel stride of its own launch, so each run of consecutive global
@@ -1784,15 +1740,15 @@ int physad_deep_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad_
             if (int rc = physad_mlp_generate_fields_deep_dev(c, g, &rs, t, dt, sc, sc + nr, sc + 2 * nr, sc + 3 * nr, sc + 6 * nr,
                                                              sc + 9 * nr, stream))
                 return rc;
-            float* dst[12] = {s_m + off, s_0 + off, s_p + off};
+            float* dst[12] = {f.s_m + off, f.s_0 + off, f.s_p + off};
             for (int k = 0; k < 3; ++k)
-                for (int ch = 0; ch < 3; ++ch) dst[3 + 3 * k + ch] = (k == 0 ? u_m : (k == 1 ? u_0 : u_p)) + ch * NL + off;
+                for (int ch = 0; ch < 3; ++ch) dst[3 + 3 * k + ch] = (k == 0 ? f.u_m : (k == 1 ? f.u_0 : f.u_p)) + ch * NL + off;
             for (int b = 0; b < 12; ++b)
                 CU(cudaMemcpyAsync(dst[b], sc + size_t(b) * nr, nr * sizeof(float), cudaMemcpyDeviceToDevice, st));
             zv += run;
         }
         // residuals of every window plane with the z neighbours clamped at its ends (exact on the planes the slab uses)
-        PhysArgs pa = phys_args(s_m, s_0, s_p, u_m, u_0, u_p, R, R + NL, R + 2 * NL, R + 3 * NL);
+        PhysArgs pa = phys_args(f.s_m, f.s_0, f.s_p, f.u_m, f.u_0, f.u_p, R, R + NL, R + 2 * NL, R + 3 * NL);
         pa.clamp_z = 1;
         if (int rc = launch_phys<true, false, false>(c, g, pa, st, npl)) return rc;
     }
@@ -1802,21 +1758,14 @@ int physad_deep_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad_
     ga.z_begin = s.z_begin; ga.z_end = s.z_end; ga.z_origin = zlo;
     ga.wrap_z = whole ? ga.periodic : 0;
     ga.cstride = NL;
-    ga.s0 = s_0; ga.u0 = u_0;
+    ga.s0 = f.s_0; ga.u0 = f.u_0;
     for (int k = 0; k < 4; ++k) ga.R[k] = R + k * NL;
-    float4* adj = reinterpret_cast<float4*>(f + 16 * NL);
-    CU(cudaError_t(adjoint_launch(ga, adj, st)));
+    CU(cudaError_t(adjoint_launch(ga, f.adj, st)));
     c->launches++;
     // back-propagation through every layer, then the block-order reduction
     const long long npts = (long long)pln * (s.z_end - s.z_begin);
     const int blocks = deep_grad_blocks(H, npts, c->sm_count);
-    const size_t ck = size_t(blocks) * deep_grad_ckpt_floats(H, L);
-    if (ck > c->dckpt_cap) {
-        if (c->dckpt) CU(cudaFree(c->dckpt));
-        c->dckpt = nullptr; c->dckpt_cap = 0;
-        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
-        c->dckpt_cap = ck;
-    }
+    if (int rc = grow(c->dckpt, c->dckpt_cap, size_t(blocks) * deep_grad_ckpt_floats(H, L))) return rc;
     if (int rc = ensure_grad_partials(c, size_t(blocks) * (P + 2))) return rc;
     DeepGradArgs a{};
     a.nx = g->nx; a.ny = g->ny; a.nz = g->nz;
@@ -1827,7 +1776,7 @@ int physad_deep_loss_grad_dev(physad_ctx* c, const physad_grid* g, const physad_
     for (int k = 0; k < 3; ++k) a.tc[k] = ga.tc[k];
     a.wh = c->d_wh; a.bh = c->d_bh;
     for (int k = 0; k < 4; ++k) a.R[k] = ga.R[k];
-    a.adj = adj;
+    a.adj = f.adj;
     a.scale_s = ga.scale_s; a.scale_u = ga.scale_u; a.inv2dt = ga.inv2dt;
     a.ckpt = c->dckpt;
     a.partials = c->gpart;
@@ -1843,43 +1792,14 @@ int physad_deep_loss_grad_host(physad_ctx* c, const physad_grid* g, const physad
     if (int rc = check_grid(g)) return rc;
     if (int rc = deep_ready(c, "deep_loss_grad")) return rc;
     DeviceGuard dg(c->device);
-    const int H = c->cfg.H, L = c->deep_layers;
-    const size_t P = deep_grad_len(H, L);
-    if (P + 2 > c->dgrad_cap) {
-        if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
-        if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
-        c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
-        CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
-        CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
-        c->dgrad_cap = P + 2;
-    }
+    if (int rc = ensure_host_grad(c)) return rc;
     if (int rc = physad_deep_loss_grad_dev(c, g, nullptr, w, t, dt, c->d_dgrad, c->d_dgrad + 2, c->stream)) return rc;
-    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 2) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    physad_finalize_loss(c->h_dgrad, w, size_t(g->nx) * g->ny * g->nz, loss_sigma, loss_u);
-    const double* gd = c->h_dgrad + 2;
-    const size_t nl = size_t(L - 1), hh = size_t(H);
-    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
-    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
-    for (int k = 0; k < 6; ++k) {
-        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
-        gd += len[k];
-    }
-    return 0;
+    return grad_to_host(c, 2, size_t(g->nx) * g->ny * g->nz, w, loss_sigma, loss_u, {dW1, db1, dWh, dbh, dW2, db2});
 }
 
 // ---- analytic loss of deeper networks and its closed loop (deep_tangent_kernels.cuh) ---------------------------------
 }  // extern "C"  (helpers below)
 namespace {
-// dc/dx of the three space inputs as physad_tangent_loss_dev forms them: f / ((n-1) h), f = 2 for MinusOneToOne (norm 1),
-// 1 for ZeroToOne, 0 for an extent of 1
-void input_scales(const physad_grid* g, int norm, float s[3]) {
-    const double f = norm == 1 ? 2.0 : 1.0;
-    s[0] = g->nx > 1 ? float(f / (double(g->nx - 1) * double(g->hx))) : 0.f;
-    s[1] = g->ny > 1 ? float(f / (double(g->ny - 1) * double(g->hy))) : 0.f;
-    s[2] = g->nz > 1 ? float(f / (double(g->nz - 1) * double(g->hz))) : 0.f;
-}
-
 // checks and arguments shared by the loss and the loss + gradient call; *npts = 0 for an empty slab
 int deep_tangent_args(physad_ctx* c, const physad_grid* g, const physad_slab* slab, float t, const char* what,
                       DeepTangentArgs& a, long long* npts, cudaStream_t st) {
@@ -1911,8 +1831,7 @@ extern "C" {
 int physad_deep_tangent_loss_dev(physad_ctx* c, const physad_grid* g, const physad_slab* slab, float t, double* acc,
                                  float* Rs, float* Rx, float* Ry, float* Rz, void* stream) {
     if (!c || !acc) return fail(PHYSAD_E_INVALID, "deep_tangent_loss: null argument");
-    const bool any = Rs || Rx || Ry || Rz, all = Rs && Rx && Ry && Rz;
-    if (any && !all) return fail(PHYSAD_E_INVALID, "deep_tangent_loss: residual outputs must be all set or all null");
+    if (int rc = check_residual_outputs(Rs, Rx, Ry, Rz, "deep_tangent_loss")) return rc;
     if (int rc = check_grid(g)) return rc;
     if (int rc = deep_ready(c, "deep_tangent_loss")) return rc;
     // one hidden layer: the one-hidden-layer analytic loss (its Jacobian products are precomputed on the host)
@@ -1922,10 +1841,7 @@ int physad_deep_tangent_loss_dev(physad_ctx* c, const physad_grid* g, const phys
     DeepTangentArgs a{};
     long long npts = 0;
     if (int rc = deep_tangent_args(c, g, slab, t, "deep_tangent_loss", a, &npts, st)) return rc;
-    if (npts == 0) {
-        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
-        return 0;
-    }
+    if (npts == 0) return zero_result(acc, 2, nullptr, 0, st);
     a.R[0] = Rs; a.R[1] = Rx; a.R[2] = Ry; a.R[3] = Rz;
     const int H = c->cfg.H;
     const int blocks = deep_tangent_blocks(H, npts, c->sm_count);
@@ -1950,20 +1866,10 @@ int physad_deep_tangent_loss_grad_dev(physad_ctx* c, const physad_grid* g, const
     if (int rc = deep_tangent_args(c, g, slab, t, "deep_tangent_loss_grad", a, &npts, st)) return rc;
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
-    if (npts == 0) {
-        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
-        CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
-        return 0;
-    }
+    if (npts == 0) return zero_result(acc, 2, grad, P, st);
     vjp_scales(g, w, &a.scale_s, &a.scale_u);   // 2 w / float(N) of the whole grid: slab results add up to the grid's
     const int blocks = deep_tangent_blocks(H, npts, c->sm_count);
-    const size_t ck = size_t(blocks) * deep_tangent_ckpt_floats(L);
-    if (ck > c->dckpt_cap) {
-        if (c->dckpt) CU(cudaFree(c->dckpt));
-        c->dckpt = nullptr; c->dckpt_cap = 0;
-        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
-        c->dckpt_cap = ck;
-    }
+    if (int rc = grow(c->dckpt, c->dckpt_cap, size_t(blocks) * deep_tangent_ckpt_floats(L))) return rc;
     if (int rc = ensure_grad_partials(c, size_t(blocks) * (P + 2))) return rc;
     a.ckpt = c->dckpt;
     a.partials = c->gpart;
@@ -1979,29 +1885,9 @@ int physad_deep_tangent_loss_grad_host(physad_ctx* c, const physad_grid* g, cons
     if (int rc = check_grid(g)) return rc;
     if (int rc = deep_ready(c, "deep_tangent_loss_grad")) return rc;
     DeviceGuard dg(c->device);
-    const int H = c->cfg.H, L = c->deep_layers;
-    const size_t P = deep_grad_len(H, L);
-    if (P + 2 > c->dgrad_cap) {
-        if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
-        if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
-        c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
-        CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
-        CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
-        c->dgrad_cap = P + 2;
-    }
+    if (int rc = ensure_host_grad(c)) return rc;
     if (int rc = physad_deep_tangent_loss_grad_dev(c, g, nullptr, w, t, c->d_dgrad, c->d_dgrad + 2, c->stream)) return rc;
-    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 2) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    physad_finalize_loss(c->h_dgrad, w, size_t(g->nx) * g->ny * g->nz, loss_sigma, loss_u);
-    const double* gd = c->h_dgrad + 2;
-    const size_t nl = size_t(L - 1), hh = size_t(H);
-    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
-    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
-    for (int k = 0; k < 6; ++k) {
-        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
-        gd += len[k];
-    }
-    return 0;
+    return grad_to_host(c, 2, size_t(g->nx) * g->ny * g->nz, w, loss_sigma, loss_u, {dW1, db1, dWh, dbh, dW2, db2});
 }
 
 // ---- deeper networks at caller-supplied points: forward and data-fit loss + gradient (deep_data_kernels.cuh) --------
@@ -2072,15 +1958,10 @@ int physad_mlp_forward_deep_host(physad_ctx* c, const float* x, float* y, size_t
     if (B && (!x || !y)) return fail(PHYSAD_E_INVALID, "mlp_forward_deep: null argument");
     if (B == 0) return 0;
     DeviceGuard dg(c->device);
-    const size_t bytes = B * 4 * sizeof(float), off_y = (bytes + 255) & ~size_t(255);
-    if (int rc = ensure_scratch(c, off_y + bytes)) return rc;
-    float* dx = reinterpret_cast<float*>(c->scratch);
-    float* dy = reinterpret_cast<float*>(c->scratch + off_y);
-    CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
-    if (int rc = physad_mlp_forward_deep_dev(c, dx, dy, B, c->stream)) return rc;
-    CU(cudaMemcpyAsync(y, dy, bytes, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
+    Staged a[2] = {{x, nullptr, B * 4 * sizeof(float)}, {nullptr, y, B * 4 * sizeof(float)}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_mlp_forward_deep_dev(c, a[0].dev, a[1].dev, B, c->stream)) return rc;
+    return stage_out(c, a);
 }
 
 }  // extern "C"  (helpers below)
@@ -2098,29 +1979,6 @@ int read_lam(const float* lam, float lw[4], const std::string& what) {
     return 0;
 }
 
-// The host forms of the deep gradients: the context's device result buffer [P + 2] and its pinned host copy ...
-int ensure_host_grad(physad_ctx* c, size_t P) {
-    if (P + 2 <= c->dgrad_cap) return 0;
-    if (c->d_dgrad) CU(cudaFree(c->d_dgrad));
-    if (c->h_dgrad) CU(cudaFreeHost(c->h_dgrad));
-    c->d_dgrad = nullptr; c->h_dgrad = nullptr; c->dgrad_cap = 0;
-    CU(cudaMalloc(&c->d_dgrad, (P + 2) * sizeof(double)));
-    CU(cudaMallocHost(&c->h_dgrad, (P + 2) * sizeof(double)));
-    c->dgrad_cap = P + 2;
-    return 0;
-}
-
-// ... and the gradient gd[P] split into physad_set_weights_deep's six arrays (a null array is skipped)
-void split_deep_grad(const double* gd, int H, int L, float* dW1, float* db1, float* dWh, float* dbh, float* dW2, float* db2) {
-    const size_t nl = size_t(L - 1), hh = size_t(H);
-    float* out[6] = {dW1, db1, dWh, dbh, dW2, db2};
-    const size_t len[6] = {4 * hh, hh, nl * hh * hh, nl * hh, 4 * hh, 4};
-    for (int k = 0; k < 6; ++k) {
-        if (out[k]) for (size_t i = 0; i < len[k]; ++i) out[k][i] = float(gd[i]);
-        gd += len[k];
-    }
-}
-
 // The launch shared by the data loss, the pair loss and the VJP at a.n > 0 rows: the weights, the grid, the checkpoint, the
 // partials, the kernel and the reduction.  `a` brings the rows and the seed inputs; the network's fields are filled here.
 // acc null (the VJP): the reduction's (zero) loss sum goes to a slot after the partials.
@@ -2129,13 +1987,7 @@ int deep_data_run(physad_ctx* c, DataSeeds seeds, DeepDataArgs& a, double* grad,
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
     const int blocks = deep_data_blocks(H, a.n, c->sm_count);
-    const size_t ck = size_t(blocks) * deep_data_ckpt_floats(H, L);
-    if (ck > c->dckpt_cap) {
-        if (c->dckpt) CU(cudaFree(c->dckpt));
-        c->dckpt = nullptr; c->dckpt_cap = 0;
-        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
-        c->dckpt_cap = ck;
-    }
+    if (int rc = grow(c->dckpt, c->dckpt_cap, size_t(blocks) * deep_data_ckpt_floats(H, L))) return rc;
     const size_t np = size_t(blocks) * (P + 1);
     if (int rc = ensure_grad_partials(c, np + (acc ? 0 : 1))) return rc;
     a.hidden_layers = L;
@@ -2169,11 +2021,7 @@ int deep_fit_dev(physad_ctx* c, const char* what, bool pairs, const float* x, co
     cudaStream_t st = cudaStream_t(stream);
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
-    if (B == 0) {   // an empty shard: zero sum, zero gradient
-        CU(cudaMemsetAsync(acc, 0, sizeof(double), st));
-        CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
-        return 0;
-    }
+    if (B == 0) return zero_result(acc, 1, grad, P, st);   // an empty shard: zero sum, zero gradient
     DeepDataArgs a{};
     a.n = (long long)(pairs ? 2 * B : B);
     a.x = reinterpret_cast<const float4*>(x);
@@ -2192,24 +2040,15 @@ int deep_fit_host(physad_ctx* c, const char* what, bool pairs, const float* x, c
     if (int rc = deep_points_ready(c, what)) return rc;
     if (B && (!x || (!pairs && !target))) return fail(PHYSAD_E_INVALID, std::string(what) + ": null argument");
     DeviceGuard dg(c->device);
-    const int H = c->cfg.H, L = c->deep_layers;
-    const size_t P = deep_grad_len(H, L);
-    if (int rc = ensure_host_grad(c, P)) return rc;
-    const size_t bytes = B * (pairs ? 8 : 4) * sizeof(float), off_t = (bytes + 255) & ~size_t(255);
-    if (int rc = ensure_scratch(c, off_t + (pairs ? 0 : bytes) + 1)) return rc;
-    float* dx = reinterpret_cast<float*>(c->scratch);
-    float* dtg = pairs ? nullptr : reinterpret_cast<float*>(c->scratch + off_t);
-    if (B) {
-        CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
-        if (!pairs) CU(cudaMemcpyAsync(dtg, target, bytes, cudaMemcpyHostToDevice, c->stream));
-    }
+    if (int rc = ensure_host_grad(c)) return rc;
+    const size_t bytes = B * (pairs ? 8 : 4) * sizeof(float);
+    Staged a[2] = {{x, nullptr, bytes}, {target, nullptr, pairs ? 0 : bytes}};
+    if (int rc = stage_in(c, a)) return rc;
     // n_norm = B; an empty set (B = 0) gives a zero loss and a zero gradient
-    if (int rc = deep_fit_dev(c, what, pairs, dx, dtg, B, lam, B ? B : 1, c->d_dgrad, c->d_dgrad + 1, c->stream)) return rc;
-    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 1) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    if (loss) *loss = float(c->h_dgrad[0] / double(B ? B : 1));
-    split_deep_grad(c->h_dgrad + 1, H, L, dW1, db1, dWh, dbh, dW2, db2);
-    return 0;
+    const size_t n = B ? B : 1;
+    if (int rc = deep_fit_dev(c, what, pairs, a[0].dev, pairs ? nullptr : a[1].dev, B, lam, n, c->d_dgrad, c->d_dgrad + 1, c->stream))
+        return rc;
+    return grad_to_host(c, 1, n, nullptr, loss, nullptr, {dW1, db1, dWh, dbh, dW2, db2});
 }
 }  // namespace
 extern "C" {
@@ -2280,13 +2119,7 @@ int colloc_grad_launch(physad_ctx* c, TangentSeeds seeds, DeepTangentArgs& a, do
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
     const int blocks = deep_tangent_blocks(H, a.n_points, c->sm_count);
-    const size_t ck = size_t(blocks) * deep_tangent_ckpt_floats(L);
-    if (ck > c->dckpt_cap) {
-        if (c->dckpt) CU(cudaFree(c->dckpt));
-        c->dckpt = nullptr; c->dckpt_cap = 0;
-        CU(cudaMalloc(&c->dckpt, ck * sizeof(float)));
-        c->dckpt_cap = ck;
-    }
+    if (int rc = grow(c->dckpt, c->dckpt_cap, size_t(blocks) * deep_tangent_ckpt_floats(L))) return rc;
     const size_t np = size_t(blocks) * (P + 2);
     const bool physics = seeds == TangentSeeds::physics;
     if (int rc = ensure_grad_partials(c, np + (physics ? 0 : 2))) return rc;
@@ -2315,10 +2148,7 @@ int physad_deep_tangent_points_loss_dev(physad_ctx* c, const float* x, size_t B,
     if (int rc = colloc_check(x, B, dcdx, "deep_tangent_points_loss")) return rc;
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
-    if (B == 0) {
-        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
-        return 0;
-    }
+    if (B == 0) return zero_result(acc, 2, nullptr, 0, st);
     DeepTangentArgs a{};
     if (int rc = colloc_args(c, x, B, dcdx, a, st)) return rc;
     a.R_pts = reinterpret_cast<float4*>(R);
@@ -2345,11 +2175,7 @@ int physad_deep_tangent_points_loss_grad_dev(physad_ctx* c, const float* x, size
     cudaStream_t st = cudaStream_t(stream);
     const int H = c->cfg.H, L = c->deep_layers;
     const size_t P = deep_grad_len(H, L);
-    if (B == 0) {   // an empty shard: zero sums, zero gradient
-        CU(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
-        CU(cudaMemsetAsync(grad, 0, P * sizeof(double), st));
-        return 0;
-    }
+    if (B == 0) return zero_result(acc, 2, grad, P, st);   // an empty shard: zero sums, zero gradient
     DeepTangentArgs a{};
     if (int rc = colloc_args(c, x, B, dcdx, a, st)) return rc;
     // vjp_scales' formula with n_norm for N: shards with the same n_norm add up to the whole set's gradient
@@ -2365,21 +2191,14 @@ int physad_deep_tangent_points_loss_grad_host(physad_ctx* c, const float* x, siz
     if (int rc = deep_points_ready(c, "deep_tangent_points_loss_grad")) return rc;
     if (!w || !dcdx || (B && !x)) return fail(PHYSAD_E_INVALID, "deep_tangent_points_loss_grad: null argument");
     DeviceGuard dg(c->device);
-    const int H = c->cfg.H, L = c->deep_layers;
-    const size_t P = deep_grad_len(H, L);
-    if (int rc = ensure_host_grad(c, P)) return rc;
-    const size_t bytes = B * 4 * sizeof(float);
-    if (int rc = ensure_scratch(c, bytes + 1)) return rc;
-    float* dx = reinterpret_cast<float*>(c->scratch);
-    if (B) CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
+    if (int rc = ensure_host_grad(c)) return rc;
+    Staged a[1] = {{x, nullptr, B * 4 * sizeof(float)}};
+    if (int rc = stage_in(c, a)) return rc;
     // n_norm = B; an empty set (B = 0) gives zero losses and a zero gradient
     const size_t n = B ? B : 1;
-    if (int rc = physad_deep_tangent_points_loss_grad_dev(c, dx, B, dcdx, w, n, c->d_dgrad, c->d_dgrad + 2, c->stream)) return rc;
-    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 2) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    physad_finalize_loss(c->h_dgrad, w, n, loss_sigma, loss_u);
-    split_deep_grad(c->h_dgrad + 2, H, L, dW1, db1, dWh, dbh, dW2, db2);
-    return 0;
+    if (int rc = physad_deep_tangent_points_loss_grad_dev(c, a[0].dev, B, dcdx, w, n, c->d_dgrad, c->d_dgrad + 2, c->stream))
+        return rc;
+    return grad_to_host(c, 2, n, w, loss_sigma, loss_u, {dW1, db1, dWh, dbh, dW2, db2});
 }
 
 // ---- Neumann boundaries at points: the Jacobian of deeper networks and the derivative-fit loss (deep_tangent_kernels.cuh)
@@ -2408,17 +2227,11 @@ int physad_mlp_jacobian_deep_host(physad_ctx* c, const float* x, float* y, float
     if (B && (!x || !y || !J)) return fail(PHYSAD_E_INVALID, "mlp_jacobian_deep: null argument");
     if (B == 0) return 0;
     DeviceGuard dg(c->device);
-    const size_t bytes = B * 4 * sizeof(float), off = (bytes + 255) & ~size_t(255);
-    if (int rc = ensure_scratch(c, 2 * off + 4 * bytes)) return rc;
-    float* dx = reinterpret_cast<float*>(c->scratch);
-    float* dy = reinterpret_cast<float*>(c->scratch + off);
-    float* dJ = reinterpret_cast<float*>(c->scratch + 2 * off);
-    CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
-    if (int rc = physad_mlp_jacobian_deep_dev(c, dx, dy, dJ, B, c->stream)) return rc;
-    CU(cudaMemcpyAsync(y, dy, bytes, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(J, dJ, 4 * bytes, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
+    const size_t bytes = B * 4 * sizeof(float);
+    Staged a[3] = {{x, nullptr, bytes}, {nullptr, y, bytes}, {nullptr, J, 4 * bytes}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_mlp_jacobian_deep_dev(c, a[0].dev, a[1].dev, a[2].dev, B, c->stream)) return rc;
+    return stage_out(c, a);
 }
 
 int physad_deep_deriv_loss_grad_dev(physad_ctx* c, const float* x, const float* dir, const float* target, size_t B,
@@ -2435,11 +2248,7 @@ int physad_deep_deriv_loss_grad_dev(physad_ctx* c, const float* x, const float* 
     if (int rc = read_lam(lam, lw, w)) return rc;
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
-    if (B == 0) {   // an empty shard: zero sum, zero gradient
-        CU(cudaMemsetAsync(acc, 0, sizeof(double), st));
-        CU(cudaMemsetAsync(grad, 0, deep_grad_len(c->cfg.H, c->deep_layers) * sizeof(double), st));
-        return 0;
-    }
+    if (B == 0) return zero_result(acc, 1, grad, deep_grad_len(c->cfg.H, c->deep_layers), st);   // an empty shard
     DeepTangentArgs a{};
     if (int rc = colloc_args(c, x, B, nullptr, a, st)) return rc;
     a.dirs = reinterpret_cast<const float4*>(dir);
@@ -2458,24 +2267,15 @@ int physad_deep_deriv_loss_grad_host(physad_ctx* c, const float* x, const float*
     if (int rc = deep_points_ready(c, "deep_deriv_loss_grad")) return rc;
     if (B && (!x || !dir || !target)) return fail(PHYSAD_E_INVALID, "deep_deriv_loss_grad: null argument");
     DeviceGuard dg(c->device);
-    const int H = c->cfg.H, L = c->deep_layers;
-    const size_t P = deep_grad_len(H, L);
-    if (int rc = ensure_host_grad(c, P)) return rc;
-    const size_t bytes = B * 4 * sizeof(float), off = (bytes + 255) & ~size_t(255);
-    if (int rc = ensure_scratch(c, 2 * off + bytes + 1)) return rc;
-    float* d[3] = {reinterpret_cast<float*>(c->scratch), reinterpret_cast<float*>(c->scratch + off),
-                   reinterpret_cast<float*>(c->scratch + 2 * off)};
-    const float* h[3] = {x, dir, target};
-    if (B)
-        for (int k = 0; k < 3; ++k) CU(cudaMemcpyAsync(d[k], h[k], bytes, cudaMemcpyHostToDevice, c->stream));
+    if (int rc = ensure_host_grad(c)) return rc;
+    const size_t bytes = B * 4 * sizeof(float);
+    Staged a[3] = {{x, nullptr, bytes}, {dir, nullptr, bytes}, {target, nullptr, bytes}};
+    if (int rc = stage_in(c, a)) return rc;
     // n_norm = B; an empty set (B = 0) gives a zero loss and a zero gradient
     const size_t n = B ? B : 1;
-    if (int rc = physad_deep_deriv_loss_grad_dev(c, d[0], d[1], d[2], B, lam, n, c->d_dgrad, c->d_dgrad + 1, c->stream)) return rc;
-    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, (P + 1) * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    if (loss) *loss = float(c->h_dgrad[0] / double(n));
-    split_deep_grad(c->h_dgrad + 1, H, L, dW1, db1, dWh, dbh, dW2, db2);
-    return 0;
+    if (int rc = physad_deep_deriv_loss_grad_dev(c, a[0].dev, a[1].dev, a[2].dev, B, lam, n, c->d_dgrad, c->d_dgrad + 1, c->stream))
+        return rc;
+    return grad_to_host(c, 1, n, nullptr, loss, nullptr, {dW1, db1, dWh, dbh, dW2, db2});
 }
 
 // ---- vector-Jacobian products of deeper networks at points (deep_data_kernels.cuh, deep_tangent_kernels.cuh) ----------
@@ -2488,10 +2288,7 @@ int physad_mlp_vjp_deep_dev(physad_ctx* c, const float* x, const float* ybar, si
     if (uintptr_t(grad) % 8) return fail(PHYSAD_E_INVALID, w + ": grad must be 8-byte aligned");
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
-    if (B == 0) {   // an empty shard: zero gradient
-        CU(cudaMemsetAsync(grad, 0, deep_grad_len(c->cfg.H, c->deep_layers) * sizeof(double), st));
-        return 0;
-    }
+    if (B == 0) return zero_result(nullptr, 0, grad, deep_grad_len(c->cfg.H, c->deep_layers), st);   // an empty shard
     DeepDataArgs a{};
     a.n = (long long)B;
     a.x = reinterpret_cast<const float4*>(x);
@@ -2505,22 +2302,11 @@ int physad_mlp_vjp_deep_host(physad_ctx* c, const float* x, const float* ybar, s
     if (int rc = deep_points_ready(c, "mlp_vjp_deep")) return rc;
     if (B && (!x || !ybar)) return fail(PHYSAD_E_INVALID, "mlp_vjp_deep: null argument");
     DeviceGuard dg(c->device);
-    const int H = c->cfg.H, L = c->deep_layers;
-    const size_t P = deep_grad_len(H, L);
-    if (int rc = ensure_host_grad(c, P)) return rc;
-    const size_t bytes = B * 4 * sizeof(float), off = (bytes + 255) & ~size_t(255);
-    if (int rc = ensure_scratch(c, off + bytes + 1)) return rc;
-    float* dx = reinterpret_cast<float*>(c->scratch);
-    float* dyb = reinterpret_cast<float*>(c->scratch + off);
-    if (B) {
-        CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
-        CU(cudaMemcpyAsync(dyb, ybar, bytes, cudaMemcpyHostToDevice, c->stream));
-    }
-    if (int rc = physad_mlp_vjp_deep_dev(c, dx, dyb, B, c->d_dgrad, c->stream)) return rc;
-    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, P * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    split_deep_grad(c->h_dgrad, H, L, dW1, db1, dWh, dbh, dW2, db2);
-    return 0;
+    if (int rc = ensure_host_grad(c)) return rc;
+    Staged a[2] = {{x, nullptr, B * 4 * sizeof(float)}, {ybar, nullptr, B * 4 * sizeof(float)}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_mlp_vjp_deep_dev(c, a[0].dev, a[1].dev, B, c->d_dgrad, c->stream)) return rc;
+    return grad_to_host(c, 0, 0, nullptr, nullptr, nullptr, {dW1, db1, dWh, dbh, dW2, db2});
 }
 
 int physad_mlp_jacobian_vjp_deep_dev(physad_ctx* c, const float* x, const float* ybar, const float* Jbar, size_t B, double* grad,
@@ -2534,10 +2320,7 @@ int physad_mlp_jacobian_vjp_deep_dev(physad_ctx* c, const float* x, const float*
     if (uintptr_t(grad) % 8) return fail(PHYSAD_E_INVALID, w + ": grad must be 8-byte aligned");
     DeviceGuard dg(c->device);
     cudaStream_t st = cudaStream_t(stream);
-    if (B == 0) {   // an empty shard: zero gradient
-        CU(cudaMemsetAsync(grad, 0, deep_grad_len(c->cfg.H, c->deep_layers) * sizeof(double), st));
-        return 0;
-    }
+    if (B == 0) return zero_result(nullptr, 0, grad, deep_grad_len(c->cfg.H, c->deep_layers), st);   // an empty shard
     DeepTangentArgs a{};
     if (int rc = colloc_args(c, x, B, nullptr, a, st)) return rc;
     a.ybar = reinterpret_cast<const float4*>(ybar);
@@ -2551,24 +2334,12 @@ int physad_mlp_jacobian_vjp_deep_host(physad_ctx* c, const float* x, const float
     if (int rc = deep_points_ready(c, "mlp_jacobian_vjp_deep")) return rc;
     if (B && (!x || !ybar || !Jbar)) return fail(PHYSAD_E_INVALID, "mlp_jacobian_vjp_deep: null argument");
     DeviceGuard dg(c->device);
-    const int H = c->cfg.H, L = c->deep_layers;
-    const size_t P = deep_grad_len(H, L);
-    if (int rc = ensure_host_grad(c, P)) return rc;
-    const size_t bytes = B * 4 * sizeof(float), off = (bytes + 255) & ~size_t(255);
-    if (int rc = ensure_scratch(c, 2 * off + 4 * bytes + 1)) return rc;
-    float* dx = reinterpret_cast<float*>(c->scratch);
-    float* dyb = reinterpret_cast<float*>(c->scratch + off);
-    float* dJb = reinterpret_cast<float*>(c->scratch + 2 * off);
-    if (B) {
-        CU(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, c->stream));
-        CU(cudaMemcpyAsync(dyb, ybar, bytes, cudaMemcpyHostToDevice, c->stream));
-        CU(cudaMemcpyAsync(dJb, Jbar, 4 * bytes, cudaMemcpyHostToDevice, c->stream));
-    }
-    if (int rc = physad_mlp_jacobian_vjp_deep_dev(c, dx, dyb, dJb, B, c->d_dgrad, c->stream)) return rc;
-    CU(cudaMemcpyAsync(c->h_dgrad, c->d_dgrad, P * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    split_deep_grad(c->h_dgrad, H, L, dW1, db1, dWh, dbh, dW2, db2);
-    return 0;
+    if (int rc = ensure_host_grad(c)) return rc;
+    const size_t bytes = B * 4 * sizeof(float);
+    Staged a[3] = {{x, nullptr, bytes}, {ybar, nullptr, bytes}, {Jbar, nullptr, 4 * bytes}};
+    if (int rc = stage_in(c, a)) return rc;
+    if (int rc = physad_mlp_jacobian_vjp_deep_dev(c, a[0].dev, a[1].dev, a[2].dev, B, c->d_dgrad, c->stream)) return rc;
+    return grad_to_host(c, 0, 0, nullptr, nullptr, nullptr, {dW1, db1, dWh, dbh, dW2, db2});
 }
 
 int physad_plan_ranges(int tiles, int planes, int slots, int* out, int out_cap) {

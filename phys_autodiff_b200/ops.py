@@ -147,6 +147,12 @@ class Context:
         import torch
         return torch.empty(n, dtype=dtype or torch.float32, device="cuda")
 
+    def _grad_arrays(self):
+        """The six float32 host arrays a deep gradient's host form fills: dW1, db1, dWh, dbh, dW2, db2 of the network set by
+        set_weights_deep (dWh and dbh are empty at one hidden layer)."""
+        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
+        return [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+
     # -- MLP -------------------------------------------------------------------------------------
     def mlp_forward(self, x):
         """y[B,Out] = MLP(x[B,In]) on device tensors (mlp_forward<ExecCuda>, include/mlp.h:5-6)."""
@@ -256,8 +262,7 @@ class Context:
 
     def deep_loss_grad_host(self, g: Grid, pw: PhysWeights, t: float, dt: float):
         """Host-buffer form with the context's deep weights: (L_sigma, L_u, dW1, db1, dWh, dbh, dW2, db2), float32."""
-        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
-        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        d = self._grad_arrays()
         ls, lu = C.c_float(), C.c_float()
         cg, cw = g.c(), pw.c()
         check(self._lib.physad_deep_loss_grad_host(self._h, C.byref(cg), C.byref(cw), C.c_float(t), C.c_float(dt), C.byref(ls),
@@ -306,8 +311,7 @@ class Context:
     def deep_tangent_loss_grad_host(self, g: Grid, pw: PhysWeights, t: float):
         """Host-buffer form with the context's deep weights: (L_sigma, L_u, dW1, db1, dWh, dbh, dW2, db2) of the analytic
         loss, float32."""
-        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
-        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        d = self._grad_arrays()
         ls, lu = C.c_float(), C.c_float()
         cg, cw = g.c(), pw.c()
         check(self._lib.physad_deep_tangent_loss_grad_host(self._h, C.byref(cg), C.byref(cw), C.c_float(t), C.byref(ls),
@@ -345,9 +349,9 @@ class Context:
 
     @staticmethod
     def _fit_allreduce(B, device, n_global, group, acc):
-        """(loss, grad float64 ndarray[P]) of a fit loss over every rank: n_global (default: the sum of B over ranks, one
-        all-reduce of one integer) normalises, acc(n_global) is the rank's device [acc, grad(P)], and ONE all-reduce of P+1
-        doubles combines the ranks."""
+        """(n_global, [sums, grad(P)] float64 ndarray) of a loss at points over every rank: n_global (default: the sum of B over
+        ranks, one all-reduce of one integer) normalises, acc(n_global) is the rank's device [sums, grad(P)], and ONE
+        all-reduce combines the ranks.  The caller finishes its loss from the sums."""
         import torch
         import torch.distributed as dist
         world = dist.get_world_size(group) if dist.is_initialized() else 1
@@ -362,8 +366,7 @@ class Context:
         buf = acc(n_global)
         if world > 1:
             dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
-        h = buf.cpu().numpy()
-        return float(h[0] / n_global), h[1:].copy()
+        return n_global, buf.cpu().numpy()
 
     def deep_data_loss_grad_acc(self, x, target, lam=None, n_norm=None, out=None):
         """Device form of the data-fit loss L_d = (1/n_norm) sum_i sum_o lam[o] (y_io - target_io)^2 of the deep network at
@@ -385,16 +388,16 @@ class Context:
         """(L_d, grad float64 ndarray[P]) of the data-fit loss over the points of every rank.  With torch.distributed
         initialised each rank passes its own points; n_global (default: the sum of B over ranks, one all-reduce of one
         integer) normalises, and ONE all-reduce of P+1 doubles combines the ranks."""
-        return self._fit_allreduce(x.numel() // 4, x.device, n_global, group,
+        n, h = self._fit_allreduce(x.numel() // 4, x.device, n_global, group,
                                    lambda n: self.deep_data_loss_grad_acc(x, target, lam, n))
+        return float(h[0] / n), h[1:].copy()
 
     def deep_data_loss_grad_host(self, x, target, lam=None):
         """Host-array form with n_norm = B: (L_d, dW1, db1, dWh, dbh, dW2, db2), float32."""
         x, target = _f32(x), _f32(target)
         B = x.size // 4
         assert target.size == 4 * B
-        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
-        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        d = self._grad_arrays()
         loss = C.c_float()
         check(self._lib.physad_deep_data_loss_grad_host(self._h, ptr(x), ptr(target), C.c_size_t(B), self._lam(lam), C.byref(loss),
                                                         *[ptr(a) if a.size else None for a in d]), "deep_data_loss_grad_host")
@@ -422,15 +425,15 @@ class Context:
         """(L_p, grad float64 ndarray[P]) of the pair loss over the pairs of every rank.  With torch.distributed initialised
         each rank passes its own pairs; n_global (default: the sum of B over ranks, one all-reduce of one integer)
         normalises, and ONE all-reduce of P+1 doubles combines the ranks."""
-        return self._fit_allreduce(x.numel() // 8, x.device, n_global, group, lambda n: self.deep_pair_loss_grad_acc(x, lam, n))
+        n, h = self._fit_allreduce(x.numel() // 8, x.device, n_global, group, lambda n: self.deep_pair_loss_grad_acc(x, lam, n))
+        return float(h[0] / n), h[1:].copy()
 
     def deep_pair_loss_grad_host(self, x, lam=None):
         """Host-array form with n_norm = B: x [B, 2, 4] -> (L_p, dW1, db1, dWh, dbh, dW2, db2), float32."""
         x = _f32(x)
         B = x.size // 8
         assert x.size == 8 * B
-        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
-        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        d = self._grad_arrays()
         loss = C.c_float()
         check(self._lib.physad_deep_pair_loss_grad_host(self._h, ptr(x), C.c_size_t(B), self._lam(lam), C.byref(loss),
                                                         *[ptr(a) if a.size else None for a in d]), "deep_pair_loss_grad_host")
@@ -481,16 +484,16 @@ class Context:
         """(L_g, grad float64 ndarray[P]) of the derivative-fit loss over the points of every rank.  With torch.distributed
         initialised each rank passes its own points; n_global (default: the sum of B over ranks, one all-reduce of one
         integer) normalises, and ONE all-reduce of P+1 doubles combines the ranks."""
-        return self._fit_allreduce(x.numel() // 4, x.device, n_global, group,
+        n, h = self._fit_allreduce(x.numel() // 4, x.device, n_global, group,
                                    lambda n: self.deep_deriv_loss_grad_acc(x, d, target, lam, n))
+        return float(h[0] / n), h[1:].copy()
 
     def deep_deriv_loss_grad_host(self, x, d, target, lam=None):
         """Host-array form with n_norm = B: x, d, target [B, 4] -> (L_g, dW1, db1, dWh, dbh, dW2, db2), float32."""
         x, d, target = _f32(x), _f32(d), _f32(target)
         B = x.size // 4
         assert x.size == 4 * B and d.size == 4 * B and target.size == 4 * B
-        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
-        g = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        g = self._grad_arrays()
         loss = C.c_float()
         check(self._lib.physad_deep_deriv_loss_grad_host(self._h, ptr(x), ptr(d), ptr(target), C.c_size_t(B), self._lam(lam),
                                                          C.byref(loss), *[ptr(a) if a.size else None for a in g]),
@@ -530,8 +533,7 @@ class Context:
         x, ybar = _f32(x), _f32(ybar)
         B = x.size // 4
         assert x.size == 4 * B and ybar.size == 4 * B
-        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
-        g = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        g = self._grad_arrays()
         check(self._lib.physad_mlp_vjp_deep_host(self._h, ptr(x), ptr(ybar), C.c_size_t(B),
                                                  *[ptr(a) if a.size else None for a in g]), "mlp_vjp_deep_host")
         return tuple(g)
@@ -541,8 +543,7 @@ class Context:
         x, ybar, Jbar = _f32(x), _f32(ybar), _f32(Jbar)
         B = x.size // 4
         assert x.size == 4 * B and ybar.size == 4 * B and Jbar.size == 16 * B
-        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
-        g = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        g = self._grad_arrays()
         check(self._lib.physad_mlp_jacobian_vjp_deep_host(self._h, ptr(x), ptr(ybar), ptr(Jbar), C.c_size_t(B),
                                                           *[ptr(a) if a.size else None for a in g]), "mlp_jacobian_vjp_deep_host")
         return tuple(g)
@@ -589,31 +590,16 @@ class Context:
         """(L_sigma, L_u, grad float64 ndarray[P]) of the analytic loss over the points of every rank.  With
         torch.distributed initialised each rank passes its own points; n_global (default: the sum of B over ranks, one
         all-reduce of one integer) normalises, and ONE all-reduce of P+2 doubles combines the ranks."""
-        import torch
-        import torch.distributed as dist
-        world = dist.get_world_size(group) if dist.is_initialized() else 1
-        B = x.numel() // 4
-        if n_global is None:
-            if world > 1:
-                nb = torch.tensor([B], dtype=torch.int64, device=x.device)
-                dist.all_reduce(nb, op=dist.ReduceOp.SUM, group=group)
-                n_global = int(nb.item())
-            else:
-                n_global = B
-        n_global = max(int(n_global), 1)
-        buf = self.deep_tangent_points_loss_grad_acc(x, dcdx, pw, n_global)
-        if world > 1:
-            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
-        h = buf.cpu().numpy()
-        ls, lu = self.finalize(h[:2], pw, n_global)
+        n, h = self._fit_allreduce(x.numel() // 4, x.device, n_global, group,
+                                   lambda n: self.deep_tangent_points_loss_grad_acc(x, dcdx, pw, n))
+        ls, lu = self.finalize(h[:2], pw, n)
         return ls, lu, h[2:].copy()
 
     def deep_tangent_points_loss_grad_host(self, x, dcdx, pw: PhysWeights):
         """Host-array form with n_norm = B: x [B, 4] (or flat) -> (L_sigma, L_u, dW1, db1, dWh, dbh, dW2, db2), float32."""
         x = _f32(x)
         B = x.size // 4
-        H, nl = self.cfg.H, (self.hidden_layers or 1) - 1
-        d = [np.empty(n, np.float32) for n in (4 * H, H, nl * H * H, nl * H, 4 * H, 4)]
+        d = self._grad_arrays()
         ls, lu = C.c_float(), C.c_float()
         cw = pw.c()
         check(self._lib.physad_deep_tangent_points_loss_grad_host(self._h, ptr(x), C.c_size_t(B), self._dcdx(dcdx), C.byref(cw),
